@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--batch-n 65536] [--d 256] [--dtype bf16|f32] [--similarity cosine]
+                    [--dump-outputs DIR]
 
 One "step" = one forward + backward of the loss over one batch of synthetic
 unit-norm embeddings (value = N^2 / t).  Default workload = BASELINE.json
@@ -39,6 +40,7 @@ if ROOT not in sys.path:
 
 METRIC = "supcon_fwd_bwd_sim_pairs_per_s"
 UNIT = "pairs/s"
+DUMP_DZ_BYTES = 32 << 20
 
 
 def parse():
@@ -76,7 +78,18 @@ def parse():
     ap.add_argument("--no-weak-leg", action="store_true",
                     help="several ranks, strong scaling: skip the additional weak-scaling measurement (per-GPU pair "
                          "count of the single-GPU workload, N = batch-n * sqrt(gpus)) reported under \"weak\"")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as float32 DIR/<name>.npy: "
+                         "loss.npy and dz.npy = d loss / d z of the whole batch (all ranks' rows), all rows or a "
+                         "fixed, seeded sample of them "
+                         f"(at most {DUMP_DZ_BYTES >> 20} MiB); the inputs are seeded, so two builds compare file "
+                         "for file")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "loss"):
+        ap.error("--dump-outputs writes the outputs of --impl ours --workload loss only")
+    return args
 
 
 def peaks():
@@ -154,6 +167,21 @@ def synth(n, d, dtype, seed=1337):
     y = torch.zeros(n, dtype=torch.int64)
     y[torch.randperm(n, generator=g)[: n // 2]] = 1
     return z, y
+
+
+def dump_outputs(out_dir, loss, dz):
+    """Write the loss and d loss / d z of one step as float32 .npy files.  dz keeps all its rows when they fit
+    DUMP_DZ_BYTES, else a sample of rows that depends only on the shape (fixed seed, ascending order)."""
+    import numpy as np
+    import torch
+    rows, cols = dz.shape
+    keep = max(1, DUMP_DZ_BYTES // (4 * cols))
+    if rows > keep:
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        dz = dz[idx.to(dz.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "dz.npy"), dz.detach().float().cpu().numpy())
 
 
 def cpu_model():
@@ -311,7 +339,7 @@ def run_stage1(args):
     n_params = sum(p_.numel() for p_ in enc.parameters())
     B = args.stage1_batch * ngpu
     g = torch.Generator().manual_seed(1337)
-    steps = max(3, min(args.steps, 8))
+    steps = args.steps
     batches = [(torch.randn(B, 64000, generator=g), (torch.arange(B) % 2).long()) for _ in range(steps)]
     cfg = SimpleNamespace(finetune_encoder=False, use_rawboost=False, topk_neg=args.topk, warmup_epochs=0,
                           alpha_ramp_epochs=1, alpha_end=args.alpha)      # epoch 1 -> alpha = alpha_end
@@ -531,6 +559,14 @@ def main():
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     ms_per_step = float(tt)
+    if args.dump_outputs:
+        dz_all = dz
+        if world > 1:       # the row shards in rank order: dz of the whole batch, whatever the number of ranks
+            parts = [torch.empty_like(dz) for _ in range(world)]
+            dist.all_gather(parts, dz.contiguous())
+            dz_all = torch.cat(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, loss, dz_all)
 
     # ---- end-to-end: pinned host inputs -> H2D -> fwd+bwd -> loss D2H, every step ----
     ev2 = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]

@@ -8,14 +8,8 @@ Resolution order of the reference root:
 
 Nothing under ``wav2vec_contr_loss_b200/`` imports this module.
 """
-import contextlib
 import importlib.util
-import io
 import os
-import re
-import runpy
-import sys
-import types
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 STAGED_ROOT = os.path.join(_HERE, "_ref")
@@ -58,96 +52,3 @@ def load_reference_module(name: str = "loss"):
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
-
-
-# ---------------------------------------------------------------------------------------------
-# Running the reference's callers UNCHANGED (SURVEY H9): train_stage1.py imports data_loader, which needs
-# soundfile / librosa / a dataset on disk.  The harness below injects a synthetic ``data_loader`` module,
-# puts a chosen directory holding a module named ``loss`` (the reference's own, or this repo's drop-in)
-# ahead on sys.path, and executes the reference's train_stage1.py as __main__ without editing any file.
-# ---------------------------------------------------------------------------------------------
-_CALLER_MODULES = ("loss", "stage1_utils", "stage1_config", "compression_module", "encoder", "RawBoost",
-                   "train_stage1", "data_loader")
-
-
-def synthetic_data_loader_module(n_items: int = 64, samples: int = 4000, seed: int = 0):
-    """A stand-in for the reference's data_loader.py exposing the two names train_stage1.py imports.
-    Items follow data_loader.py:207-214: (waveform, binary label, multi-class label, speaker, audio name);
-    ``dataset.data[i][1]`` is the binary label BalancedBatchSampler reads (stage1_utils.py:26-27)."""
-    import torch
-
-    class ASVspoof2019Dataset(torch.utils.data.Dataset):
-        def __init__(self, root_dir="", protocol_file="", subset="all", num_samples=None, **kwargs):
-            salt = 1 if "dev" in str(protocol_file).lower() else 0
-            g = torch.Generator().manual_seed(seed + 7919 * salt)
-            n = n_items if num_samples is None else min(int(num_samples), n_items)
-            self.data = [(f"utt{i:05d}.flac", i % 2, (i % 2) * (1 + i % 3), f"p{i % 5}", f"utt{i:05d}.flac")
-                         for i in range(n)]
-            # class-dependent tone + noise so the head has something to separate
-            t = torch.arange(samples) / 16000.0
-            self.wave = [0.1 * torch.randn(samples, generator=g) +
-                         0.2 * torch.sin(2 * 3.14159265 * (220.0 + 220.0 * lab) * t) for (_, lab, *_r) in self.data]
-
-        def __len__(self):
-            return len(self.data)
-
-        def __getitem__(self, idx):
-            _, b, m, spk, name = self.data[idx]
-            return self.wave[idx], torch.tensor(b, dtype=torch.long), torch.tensor(m, dtype=torch.long), spk, name
-
-    def pad_collate_fn_speaker_source_multiclass(batch):   # collate.py:71-86
-        waves, bl, ml, spk, src = zip(*batch)
-        padded = torch.nn.utils.rnn.pad_sequence(list(waves), batch_first=True, padding_value=0.0)
-        return padded, torch.stack(list(bl)), torch.stack(list(ml)), spk, src
-
-    mod = types.ModuleType("data_loader")
-    mod.ASVspoof2019Dataset = ASVspoof2019Dataset
-    mod.pad_collate_fn_speaker_source_multiclass = pad_collate_fn_speaker_source_multiclass
-    return mod
-
-
-def save_tiny_wav2vec2(path: str, hidden_size: int = 1024, layers: int = 2, seed: int = 0):
-    """Random-init Wav2Vec2 saved with save_pretrained so ``--model_name <path>`` works offline.  hidden_size
-    must stay 1024: stage1_config.py:17 hard-codes INPUT_DIM = 1024 for the compression head."""
-    import torch
-    from transformers import Wav2Vec2Config, Wav2Vec2Model
-    torch.manual_seed(seed)
-    cfg = Wav2Vec2Config(hidden_size=hidden_size, num_hidden_layers=layers, num_attention_heads=8,
-                         intermediate_size=256, feat_extract_norm="layer", do_stable_layer_norm=True, conv_bias=True,
-                         conv_dim=(32, 32, 32), conv_stride=(5, 4, 4), conv_kernel=(10, 8, 4),
-                         num_conv_pos_embeddings=16, num_conv_pos_embedding_groups=4, layerdrop=0.0,
-                         hidden_dropout=0.0, attention_dropout=0.0, feat_proj_dropout=0.0, activation_dropout=0.0,
-                         mask_time_prob=0.0, mask_feature_prob=0.0)
-    Wav2Vec2Model(cfg).save_pretrained(path)
-    return path
-
-
-_EPOCH_LINE = re.compile(r"\[epoch (\d+)\] alpha=([0-9.]+) \| train_loss=([0-9.eE+-]+) \| dev_loss=([0-9.eE+-]+)")
-
-
-def run_unchanged_train_stage1(loss_dir: str, argv, data_loader_module=None):
-    """Execute the reference's train_stage1.py as __main__, unedited, with ``loss_dir`` (a directory holding a
-    module named ``loss``) ahead of the reference root on sys.path.  Returns (epoch records, captured stdout)."""
-    root = reference_root()
-    if root is None:
-        raise FileNotFoundError("reference not staged: run oracle/build_ref.py in the build container")
-    saved_mods = {k: sys.modules.pop(k) for k in _CALLER_MODULES if k in sys.modules}
-    saved_path, saved_argv = list(sys.path), list(sys.argv)
-    buf = io.StringIO()
-    try:
-        sys.modules["data_loader"] = data_loader_module or synthetic_data_loader_module()
-        sys.path[:0] = [loss_dir, root]
-        sys.argv = ["train_stage1.py"] + list(argv)
-        with contextlib.redirect_stdout(buf):
-            runpy.run_path(os.path.join(root, "train_stage1.py"), run_name="__main__")
-        loss_file = getattr(sys.modules.get("loss"), "__file__", None)
-    finally:
-        for k in _CALLER_MODULES:
-            sys.modules.pop(k, None)
-        sys.modules.update(saved_mods)
-        sys.path[:] = saved_path
-        sys.argv = saved_argv
-    out = buf.getvalue()
-    recs = [dict(epoch=int(m.group(1)), alpha=float(m.group(2)), train_loss=float(m.group(3)),
-                 dev_loss=float(m.group(4))) for m in _EPOCH_LINE.finditer(out)]
-    return recs, out, loss_file

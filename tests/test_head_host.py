@@ -3,7 +3,6 @@ the reference's CompressionModule checkpoints, no CPU path, launch-geometry rule
 import pytest
 import torch
 
-from oracle.ref_loader import load_reference_module, reference_available
 from wav2vec_contr_loss_b200 import FusedCompressionHead, layer_time_pool
 
 
@@ -13,17 +12,6 @@ def test_parameters_are_the_reference_modules():
     assert head.mlp3.weight.shape == (256, 1024) and head.dropout_head.p == 0.1
     assert head.activation_head.negative_slope == 0.01
     assert "rng_state" not in head.state_dict() and head.rng_state.dtype == torch.int64
-
-
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference (build container only)")
-def test_loads_a_reference_checkpoint():
-    ref = load_reference_module("compression_module")
-    theirs = ref.CompressionModule(input_dim=48, hidden_dim=12, dropout_rate=0.2)
-    ours = FusedCompressionHead(48, 12, 0.2)
-    missing, unexpected = ours.load_state_dict(theirs.state_dict(), strict=True)
-    assert not missing and not unexpected
-    assert torch.equal(ours.mlp3.weight, theirs.mlp3.weight)
-    assert [n for n, _ in ours.named_parameters()] == [n for n, _ in theirs.named_parameters()]
 
 
 def test_dropout_stream_follows_manual_seed():

@@ -53,9 +53,19 @@ def nvcc_path():
     return None
 
 
+def _is_current(digest: str) -> bool:
+    if not (os.path.isfile(LIB_PATH) and os.path.isfile(TEST_LIB_PATH) and os.path.isfile(STAMP)):
+        return False
+    with open(STAMP) as fh:
+        return fh.read().strip() == digest
+
+
 def build(force: bool = False, verbose: bool = False) -> str:
     """Compile (if stale) and return the path of the shared library.  Safe to call from several processes at
-    once (one rank per GPU): the build runs under an exclusive file lock and the others find it done."""
+    once (one rank per GPU): the build runs under an exclusive file lock and the others find it done.  A current
+    build is returned without writing anything, so a read-only tree that was built before still works."""
+    if not force and _is_current(_digest()):
+        return LIB_PATH
     import fcntl
     os.makedirs(LIB_DIR, exist_ok=True)
     with open(os.path.join(LIB_DIR, ".build.lock"), "w") as lock:
@@ -68,13 +78,15 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
 def _build_locked(force: bool, verbose: bool) -> str:
     digest = _digest()
-    if not force and os.path.isfile(LIB_PATH) and os.path.isfile(TEST_LIB_PATH) and os.path.isfile(STAMP):
-        with open(STAMP) as fh:
-            if fh.read().strip() == digest:
-                return LIB_PATH
+    if not force and _is_current(digest):
+        return LIB_PATH
     nvcc = nvcc_path()
     if nvcc is None:
         raise RuntimeError("nvcc not found: cannot build libsupcon_b200.so")
+    # the stamp marks a complete build: drop it before any file is rewritten, so that the unlocked check in build()
+    # never hands out a library that is being relinked
+    if os.path.isfile(STAMP):
+        os.remove(STAMP)
     objs = []
     procs = []
     for src in _sources():
