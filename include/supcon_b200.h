@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SUPCON_ABI_VERSION 2
+#define SUPCON_ABI_VERSION 3
 
 /* element type of z / dz buffers */
 #define SUPCON_F32 0
@@ -145,20 +145,6 @@ int supcon_forward_rows_remote(const supcon_problem_t* p, const void* z_all, con
                                float* row_stats, double* partials, void* workspace, size_t workspace_bytes,
                                void* stream);
 
-/* Multi-pass form of the forward for a rank whose peers' rows ARRIVE OVER TIME (equal, 128-aligned row blocks;
- * block b = rows [b n_rows, (b+1) n_rows) of z_all = rank b's rows).  `blocks` (HOST array) lists every rank
- * block exactly once, in the order the columns are to be swept -- the own block first, then the peers in arrival
- * order -- and `pass_sizes` (HOST array, n_passes <= 4 entries) cuts that list into passes.  Pass i is one call:
- * it needs only ITS blocks of z_all / labels_all to be valid, sweeps them in one launch and leaves partial
- * records in the workspace; the last pass also merges all passes and writes row_stats / partials exactly as
- * supcon_forward_rows would (row_stats / partials may be NULL in the other passes).  All passes share the
- * workspace.  skip_norms != 0: passes > 0 do not read z in their O(N) preparation (no squared norms, no
- * unit-rows check of the peers' rows -- every rank checks its own in pass 0); ignored with a uniformity term. */
-int supcon_forward_rows_pass(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
-                             const int32_t* blocks, const int32_t* pass_sizes, int32_t n_passes,
-                             int32_t pass_index, int32_t skip_norms, float* row_stats, double* partials,
-                             void* workspace, size_t workspace_bytes, void* stream);
-
 /* Scalar loss from globally summed partials (alpha blend, empty-set fall-backs,
  * uniformity term): loss.py:137-153. */
 int supcon_finalize(const supcon_problem_t* p, const double* partials_global, float* loss_out,
@@ -211,8 +197,9 @@ int supcon_backward_rows_remote(const supcon_problem_t* p, const void* z_all, co
 #define SUPCON_PEER_FLAG_STATS 1  /* row statistics + partial sums of step e have landed */
 #define SUPCON_PEER_FLAG_DONE 2   /* rank has finished step e (its buffers may be overwritten) */
 #define SUPCON_PEER_NFLAGS 3
-/* bytes every buffer reserves at off_flags, zeroed once at set-up: int32 flags[NFLAGS][world] + ticket words */
-#define SUPCON_PEER_FLAG_BYTES(world) ((SUPCON_PEER_NFLAGS * (world) + 4 + (world)) * 4)
+/* bytes every buffer reserves at off_flags, zeroed once at set-up: int32 flags[NFLAGS][world] + 4 words, the first
+ * of which is the push kernel's block ticket */
+#define SUPCON_PEER_FLAG_BYTES(world) ((SUPCON_PEER_NFLAGS * (world) + 4) * 4)
 
 typedef struct supcon_peer {
   int32_t rank, world;
@@ -230,17 +217,8 @@ typedef struct supcon_peer {
 int supcon_peer_push(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0,
                      const void* src1, size_t bytes1, uint64_t dst_off1, int32_t flag_id, int32_t wait_flag_id,
                      int32_t include_self, void* stream);
-/* Ordered form of supcon_peer_push (unicast, never into the own buffer): the ranges go to rank+1 first, then
- * rank+2, ... and the flag of each destination is raised as soon as its copy is complete (the own buffer's flag at
- * the end).  With every rank pushing like this a receiver gets its peers' blocks one after the other, from rank-1
- * first, and can start computing on the early ones (supcon_forward_rows_pass + supcon_peer_wait_mask). */
-int supcon_peer_push_ordered(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0,
-                             const void* src1, size_t bytes1, uint64_t dst_off1, int32_t flag_id,
-                             int32_t wait_flag_id, void* stream);
-/* One-block kernel: returns (on the stream) when flag[flag_id][p] >= epoch for every rank p
- * (_mask: for the ranks p whose bit is set in rank_mask). */
+/* One-block kernel: returns (on the stream) when flag[flag_id][p] >= epoch for every rank p. */
 int supcon_peer_wait(const supcon_peer_t* pe, int32_t flag_id, void* stream);
-int supcon_peer_wait_mask(const supcon_peer_t* pe, int32_t flag_id, uint64_t rank_mask, void* stream);
 /* End of a step: flag[flag_id][rank] = epoch in every buffer, then epoch += 1. */
 int supcon_peer_end_step(const supcon_peer_t* pe, int32_t flag_id, void* stream);
 

@@ -27,7 +27,7 @@ def test_library_exports_every_declared_symbol(lib_built):
     for name in names:
         assert hasattr(lib, name), f"{name} declared in supcon_b200.h but not exported"
     assert sorted(_cabi.EXPORTS) == names
-    assert _cabi.load().supcon_abi_version() == _cabi.ABI_VERSION == 2
+    assert _cabi.load().supcon_abi_version() == _cabi.ABI_VERSION == 3
     # diagnostics live in the test-only library, not in the product or its public header
     assert not any("debug" in n for n in names)
     assert not hasattr(lib, "supcon_debug_plan") and not hasattr(lib, "supcon_debug_tc_tile")

@@ -352,38 +352,6 @@ def test_mid_size_single_launch_kernel_fp32(cuda_device, n, d, kind, classes, si
 
 
 # ---------------------------------------------------------------------------------------------------------
-# multi-pass forward (the peers' rows arrive over time): any grouping / order of the rank blocks == one sweep
-# ---------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("sim,alpha,k", [("cosine", 0.0, 15), ("cosine", 0.5, 15), ("geodesic", 1.0, 7)])
-def test_multi_pass_forward_equals_single_sweep(cuda_device, sim, alpha, k):
-    """supcon_forward_rows_pass over [own block] + [first arrivals] + [later arrivals] (ring order, as
-    distributed.PeerExchange issues it) == supcon_forward_rows: counts and hard-negative thresholds exactly, sums to
-    rounding (the order of summation differs), partial sums likewise."""
-    n, world = 2048, 8
-    nl = n // world
-    x, y = O.make_inputs(n, 256, "ties" if sim == "cosine" else "iso", classes=3)
-    z = Fn.canonical_z(F.normalize(x, dim=1).to(torch.bfloat16).to(cuda_device))
-    yy = Fn.canonical_labels(y.to(cuda_device), n)
-    for rank in (0, 3, 7):
-        prob = _tc_problem(n, sim=sim, topk=k, alpha=alpha, row_offset=rank * nl, n_rows=nl,
-                           flags=_cabi.FLAG_UNIT_ROWS | _cabi.FLAG_FORCE_TENSOR)
-        s1, p1, _ = Fn.forward_rows(z, yy, prob, want_loss=False)
-        order = [(rank - j) % world for j in range(1, world)]
-        for groups in ([order[:3], order[3:]], [order[:1], order[1:4], order[4:]], [order]):
-            passes = Fn.ForwardPasses([[rank]] + groups)
-            ws = Fn.forward_rows_pass(z, yy, prob, passes, 0)
-            out = None
-            for i in range(1, passes.n):
-                out = Fn.forward_rows_pass(z, yy, prob, passes, i, ws)
-            s2, p2 = out
-            assert torch.equal(s1.view(torch.int32)[:, [2, 3, 5]], s2.view(torch.int32)[:, [2, 3, 5]])
-            assert torch.equal(s1[:, 4], s2[:, 4])                                       # threshold values
-            assert torch.allclose(s1[:, [0, 1, 6, 7]], s2[:, [0, 1, 6, 7]], rtol=1e-5, atol=1e-6)
-            assert torch.allclose(p1[:5], p2[:5], rtol=1e-6)
-            assert torch.equal(p1[5:], p2[5:])                                           # global counts, fixed maximum
-
-
-# ---------------------------------------------------------------------------------------------------------
 # backward beyond L2: the work list ordered by column panels (z > 48 MB)
 # ---------------------------------------------------------------------------------------------------------
 def test_backward_column_panels_beyond_l2(cuda_device):

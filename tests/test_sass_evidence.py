@@ -43,8 +43,8 @@ def test_sweeps_are_tcgen05_tmem_tma(sass_per_kernel):
 
 
 def test_unmasked_cosine_sweeps_use_packed_fp32_pairs(sass_per_kernel):
-    # mangled template arguments: tc_fwd_kernel<SIM, UNI, MINE, POLY, NCH, PLIN>, tc_bwd_kernel<SIM, UNI, MINE, NCH, PLIN>
-    fwd_plin = [v for k, v in sass_per_kernel.items() if "tc_fwd_kernelILi0ELb0ELb0ELi0ELi2ELb1EE" in k]
+    # mangled template arguments: tc_fwd_kernel<SIM, UNI, MINE, NCH, PLIN>, tc_bwd_kernel<SIM, UNI, MINE, NCH, PLIN>
+    fwd_plin = [v for k, v in sass_per_kernel.items() if "tc_fwd_kernelILi0ELb0ELb0ELi2ELb1EE" in k]
     bwd_plin = [v for k, v in sass_per_kernel.items() if "tc_bwd_kernelILi0ELb0ELb0ELi1ELb1EE" in k]
     assert len(fwd_plin) == 1 and len(bwd_plin) == 1
     assert fwd_plin[0]["FFMA2"] >= 32 and fwd_plin[0]["FADD2"] >= 32

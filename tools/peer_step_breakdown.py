@@ -3,8 +3,6 @@
 Captures the step (ShardedSupConLoss + autograd, exactly bench.py's) as a CUDA graph under several settings and
 times 20 replays each (CUDA events, L2 flushed, max over ranks):
   full           the real step
-  pipe           ordered push (rank+1 first, ...) + multi-pass forward (own block, first arrivals, later arrivals)
-                 instead of one push to all peers and a two-phase forward
   noz            rows are NOT pushed / waited for (stale z: timing only)  -> full - noz  = exposed z exchange
   nostats        statistics are NOT pushed / waited for                   -> full - this = exposed stats exchange
   noz,nostats    neither                                                  -> kernels + launch structure only
@@ -14,7 +12,25 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch
 import torch.distributed as dist
-from wav2vec_contr_loss_b200 import distributed as D
+from wav2vec_contr_loss_b200 import _cabi, distributed as D
+
+# The variants leave an exchange out by skipping its push and its wait (the flag ids of the exchanges they drop)
+SKIPS = {"noz": _cabi.PEER_FLAG_Z, "nostats": _cabi.PEER_FLAG_STATS}
+skipped = set()
+_peer_push, _peer_wait = D.Fn.peer_push, D.Fn.peer_wait
+
+
+def peer_push(desc, src0, dst_off0, src1, dst_off1, flag_id, **kw):
+    if flag_id not in skipped:
+        _peer_push(desc, src0, dst_off0, src1, dst_off1, flag_id, **kw)
+
+
+def peer_wait(desc, flag_id, device):
+    if flag_id not in skipped:
+        _peer_wait(desc, flag_id, device)
+
+
+D.Fn.peer_push, D.Fn.peer_wait = peer_push, peer_wait
 
 rank, world, lr = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 dev = torch.device("cuda", lr)
@@ -31,8 +47,8 @@ out = {"world": world, "N": n}
 keep = []      # modules, graphs and outputs stay alive: freeing symmetric memory during a later capture is an error
 rounds = int(sys.argv[2]) if len(sys.argv) > 2 else 2     # the whole list is measured `rounds` times: order effects show
 for rnd, exchange in [(r_, e_) for r_ in range(rounds) for e_ in ("peer", "nccl")]:
-    for variant in (("", "pipe", "noz", "nostats", "noz,nostats") if exchange == "peer" else ("",)):
-        D._EXPERIMENT = variant
+    for variant in (("", "noz", "nostats", "noz,nostats") if exchange == "peer" else ("",)):
+        skipped = {SKIPS[v] for v in variant.split(",") if v}
         mod = D.ShardedSupConLoss(0.07, "cosine", exchange=exchange)
         mod.assume_unit_rows = True
         keep.append(mod)

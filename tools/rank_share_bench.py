@@ -54,5 +54,4 @@ for R in ranks:
     except Exception as ex:  # noqa: BLE001
         gms = str(ex)
     fl = 6.0 * n * nl * 256
-    print(json.dumps(dict(N=n, R=R, rows=nl, fwd_ms=round(fw, 4), bwd_ms=round(bw, 4), graph_ms=(round(gms, 4) if isinstance(gms, float) else gms), graph_tflops=(round(fl / gms / 1e9, 1) if isinstance(gms, float) else None), tflops=round(fl / (fw + bw) / 1e9, 1),
-                          env={k: v for k, v in os.environ.items() if k.startswith("SUPCON_")})), flush=True)
+    print(json.dumps(dict(N=n, R=R, rows=nl, fwd_ms=round(fw, 4), bwd_ms=round(bw, 4), graph_ms=(round(gms, 4) if isinstance(gms, float) else gms), graph_tflops=(round(fl / gms / 1e9, 1) if isinstance(gms, float) else None), tflops=round(fl / (fw + bw) / 1e9, 1))), flush=True)

@@ -22,7 +22,7 @@ FLAG_WS_FROM_FORWARD = 512
 STATS_STRIDE = 8
 N_PARTIALS = 8
 P_SUM_FULL, P_CNT_FULL, P_SUM_MINED, P_CNT_MINED, P_SUM_W, P_GCNT_FULL, P_GCNT_MINED, P_FIXMAX = range(8)
-ABI_VERSION = 2
+ABI_VERSION = 3
 ST_LSE, ST_LSE_M, ST_NPOS, ST_NNEG, ST_THR_VAL, ST_THR_IDX, ST_WSUM, ST_POS_MEAN = range(8)
 
 EXPORTS = (
@@ -32,7 +32,6 @@ EXPORTS = (
     "supcon_forward_rows_remote", "supcon_head_pool_forward", "supcon_head_pool_backward",
     "supcon_finalize_sets", "supcon_backward_rows_local", "supcon_backward_rows_remote",
     "supcon_peer_push", "supcon_peer_wait", "supcon_peer_end_step", "supcon_label_keys",
-    "supcon_peer_push_ordered", "supcon_peer_wait_mask", "supcon_forward_rows_pass",
 )
 
 
@@ -55,7 +54,7 @@ PEER_FLAG_Z, PEER_FLAG_STATS, PEER_FLAG_DONE, PEER_NFLAGS = 0, 1, 2, 3
 
 
 def peer_flag_bytes(world: int) -> int:
-    return (PEER_NFLAGS * world + 4 + world) * 4
+    return (PEER_NFLAGS * world + 4) * 4
 
 
 _lib = None
@@ -123,14 +122,6 @@ def load():
     lib.supcon_peer_push.restype = c_int32
     lib.supcon_peer_push.argtypes = [PP, c_void_p, c_size_t, ctypes.c_uint64, c_void_p, c_size_t, ctypes.c_uint64,
                                      c_int32, c_int32, c_int32, c_void_p]
-    lib.supcon_peer_push_ordered.restype = c_int32
-    lib.supcon_peer_push_ordered.argtypes = [PP, c_void_p, c_size_t, ctypes.c_uint64, c_void_p, c_size_t,
-                                             ctypes.c_uint64, c_int32, c_int32, c_void_p]
-    lib.supcon_peer_wait_mask.restype = c_int32
-    lib.supcon_peer_wait_mask.argtypes = [PP, c_int32, ctypes.c_uint64, c_void_p]
-    lib.supcon_forward_rows_pass.restype = c_int32
-    lib.supcon_forward_rows_pass.argtypes = [P, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32,
-                                             c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
     lib.supcon_peer_wait.restype = c_int32
     lib.supcon_peer_wait.argtypes = [PP, c_int32, c_void_p]
     lib.supcon_peer_end_step.restype = c_int32

@@ -292,26 +292,6 @@ int supcon_forward_rows_remote(const supcon_problem_t* p, const void* z_all, con
   return 0;
 }
 
-int supcon_forward_rows_pass(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
-                             const int32_t* blocks, const int32_t* pass_sizes, int32_t n_passes, int32_t pass_index,
-                             int32_t skip_norms, float* row_stats, double* partials, void* workspace,
-                             size_t workspace_bytes, void* stream) {
-  if (int rc = validate(p)) return rc;
-  if (!(use_tc(p, false) && tc_two_phase(p)))
-    return fail(SUPCON_E_UNSUPPORTED, "supcon_forward_rows_pass needs the tensor path with equal, 128-aligned row blocks");
-  if (!z_all || !labels_all || !blocks || !pass_sizes || !workspace)
-    return fail(SUPCON_E_INVALID, "NULL buffer passed to supcon_forward_rows_pass");
-  if (pass_index == n_passes - 1 && (!row_stats || !partials))
-    return fail(SUPCON_E_INVALID, "the last pass needs row_stats and partials");
-  if (workspace_bytes < workspace_need(p))
-    return fail(SUPCON_E_WORKSPACE, "workspace too small: %zu < %zu", workspace_bytes, workspace_need(p));
-  const char* err = "";
-  int rc = tc_forward_pass(p, z_all, labels_all, blocks, pass_sizes, n_passes, pass_index, skip_norms, row_stats,
-                           partials, workspace, reinterpret_cast<cudaStream_t>(stream), &err);
-  if (rc) return fail(rc, "tc_forward_pass: %s", err);
-  return 0;
-}
-
 int supcon_finalize(const supcon_problem_t* p, const double* partials_global, float* loss_out,
                     void* stream) {
   if (int rc = validate(p)) return rc;
@@ -538,31 +518,13 @@ int supcon_peer_push(const supcon_peer_t* pe, const void* src0, size_t bytes0, u
   return 0;
 }
 
-int supcon_peer_push_ordered(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0,
-                             const void* src1, size_t bytes1, uint64_t dst_off1, int32_t flag_id,
-                             int32_t wait_flag_id, void* stream) {
-  const char* err = "";
-  if (int rc = peer_check(pe, &err)) return fail(rc, "supcon_peer_push_ordered: %s", err);
-  if (!src0 || (bytes0 % 4) || (src1 && (bytes1 % 4)) || flag_id < 0 || flag_id >= SUPCON_PEER_NFLAGS ||
-      wait_flag_id >= SUPCON_PEER_NFLAGS)
-    return fail(SUPCON_E_INVALID, "bad arguments to supcon_peer_push_ordered");
-  cudaError_t e = peer_push_ordered(*pe, src0, bytes0, dst_off0, src1, bytes1, dst_off1, flag_id, wait_flag_id,
-                                    reinterpret_cast<cudaStream_t>(stream));
-  if (e != cudaSuccess) return cuda_fail(e, "peer_push_ordered_kernel");
-  return 0;
-}
-
-int supcon_peer_wait_mask(const supcon_peer_t* pe, int32_t flag_id, uint64_t rank_mask, void* stream) {
+int supcon_peer_wait(const supcon_peer_t* pe, int32_t flag_id, void* stream) {
   const char* err = "";
   if (int rc = peer_check(pe, &err)) return fail(rc, "supcon_peer_wait: %s", err);
   if (flag_id < 0 || flag_id >= SUPCON_PEER_NFLAGS) return fail(SUPCON_E_INVALID, "bad flag id");
-  cudaError_t e = peer_wait(*pe, flag_id, rank_mask, reinterpret_cast<cudaStream_t>(stream));
+  cudaError_t e = peer_wait(*pe, flag_id, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "peer_wait_kernel");
   return 0;
-}
-
-int supcon_peer_wait(const supcon_peer_t* pe, int32_t flag_id, void* stream) {
-  return supcon_peer_wait_mask(pe, flag_id, ~0ull, stream);
 }
 
 int supcon_peer_end_step(const supcon_peer_t* pe, int32_t flag_id, void* stream) {

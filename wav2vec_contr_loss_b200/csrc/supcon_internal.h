@@ -72,12 +72,7 @@ struct TcPlan {
   uint32_t hash_size;
 };
 constexpr int TC_CMAX = 32;         // most classes the class-sum route handles (more: per-pair sums in the sweep)
-constexpr int TC_MAX_PASSES = 4;    // passes of a multi-pass forward (own columns + up to three groups of peers)
-constexpr int TC_MAX_BLOCKS = 16;   // rank blocks one pass may list
-struct TcBlockList {                // column blocks a launch sweeps, in sweep order: block b covers `len` units from start[b]
-  int n, len;
-  int start[TC_MAX_BLOCKS];
-};
+constexpr int TC_FWD_PASSES = 2;    // passes the forward merge sums: the whole sweep, or own columns + the others
 struct TcFwdArgs {
   const int32_t* lab_pad;
   const float* nrm_pad;
@@ -98,11 +93,10 @@ struct TcFwdArgs {
   int32_t* topk_i;
   TcSched sched;
   int ct_base, ex_lo, ex_len, slot_base;
-  TcBlockList blocks;   // n > 0: the logical -> physical column-tile map of this launch (instead of ct_base / ex_*)
   // merge only: every pass whose partial records are summed (sched + first slot)
   int npass;
-  TcSched msched[TC_MAX_PASSES];
-  int mslot[TC_MAX_PASSES];
+  TcSched msched[TC_FWD_PASSES];
+  int mslot[TC_FWD_PASSES];
   int n_total, n_pad, row_offset, n_rows, rows_pad, topk, mine, kcap;
   float inv_tau, c1, c0, ut2;
   float m_limit;     // tau / 0.025: largest fixed maximum that cannot underflow a row's dominant terms
@@ -160,11 +154,6 @@ int tc_debug_sched(int T, int P, long long U, int cta, int row_block, long long*
 int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, float* row_stats,
                double* partials, float* loss_out, void* workspace, cudaStream_t stream, const char** err,
                int phase = 0);
-// multi-pass forward: pass `pass_index` sweeps the rank blocks blocks[first .. first + pass_sizes[pass_index]);
-// pass 0 clears the workspace, the last pass merges all of them
-int tc_forward_pass(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const int32_t* blocks,
-                    const int32_t* pass_sizes, int n_passes, int pass_index, int skip_norms, float* row_stats,
-                    double* partials, void* workspace, cudaStream_t stream, const char** err);
 // phase: 0 = whole backward; 1 = only the columns this rank owns (`stats` = the rank's OWN statistics
 // [n_rows][STRIDE], `partials` = its own forward partials; partial dz records, nothing else is written);
 // 2 = all other columns (`stats` = everyone's, `partials` = the global sums) + reduce over both phases.
@@ -177,9 +166,7 @@ int peer_check(const supcon_peer_t* pe, const char** err);
 cudaError_t peer_push(const supcon_peer_t& pe, const void* src0, size_t bytes0, uint64_t off0, const void* src1,
                       size_t bytes1, uint64_t off1, int flag_id, int wait_flag_id, int include_self,
                       cudaStream_t stream);
-cudaError_t peer_push_ordered(const supcon_peer_t& pe, const void* src0, size_t bytes0, uint64_t off0, const void* src1,
-                              size_t bytes1, uint64_t off1, int flag_id, int wait_flag_id, cudaStream_t stream);
-cudaError_t peer_wait(const supcon_peer_t& pe, int flag_id, uint64_t mask, cudaStream_t stream);
+cudaError_t peer_wait(const supcon_peer_t& pe, int flag_id, cudaStream_t stream);
 cudaError_t peer_end_step(const supcon_peer_t& pe, int flag_id, cudaStream_t stream);
 
 // ---- single-launch small-batch path (supcon_small.cu) ----

@@ -16,7 +16,6 @@
 // before the consumers' loads.  Every spin is bounded (trap after ~seconds) so a protocol error cannot hang a GPU.
 // Kernels of DIFFERENT GPUs wait on one another; kernels of one GPU never do.
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "supcon_common.cuh"
 #include "supcon_internal.h"
@@ -130,64 +129,9 @@ __global__ void __launch_bounds__(256, 6) peer_push_kernel(PushArgs a) {
   if (threadIdx.x == 0) *ticket = 0u;
 }
 
-// Ordered form of the push: the block goes to rank+1 first, then rank+2, ... and each destination's flag is raised
-// as soon as ITS copy is complete.  Every rank doing the same, a receiver sees its peers' blocks arrive one after
-// another (from rank-1 first), each at the full rate of the link, instead of all of them at the very end -- so its
-// forward can start on the first blocks while the later ones are still in flight.
-__global__ void __launch_bounds__(256, 6) peer_push_ordered_kernel(PushArgs a) {
-  const supcon_peer_t& pe = a.pe;
+__global__ void peer_wait_kernel(supcon_peer_t pe, int flag_id) {
   const int e = *pe.epoch;
-  // per-destination block counters behind the flags and the ticket word of the own buffer (zero between launches)
-  unsigned* tickets = reinterpret_cast<unsigned*>(flag_ptr(pe, pe.rank, SUPCON_PEER_NFLAGS, 0)) + 4;
-  __shared__ int is_last;
-  if (a.wait_flag_id >= 0) {
-    if ((int)threadIdx.x < pe.world) wait_flag(pe, a.wait_flag_id, threadIdx.x, e - 1);
-    __syncthreads();
-  }
-  const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x, nthr = (long long)gridDim.x * blockDim.x;
-  constexpr int U = 4;
-  for (int k = 1; k < pe.world; ++k) {
-    const int p = (pe.rank + k) % pe.world;
-    for (int sgm = 0; sgm < 2; ++sgm) {
-      const unsigned long long nb = a.bytes[sgm];
-      if (nb == 0) continue;
-      const char* src = a.src[sgm];
-      const bool vec = ((reinterpret_cast<uintptr_t>(src) | a.dst_off[sgm]) & 15) == 0;
-      const long long n16 = vec ? (long long)(nb / 16) : 0;
-      const uint4* s16 = reinterpret_cast<const uint4*>(src);
-      uint4* d16 = reinterpret_cast<uint4*>(pe.peer_bases[p] + a.dst_off[sgm]);
-      for (long long i = tid; i < n16; i += U * nthr) {
-        uint4 v[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u)
-          if (i + u * nthr < n16) v[u] = __ldg(s16 + i + u * nthr);
-#pragma unroll
-        for (int u = 0; u < U; ++u)
-          if (i + u * nthr < n16) d16[i + u * nthr] = v[u];
-      }
-      const int* s4 = reinterpret_cast<const int*>(src);
-      int* d4 = reinterpret_cast<int*>(pe.peer_bases[p] + a.dst_off[sgm]);
-      for (long long i = n16 * 4 + tid; i < (long long)(nb / 4); i += nthr) d4[i] = __ldg(s4 + i);
-    }
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      is_last = (atomicAdd(&tickets[k], 1u) == gridDim.x - 1);
-      if (is_last) {
-        __threadfence_system();
-        st_flag(flag_ptr(pe, p, a.flag_id, pe.rank), e);
-        tickets[k] = 0u;
-      }
-    }
-    __syncthreads();
-  }
-  // the own buffer's flag: the caller has put this rank's own block there itself
-  if (blockIdx.x == 0 && threadIdx.x == 0) st_flag(flag_ptr(pe, pe.rank, a.flag_id, pe.rank), e);
-}
-
-__global__ void peer_wait_kernel(supcon_peer_t pe, int flag_id, unsigned long long mask) {
-  const int e = *pe.epoch;
-  if ((int)threadIdx.x < pe.world && ((mask >> threadIdx.x) & 1ull)) wait_flag(pe, flag_id, threadIdx.x, e);
+  if ((int)threadIdx.x < pe.world) wait_flag(pe, flag_id, threadIdx.x, e);
   __syncthreads();
   __threadfence_system();
 }
@@ -222,13 +166,7 @@ cudaError_t peer_push(const supcon_peer_t& pe, const void* src0, size_t bytes0, 
   // enough threads in flight to fill the NVLink egress (16 B per store), few enough to sit beside a compute kernel
   const size_t chunks = (bytes0 + a.bytes[1]) / 16 + 1;
   int blocks = (int)((chunks + 255) / 256);
-  static const int max_blocks = [] {   // tuning knob, read once
-    const char* v = getenv("SUPCON_PEER_PUSH_BLOCKS");
-    const int n = (v && *v) ? atoi(v) : 0;
-    return n > 0 ? n : 0;
-  }();
-  const int cap = max_blocks > 0 ? max_blocks : 64;
-  if (blocks > cap) blocks = cap;
+  if (blocks > 64) blocks = 64;
   // The push runs BESIDE the own-column forward, whose CTAs need the SM's maximum shared-memory carve-out.  CTAs
   // of kernels that prefer different carve-outs cannot share an SM (the SM would have to drain to re-partition
   // L1 / shared memory), so without this the 1-CTA-per-SM compute kernel waits for the push on every SM the push
@@ -240,26 +178,8 @@ cudaError_t peer_push(const supcon_peer_t& pe, const void* src0, size_t bytes0, 
   peer_push_kernel<<<blocks, 256, 0, stream>>>(a);
   return cudaGetLastError();
 }
-cudaError_t peer_push_ordered(const supcon_peer_t& pe, const void* src0, size_t bytes0, uint64_t off0, const void* src1,
-                              size_t bytes1, uint64_t off1, int flag_id, int wait_flag_id, cudaStream_t stream) {
-  PushArgs a;
-  a.pe = pe;
-  a.src[0] = reinterpret_cast<const char*>(src0); a.bytes[0] = bytes0; a.dst_off[0] = off0;
-  a.src[1] = reinterpret_cast<const char*>(src1); a.bytes[1] = src1 ? bytes1 : 0; a.dst_off[1] = off1;
-  a.flag_id = flag_id; a.wait_flag_id = wait_flag_id; a.include_self = 0;
-  static const cudaError_t carve = cudaFuncSetAttribute(peer_push_ordered_kernel,
-                                                        cudaFuncAttributePreferredSharedMemoryCarveout,
-                                                        (int)cudaSharedmemCarveoutMaxShared);
-  (void)carve;
-  const size_t chunks = (bytes0 + a.bytes[1]) / 64 + 1;   // four 16-byte chunks per thread per sweep
-  int blocks = (int)((chunks + 255) / 256);
-  if (blocks > 64) blocks = 64;
-  if (blocks < 1) blocks = 1;
-  peer_push_ordered_kernel<<<blocks, 256, 0, stream>>>(a);
-  return cudaGetLastError();
-}
-cudaError_t peer_wait(const supcon_peer_t& pe, int flag_id, uint64_t mask, cudaStream_t stream) {
-  peer_wait_kernel<<<1, 64, 0, stream>>>(pe, flag_id, mask);
+cudaError_t peer_wait(const supcon_peer_t& pe, int flag_id, cudaStream_t stream) {
+  peer_wait_kernel<<<1, 64, 0, stream>>>(pe, flag_id);
   return cudaGetLastError();
 }
 cudaError_t peer_end_step(const supcon_peer_t& pe, int flag_id, cudaStream_t stream) {

@@ -31,7 +31,6 @@
 // result: every exponential becomes NaN and so do the loss and dz -- loud, never silently wrong.  Without the
 // promise such inputs take the exact path (online maximum), which handles any norms.
 #include <stdio.h>
-#include <stdlib.h>
 
 #include "supcon_common.cuh"
 #include "supcon_internal.h"
@@ -84,36 +83,8 @@ __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) {
   asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
   return r;
 }
-// 2^x on the FMA / ALU pipes (no MUFU), for x in (-126, 127): Cody-Waite split x = n + f with n = floor(x) taken
-// from the low mantissa bits of x + 1.5 * 2^23 (rounded toward -inf), 2^f on [0, 1) by the degree-4 minimax
-// polynomial (relative error 2.7e-6, fp32 Horner included), 2^n added into the exponent field.  Built to take a
-// fixed fraction of the forward's exponentials off the MUFU unit (at d = 256 a 128 x 128 tile costs the tensor
-// pipe and the MUFU unit the same ~1024 cycles per SM); see poly_elem for what the measurement said.
-// The exponents of this path lie in [-2 M log2(e) / tau, ~1] with M / tau <= 40 (tc_supported / m_limit), i.e.
-// above -116: no clamp is needed.  Which elements take this route depends only on the column index (mod 8), so
-// the result does not depend on how rows or columns are split over CTAs or ranks.
-__device__ __forceinline__ float ex2_poly(float x) {
-  constexpr float MAGIC = 12582912.f;   // 1.5 * 2^23
-  float r;
-  asm("add.rm.ftz.f32 %0, %1, %2;" : "=f"(r) : "f"(x), "f"(MAGIC));
-  const float f = x - (r - MAGIC);      // in [0, 1)
-  float p = 0.013534167781472206f;
-  p = fmaf(p, f, 0.052011460065841675f);
-  p = fmaf(p, f, 0.2414427548646927f);
-  p = fmaf(p, f, 0.6930038332939148f);
-  p = fmaf(p, f, 1.0000026226043701f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(r) << 23));
-}
-// element e of a 32-column chunk takes the polynomial route when POLY says so: 4 = every fourth, 8 = every
-// eighth, 2 = every second, 0 = none.  MEASURED (profiles/r02_fwd_poly_ab.md, N = 65536): forward 1.573 ms with
-// none, 1.636 / 1.763 / 2.041 ms with 1/8, 1/4, 1/2 of the exponentials here -- the sweep is bound by the
-// dependent instruction stream of its two softmax warps per scheduler, not by MUFU throughput, and the
-// polynomial's eight dependent FMA-pipe instructions lengthen exactly that.  So the default is 0; the 1/4
-// variant stays selectable (SUPCON_TC_FWD_POLY=4) to reproduce the measurement.
-template <int POLY>
-__device__ __forceinline__ constexpr bool poly_elem(int e) {
-  return POLY == 2 ? (e & 1) == 1 : POLY == 4 ? (e & 3) == 3 : POLY == 8 ? (e & 7) == 7 : false;
-}
+// Every exponential stays on the MUFU unit: moving a share of them to the FMA pipe was slower at every ratio tried
+// (profiles/r02_fwd_poly_ab.md).
 __device__ __forceinline__ float sqrt_approx(float x) {
   float y;
   asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -179,12 +150,6 @@ __device__ __forceinline__ float fixmax_from_bits(unsigned bits, float m_limit) 
   return m2 <= m_limit ? m2 : __int_as_float(0x7fc00000);   // beyond tau / 0.025: poison (NaN), see the header
 }
 
-// logical unit w of a launch that sweeps a list of equal-length blocks -> physical unit
-__host__ __device__ __forceinline__ int block_list_map(const TcBlockList& bl, int w) {
-  const int b = w / bl.len;
-  return bl.start[b] + (w - b * bl.len);
-}
-
 // padded labels + squared norms of `count` columns of [j_lo, n_pad) minus the window [ex_lo, ex_lo + ex_len),
 // and their running maximum (one atomic per block).  One warp per column, grid-stride.
 __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* __restrict__ z,
@@ -192,18 +157,16 @@ __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* _
                                                           int32_t* __restrict__ lab_pad, float* __restrict__ nrm_pad,
                                                           unsigned* __restrict__ nrm2_max, int count, int j_lo = 0,
                                                           int ex_lo = 0x7fffffff, int ex_len = 0,
-                                                          int track_max = 1, TcBlockList bl = TcBlockList{0, 1, {0}},
-                                                          int read_z = 1) {
+                                                          int track_max = 1) {
   __shared__ float wmax[8];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   float mx = 0.f;
   for (int w = blockIdx.x * 8 + wib; w < count; w += gridDim.x * 8) {
     int j = j_lo + w;
     if (j >= ex_lo) j += ex_len;
-    if (bl.n > 0) j = block_list_map(bl, w);
     if (j >= n_pad) break;
     float s = 0.f;
-    if (j < n && read_z) {
+    if (j < n) {
       const __nv_bfloat16* zr = z + (int64_t)j * d;
       for (int k = 8 * lane; k < d; k += 256) {   // d % 8 == 0 on this path (d == 256): 16-byte loads
         const uint4 v = __ldg(reinterpret_cast<const uint4*>(zr + k));
@@ -237,14 +200,9 @@ __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* _
 // hids / n_classes (optional): the thread that claims a slot also gives it the next dense class id
 __global__ void tc_label_table_kernel(const int32_t* __restrict__ labels, int n, unsigned long long* hkeys,
                                       int* hcounts, uint32_t hmask, int j_lo, int ex_lo, int ex_len,
-                                      TcBlockList bl = TcBlockList{0, 1, {0}}, int* hids = nullptr,
-                                      int* n_classes = nullptr) {
+                                      int* hids = nullptr, int* n_classes = nullptr) {
   int j = j_lo + blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= ex_lo) j += ex_len;
-  if (bl.n > 0) {
-    const int w = blockIdx.x * blockDim.x + threadIdx.x;
-    j = w < bl.n * bl.len ? block_list_map(bl, w) : n;
-  }
   const bool ok = j < n;
   const unsigned active = __ballot_sync(0xffffffffu, ok);
   if (!ok) return;
@@ -464,14 +422,14 @@ __device__ __noinline__ MineState mine_candidates(int sim, uint32_t taddr_chunk,
   return ms;
 }
 
-template <int SIM, bool UNI, bool MINE, bool MASKED, int POLY, bool PLIN>
+template <int SIM, bool UNI, bool MINE, bool MASKED, bool PLIN>
 __device__ __forceinline__ void fwd_chunk(const uint32_t (&r)[32], int gj0, int gi, int n_total, int lab_r,
                                           float nrm_r, const int32_t* __restrict__ lab_s,
                                           const float* __restrict__ nrm_s, float c1, float c0, float ut2,
                                           RowSums& st, MineState& ms, float* wl_v, int* wl_i, int lane, int K,
                                           uint32_t taddr_chunk) {
   // lab_s / nrm_s: this chunk's 32 column labels / squared norms in shared memory (broadcast reads)
-  if constexpr (SIM == SUPCON_COSINE && !MINE && !MASKED && POLY == 0) {
+  if constexpr (SIM == SUPCON_COSINE && !MINE && !MASKED) {
     // packed pairs: exponent arguments and the running sum, two columns per instruction
     const f32x2 c1p = pk2(c1, c1), c0p = pk2(c0, c0);
 #pragma unroll
@@ -512,7 +470,7 @@ __device__ __forceinline__ void fwd_chunk(const uint32_t (&r)[32], int gj0, int 
     for (int e = 0; e < 4; ++e) {
       const float c = __uint_as_float(r[4 * q + e]);
       const float s = (SIM == SUPCON_GEODESIC) ? geodesic_sim_fast(c) : c;
-      float ex = poly_elem<POLY>(4 * q + e) ? ex2_poly(fmaf(s, c1, c0)) : ex2f(fmaf(s, c1, c0));
+      float ex = ex2f(fmaf(s, c1, c0));
       bool pos = PLIN ? false : labs[e] == lab_r;   // PLIN: the positives' sum comes from the class sums (merge)
       bool neg = !pos;
       if (MASKED) {
@@ -547,7 +505,6 @@ __device__ __forceinline__ void fwd_chunk(const uint32_t (&r)[32], int gj0, int 
 // logical column tile of this launch -> physical tile: a launch covers [ct_base, ...) minus an excluded window
 // (the two-phase multi-GPU forward first sweeps the rank's own columns, then everything else)
 __device__ __forceinline__ int fwd_col_tile(const TcFwdArgs& a, int ct) {
-  if (a.blocks.n > 0) return block_list_map(a.blocks, ct);
   return a.ct_base + ct + (ct >= a.ex_lo ? a.ex_len : 0);
 }
 
@@ -578,7 +535,7 @@ __device__ __forceinline__ void load_rows_to_tmem(const __nv_bfloat16* __restric
 // releases the TMEM buffer at once (the next MMA into it overlaps the exp work) and then reduces
 // from registers.  All pipeline barriers are indexed by a running tile counter, so segments
 // follow each other without draining the TMA ring.
-template <int SIM, bool UNI, bool MINE, int POLY, int NCH, bool PLIN>
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
 __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid_constant__ CUtensorMap tmap,
                                                                     const __nv_bfloat16* __restrict__ z, TcFwdArgs a) {
   static_assert(NCH == 1 || (NCH == 2 && !MINE), "the top-K lists are kept by one thread per row");
@@ -732,18 +689,18 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid
         const int32_t* lab_s = lab_ring[slot] + cc;
         const float* nrm_s = nrm_ring[UNI ? slot : 0] + cc;
         if (masked) {
-          fwd_chunk<SIM, UNI, MINE, true, POLY, PLIN>(r0, col0 + cc, gi, a.n_total, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
-          fwd_chunk<SIM, UNI, MINE, true, POLY, PLIN>(r1, col0 + cc + 32, gi, a.n_total, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
+          fwd_chunk<SIM, UNI, MINE, true, PLIN>(r0, col0 + cc, gi, a.n_total, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
+          fwd_chunk<SIM, UNI, MINE, true, PLIN>(r1, col0 + cc + 32, gi, a.n_total, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
           if constexpr (NCH == 1) {
-            fwd_chunk<SIM, UNI, MINE, true, POLY, PLIN>(r2, col0 + 64, gi, a.n_total, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
-            fwd_chunk<SIM, UNI, MINE, true, POLY, PLIN>(r3, col0 + 96, gi, a.n_total, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
+            fwd_chunk<SIM, UNI, MINE, true, PLIN>(r2, col0 + 64, gi, a.n_total, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
+            fwd_chunk<SIM, UNI, MINE, true, PLIN>(r3, col0 + 96, gi, a.n_total, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
           }
         } else {
-          fwd_chunk<SIM, UNI, MINE, false, POLY, PLIN>(r0, col0 + cc, gi, a.n_total, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
-          fwd_chunk<SIM, UNI, MINE, false, POLY, PLIN>(r1, col0 + cc + 32, gi, a.n_total, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
+          fwd_chunk<SIM, UNI, MINE, false, PLIN>(r0, col0 + cc, gi, a.n_total, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
+          fwd_chunk<SIM, UNI, MINE, false, PLIN>(r1, col0 + cc + 32, gi, a.n_total, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
           if constexpr (NCH == 1) {
-            fwd_chunk<SIM, UNI, MINE, false, POLY, PLIN>(r2, col0 + 64, gi, a.n_total, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
-            fwd_chunk<SIM, UNI, MINE, false, POLY, PLIN>(r3, col0 + 96, gi, a.n_total, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
+            fwd_chunk<SIM, UNI, MINE, false, PLIN>(r2, col0 + 64, gi, a.n_total, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
+            fwd_chunk<SIM, UNI, MINE, false, PLIN>(r3, col0 + 96, gi, a.n_total, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
           }
         }
         if (MINE) {   // candidates re-read S from tensor memory: release the buffer only now
@@ -833,10 +790,10 @@ __global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishAr
     // partial records of this row: one per CTA whose unit range touches the row's 256-row block,
     // in CTA order = ascending column order
     const int rb = lr / (2 * TBM);
-    // slot list of this row: one range of slots per pass of the forward (one, two or more passes)
-    int slot_lo[TC_MAX_PASSES], slot_n[TC_MAX_PASSES];
+    // slot list of this row: one range of slots per pass of the forward (one or two passes)
+    int slot_lo[TC_FWD_PASSES], slot_n[TC_FWD_PASSES];
     const int npass = a.npass;
-    for (int ps = 0; ps < TC_MAX_PASSES; ++ps) {
+    for (int ps = 0; ps < TC_FWD_PASSES; ++ps) {
       slot_lo[ps] = 0; slot_n[ps] = 0;
       if (ps < npass) {
         const TcSched& ms = a.msched[ps];
@@ -1367,38 +1324,15 @@ __global__ void __launch_bounds__(256) tc_bwd_reduce_kernel(TcBwdArgs a, const _
   }
 }
 
-// Tuning knobs: read from the environment ONCE, when the library is first used (never on the launch path),
-// so that a plan is a pure function of the problem afterwards.  0 / unset = the built-in choice.
-struct TcKnobs {
-  int fwd_ctas, bwd_ctas, local_ctas, local_free_sms, bwd_local_free_sms, bwd_panels;
-  int fwd_poly;   // 4: a quarter of the forward's exponentials evaluated off the MUFU unit (A/B only); else none
-  int fwd_nch, bwd_nch;   // threads per tile row (1 or 2; 0 = built-in choice), see tc_threads()
-  int fwd_plin, bwd_plin; // positives by linearity (cosine, no mining) in the forward / backward: 0 = off, else on
-};
-int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return (v && *v) ? atoi(v) : dflt;
-}
-const TcKnobs& knobs() {
-  static const TcKnobs k = {env_int("SUPCON_TC_FWD_CTAS", 0), env_int("SUPCON_TC_BWD_CTAS", 0),
-                            env_int("SUPCON_TC_LOCAL_CTAS", 0), env_int("SUPCON_TC_LOCAL_FREE_SMS", 32),
-                            env_int("SUPCON_TC_BWD_LOCAL_FREE_SMS", 16), env_int("SUPCON_TC_BWD_PANELS", 0),
-                            env_int("SUPCON_TC_FWD_POLY", -1), env_int("SUPCON_TC_FWD_NCH", 0),
-                            env_int("SUPCON_TC_BWD_NCH", 0), env_int("SUPCON_TC_FWD_PLIN", 1),
-                            env_int("SUPCON_TC_BWD_PLIN", 1)};
-  return k;
-}
-
-TcSched make_sched(int row_blocks, int col_tiles, int num_sms, int forced_ctas, int leave_free = 0) {
+TcSched make_sched(int row_blocks, int col_tiles, int num_sms, int leave_free = 0) {
   TcSched sc;
   sc.T = col_tiles;
   sc.U = (long long)row_blocks * col_tiles;
   sc.RB = row_blocks; sc.NP = 1; sc.Tp = col_tiles;
   // two CTAs' worth of work per SM: the hardware scheduler evens out SM-to-SM speed differences
   // (measured: rank share of N/8 rows 0.714 -> 0.694 ms), as long as a CTA still gets >= 32 tiles
-  long long p = forced_ctas;
-  if (p <= 0 && leave_free > 0) p = num_sms > leave_free ? num_sms - leave_free : 1;   // one CTA per used SM
-  if (p <= 0) p = (sc.U / (2LL * num_sms) >= 32) ? 2LL * num_sms : num_sms;
+  long long p = (sc.U / (2LL * num_sms) >= 32) ? 2LL * num_sms : num_sms;
+  if (leave_free > 0) p = num_sms > leave_free ? num_sms - leave_free : 1;   // one CTA per used SM
   if (p > sc.U) p = sc.U;
   if (p < 1) p = 1;
   sc.P = (int)p;
@@ -1459,7 +1393,6 @@ const char* tmap_error(int code, const void* base, int rows) {
 // ---- workspace layout shared by forward and backward ----
 TcPlan tc_plan(const supcon_problem_t* p) {
   TcPlan pl;
-  const TcKnobs& kn = knobs();
   const int sms = num_sms();
   pl.n_pad = (int)align_up((size_t)p->n_total, 128);
   pl.rows_pad = (int)align_up((size_t)p->n_rows, 128);
@@ -1467,8 +1400,8 @@ TcPlan tc_plan(const supcon_problem_t* p) {
   pl.fwd_row_blocks = (pl.row_blocks + 1) / 2;   // forward CTAs own two 128-row blocks
   pl.fwd_col_tiles = pl.n_pad / 128;
   pl.bwd_col_tiles = (p->n_total + 63) / 64;
-  pl.fwd_sched = make_sched(pl.fwd_row_blocks, pl.fwd_col_tiles, sms, kn.fwd_ctas);
-  pl.bwd_sched = make_sched(pl.row_blocks, pl.bwd_col_tiles, sms, kn.bwd_ctas);
+  pl.fwd_sched = make_sched(pl.fwd_row_blocks, pl.fwd_col_tiles, sms);
+  pl.bwd_sched = make_sched(pl.row_blocks, pl.bwd_col_tiles, sms);
   pl.fwd_slots = sched_max_slots(pl.fwd_sched, pl.fwd_row_blocks);
   // Backward beyond L2: with z larger than ~48 MB the CTAs of a wave, each somewhere else in its own column sweep,
   // stream ALL of z concurrently and the 64-column Z_J tiles miss L2 (measured at N = 186368, a rank's 23296 rows:
@@ -1481,7 +1414,6 @@ TcPlan tc_plan(const supcon_problem_t* p) {
     if (z_bytes <= (48u << 20)) np = 1;
     if (np > 16) np = 16;
     while (np > 1 && pl.bwd_col_tiles < 64 * np) --np;
-    if (knobs().bwd_panels > 0) np = knobs().bwd_panels;
     if (np > 1) {
       pl.bwd_sched.NP = np;
       pl.bwd_sched.Tp = (pl.bwd_col_tiles + np - 1) / np;
@@ -1501,26 +1433,15 @@ TcPlan tc_plan(const supcon_problem_t* p) {
     // an own-column phase runs beside an NCCL all-gather kernel: leave SMs free for its channels (a CTA of
     // these kernels fills an SM, so the collective could not co-reside and the two would serialise)
     // (only when that phase is short, i.e. the rank owns at most a quarter of the columns)
+    constexpr int LOCAL_FREE_SMS = 32, BWD_LOCAL_FREE_SMS = 16;   // forward / backward
     const bool small_share = (4 * pl.local_cts <= pl.fwd_col_tiles) && !(p->flags & SUPCON_FLAG_PEER_EXCHANGE);
-    pl.fwd_sched_local = make_sched(pl.fwd_row_blocks, pl.local_cts, sms, kn.local_ctas,
-                                    small_share ? kn.local_free_sms : 0);
-    pl.fwd_sched_remote = make_sched(pl.fwd_row_blocks, pl.fwd_col_tiles - pl.local_cts, sms, kn.fwd_ctas);
+    pl.fwd_sched_local = make_sched(pl.fwd_row_blocks, pl.local_cts, sms, small_share ? LOCAL_FREE_SMS : 0);
+    pl.fwd_sched_remote = make_sched(pl.fwd_row_blocks, pl.fwd_col_tiles - pl.local_cts, sms);
     pl.slots_local = sched_max_slots(pl.fwd_sched_local, pl.fwd_row_blocks);
     int both = pl.slots_local + sched_max_slots(pl.fwd_sched_remote, pl.fwd_row_blocks);
     if (both > pl.fwd_slots) pl.fwd_slots = both;
-    // multi-pass forward (tc_forward_pass): up to TC_MAX_PASSES passes over groups of rank blocks; a row block's
-    // records per pass never exceed those of the widest single-pass schedule seen over all group sizes
-    if (p->n_total % p->n_rows == 0) {
-      const int world = p->n_total / p->n_rows;
-      int worst = 1;
-      for (int k = 1; k <= world && k <= TC_MAX_BLOCKS; ++k) {
-        const int sl = sched_max_slots(make_sched(pl.fwd_row_blocks, k * pl.local_cts, sms, 0), pl.fwd_row_blocks);
-        if (sl > worst) worst = sl;
-      }
-      if (TC_MAX_PASSES * worst > pl.fwd_slots) pl.fwd_slots = TC_MAX_PASSES * worst;
-    }
-    pl.bwd_sched_local = make_sched(pl.row_blocks, pl.bwd_local_cts, sms, 0, small_share ? kn.bwd_local_free_sms : 0);
-    pl.bwd_sched_remote = make_sched(pl.row_blocks, pl.bwd_col_tiles - pl.bwd_local_cts, sms, kn.bwd_ctas);
+    pl.bwd_sched_local = make_sched(pl.row_blocks, pl.bwd_local_cts, sms, small_share ? BWD_LOCAL_FREE_SMS : 0);
+    pl.bwd_sched_remote = make_sched(pl.row_blocks, pl.bwd_col_tiles - pl.bwd_local_cts, sms);
     pl.bwd_slots_local = sched_max_slots(pl.bwd_sched_local, pl.row_blocks);
     both = pl.bwd_slots_local + sched_max_slots(pl.bwd_sched_remote, pl.row_blocks);
     if (both > pl.bwd_slots) pl.bwd_slots = both;
@@ -1593,45 +1514,34 @@ bool tc_supported(const supcon_problem_t* p) {
   return true;
 }
 
-constexpr int FWD_POLY_DEFAULT = 0;
 // Threads per tile row, measured at N = 65536 (profiles/r02_nch_ab.md): the unmined forward gains 4 % from two
 // (1.663 -> 1.595 ms), the mined backward 13 % (6.93 -> 6.01 ms: its membership tests make it issue-bound and more
 // warps fill the slots); the unmined backward gets SLOWER and unsteady with two (3.11 -> 3.36-3.51 ms median).
-constexpr int FWD_NCH_DEFAULT = 2, BWD_NCH_DEFAULT = 1, BWD_MINE_NCH_DEFAULT = 2;
-template <int SIM, bool UNI, bool MINE, int POLY, int NCH, bool PLIN = false>
+// The mined forward keeps one: its top-K lists are kept by one thread per row.
+constexpr int FWD_NCH = 2, BWD_NCH = 1, BWD_MINE_NCH = 2;
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN = false>
 static cudaError_t launch_fwd(const CUtensorMap& tm, const __nv_bfloat16* z, const TcFwdArgs& a, int ctas, size_t smem,
                               cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute(tc_fwd_kernel<SIM, UNI, MINE, POLY, NCH, PLIN>,
+  cudaError_t e = cudaFuncSetAttribute(tc_fwd_kernel<SIM, UNI, MINE, NCH, PLIN>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  tc_fwd_kernel<SIM, UNI, MINE, POLY, NCH, PLIN><<<ctas, tc_threads(NCH), smem, st>>>(tm, z, a);
+  tc_fwd_kernel<SIM, UNI, MINE, NCH, PLIN><<<ctas, tc_threads(NCH), smem, st>>>(tm, z, a);
   return cudaGetLastError();
 }
 template <int SIM, bool UNI>
 static cudaError_t launch_fwd_m(bool mine, const CUtensorMap& tm, const __nv_bfloat16* z, const TcFwdArgs& a, int ctas,
                                 size_t smem, cudaStream_t st) {
-  // mining: the sorted inserts, not the exponentials, bound that sweep -> all exponentials stay on the MUFU unit
-  // (and its top-K lists are kept by one thread per row)
-  if (mine) return launch_fwd<SIM, UNI, true, 0, 1>(tm, z, a, ctas, smem, st);
-  const int poly = knobs().fwd_poly < 0 ? FWD_POLY_DEFAULT : knobs().fwd_poly;
-  const int nch = knobs().fwd_nch == 1 || knobs().fwd_nch == 2 ? knobs().fwd_nch : FWD_NCH_DEFAULT;
+  if (mine) return launch_fwd<SIM, UNI, true, 1>(tm, z, a, ctas, smem, st);
   // positives by linearity (the caller set it up: cosine only): the class-sum kernel first, then its per-pair twin;
   // exactly one of the two does the sweep, decided on the device by the class count
   if (SIM == SUPCON_COSINE && a.n_classes != nullptr) {
-    cudaError_t e = launch_fwd<SUPCON_COSINE, UNI, false, 0, 2, true>(tm, z, a, ctas, smem, st);
+    cudaError_t e = launch_fwd<SUPCON_COSINE, UNI, false, FWD_NCH, true>(tm, z, a, ctas, smem, st);
     if (e != cudaSuccess) return e;
     TcFwdArgs b = a;
     b.plin_twin = 1;
-    if (nch == 2) return launch_fwd<SUPCON_COSINE, UNI, false, 0, 2>(tm, z, b, ctas, smem, st);
-    return launch_fwd<SUPCON_COSINE, UNI, false, 0, 1>(tm, z, b, ctas, smem, st);
+    return launch_fwd<SUPCON_COSINE, UNI, false, FWD_NCH>(tm, z, b, ctas, smem, st);
   }
-  // the polynomial share exists for the headline variant only (A/B measurement: profiles/r02_fwd_poly_ab.md)
-  if (SIM == SUPCON_COSINE && !UNI && poly == 4) {
-    if (nch == 2) return launch_fwd<SUPCON_COSINE, false, false, 4, 2>(tm, z, a, ctas, smem, st);
-    return launch_fwd<SUPCON_COSINE, false, false, 4, 1>(tm, z, a, ctas, smem, st);
-  }
-  if (nch == 2) return launch_fwd<SIM, UNI, false, FWD_POLY_DEFAULT, 2>(tm, z, a, ctas, smem, st);
-  return launch_fwd<SIM, UNI, false, FWD_POLY_DEFAULT, 1>(tm, z, a, ctas, smem, st);
+  return launch_fwd<SIM, UNI, false, FWD_NCH>(tm, z, a, ctas, smem, st);
 }
 
 bool tc_two_phase(const supcon_problem_t* p) { return tc_supported(p) && tc_plan(p).two_phase; }
@@ -1641,7 +1551,7 @@ bool tc_bwd_two_phase(const supcon_problem_t* p) { return tc_two_phase(p) && !(p
 
 // phase: 0 = whole forward; 1 = only the columns this rank owns (partial records, needs nothing from other
 // ranks); 2 = all other columns + merge.  Phases 1 and 2 must use the same workspace.
-// common part of the forward launches: argument block that does not depend on the pass
+// common part of the forward launches: argument block that does not depend on the phase
 static TcFwdArgs fwd_base_args(const supcon_problem_t* p, const TcPlan& pl, char* ws) {
   TcFwdArgs a;
   a.hkeys = reinterpret_cast<const unsigned long long*>(ws + pl.off_hkeys);
@@ -1650,7 +1560,6 @@ static TcFwdArgs fwd_base_args(const supcon_problem_t* p, const TcPlan& pl, char
   a.nrm2_max = reinterpret_cast<unsigned*>(ws) + WS_NRM2_MAX_WORD;
   a.n_classes = nullptr; a.hids = nullptr; a.csum = nullptr; a.z_rows = nullptr; a.plin_twin = 0;
   a.ct_base = 0; a.ex_lo = 0x7fffffff; a.ex_len = 0; a.slot_base = 0;
-  a.blocks.n = 0; a.blocks.len = 1;
   a.npass = 0;
   a.lab_pad = reinterpret_cast<const int32_t*>(ws + pl.off_lab);
   a.nrm_pad = reinterpret_cast<const float*>(ws + pl.off_nrm);
@@ -1688,7 +1597,7 @@ static bool plin_size_ok(const supcon_problem_t* p) {
 // positives by linearity in the forward: whole forward (one phase), cosine, no mining, large enough
 static bool fwd_class_sums(const supcon_problem_t* p, int phase) {
   return phase == 0 && p->similarity == SUPCON_COSINE && !(p->alpha != 0.f && p->topk >= 1) &&
-         knobs().fwd_plin != 0 && !(p->flags & SUPCON_FLAG_NO_CLASS_SUMS) && plin_size_ok(p);
+         !(p->flags & SUPCON_FLAG_NO_CLASS_SUMS) && plin_size_ok(p);
 }
 
 int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, float* row_stats,
@@ -1735,7 +1644,7 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
       tc_label_table_kernel<<<(jn_count + 255) / 256, 256, 0, stream>>>(
           labels_all, p->n_total, reinterpret_cast<unsigned long long*>(ws + pl.off_hkeys),
           reinterpret_cast<int*>(ws + pl.off_hcounts), pl.hash_size - 1, jn_lo, jn_ex_lo, jn_ex_len,
-          TcBlockList{0, 1, {0}}, plin ? hids : nullptr, plin ? n_classes : nullptr);
+          plin ? hids : nullptr, plin ? n_classes : nullptr);
     if (plin) {
       tc_class_sum_kernel<<<pl.csum_blocks, 256, 0, stream>>>(
           reinterpret_cast<const __nv_bfloat16*>(z_all), labels_all, p->n_total,
@@ -1775,86 +1684,6 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
   return 0;
 }
 
-// Multi-pass forward for a rank of a row-sharded job whose peers' rows arrive over time: the columns are swept
-// rank block by rank block in the order given (own block first, then the peers in arrival order), grouped into
-// passes; each pass is one launch over all its blocks and needs only those blocks of z_all / labels_all.
-// blocks[] lists every pass's blocks back to back, pass_sizes[i] how many belong to pass i.
-int tc_forward_pass(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const int32_t* blocks,
-                    const int32_t* pass_sizes, int n_passes, int pass_index, int skip_norms, float* row_stats,
-                    double* partials, void* workspace, cudaStream_t stream, const char** err) {
-  const TcPlan pl = tc_plan(p);
-  char* ws = reinterpret_cast<char*>(workspace);
-  if (!pl.two_phase || p->n_total % p->n_rows != 0) { *err = "multi-pass forward needs equal, 128-aligned row blocks"; return SUPCON_E_UNSUPPORTED; }
-  const int world = p->n_total / p->n_rows;
-  if (n_passes < 1 || n_passes > TC_MAX_PASSES || pass_index < 0 || pass_index >= n_passes) { *err = "bad pass index"; return SUPCON_E_INVALID; }
-  // schedules and first slots of every pass (the merge needs them all; each launch its own)
-  TcSched sched[TC_MAX_PASSES];
-  int slot0[TC_MAX_PASSES], first_block[TC_MAX_PASSES], total_blocks = 0, slots = 0;
-  const int sms = num_sms();
-  for (int i = 0; i < n_passes; ++i) {
-    if (pass_sizes[i] < 1 || pass_sizes[i] > TC_MAX_BLOCKS) { *err = "bad pass size"; return SUPCON_E_INVALID; }
-    first_block[i] = total_blocks;
-    total_blocks += pass_sizes[i];
-    sched[i] = make_sched(pl.fwd_row_blocks, pass_sizes[i] * pl.local_cts, sms, 0);
-    slot0[i] = slots;
-    slots += sched_max_slots(sched[i], pl.fwd_row_blocks);
-  }
-  if (total_blocks != world) { *err = "the passes must list every rank block exactly once"; return SUPCON_E_INVALID; }
-  if (slots > pl.fwd_slots) { *err = "multi-pass forward: more partial-record slots than the workspace holds"; return SUPCON_E_WORKSPACE; }
-  CUtensorMap tm;
-  if (int trc = make_bf16_rowmajor_tmap(&tm, z_all, (uint64_t)p->n_total, (uint64_t)p->d, 128)) {
-    *err = tmap_error(trc, z_all, p->n_total);
-    return SUPCON_E_INVALID;
-  }
-  cudaError_t e = cudaSuccess;
-  if (pass_index == 0) {
-    e = cudaMemsetAsync(workspace, 0, 256, stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ws + pl.off_hkeys, 0, (size_t)pl.hash_size * 12, stream);
-    if (e != cudaSuccess) { *err = cudaGetErrorString(e); return (int)e; }
-  }
-  TcBlockList cols, tiles;   // this pass's blocks in column units and in 128-column tiles
-  cols.n = tiles.n = pass_sizes[pass_index];
-  cols.len = p->n_rows; tiles.len = pl.local_cts;
-  for (int b = 0; b < cols.n; ++b) {
-    const int blk = blocks[first_block[pass_index] + b];
-    if (blk < 0 || blk >= world) { *err = "bad block index"; return SUPCON_E_INVALID; }
-    cols.start[b] = blk * p->n_rows;
-    tiles.start[b] = blk * pl.local_cts;
-  }
-  const int count = cols.n * cols.len;
-  {
-    int nb = (count + 7) / 8;
-    const int cap = 8 * sms;
-    if (nb > cap) nb = cap;
-    // skip_norms: labels only (rows of z not read): the caller vouches for unit rows of the peers' blocks, which
-    // each rank checks for its own rows (pass 0 always reads its rows)
-    const int read_z = (skip_norms && pass_index > 0 && !(p->lambda_uni > 0.f)) ? 0 : 1;
-    tc_prep_fwd_kernel<<<nb, 256, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(z_all), labels_all, p->n_total,
-                                               pl.n_pad, p->d, reinterpret_cast<int32_t*>(ws + pl.off_lab),
-                                               reinterpret_cast<float*>(ws + pl.off_nrm),
-                                               reinterpret_cast<unsigned*>(ws) + WS_NRM2_MAX_WORD, count, 0, 0x7fffffff, 0,
-                                               (p->similarity == SUPCON_COSINE && read_z) ? 1 : 0, cols, read_z);
-    tc_label_table_kernel<<<(count + 255) / 256, 256, 0, stream>>>(
-        labels_all, p->n_total, reinterpret_cast<unsigned long long*>(ws + pl.off_hkeys),
-        reinterpret_cast<int*>(ws + pl.off_hcounts), pl.hash_size - 1, 0, 0x7fffffff, 0, cols);
-  }
-  TcFwdArgs a = fwd_base_args(p, pl, ws);
-  a.sched = sched[pass_index];
-  a.slot_base = slot0[pass_index];
-  a.blocks = tiles;
-  e = fwd_launch_kernel(p, tm, z_all, a, stream);
-  if (e != cudaSuccess) { *err = cudaGetErrorString(e); return (int)e; }
-  if (pass_index + 1 < n_passes) return 0;
-  a.npass = n_passes;
-  for (int i = 0; i < n_passes; ++i) { a.msched[i] = sched[i]; a.mslot[i] = slot0[i]; }
-  FinishArgs f{reinterpret_cast<double*>(ws + pl.off_block_partials), reinterpret_cast<unsigned*>(ws), partials,
-               nullptr, p->n_total, p->tau, p->alpha, p->lambda_uni, p->uni_t};
-  tc_fwd_merge_kernel<<<pl.merge_blocks, 128, 0, stream>>>(a, f, row_stats);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) { *err = cudaGetErrorString(e); return (int)e; }
-  return 0;
-}
-
 template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN = false>
 static cudaError_t launch_bwd(const CUtensorMap& tmJ, const __nv_bfloat16* z, const TcBwdArgs& a, int ctas, size_t smem,
                               cudaStream_t st) {
@@ -1867,22 +1696,16 @@ static cudaError_t launch_bwd(const CUtensorMap& tmJ, const __nv_bfloat16* z, co
 template <int SIM, bool UNI>
 static cudaError_t launch_bwd_m(bool mine, const CUtensorMap& tmJ, const __nv_bfloat16* z, const TcBwdArgs& a, int ctas,
                                 size_t smem, cudaStream_t st) {
-  const int nch = knobs().bwd_nch == 1 || knobs().bwd_nch == 2 ? knobs().bwd_nch
-                                                                : (mine ? BWD_MINE_NCH_DEFAULT : BWD_NCH_DEFAULT);
+  if (mine) return launch_bwd<SIM, UNI, true, BWD_MINE_NCH>(tmJ, z, a, ctas, smem, st);
   // positives by linearity (the caller set it up: cosine, no mining): the class-sum kernel, then its per-pair twin
-  if (SIM == SUPCON_COSINE && !mine && a.n_classes != nullptr) {
-    cudaError_t e = launch_bwd<SUPCON_COSINE, UNI, false, 1, true>(tmJ, z, a, ctas, smem, st);
+  if (SIM == SUPCON_COSINE && a.n_classes != nullptr) {
+    cudaError_t e = launch_bwd<SUPCON_COSINE, UNI, false, BWD_NCH, true>(tmJ, z, a, ctas, smem, st);
     if (e != cudaSuccess) return e;
     TcBwdArgs b = a;
     b.plin_twin = 1;
-    if (nch == 2) return launch_bwd<SUPCON_COSINE, UNI, false, 2>(tmJ, z, b, ctas, smem, st);
-    return launch_bwd<SUPCON_COSINE, UNI, false, 1>(tmJ, z, b, ctas, smem, st);
+    return launch_bwd<SUPCON_COSINE, UNI, false, BWD_NCH>(tmJ, z, b, ctas, smem, st);
   }
-  if (nch == 2)
-    return mine ? launch_bwd<SIM, UNI, true, 2>(tmJ, z, a, ctas, smem, st)
-                : launch_bwd<SIM, UNI, false, 2>(tmJ, z, a, ctas, smem, st);
-  return mine ? launch_bwd<SIM, UNI, true, 1>(tmJ, z, a, ctas, smem, st)
-              : launch_bwd<SIM, UNI, false, 1>(tmJ, z, a, ctas, smem, st);
+  return launch_bwd<SIM, UNI, false, BWD_NCH>(tmJ, z, a, ctas, smem, st);
 }
 
 int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const float* stats,
@@ -1910,7 +1733,7 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
   }
   // positives by linearity: single-phase cosine backward without mining, when the sweep is long enough
   const bool mine_b = p->alpha != 0.f && p->topk >= 1;
-  const bool plin = phase == 0 && p->similarity == SUPCON_COSINE && !mine_b && knobs().bwd_plin != 0 &&
+  const bool plin = phase == 0 && p->similarity == SUPCON_COSINE && !mine_b &&
                     !(p->flags & SUPCON_FLAG_NO_CLASS_SUMS) && plin_size_ok(p);
   int* n_classes = reinterpret_cast<int*>(ws) + WS_NCLASSES_WORD;
   int* hids = reinterpret_cast<int*>(ws + pl.off_hids);
@@ -1923,8 +1746,7 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
     if (e != cudaSuccess) { *err = cudaGetErrorString(e); return (int)e; }
     tc_label_table_kernel<<<(p->n_total + 255) / 256, 256, 0, stream>>>(
         labels_all, p->n_total, reinterpret_cast<unsigned long long*>(ws + pl.off_hkeys),
-        reinterpret_cast<int*>(ws + pl.off_hcounts), pl.hash_size - 1, 0, 0x7fffffff, 0, TcBlockList{0, 1, {0}}, hids,
-        n_classes);
+        reinterpret_cast<int*>(ws + pl.off_hcounts), pl.hash_size - 1, 0, 0x7fffffff, 0, hids, n_classes);
     tc_class_sum_kernel<<<pl.csum_blocks, 256, 0, stream>>>(
         reinterpret_cast<const __nv_bfloat16*>(z_all), labels_all, p->n_total,
         reinterpret_cast<const unsigned long long*>(ws + pl.off_hkeys), hids, pl.hash_size - 1, n_classes,

@@ -55,7 +55,6 @@ class _CudaKernels:
     # two-phase forward: own columns while the all-gather is in flight, then the rest
     forward_rows_local = staticmethod(Fn.forward_rows_local)
     forward_rows_remote = staticmethod(Fn.forward_rows_remote)
-    forward_rows_pass = staticmethod(Fn.forward_rows_pass)
     # two-phase backward: own columns while the statistics are exchanged, then the rest
     backward_rows_local = staticmethod(Fn.backward_rows_local)
     backward_rows_remote = staticmethod(Fn.backward_rows_remote)
@@ -63,8 +62,6 @@ class _CudaKernels:
 
 
 _COMM_STREAMS = {}
-import os as _os
-_EXPERIMENT = _os.environ.get("SUPCON_PEER_EXPERIMENT", "")    # "noz", "nostats": skip an exchange (timing breakdown)
 
 
 def _comm_stream(device) -> "torch.cuda.Stream":
@@ -118,59 +115,14 @@ class PeerExchange:
             torch.float64).view(self.world, _cabi.N_PARTIALS)
         # NVSwitch multicast mapping of the same buffers, when the fabric offers one: a single store per 16 bytes
         # reaches every rank (multimem.st), so a rank's egress is its block, not (world - 1) copies of it
-        mc = 0
-        if _os.environ.get("SUPCON_PEER_MULTICAST", "1") != "0":
-            try:
-                mc = int(getattr(self.handle, "multicast_ptr", 0) or 0)
-            except Exception:  # noqa: BLE001
-                mc = 0
+        try:
+            mc = int(getattr(self.handle, "multicast_ptr", 0) or 0)
+        except Exception:  # noqa: BLE001
+            mc = 0
         self.multicast = mc != 0
         self.desc = _cabi.Peer(rank=self.rank, world=self.world, peer_bases=self.peer_bases.data_ptr(),
                                off_flags=self.off_flags, epoch=self.epoch.data_ptr(), mc_base=mc)
         self.pending = False                      # a forward whose backward has not run yet
-        # Arrival order of the peers' blocks under the ordered push (everybody sends to rank+1 first): rank-1, rank-2,
-        # ...  The forward sweeps the own block, then the first ~3/7 of the peers, then the rest: while it works on a
-        # group the next one is still landing.
-        order = [(self.rank - k) % self.world for k in range(1, self.world)]
-        n_first = max(1, round(len(order) * 3 / 7)) if len(order) >= 3 else len(order)
-        groups = [order[:n_first], order[n_first:]] if len(order) > n_first else [order]
-        self.groups = [g_ for g_ in groups if g_]
-        self.passes = Fn.ForwardPasses([[self.rank]] + self.groups)
-        self.masks = [sum(1 << p_ for p_ in g_) for g_ in self.groups]
-
-    def pipelined_ok(self, prob, kernels) -> bool:
-        """Ordered push + multi-pass forward: tensor path, aligned equal blocks, no uniformity term (its norms and
-        coefficient need every row before the sweep), at least three ranks.  OFF unless SUPCON_PEER_EXPERIMENT=pipe:
-        measured on 8 B200s it is SLOWER than pushing to all peers at once (0.83-0.85 ms vs 0.78 ms per step,
-        profiles/r02_peer_exchange_breakdown.md): three forward launches and a push serialised by destination cost more
-        than the earlier start buys."""
-        from . import _cabi
-        return (self.world >= 3 and hasattr(kernels, "forward_rows_pass") and prob.z_dtype == _cabi.BF16
-                and prob.d == 256 and self.n_local % 128 == 0 and prob.lambda_uni == 0.0 and prob.tau >= 0.025
-                and (prob.similarity == _cabi.GEODESIC or (prob.flags & (_cabi.FLAG_UNIT_ROWS | _cabi.FLAG_FORCE_TENSOR)))
-                and not (prob.flags & _cabi.FLAG_FORCE_EXACT) and (prob.alpha == 0.0 or prob.topk <= 32)
-                and "pipe" in _EXPERIMENT.split(","))
-
-    def forward_pipelined(self, zc, labels_local, prob, kernels, want_grad: bool):
-        """rows to the peers in ring order | own columns -> first arrivals -> later arrivals -> statistics out."""
-        from . import _cabi
-        r, nl, dev = self.rank, self.n_local, self.device
-        cur, comm = torch.cuda.current_stream(dev), _comm_stream(dev)
-        zb, yb = self.z_all[r * nl:(r + 1) * nl], self.labels_all[r * nl:(r + 1) * nl]
-        zb.copy_(zc)
-        yb.copy_(labels_local)
-        comm.wait_stream(cur)
-        with torch.cuda.stream(comm):
-            Fn.peer_push_ordered(self.desc, zb, self.off_z + r * nl * self.row_bytes, yb, self.off_labels + r * nl * 4,
-                                 _cabi.PEER_FLAG_Z, wait_flag_id=_cabi.PEER_FLAG_DONE)
-        ws = kernels.forward_rows_pass(self.z_all, self.labels_all, prob, self.passes, 0)
-        out = None
-        for i, mask in enumerate(self.masks):
-            Fn.peer_wait(self.desc, _cabi.PEER_FLAG_Z, dev, rank_mask=mask)
-            out = kernels.forward_rows_pass(self.z_all, self.labels_all, prob, self.passes, i + 1, ws)
-        stats, partials = out
-        cur.wait_stream(comm)                      # the own push has long finished; joins the side stream
-        return stats, partials
 
     def forward(self, zc, labels_local, prob, kernels, want_grad: bool):
         """push rows | own-column forward -> wait -> other columns -> push statistics -> wait -> loss."""
@@ -179,34 +131,27 @@ class PeerExchange:
             raise RuntimeError("ShardedSupConLoss (peer exchange): forward() called again before the backward of the "
                                "previous call; the exchange buffers hold what that backward reads")
         r, nl, dev = self.rank, self.n_local, self.device
-        skip = _EXPERIMENT                         # timing experiments only (results are then stale): see tools/
-        if self.pipelined_ok(prob, kernels) and "noz" not in skip:
-            stats, partials = self.forward_pipelined(zc, labels_local, prob, kernels, want_grad)
-            return self._finish_forward(stats, partials, prob, kernels, want_grad, skip)
         cur, comm = torch.cuda.current_stream(dev), _comm_stream(dev)
         zb, yb = self.z_all[r * nl:(r + 1) * nl], self.labels_all[r * nl:(r + 1) * nl]
         zb.copy_(zc)                               # own block of the own buffer: only this rank's kernels read it
         yb.copy_(labels_local)
-        if "noz" not in skip:
-            comm.wait_stream(cur)
-            with torch.cuda.stream(comm):          # rows + labels to every peer, beside the own-column forward
-                Fn.peer_push(self.desc, zb, self.off_z + r * nl * self.row_bytes, yb, self.off_labels + r * nl * 4,
-                             _cabi.PEER_FLAG_Z, wait_flag_id=_cabi.PEER_FLAG_DONE, include_self=False)
+        comm.wait_stream(cur)
+        with torch.cuda.stream(comm):              # rows + labels to every peer, beside the own-column forward
+            Fn.peer_push(self.desc, zb, self.off_z + r * nl * self.row_bytes, yb, self.off_labels + r * nl * 4,
+                         _cabi.PEER_FLAG_Z, wait_flag_id=_cabi.PEER_FLAG_DONE, include_self=False)
         ws = kernels.forward_rows_local(self.z_all, self.labels_all, prob)
-        if "noz" not in skip:
-            cur.wait_stream(comm)
-            Fn.peer_wait(self.desc, _cabi.PEER_FLAG_Z, dev)
+        cur.wait_stream(comm)
+        Fn.peer_wait(self.desc, _cabi.PEER_FLAG_Z, dev)
         stats, partials = kernels.forward_rows_remote(self.z_all, self.labels_all, prob, ws)
-        return self._finish_forward(stats, partials, prob, kernels, want_grad, skip)
+        return self._finish_forward(stats, partials, prob, kernels, want_grad)
 
-    def _finish_forward(self, stats, partials, prob, kernels, want_grad, skip):
+    def _finish_forward(self, stats, partials, prob, kernels, want_grad):
         """statistics + partial sums to every rank, wait for everybody's, loss."""
         from . import _cabi
         r, nl, dev = self.rank, self.n_local, self.device
-        if "nostats" not in skip:
-            Fn.peer_push(self.desc, stats, self.off_stats + r * nl * 4 * _cabi.STATS_STRIDE, partials,
-                         self.off_partials + r * 8 * _cabi.N_PARTIALS, _cabi.PEER_FLAG_STATS, include_self=True)
-            Fn.peer_wait(self.desc, _cabi.PEER_FLAG_STATS, dev)
+        Fn.peer_push(self.desc, stats, self.off_stats + r * nl * 4 * _cabi.STATS_STRIDE, partials,
+                     self.off_partials + r * 8 * _cabi.N_PARTIALS, _cabi.PEER_FLAG_STATS, include_self=True)
+        Fn.peer_wait(self.desc, _cabi.PEER_FLAG_STATS, dev)
         partials_global, loss = kernels.finalize_sets(prob, self.partial_sets)
         if want_grad:
             self.pending = True

@@ -293,58 +293,11 @@ def peer_push(desc: _cabi.Peer, src0: torch.Tensor, dst_off0: int, src1, dst_off
                                          _stream(dev)), "supcon_peer_push")
 
 
-def peer_wait(desc: _cabi.Peer, flag_id: int, device, rank_mask=None):
-    """Block the stream until the flag of every rank (or of the ranks in rank_mask) carries the current step."""
+def peer_wait(desc: _cabi.Peer, flag_id: int, device):
+    """Block the stream until the flag of every rank carries the current step."""
     lib = _cabi.load()
-    mask = (1 << 64) - 1 if rank_mask is None else int(rank_mask)
     with _on(device):
-        _cabi.check(lib.supcon_peer_wait_mask(ctypes.byref(desc), int(flag_id), ctypes.c_uint64(mask), _stream(device)),
-                    "supcon_peer_wait_mask")
-
-
-def peer_push_ordered(desc: _cabi.Peer, src0: torch.Tensor, dst_off0: int, src1, dst_off1: int, flag_id: int,
-                      wait_flag_id: int = -1):
-    """supcon_peer_push_ordered: the ranges go to rank+1 first, then rank+2, ...; each destination's flag as soon as
-    its copy is complete."""
-    lib = _cabi.load()
-    dev = src0.device
-    with _on(dev):
-        _cabi.check(lib.supcon_peer_push_ordered(ctypes.byref(desc), _p(src0), src0.numel() * src0.element_size(),
-                                                 int(dst_off0), _p(src1),
-                                                 0 if src1 is None else src1.numel() * src1.element_size(),
-                                                 int(dst_off1), int(flag_id), int(wait_flag_id), _stream(dev)),
-                    "supcon_peer_push_ordered")
-
-
-class ForwardPasses:
-    """Host-side description of a multi-pass forward (supcon_forward_rows_pass): which rank blocks each pass sweeps."""
-
-    def __init__(self, passes):
-        self.passes = [list(map(int, p_)) for p_ in passes]
-        flat = [b for p_ in self.passes for b in p_]
-        self.blocks = (ctypes.c_int32 * len(flat))(*flat)
-        self.sizes = (ctypes.c_int32 * len(self.passes))(*[len(p_) for p_ in self.passes])
-        self.n = len(self.passes)
-
-
-def forward_rows_pass(z_all, labels_i32, prob: _cabi.Problem, passes: ForwardPasses, index: int, ws=None,
-                      skip_norms: bool = True):
-    """One pass of the multi-pass row-block forward.  Returns the workspace (passes before the last) or
-    (row_stats, partials) (last pass)."""
-    lib = _cabi.load()
-    dev = z_all.device
-    with _on(dev):
-        if ws is None:
-            ws = workspace_for(prob, dev)
-        last = index == passes.n - 1
-        stats = partials = None
-        if last:
-            stats, partials, _ = _stats_buffers(prob.n_rows, dev, False)
-        _cabi.check(lib.supcon_forward_rows_pass(ctypes.byref(prob), _p(z_all), _p(labels_i32), passes.blocks,
-                                                 passes.sizes, passes.n, int(index), 1 if skip_norms else 0,
-                                                 _p(stats), _p(partials), _p(ws), ws.numel(), _stream(dev)),
-                    "supcon_forward_rows_pass")
-    return (stats, partials) if last else ws
+        _cabi.check(lib.supcon_peer_wait(ctypes.byref(desc), int(flag_id), _stream(device)), "supcon_peer_wait")
 
 
 def peer_end_step(desc: _cabi.Peer, flag_id: int, device):
