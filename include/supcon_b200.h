@@ -67,6 +67,20 @@ extern "C" {
  * forward left there instead of rebuilding them (three launches, ~40 us at N = 65536).  Without the flag the
  * backward needs nothing from the forward but the row statistics and partial sums. */
 #define SUPCON_FLAG_WS_FROM_FORWARD 512u
+/* Cross-batch memory (XBM): rows [0, n_rows) of z_all are the batch and its anchors; columns [n_rows, n_total) are
+ * a memory of earlier batches' embeddings and labels.  Every anchor is contrasted against batch + memory (lse,
+ * positives, negatives and the mined top-K run over all n_total columns), but only the batch carries statistics:
+ *   - memory columns are constants: they get no gradient and no column-side term (H_ij = G_ij for j >= n_rows);
+ *   - |A_f| and |A_m| count anchors only, and SUPCON_P_GCNT_* equal SUPCON_P_CNT_*;
+ *   - the uniformity term stays over the batch's own pairs: log mean_{i<j<n_rows} exp(-t |z_i - z_j|^2), so its
+ *     pair count comes from n_rows in supcon_finalize and everywhere else;
+ *   - supcon_backward_rows reads stats_all as the anchors' [n_rows][STRIDE] statistics the forward wrote.
+ * Requires row_offset == 0 and, when lambda_uni > 0, uni_t > 0 (SUPCON_E_INVALID otherwise).  Single rank only: the
+ * two-phase _local / _remote calls treat the problem as not eligible, and supcon_finalize_sets with n_sets > 1
+ * returns SUPCON_E_UNSUPPORTED.  With n_rows == n_total the loss is the plain loss; the problem still takes the tiled
+ * kernels, never the single-launch small / mid ones, so that a separately issued forward and backward rank the hard
+ * negatives with the same Gram arithmetic. */
+#define SUPCON_FLAG_MEMORY_COLUMNS 1024u
 
 /* error codes */
 #define SUPCON_E_INVALID (-1)
@@ -125,8 +139,8 @@ int supcon_workspace_bytes(const supcon_problem_t* p, size_t* bytes_out);
  *   z_all      [n_total][d]   labels_all [n_total] int32
  *   row_stats  [n_rows][SUPCON_STATS_STRIDE]      (out)
  *   partials   [SUPCON_N_PARTIALS] doubles         (out; this rank's sums)
- *   loss_out   optional; only when the rank owns every row: the scalar loss
- *              (loss.py:137-153) is written by the same launch */
+ *   loss_out   optional; only when the rank owns every row (or with SUPCON_FLAG_MEMORY_COLUMNS, whose
+ *              anchors are every row): the scalar loss (loss.py:137-153) is written by the same launch */
 int supcon_forward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
                         float* row_stats, double* partials, float* loss_out, void* workspace,
                         size_t workspace_bytes, void* stream);
@@ -160,7 +174,8 @@ int supcon_finalize_sets(const supcon_problem_t* p, const double* partial_sets, 
 /* Backward for the owned rows (replaces autograd through loss.py:96-153):
  *   dz_i = grad_out * sum_j (G_ij + G_ji) z_j (+ uniformity), recomputing the
  *   similarity tiles; needs the statistics of ALL rows and the global partials.
- *   stats_all  [n_total][SUPCON_STATS_STRIDE]
+ *   stats_all  [n_total][SUPCON_STATS_STRIDE]  (SUPCON_FLAG_MEMORY_COLUMNS: [n_rows][SUPCON_STATS_STRIDE], the
+ *              anchors' statistics; memory columns have none)
  *   grad_out   device scalar (NULL = 1.0)
  *   dz_out     [n_rows][d] in dz_dtype */
 int supcon_backward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,

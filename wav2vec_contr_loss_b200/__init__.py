@@ -9,5 +9,6 @@ from .loss import (BCEBinaryLoss, SupConBinaryLoss, SupConMultiClassLoss,  # noq
                    compute_pos_weight_from_dataset)
 from .functional import l2_normalize, supcon_loss  # noqa: F401
 from .head import FusedCompressionHead, layer_time_pool  # noqa: F401
+from .memory import CrossBatchMemory, MemorySupConLoss  # noqa: F401
 
 __version__ = "0.1.0"

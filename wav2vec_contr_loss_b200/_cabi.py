@@ -19,6 +19,7 @@ FLAG_UNIT_ROWS = 32
 FLAG_PEER_EXCHANGE = 64
 FLAG_CLASS_SUMS, FLAG_NO_CLASS_SUMS = 128, 256
 FLAG_WS_FROM_FORWARD = 512
+FLAG_MEMORY_COLUMNS = 1024
 STATS_STRIDE = 8
 N_PARTIALS = 8
 P_SUM_FULL, P_CNT_FULL, P_SUM_MINED, P_CNT_MINED, P_SUM_W, P_GCNT_FULL, P_GCNT_MINED, P_FIXMAX = range(8)

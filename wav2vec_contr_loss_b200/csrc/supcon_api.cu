@@ -47,7 +47,19 @@ int validate(const supcon_problem_t* p) {
   if (p->similarity != SUPCON_COSINE && p->similarity != SUPCON_GEODESIC)
     return fail(SUPCON_E_INVALID, "Unknown similarity: %d", p->similarity);
   if (!(p->tau > 0.f)) return fail(SUPCON_E_INVALID, "tau must be > 0");
+  if (p->flags & SUPCON_FLAG_MEMORY_COLUMNS) {
+    if (p->row_offset != 0)
+      return fail(SUPCON_E_INVALID, "SUPCON_FLAG_MEMORY_COLUMNS needs row_offset == 0 (got %d)", p->row_offset);
+    // the tensor path masks memory columns out of the uniformity sums through exp(-t * inf) == 0
+    if (p->lambda_uni > 0.f && !(p->uni_t > 0.f))
+      return fail(SUPCON_E_INVALID, "SUPCON_FLAG_MEMORY_COLUMNS with lambda_uni > 0 needs uni_t > 0");
+  }
   return 0;
+}
+
+// the rank owns every anchor: a whole batch, or a batch contrasted against a memory of earlier batches
+bool owns_all_anchors(const supcon_problem_t* p) {
+  return p->row_offset == 0 && (p->n_rows == p->n_total || (p->flags & SUPCON_FLAG_MEMORY_COLUMNS));
 }
 
 constexpr uint32_t FLAG_TC_FWD_ONLY = SUPCON_FLAG_DEBUG_TC_FWD_ONLY, FLAG_TC_BWD_ONLY = SUPCON_FLAG_DEBUG_TC_BWD_ONLY;
@@ -76,13 +88,18 @@ bool vec_ok(const void* z, const supcon_problem_t* p) {
   return (p->d % 4 == 0) && ((reinterpret_cast<uintptr_t>(z) % al) == 0);
 }
 
+// A memory problem (SUPCON_FLAG_MEMORY_COLUMNS) never takes the single-launch kernels, not even with an empty memory
+// (n_rows == n_total): its forward and backward are separate calls, and the backward's hard-negative membership test
+// (s == thr) needs the forward's Gram arithmetic, which the small / mid kernels do not share with the tiled ones.
+constexpr uint32_t NOT_SINGLE_LAUNCH = SUPCON_FLAG_NO_SMALL | SUPCON_FLAG_FORCE_TENSOR | SUPCON_FLAG_MEMORY_COLUMNS;
+
 bool use_small(const supcon_problem_t* p, const void* z) {
-  if (p->flags & (SUPCON_FLAG_NO_SMALL | SUPCON_FLAG_FORCE_TENSOR)) return false;
+  if (p->flags & NOT_SINGLE_LAUNCH) return false;
   return small_supported(p, z);
 }
 // mid-size single-launch kernel: exact fp32 math, so it yields to the tensor path where that one is eligible
 bool use_mid(const supcon_problem_t* p, const void* z) {
-  if (p->flags & (SUPCON_FLAG_NO_SMALL | SUPCON_FLAG_FORCE_TENSOR)) return false;
+  if (p->flags & NOT_SINGLE_LAUNCH) return false;
   if (use_tc(p, false) || use_tc(p, true)) return false;
   return !small_supported(p, z) && mid_supported(p, z);
 }
@@ -105,6 +122,7 @@ FfmaArgs make_ffma(const supcon_problem_t* p, const void* z, const int32_t* labe
   a.splits = 1; a.col_tiles = (p->n_total + 63) / 64; a.rows_pad = (p->n_rows + 63) / 64 * 64;
   if (use_plan && ws) ffma_bind_plan(a, ffma_plan(p), ws, backward);
   a.n_total = p->n_total; a.row_offset = p->row_offset; a.n_rows = p->n_rows; a.d = p->d;
+  a.n_batch = batch_columns(p);
   a.z_dtype = p->z_dtype; a.similarity = p->similarity; a.topk = p->topk < 0 ? 0 : p->topk;
   a.mine = needs_mining(p) ? 1 : 0;
   int cap = ffma_kcap();
@@ -114,16 +132,16 @@ FfmaArgs make_ffma(const supcon_problem_t* p, const void* z, const int32_t* labe
   return a;
 }
 
-__global__ void finalize_kernel(const double* pg, float* loss_out, int n_total, float tau, float alpha,
+__global__ void finalize_kernel(const double* pg, float* loss_out, int n_batch, float tau, float alpha,
                                 float lambda_uni, float uni_t) {
   if (threadIdx.x == 0 && blockIdx.x == 0)
-    *loss_out = global_coef(pg, n_total, tau, alpha, lambda_uni, uni_t).loss;
+    *loss_out = global_coef(pg, n_batch, tau, alpha, lambda_uni, uni_t).loss;
 }
 
 // sums the per-rank partial sums in rank order (deterministic, identical on every rank) and writes the loss.
 // Slots SUPCON_P_GCNT_* / SUPCON_P_FIXMAX are global quantities every rank derived identically: copied, not summed.
 __global__ void finalize_sets_kernel(const double* sets, int n_sets, double* partials_out, float* loss_out,
-                                     int n_total, float tau, float alpha, float lambda_uni, float uni_t) {
+                                     int n_batch, float tau, float alpha, float lambda_uni, float uni_t) {
   __shared__ double pg[SUPCON_N_PARTIALS];
   const int k = threadIdx.x;
   if (k < SUPCON_N_PARTIALS) {
@@ -134,7 +152,7 @@ __global__ void finalize_sets_kernel(const double* sets, int n_sets, double* par
     partials_out[k] = s;
   }
   __syncthreads();
-  if (k == 0 && loss_out) *loss_out = global_coef(pg, n_total, tau, alpha, lambda_uni, uni_t).loss;
+  if (k == 0 && loss_out) *loss_out = global_coef(pg, n_batch, tau, alpha, lambda_uni, uni_t).loss;
 }
 
 // ---- labels of any width -> int32 class keys: equal labels <-> equal keys (loss.py:123 compares with ==) ----
@@ -228,7 +246,7 @@ int supcon_forward_rows(const supcon_problem_t* p, const void* z_all, const int3
     return fail(SUPCON_E_WORKSPACE, "workspace too small: %zu < %zu", workspace_bytes, workspace_need(p));
   if ((p->flags & SUPCON_FLAG_FORCE_TENSOR) && !tc_supported(p))
     return fail(SUPCON_E_UNSUPPORTED, "tensor-core path needs bf16 z, d == 256, tau >= 0.025, N >= 256, top-K <= 32");
-  if (loss_out && (p->row_offset != 0 || p->n_rows != p->n_total))
+  if (loss_out && !owns_all_anchors(p))
     return fail(SUPCON_E_INVALID, "loss_out needs a rank that owns every row; use supcon_finalize");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (use_small(p, z_all)) {   // whole batch on this rank, small N: one launch, statistics + loss only
@@ -297,7 +315,7 @@ int supcon_finalize(const supcon_problem_t* p, const double* partials_global, fl
   if (int rc = validate(p)) return rc;
   if (!partials_global || !loss_out) return fail(SUPCON_E_INVALID, "NULL buffer passed to supcon_finalize");
   finalize_kernel<<<1, 32, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      partials_global, loss_out, p->n_total, p->tau, p->alpha, p->lambda_uni, p->uni_t);
+      partials_global, loss_out, batch_columns(p), p->tau, p->alpha, p->lambda_uni, p->uni_t);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "finalize_kernel");
   return 0;
@@ -308,8 +326,10 @@ int supcon_finalize_sets(const supcon_problem_t* p, const double* partial_sets, 
   if (int rc = validate(p)) return rc;
   if (!partial_sets || !partials_out || n_sets < 1)
     return fail(SUPCON_E_INVALID, "bad arguments to supcon_finalize_sets");
+  if ((p->flags & SUPCON_FLAG_MEMORY_COLUMNS) && n_sets > 1)
+    return fail(SUPCON_E_UNSUPPORTED, "SUPCON_FLAG_MEMORY_COLUMNS is single-rank: n_sets must be 1 (got %d)", n_sets);
   finalize_sets_kernel<<<1, 32, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      partial_sets, n_sets, partials_out, loss_out, p->n_total, p->tau, p->alpha, p->lambda_uni, p->uni_t);
+      partial_sets, n_sets, partials_out, loss_out, batch_columns(p), p->tau, p->alpha, p->lambda_uni, p->uni_t);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "finalize_sets_kernel");
   return 0;
@@ -385,7 +405,7 @@ int supcon_loss_and_grad(const supcon_problem_t* p, const void* z, const int32_t
                          void* dz_out, int32_t dz_dtype, float* row_stats, double* partials,
                          void* workspace, size_t workspace_bytes, void* stream) {
   if (int rc = validate(p)) return rc;
-  if (p->row_offset != 0 || p->n_rows != p->n_total)
+  if (!owns_all_anchors(p))
     return fail(SUPCON_E_INVALID, "supcon_loss_and_grad needs the whole batch on one rank");
   if (!loss_out) return fail(SUPCON_E_INVALID, "loss_out is NULL");
   if (!z || !labels) return fail(SUPCON_E_INVALID, "NULL buffer passed to supcon_loss_and_grad");

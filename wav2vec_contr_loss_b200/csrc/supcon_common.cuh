@@ -50,7 +50,8 @@ struct GlobalCoef {
 
 // use_label_counts: take |A_f|, |A_m| from the label-derived GLOBAL counts (SUPCON_P_GCNT_*) that the tensor
 // path's forward leaves in a rank's own partials, so coefficients are known before any exchange.
-__device__ __forceinline__ GlobalCoef global_coef(const double* pg, int n_total, float tau, float alpha,
+// n_batch: rows of the uniformity term (batch_columns(): n_total, or n_rows with SUPCON_FLAG_MEMORY_COLUMNS).
+__device__ __forceinline__ GlobalCoef global_coef(const double* pg, int n_batch, float tau, float alpha,
                                                   float lambda_uni, float uni_t, bool use_label_counts = false) {
   GlobalCoef g;
   double cnt_f = pg[use_label_counts ? SUPCON_P_GCNT_FULL : SUPCON_P_CNT_FULL];
@@ -73,8 +74,8 @@ __device__ __forceinline__ GlobalCoef global_coef(const double* pg, int n_total,
   g.a_full = (cnt_f > 0.0) ? (float)(wf / (cnt_f * (double)tau)) : 0.0f;
   g.a_mined = (cnt_m > 0.0) ? (float)(wm / (cnt_m * (double)tau)) : 0.0f;
   g.cu = 0.0f;
-  if (lambda_uni > 0.0f && n_total > 1) {
-    double pairs2 = (double)n_total * (double)(n_total - 1);
+  if (lambda_uni > 0.0f && n_batch > 1) {
+    double pairs2 = (double)n_batch * (double)(n_batch - 1);
     double m = pg[SUPCON_P_SUM_W] / pairs2;
     main_loss += (double)lambda_uni * log(m + 1e-8);
     g.cu = (float)((double)lambda_uni * (-2.0 * (double)uni_t) / ((pairs2 * 0.5) * (m + 1e-8)));
@@ -91,7 +92,7 @@ struct FinishArgs {
   unsigned* ticket;        // zero before the launch
   double* partials;        // [SUPCON_N_PARTIALS] out
   float* loss_out;         // optional
-  int n_total;
+  int n_batch;             // rows of the uniformity term (global_coef)
   float tau, alpha, lambda_uni, uni_t;
 };
 
@@ -129,7 +130,7 @@ __device__ inline void block_partials_and_finish(const FinishArgs& a, const doub
   if (tid == 0) {
     *a.ticket = 0u;
     if (a.loss_out) {
-      GlobalCoef g = global_coef(a.partials, a.n_total, a.tau, a.alpha, a.lambda_uni, a.uni_t);
+      GlobalCoef g = global_coef(a.partials, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t);
       *a.loss_out = g.loss;
     }
   }

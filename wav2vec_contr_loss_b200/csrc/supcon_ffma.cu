@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
             st.sum_all += e;
             if (lab_c[c] == lab_r) { st.npos++; st.sum_pos_e += e; st.sum_pos_s += s; }
             else st.nneg++;
-            if (uni) st.wsum += Ws[pr * LDS_ + c];
+            if (uni && gj < a.n_batch) st.wsum += Ws[pr * LDS_ + c];   // memory columns: no uniformity
           }
         }
       }
@@ -320,7 +320,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
     red[3 * BM + pr] = c_mined; red[4 * BM + pr] = w;
   }
   __syncthreads();
-  FinishArgs fa{a.block_partials, a.ticket, a.partials, a.loss_out, a.n_total, a.tau, a.alpha, a.lambda_uni, a.uni_t};
+  FinishArgs fa{a.block_partials, a.ticket, a.partials, a.loss_out, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t};
   block_partials_and_finish(fa, red, BM);
 }
 
@@ -386,7 +386,7 @@ __global__ void __launch_bounds__(128) ffma_fwd_merge_kernel(FfmaArgs a) {
   red[0 * 128 + threadIdx.x] = l_full; red[1 * 128 + threadIdx.x] = c_full; red[2 * 128 + threadIdx.x] = l_mined;
   red[3 * 128 + threadIdx.x] = c_mined; red[4 * 128 + threadIdx.x] = w;
   __syncthreads();
-  FinishArgs fa{a.block_partials, a.ticket, a.partials, a.loss_out, a.n_total, a.tau, a.alpha, a.lambda_uni, a.uni_t};
+  FinishArgs fa{a.block_partials, a.ticket, a.partials, a.loss_out, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t};
   block_partials_and_finish(fa, red, 128);
 }
 
@@ -398,7 +398,7 @@ __global__ void __launch_bounds__(256) ffma_bwd_reduce_kernel(FfmaArgs a) {
   const int lr = (int)(idx / a.d), dd = (int)(idx % a.d);
   float v = 0.f;
   for (int s = 0; s < a.splits; ++s) v += a.dz_part[((int64_t)s * a.rows_pad + lr) * a.d + dd];
-  const GlobalCoef g = global_coef(a.partials, a.n_total, a.tau, a.alpha, a.lambda_uni, a.uni_t);
+  const GlobalCoef g = global_coef(a.partials, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t);
   const int gi = a.row_offset + lr;
   if (g.cu != 0.f)
     v = fmaf(g.cu * a.stats_all[(int64_t)gi * SUPCON_STATS_STRIDE + SUPCON_ST_WSUM],
@@ -417,6 +417,13 @@ __device__ __forceinline__ void load_coef(const FfmaArgs& a, const GlobalCoef& g
   // layout: f[0]=lse f[1]=rm f[2]=af f[3]=am f[4]=bp f[5]=thr ; n[0]=thr_idx n[1]=lab
   float lse = 0.f, rm = 0.f, af = 0.f, am = 0.f, bp = 0.f, thr = INFINITY;
   int ti = -1, lab = 0;
+  if (ok && gidx >= a.n_batch) {
+    // memory column (SUPCON_FLAG_MEMORY_COLUMNS): its label decides the row side's positives, but it has no
+    // statistics and no column-side term; lse = +inf makes its exp(s/tau - lse) exactly 0
+    lse = INFINITY;
+    lab = a.labels[gidx];
+    ok = false;
+  }
   if (ok) {
     const float* s = a.stats_all + (int64_t)gidx * SUPCON_STATS_STRIDE;
     const int* si = reinterpret_cast<const int*>(s);
@@ -458,7 +465,7 @@ __global__ void __launch_bounds__(NT) ffma_bwd_kernel(FfmaArgs a) {
   const int row_end = a.row_offset + a.n_rows;
   const int dc0 = blockIdx.y * DC;
   const bool geo = a.similarity == SUPCON_GEODESIC;
-  const GlobalCoef g = global_coef(a.partials, a.n_total, a.tau, a.alpha, a.lambda_uni, a.uni_t);
+  const GlobalCoef g = global_coef(a.partials, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t);
   const bool uni = g.cu != 0.f;
   const bool mining = g.a_mined != 0.f;
 
@@ -508,7 +515,7 @@ __global__ void __launch_bounds__(NT) ffma_bwd_kernel(FfmaArgs a) {
           }
           if (pos) h -= rf[4 * BM + r] + cf[4 * BN + c];
           if (geo) h *= geodesic_slope_exact(cv);
-          if (uni) {
+          if (uni && gj < a.n_batch) {   // memory columns: no uniformity
             float d2 = fmaxf(nrm_r[r] + nrm_c[c] - 2.f * cv, 0.f);
             h = fmaf(-g.cu, expf(-a.uni_t * d2), h);
           }

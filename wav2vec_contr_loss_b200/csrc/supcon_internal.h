@@ -8,6 +8,13 @@
 
 namespace supcon {
 
+// Columns [0, n_batch) are the batch: they carry row statistics, get column-side gradient terms and enter the
+// uniformity term (whose pair count is n_batch (n_batch - 1) / 2).  n_batch == n_total unless the problem has
+// SUPCON_FLAG_MEMORY_COLUMNS, whose columns [n_rows, n_total) are a memory of constants.
+inline int batch_columns(const supcon_problem_t* p) {
+  return (p->flags & SUPCON_FLAG_MEMORY_COLUMNS) ? p->n_rows : p->n_total;
+}
+
 struct FfmaArgs {
   const void* z;             // [n_total][d]
   const int32_t* labels;     // [n_total]
@@ -20,6 +27,7 @@ struct FfmaArgs {
   const float* grad_out;     // bwd: optional device scalar
   void* dz_out;              // bwd: [n_rows][d]
   int n_total, row_offset, n_rows, d;
+  int n_batch;               // batch_columns(): columns from n_batch on are memory (no statistics, no uniformity)
   int z_dtype, similarity, topk, kcap, mine, vec_ok;
   float tau, alpha, lambda_uni, uni_t;
   // column splits (ffma_plan): partial records / candidate lists / partial dz in the workspace
@@ -117,6 +125,7 @@ struct TcBwdPrepArgs {
   int32_t* cls_pad;
   float* scalars;
   int n_total, n_pad, topk;
+  int n_batch;               // batch_columns(): columns from n_batch on are memory (zero coefficients, no statistics)
   float tau, alpha, lambda_uni, uni_t;
 };
 struct TcBwdArgs {

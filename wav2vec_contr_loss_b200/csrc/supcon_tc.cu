@@ -152,12 +152,15 @@ __device__ __forceinline__ float fixmax_from_bits(unsigned bits, float m_limit) 
 
 // padded labels + squared norms of `count` columns of [j_lo, n_pad) minus the window [ex_lo, ex_lo + ex_len),
 // and their running maximum (one atomic per block).  One warp per column, grid-stride.
+// Memory columns [mem_lo, n) (SUPCON_FLAG_MEMORY_COLUMNS) feed the maximum but store nrm_pad = +inf: the sweeps'
+// uniformity weight ex2(-ut2 * max(n_i + n_j - 2 c, 0)) is then exactly 0 for them (ut2 > 0 is validated), so
+// they drop out of the uniformity sums without a test in the sweep kernels.
 __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* __restrict__ z,
                                                           const int32_t* __restrict__ labels, int n, int n_pad, int d,
                                                           int32_t* __restrict__ lab_pad, float* __restrict__ nrm_pad,
                                                           unsigned* __restrict__ nrm2_max, int count, int j_lo = 0,
                                                           int ex_lo = 0x7fffffff, int ex_len = 0,
-                                                          int track_max = 1) {
+                                                          int track_max = 1, int mem_lo = 0x7fffffff) {
   __shared__ float wmax[8];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   float mx = 0.f;
@@ -181,7 +184,7 @@ __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* _
     }
     if (lane == 0) {
       lab_pad[j] = j < n ? labels[j] : 0;
-      nrm_pad[j] = s;
+      nrm_pad[j] = (j >= mem_lo && j < n) ? INFINITY : s;
     }
     mx = fmaxf(mx, s);
   }
@@ -288,6 +291,8 @@ __global__ void __launch_bounds__(1024) tc_class_reduce_kernel(const float* __re
 // column coefficient vectors of H (SURVEY Appendix A with the fixed maximum 1/tau):
 //   e0_ij = exp((s_ij - 1)/tau);  H_ij = e0 (A_i + A_j) [+ mined terms] - pos_ij (B_i + B_j)
 //   A = a_f exp(1/tau - lse),  Am = a_m exp(1/tau - lse_m),  B = (a_f + a_m)/|pos|
+// Memory columns [n_batch, n_total) (SUPCON_FLAG_MEMORY_COLUMNS) are constants: A = Am = B = 0, thr = +inf, idx = -1
+// and no statistics are read; only their label is needed (positives of the rows).
 __global__ void tc_prep_bwd_kernel(TcBwdPrepArgs a) {
   int j = a.j_lo + blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= a.j_lo + a.j_cnt) return;
@@ -297,19 +302,21 @@ __global__ void tc_prep_bwd_kernel(TcBwdPrepArgs a) {
   const float Mp = (float)a.partials[SUPCON_P_FIXMAX];   // NaN = the forward poisoned the result: stays NaN
   const float M = (Mp >= 1.0f || Mp != Mp) ? Mp : 1.0f;
   if (j < a.n_total) {
-    const GlobalCoef g = global_coef(a.partials, a.n_total, a.tau, a.alpha, a.lambda_uni, a.uni_t,
+    const GlobalCoef g = global_coef(a.partials, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t,
                                      a.use_label_counts != 0);
-    const float* s = a.stats + (int64_t)(j - a.stats_row0) * SUPCON_STATS_STRIDE;
-    const int* si = reinterpret_cast<const int*>(s);
-    int npos = si[SUPCON_ST_NPOS], nneg = si[SUPCON_ST_NNEG];
-    bool in_f = npos > 0, in_m = in_f && nneg > 0 && a.topk >= 1;
-    float af = in_f ? g.a_full : 0.f, am = in_m ? g.a_mined : 0.f;
-    float m_tau = M / a.tau;
-    A = af * expf(m_tau - s[SUPCON_ST_LSE]);
-    Am = (am != 0.f) ? am * expf(m_tau - s[SUPCON_ST_LSE_M]) : 0.f;
-    B = in_f ? (af + am) / (float)npos : 0.f;
-    thr = s[SUPCON_ST_THR_VAL];
-    ti = si[SUPCON_ST_THR_IDX];
+    if (j < a.n_batch) {
+      const float* s = a.stats + (int64_t)(j - a.stats_row0) * SUPCON_STATS_STRIDE;
+      const int* si = reinterpret_cast<const int*>(s);
+      int npos = si[SUPCON_ST_NPOS], nneg = si[SUPCON_ST_NNEG];
+      bool in_f = npos > 0, in_m = in_f && nneg > 0 && a.topk >= 1;
+      float af = in_f ? g.a_full : 0.f, am = in_m ? g.a_mined : 0.f;
+      float m_tau = M / a.tau;
+      A = af * expf(m_tau - s[SUPCON_ST_LSE]);
+      Am = (am != 0.f) ? am * expf(m_tau - s[SUPCON_ST_LSE_M]) : 0.f;
+      B = in_f ? (af + am) / (float)npos : 0.f;
+      thr = s[SUPCON_ST_THR_VAL];
+      ti = si[SUPCON_ST_THR_IDX];
+    }
     lab = a.labels[j];
     if (j == a.j_lo) { a.scalars[0] = g.cu; a.scalars[1] = -(LOG2E / a.tau) * M; }
   }
@@ -746,7 +753,10 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid
 }
 
 // merge the column splits into row statistics + loss partial sums
-__global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishArgs f, float* __restrict__ row_stats) {
+// anchor_counts (SUPCON_FLAG_MEMORY_COLUMNS): SUPCON_P_GCNT_* count the anchors, as SUPCON_P_CNT_* do, instead of every
+// column of the label table (memory columns are not anchors)
+__global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishArgs f, float* __restrict__ row_stats,
+                                                           int anchor_counts) {
   __shared__ double red[7 * 128];
   __shared__ float mrg_v[TC_KCAP * 128];   // per-thread merge lists, entry-major (conflict-free)
   __shared__ int mrg_i[TC_KCAP * 128];
@@ -864,8 +874,9 @@ __global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishAr
   // |A_f|, |A_m| of the GLOBAL batch from the class-size table (it holds every column by now): a class of
   // size c contributes its c rows to A_f when c >= 2 and to A_m when also c < N (some negative exists).
   // Every rank derives the same two integers, so the backward's coefficients need no exchange.
-  double g_full = 0.0, g_mined = 0.0;
-  {
+  double g_full = c_full, g_mined = c_mined;
+  if (!anchor_counts) {
+    g_full = 0.0; g_mined = 0.0;
     const uint32_t hsize = a.hmask + 1u;
     const uint32_t per = (hsize + gridDim.x - 1) / gridDim.x;
     const uint32_t h_end = min(hsize, (blockIdx.x + 1u) * per);
@@ -1423,7 +1434,9 @@ TcPlan tc_plan(const supcon_problem_t* p) {
   pl.bwd_spp = sched_max_slots_panels(pl.bwd_sched);
   pl.bwd_slots = pl.bwd_sched.NP * pl.bwd_spp;
   // two-phase sweeps (multi-GPU overlap): phase 1 covers the rank's own columns, phase 2 the others
-  pl.two_phase = (p->n_rows < p->n_total) && (p->row_offset % 128 == 0) && (p->n_rows % 128 == 0);
+  // (not with SUPCON_FLAG_MEMORY_COLUMNS: the memory is single-rank, there is no exchange to overlap)
+  pl.two_phase = (p->n_rows < p->n_total) && (p->row_offset % 128 == 0) && (p->n_rows % 128 == 0) &&
+                 !(p->flags & SUPCON_FLAG_MEMORY_COLUMNS);
   pl.local_ct0 = p->row_offset / 128;
   pl.local_cts = p->n_rows / 128;
   pl.bwd_local_ct0 = p->row_offset / 64;
@@ -1630,7 +1643,8 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
                                                      p->n_total, pl.n_pad, p->d,
                                                      reinterpret_cast<int32_t*>(ws + pl.off_lab),
                                                      reinterpret_cast<float*>(ws + pl.off_nrm), nrm2_max, count, j_lo,
-                                                     ex_lo, ex_len, p->similarity == SUPCON_COSINE ? 1 : 0);
+                                                     ex_lo, ex_len, p->similarity == SUPCON_COSINE ? 1 : 0,
+                                                     batch_columns(p));
     }
     // class-size table over the (real) columns of this phase
     int jn_lo = j_lo, jn_ex_lo = ex_lo, jn_ex_len = ex_len, jn_count = p->n_total;
@@ -1677,8 +1691,9 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
     a.msched[0] = pl.fwd_sched; a.mslot[0] = 0;
   }
   FinishArgs f{reinterpret_cast<double*>(ws + pl.off_block_partials), reinterpret_cast<unsigned*>(ws), partials,
-               loss_out, p->n_total, p->tau, p->alpha, p->lambda_uni, p->uni_t};
-  tc_fwd_merge_kernel<<<pl.merge_blocks, 128, 0, stream>>>(a, f, row_stats);
+               loss_out, batch_columns(p), p->tau, p->alpha, p->lambda_uni, p->uni_t};
+  tc_fwd_merge_kernel<<<pl.merge_blocks, 128, 0, stream>>>(a, f, row_stats,
+                                                           (p->flags & SUPCON_FLAG_MEMORY_COLUMNS) ? 1 : 0);
   e = cudaGetLastError();
   if (e != cudaSuccess) { *err = cudaGetErrorString(e); return (int)e; }
   return 0;
@@ -1729,12 +1744,15 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
                                                    p->n_total, pl.n_pad, p->d,
                                                    reinterpret_cast<int32_t*>(ws + pl.off_lab),
                                                    reinterpret_cast<float*>(ws + pl.off_nrm),
-                                                   reinterpret_cast<unsigned*>(ws + pl.off_scalars) + 8, pl.n_pad);
+                                                   reinterpret_cast<unsigned*>(ws + pl.off_scalars) + 8, pl.n_pad,
+                                                   0, 0x7fffffff, 0, 1, batch_columns(p));
   }
-  // positives by linearity: single-phase cosine backward without mining, when the sweep is long enough
+  // positives by linearity: single-phase cosine backward without mining, when the sweep is long enough.  Not with
+  // SUPCON_FLAG_MEMORY_COLUMNS: -2 B_i (C[c] - z_i) assumes every same-class column j carries B_j = B_i, and a memory
+  // column carries B_j = 0 (the forward's class sums stay valid: they only need the positives' similarities)
   const bool mine_b = p->alpha != 0.f && p->topk >= 1;
   const bool plin = phase == 0 && p->similarity == SUPCON_COSINE && !mine_b &&
-                    !(p->flags & SUPCON_FLAG_NO_CLASS_SUMS) && plin_size_ok(p);
+                    !(p->flags & (SUPCON_FLAG_NO_CLASS_SUMS | SUPCON_FLAG_MEMORY_COLUMNS)) && plin_size_ok(p);
   int* n_classes = reinterpret_cast<int*>(ws) + WS_NCLASSES_WORD;
   int* hids = reinterpret_cast<int*>(ws + pl.off_hids);
   // the forward of the same problem left its label table and class sums in this very workspace (caller's promise)
@@ -1764,7 +1782,7 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
   pa.colThrIdx = reinterpret_cast<int32_t*>(ws + pl.off_colThrIdx);
   pa.lab_pad = reinterpret_cast<int32_t*>(ws + pl.off_lab);
   pa.scalars = reinterpret_cast<float*>(ws + pl.off_scalars);
-  pa.n_total = p->n_total; pa.n_pad = pl.n_pad; pa.topk = p->topk;
+  pa.n_total = p->n_total; pa.n_pad = pl.n_pad; pa.topk = p->topk; pa.n_batch = batch_columns(p);
   pa.tau = p->tau; pa.alpha = p->alpha; pa.lambda_uni = p->lambda_uni; pa.uni_t = p->uni_t;
   pa.hkeys = plin ? reinterpret_cast<const unsigned long long*>(ws + pl.off_hkeys) : nullptr;
   pa.hids = hids; pa.hmask = pl.hash_size - 1;
