@@ -22,6 +22,8 @@ def load():
         lib.supcon_debug_tc_tile.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p]
         lib.supcon_debug_plan.restype = c_int32
         lib.supcon_debug_plan.argtypes = [P, c_void_p, c_int32]
+        lib.supcon_debug_ffma_plan.restype = c_int32
+        lib.supcon_debug_ffma_plan.argtypes = [P, c_void_p, c_int32]
         lib.supcon_debug_sched.restype = c_int32
         lib.supcon_debug_sched.argtypes = [c_int32, c_int32, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                            c_void_p]

@@ -30,9 +30,11 @@ def test_library_exports_every_declared_symbol(lib_built):
     assert _cabi.load().supcon_abi_version() == _cabi.ABI_VERSION == 3
     # diagnostics live in the test-only library, not in the product or its public header
     assert not any("debug" in n for n in names)
-    assert not hasattr(lib, "supcon_debug_plan") and not hasattr(lib, "supcon_debug_tc_tile")
+    for name in ("supcon_debug_plan", "supcon_debug_tc_tile", "supcon_debug_ffma_plan"):
+        assert not hasattr(lib, name)
     import debug_lib
-    assert hasattr(debug_lib.load(), "supcon_debug_plan") and hasattr(debug_lib.load(), "supcon_forward_rows")
+    for name in ("supcon_debug_plan", "supcon_debug_ffma_plan", "supcon_forward_rows"):
+        assert hasattr(debug_lib.load(), name)
 
 
 def test_flag_constants_match_the_header():

@@ -50,10 +50,15 @@ def _index_sets(member, k):
     return out
 
 
-@pytest.mark.parametrize("m", [0, 1000, 4096])
+# K > 32 runs only on the exact path: 64 keeps one top-K list per column split and merges them (M >= 1000), 129
+# takes two selection rounds over one sweep
+EXACT_PATH_MEMORY, EXACT_PATH_TOPK = [0, 1000, 4096], [15, 32, 64, 129]
+
+
+@pytest.mark.parametrize("m", EXACT_PATH_MEMORY)
 @pytest.mark.parametrize("sim", ["cosine", "geodesic"])
 @pytest.mark.parametrize("lam", [0.0, 0.2])
-@pytest.mark.parametrize("k", [15, 32])
+@pytest.mark.parametrize("k", EXACT_PATH_TOPK)
 @pytest.mark.parametrize("alpha", [0.0, 0.5, 1.0])
 def test_exact_path_fp32(cuda_device, m, sim, lam, k, alpha):
     zb, yb, zm, ym = _inputs(64, m, seed=m + k)

@@ -25,6 +25,9 @@ int supcon_debug_tc_tile(const void* z_bf16, int32_t n, int32_t d, int32_t row_i
  *   supcon_debug_sched the contiguous unit range of one CTA and the first/last CTA touching a row block for a
  *                      flattened (row block, column tile) list of `units` = row_blocks * col_tiles entries */
 int supcon_debug_plan(const supcon_problem_t* p, int32_t* out, int32_t n_out);
+/* Host-only plan of the exact fp32 path (no device work): out[0..3] = {forward column splits, backward column
+ * splits, top-K list capacity per row, selection rounds}; rounds = ceil(K / capacity) when mining, else 0. */
+int supcon_debug_ffma_plan(const supcon_problem_t* p, int32_t* out, int32_t n_out);
 int supcon_debug_sched(int32_t col_tiles, int32_t ctas, int64_t units, int32_t cta, int32_t row_block,
                        int64_t* range_begin, int64_t* range_end, int32_t* first_cta, int32_t* last_cta);
 

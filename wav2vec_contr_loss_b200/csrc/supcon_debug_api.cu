@@ -1,5 +1,6 @@
 // TEST-ONLY entry points (libsupcon_b200_test.so; declared in csrc/supcon_debug.h, not in the public header):
-// the tcgen05/TMA building-block diagnostic and host-side introspection of the tensor path's work distribution.
+// the tcgen05/TMA building-block diagnostic, host-side introspection of the tensor path's work distribution and
+// of the exact path's column splits and top-K selection rounds.
 // The product library libsupcon_b200.so does not contain this file.
 #include <string>
 
@@ -40,6 +41,18 @@ int supcon_debug_plan(const supcon_problem_t* p, int32_t* out, int32_t n_out) {
   if (!out || n_out < 1) return dbg_fail(SUPCON_E_INVALID, "bad arguments to supcon_debug_plan");
   if (!tc_supported(p)) return dbg_fail(SUPCON_E_UNSUPPORTED, "problem does not take the tensor path");
   return tc_debug_plan(p, out, n_out);
+}
+
+int supcon_debug_ffma_plan(const supcon_problem_t* p, int32_t* out, int32_t n_out) {
+  if (int rc = dbg_validate(p)) return rc;
+  if (!out || n_out < 4) return dbg_fail(SUPCON_E_INVALID, "bad arguments to supcon_debug_ffma_plan");
+  const FfmaPlan pl = ffma_plan(p);
+  const bool mine = p->alpha != 0.f && p->topk >= 1;
+  out[0] = pl.fwd_splits;
+  out[1] = pl.bwd_splits;
+  out[2] = pl.kcap;
+  out[3] = mine ? (p->topk + pl.kcap - 1) / pl.kcap : 0;
+  return 0;
 }
 
 int supcon_debug_sched(int32_t col_tiles, int32_t ctas, int64_t units, int32_t cta, int32_t row_block,
