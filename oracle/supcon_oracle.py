@@ -157,9 +157,11 @@ def rowblock_forward(z_all, labels_all, row_offset, n_rows, *, tau, similarity, 
     per-anchor full losses, |A_f|, sum of mined losses, |A_m|, sum_{i,j!=i} w_ij).
     ``thr_val/thr_idx`` is the lowest-ranked selected hard negative under the
     (value desc, index asc) order; (-inf, INT_MAX) when every negative is selected.
+    Everything is computed on ``z_all``'s device (``labels_all`` must live there too), so
+    large batches can be evaluated in fp64 on a GPU; ``rowblock_backward`` likewise.
     """
     n = z_all.size(0)
-    dt = z_all.dtype
+    dt, dev = z_all.dtype, z_all.device
     lab = labels_all.view(-1)
     INT_MAX = 2**31 - 1
     out = {k: [] for k in ("lse", "lse_m", "npos", "nneg", "thr_val", "thr_idx", "wsum", "pos_mean")}
@@ -167,12 +169,12 @@ def rowblock_forward(z_all, labels_all, row_offset, n_rows, *, tau, similarity, 
     nrm_all = (z_all * z_all).sum(1)
     for r0 in range(row_offset, row_offset + n_rows, block):
         r1 = min(r0 + block, row_offset + n_rows)
-        rows = torch.arange(r0, r1)
+        rows = torch.arange(r0, r1, device=dev)
         c = z_all[r0:r1] @ z_all.t()
         s, _ = _sim_and_slope(c, similarity)
         lg = s / tau
         self_m = torch.zeros_like(lg, dtype=torch.bool)
-        self_m[torch.arange(r1 - r0), rows] = True
+        self_m[torch.arange(r1 - r0, device=dev), rows] = True
         pos = (lab[r0:r1].view(-1, 1) == lab.view(1, -1)) & ~self_m
         neg = ~pos & ~self_m
         lgm = lg.masked_fill(self_m, float("-inf"))
@@ -184,7 +186,7 @@ def rowblock_forward(z_all, labels_all, row_offset, n_rows, *, tau, similarity, 
         negval = s.masked_fill(~neg, float("-inf"))
         order = torch.sort(negval, dim=1, descending=True, stable=True).indices
         k_i = nneg.clamp_max(max(int(topk), 0))
-        rank = torch.arange(n).view(1, -1)
+        rank = torch.arange(n, device=dev).view(1, -1)
         sel_sorted = rank < k_i.view(-1, 1)
         member = torch.zeros_like(neg)
         member.scatter_(1, order, sel_sorted)
@@ -201,7 +203,7 @@ def rowblock_forward(z_all, labels_all, row_offset, n_rows, *, tau, similarity, 
             w = torch.exp(-uni_t * d2).masked_fill(self_m, 0.0)
             wsum = w.sum(1)
         else:
-            wsum = torch.zeros(r1 - r0, dtype=dt)
+            wsum = torch.zeros(r1 - r0, dtype=dt, device=dev)
         for k, v in (("lse", lse), ("lse_m", lse_m), ("npos", npos), ("nneg", nneg),
                      ("thr_val", thr_val), ("thr_idx", thr_idx), ("wsum", wsum), ("pos_mean", pos_mean)):
             out[k].append(v)
@@ -213,7 +215,7 @@ def rowblock_forward(z_all, labels_all, row_offset, n_rows, *, tau, similarity, 
     in_m = in_f & (stats["nneg"] > 0) & (int(topk) >= 1)
     l_full = stats["lse"] - stats["pos_mean"]
     l_mined = stats["lse_m"] - stats["pos_mean"]
-    partials = torch.zeros(N_PARTIALS, dtype=torch.float64)
+    partials = torch.zeros(N_PARTIALS, dtype=torch.float64, device=dev)
     partials[P_SUM_FULL] = l_full[in_f].double().sum()
     partials[P_CNT_FULL] = in_f.sum()
     partials[P_SUM_MINED] = l_mined[in_m].double().sum()
@@ -255,7 +257,7 @@ def rowblock_backward(z_all, labels_all, row_offset, n_rows, stats_all, coef, *,
     """dz for the owned rows using only column *stats* of the other rows:
     dz_i = sum_j (G_ij + G_ji) z_j (+ uniformity), Appendix A with H = G + G^T."""
     n = z_all.size(0)
-    dt = z_all.dtype
+    dt, dev = z_all.dtype, z_all.device
     lab = labels_all.view(-1)
     npos_all = stats_all["npos"].to(dt)
     in_f = stats_all["npos"] > 0
@@ -264,17 +266,17 @@ def rowblock_backward(z_all, labels_all, row_offset, n_rows, stats_all, coef, *,
     a_m = in_m.to(dt) * (coef["w_mined"] / max(coef["cnt_m"], 1.0) / tau)
     inv_p = torch.where(in_f, 1.0 / npos_all.clamp_min(1), torch.zeros_like(npos_all))
     nrm_all = (z_all * z_all).sum(1)
-    idx_all = torch.arange(n)
-    dz = torch.zeros(n_rows, z_all.size(1), dtype=dt)
+    idx_all = torch.arange(n, device=dev)
+    dz = torch.zeros(n_rows, z_all.size(1), dtype=dt, device=dev)
     for r0 in range(row_offset, row_offset + n_rows, block):
         r1 = min(r0 + block, row_offset + n_rows)
         R = slice(r0, r1)
-        rows = torch.arange(r0, r1)
+        rows = torch.arange(r0, r1, device=dev)
         c = z_all[R] @ z_all.t()
         s, slope = _sim_and_slope(c, similarity)
         lg = s / tau
         self_m = torch.zeros_like(lg, dtype=torch.bool)
-        self_m[torch.arange(r1 - r0), rows] = True
+        self_m[torch.arange(r1 - r0, device=dev), rows] = True
         pos = (lab[R].view(-1, 1) == lab.view(1, -1)) & ~self_m
         neg = ~pos & ~self_m
         # row-side membership: j in top_i ; column-side: i in top_j
