@@ -265,9 +265,22 @@ int supcon_normalize_backward(const void* z, int32_t z_dtype, const float* norms
  * (compression_module.py:48-65 + the seq.mean(dim=-1) of stage1_utils.py:122-123).  Because the Linear layer and the
  * time mean commute, mean_t Linear(x_t) = Linear(mean_t x_t), and what is left of the head is one pass over hs:
  *   pooled[b][f] = (1/T) sum_t LeakyReLU(Dropout((1/K) sum_k hs[b][k][f][t]))
- * hs is (batch, layers, feat, frames) fp32 contiguous.  rng_state = device {seed, offset} (two 64-bit words) of the
+ * hs is (batch, layers, feat, frames) contiguous.  rng_state = device {seed, offset} (two 64-bit words) of the
  * counter-based dropout mask, or NULL / dropout_p == 0 for eval mode; the backward must be given the same values.
- * supcon_head_pool_backward writes d loss / d hs (same shape as hs) and is only needed when the encoder trains. */
+ * supcon_head_pool_backward writes d loss / d hs (same shape as hs) and is only needed when the encoder trains.
+ * pooled_out and dpooled are fp32.
+ *
+ * hs_dtype (the _typed entry points) is the element type of hs and of dhs_out: SUPCON_F32, or SUPCON_BF16 for the
+ * output of an encoder run in bf16, read as it is (no fp32 copy).  bf16 elements are widened to fp32 exactly and the
+ * arithmetic after the load is the fp32 one, so pooled_out equals bit for bit that of the fp32 call on the widened
+ * hs, and dhs_out is that call's fp32 dhs rounded to nearest even.  Any other hs_dtype returns SUPCON_E_INVALID.
+ * supcon_head_pool_forward / _backward are the SUPCON_F32 case. */
+int supcon_head_pool_forward_typed(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                                   int32_t frames, float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                   float* pooled_out /*[batch][feat]*/, void* stream);
+int supcon_head_pool_backward_typed(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                                    int32_t frames, float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                    const float* dpooled /*[batch][feat]*/, void* dhs_out, void* stream);
 int supcon_head_pool_forward(const float* hs, int32_t batch, int32_t layers, int32_t feat, int32_t frames,
                              float dropout_p, float negative_slope, const uint64_t* rng_state,
                              float* pooled_out /*[batch][feat]*/, void* stream);

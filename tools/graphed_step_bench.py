@@ -1,16 +1,21 @@
 """Head step of BASELINE configs[4] (frozen encoder): eager launches vs one CUDA-graph replay.
 
-    python tools/graphed_step_bench.py [--batch 64] [--iters 30] > gpurun_out/graphed_step.json
+    python tools/graphed_step_bench.py [--batch 64] [--iters 30] [--head fused] [--hs-dtype bfloat16]
 
-hs is the encoder output the reference hands the head: (B, 25, 1024, 199) fp32 (1.3 GB at B = 64), synthetic.
+hs is the encoder output the reference hands the head: (B, 25, 1024, 199) fp32 (1.3 GB at B = 64), synthetic; with
+--hs-dtype bfloat16 it is the output of an encoder run in bf16 (0.65 GB), which the fused head reads as it is.
 The head has the shape/ops of the reference's compression head (compression_module.py:35-67): layer mean,
 Dropout(0.1), LeakyReLU, Linear(1024 -> 256) per frame.  Step = stage1_utils.py:121-130 without the encoder.
-Times are CUDA events on the launching stream, median of --iters steps after warm-up.
+Times are CUDA events on the launching stream, median of --iters steps after warm-up; hs is far larger than the L2,
+so every pass reads it from HBM.  Rates are over algorithmic bytes: hs read once by the forward; hs read once and d hs
+(K copies of the (B, F, T) gradient) written once by the backward.  The card's name and power limit are read in the
+same run and printed with the times.
 """
 import argparse
 import json
 import os
 import statistics
+import subprocess
 import sys
 
 import torch
@@ -42,6 +47,18 @@ def median_ms(fn, iters):
     return statistics.median(s.elapsed_time(e) for s, e in ev)
 
 
+def card():
+    """name and power limit of device 0 (the limit is part of any time measured on it)"""
+    out = {"name": torch.cuda.get_device_name(0)}
+    try:
+        r = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30)
+        out["power_limit_and_max_sm_clock"] = r.stdout.strip() or r.stderr.strip()
+    except (OSError, subprocess.SubprocessError) as e:
+        out["power_limit_and_max_sm_clock"] = f"not read: {e}"
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", type=int, default=64)
@@ -49,7 +66,11 @@ def main():
     ap.add_argument("--frames", type=int, default=199)
     ap.add_argument("--head", choices=("torch", "fused"), default="torch",
                     help="torch: the reference's op chain; fused: FusedCompressionHead (csrc/supcon_head.cu)")
+    ap.add_argument("--hs-dtype", choices=("float32", "bfloat16"), default="float32",
+                    help="element type of the encoder output hs (bfloat16 needs --head fused)")
     args = ap.parse_args()
+    if args.hs_dtype == "bfloat16" and args.head != "fused":
+        ap.error("--hs-dtype bfloat16 needs --head fused (the torch op chain's Linear layer is fp32)")
     from wav2vec_contr_loss_b200 import build
     build.build()
     from wav2vec_contr_loss_b200 import FusedCompressionHead, SupConBinaryLoss, layer_time_pool
@@ -58,19 +79,36 @@ def main():
     dev = torch.device("cuda", 0)
     torch.manual_seed(1337)
     B = args.batch
-    hs = torch.randn(B, 25, 1024, args.frames, device=dev)
+    hs = torch.randn(B, 25, 1024, args.frames, device=dev, dtype=getattr(torch, args.hs_dtype))
     y = (torch.arange(B, device=dev) % 2).long()
     loss_fn = SupConBinaryLoss(temperature=0.07, similarity="cosine", uniformity_weight=0.0)
-    out = {"batch": B, "hs_shape": list(hs.shape), "hs_GB": hs.numel() * 4 / 1e9, "iters": args.iters,
-           "head": args.head}
+    hs_bytes = hs.numel() * hs.element_size()
+    out = {"batch": B, "hs_shape": list(hs.shape), "hs_dtype": args.hs_dtype, "hs_GB": hs_bytes / 1e9,
+           "iters": args.iters, "head": args.head, "card": card()}
     if args.head == "fused":
         rng = torch.tensor([1337, 0], dtype=torch.int64, device=dev)
         with torch.no_grad():
             t_eval = median_ms(lambda: layer_time_pool(hs, 0.0, 0.01, None), args.iters)
             t_drop = median_ms(lambda: layer_time_pool(hs, 0.1, 0.01, rng), args.iters)
-        out["head_pool_kernel"] = {"eval_ms": t_eval, "dropout_ms": t_drop,
-                                   "eval_GBps": hs.numel() * 4 / 1e6 / t_eval,
-                                   "dropout_GBps": hs.numel() * 4 / 1e6 / t_drop}
+        kern = {"eval_ms": t_eval, "dropout_ms": t_drop,
+                "eval_GBps": hs_bytes / 1e6 / t_eval, "dropout_GBps": hs_bytes / 1e6 / t_drop}
+        # the backward (encoder fine-tuned), dropout on: d hs in hs's dtype
+        x = hs.detach().requires_grad_(True)
+        pooled = layer_time_pool(x, 0.1, 0.01, rng)
+        up = torch.randn_like(pooled)
+        t_bwd = median_ms(lambda: torch.autograd.grad(pooled, x, up, retain_graph=True), args.iters)
+        kern.update(backward_ms=t_bwd, backward_GBps=2 * hs_bytes / 1e6 / t_bwd)
+        if hs.dtype != torch.float32:
+            # the route without a kernel for hs's dtype: an fp32 copy of hs, the fp32 kernel, and in the backward the
+            # fp32 d hs converted back to hs's dtype
+            with torch.no_grad():
+                t_up = median_ms(lambda: layer_time_pool(hs.float(), 0.0, 0.01, None), args.iters)
+            pooled_up = layer_time_pool(x.float(), 0.1, 0.01, rng)
+            t_up_bwd = median_ms(lambda: torch.autograd.grad(pooled_up, x, up, retain_graph=True), args.iters)
+            del pooled_up
+            kern.update(upcast_route_eval_ms=t_up, upcast_route_backward_ms=t_up_bwd)
+        del x, pooled
+        out["head_pool_kernel"] = kern
 
     for alpha in (0.0, 0.5):
         head = (FusedCompressionHead() if args.head == "fused" else LayerMeanHead()).to(dev).train()
@@ -102,7 +140,7 @@ def main():
         out[f"alpha_{alpha}"] = {"eager_step_ms": t_eager, "graphed_step_ms": t_graph,
                                  "graphed_step_with_input_copy_ms": t_graph_copy,
                                  "loss_fwd_bwd_eager_ms": t_loss, "layer_mean_only_ms": t_mean,
-                                 "layer_mean_GBps": hs.numel() * 4 / 1e6 / t_mean}
+                                 "layer_mean_GBps": hs_bytes / 1e6 / t_mean}
     print(json.dumps(out))
 
 

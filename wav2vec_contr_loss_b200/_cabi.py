@@ -33,6 +33,7 @@ EXPORTS = (
     "supcon_forward_rows_remote", "supcon_head_pool_forward", "supcon_head_pool_backward",
     "supcon_finalize_sets", "supcon_backward_rows_local", "supcon_backward_rows_remote",
     "supcon_peer_push", "supcon_peer_wait", "supcon_peer_end_step", "supcon_label_keys",
+    "supcon_head_pool_forward_typed", "supcon_head_pool_backward_typed",
 )
 
 
@@ -117,6 +118,12 @@ def load():
     lib.supcon_head_pool_backward.restype = c_int32
     lib.supcon_head_pool_backward.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_float, c_float,
                                               c_void_p, c_void_p, c_void_p, c_void_p]
+    lib.supcon_head_pool_forward_typed.restype = c_int32
+    lib.supcon_head_pool_forward_typed.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_float,
+                                                   c_float, c_void_p, c_void_p, c_void_p]
+    lib.supcon_head_pool_backward_typed.restype = c_int32
+    lib.supcon_head_pool_backward_typed.argtypes = [c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_float,
+                                                    c_float, c_void_p, c_void_p, c_void_p, c_void_p]
     lib.supcon_label_keys.restype = c_int32
     lib.supcon_label_keys.argtypes = [c_void_p, c_int32, c_int32, c_void_p, c_void_p]
     PP = POINTER(Peer)

@@ -483,25 +483,27 @@ int supcon_normalize_backward(const void* z, int32_t z_dtype, const float* norms
   return 0;
 }
 
-static int head_pool_check(const float* hs, int32_t batch, int32_t layers, int32_t feat, int32_t frames,
-                           float dropout_p, const void* out, const char* who) {
+static int head_pool_check(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                           int32_t frames, float dropout_p, const void* out, const char* who) {
   if (!hs || !out) return fail(SUPCON_E_INVALID, "NULL buffer passed to %s", who);
+  if (hs_dtype != SUPCON_F32 && hs_dtype != SUPCON_BF16)
+    return fail(SUPCON_E_INVALID, "%s: unknown hs_dtype %d (SUPCON_F32 or SUPCON_BF16)", who, hs_dtype);
   if (batch < 1 || layers < 1 || feat < 1 || frames < 1)
     return fail(SUPCON_E_INVALID, "%s: bad shape (%d, %d, %d, %d)", who, batch, layers, feat, frames);
   if (batch > 65535) return fail(SUPCON_E_UNSUPPORTED, "%s: batch %d > 65535", who, batch);
   if (!(dropout_p >= 0.f && dropout_p < 1.f)) return fail(SUPCON_E_INVALID, "%s: dropout_p must be in [0, 1)", who);
-  if (head_pool_rows_per_block(feat, frames) < 1)
+  if (head_pool_rows_per_block(feat, frames, hs_dtype) < 1)
     return fail(SUPCON_E_UNSUPPORTED, "%s: %d frames exceed the 12288 a block can stage", who, frames);
   return 0;
 }
 
-int supcon_head_pool_forward(const float* hs, int32_t batch, int32_t layers, int32_t feat, int32_t frames,
-                             float dropout_p, float negative_slope, const uint64_t* rng_state, float* pooled_out,
-                             void* stream) {
-  if (int rc = head_pool_check(hs, batch, layers, feat, frames, dropout_p, pooled_out, "supcon_head_pool_forward"))
-    return rc;
+static int head_pool_fwd(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                         int32_t frames, float dropout_p, float negative_slope, const uint64_t* rng_state,
+                         float* pooled_out, void* stream, const char* who) {
+  if (int rc = head_pool_check(hs, hs_dtype, batch, layers, feat, frames, dropout_p, pooled_out, who)) return rc;
   HeadPoolArgs a{};
-  a.hs = hs; a.pooled = pooled_out; a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
+  a.hs = hs; a.hs_dtype = hs_dtype; a.pooled = pooled_out;
+  a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
   a.B = batch; a.K = layers; a.F = feat; a.T = frames;
   a.dropout_p = dropout_p; a.negative_slope = negative_slope;
   cudaError_t e = head_pool_forward(a, reinterpret_cast<cudaStream_t>(stream));
@@ -509,19 +511,47 @@ int supcon_head_pool_forward(const float* hs, int32_t batch, int32_t layers, int
   return 0;
 }
 
-int supcon_head_pool_backward(const float* hs, int32_t batch, int32_t layers, int32_t feat, int32_t frames,
-                              float dropout_p, float negative_slope, const uint64_t* rng_state,
-                              const float* dpooled, float* dhs_out, void* stream) {
-  if (int rc = head_pool_check(hs, batch, layers, feat, frames, dropout_p, dhs_out, "supcon_head_pool_backward"))
-    return rc;
-  if (!dpooled) return fail(SUPCON_E_INVALID, "NULL dpooled passed to supcon_head_pool_backward");
+static int head_pool_bwd(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                         int32_t frames, float dropout_p, float negative_slope, const uint64_t* rng_state,
+                         const float* dpooled, void* dhs_out, void* stream, const char* who) {
+  if (int rc = head_pool_check(hs, hs_dtype, batch, layers, feat, frames, dropout_p, dhs_out, who)) return rc;
+  if (!dpooled) return fail(SUPCON_E_INVALID, "NULL dpooled passed to %s", who);
   HeadPoolArgs a{};
-  a.hs = hs; a.pooled = nullptr; a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
+  a.hs = hs; a.hs_dtype = hs_dtype; a.pooled = nullptr;
+  a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
   a.B = batch; a.K = layers; a.F = feat; a.T = frames;
   a.dropout_p = dropout_p; a.negative_slope = negative_slope;
   cudaError_t e = head_pool_backward(a, dpooled, dhs_out, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "head_pool_bwd_kernel");
   return 0;
+}
+
+int supcon_head_pool_forward_typed(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                                   int32_t frames, float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                   float* pooled_out, void* stream) {
+  return head_pool_fwd(hs, hs_dtype, batch, layers, feat, frames, dropout_p, negative_slope, rng_state, pooled_out,
+                       stream, "supcon_head_pool_forward_typed");
+}
+
+int supcon_head_pool_backward_typed(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                                    int32_t frames, float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                    const float* dpooled, void* dhs_out, void* stream) {
+  return head_pool_bwd(hs, hs_dtype, batch, layers, feat, frames, dropout_p, negative_slope, rng_state, dpooled,
+                       dhs_out, stream, "supcon_head_pool_backward_typed");
+}
+
+int supcon_head_pool_forward(const float* hs, int32_t batch, int32_t layers, int32_t feat, int32_t frames,
+                             float dropout_p, float negative_slope, const uint64_t* rng_state, float* pooled_out,
+                             void* stream) {
+  return head_pool_fwd(hs, SUPCON_F32, batch, layers, feat, frames, dropout_p, negative_slope, rng_state, pooled_out,
+                       stream, "supcon_head_pool_forward");
+}
+
+int supcon_head_pool_backward(const float* hs, int32_t batch, int32_t layers, int32_t feat, int32_t frames,
+                              float dropout_p, float negative_slope, const uint64_t* rng_state,
+                              const float* dpooled, float* dhs_out, void* stream) {
+  return head_pool_bwd(hs, SUPCON_F32, batch, layers, feat, frames, dropout_p, negative_slope, rng_state, dpooled,
+                       dhs_out, stream, "supcon_head_pool_backward");
 }
 
 int supcon_peer_push(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0, const void* src1,

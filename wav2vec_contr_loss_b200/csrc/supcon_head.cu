@@ -8,17 +8,23 @@
 // GEMM over (B*T, F) collapses to one over (B, F), and everything left of it is ONE pass over hs:
 //     pooled[b,f] = (1/T) sum_t LeakyReLU(Dropout((1/K) sum_k hs[b,k,f,t]))
 // This file is that pass (forward) and its transpose (backward, only needed when the encoder is fine-tuned).
-// HBM-bound: the algorithmic traffic is hs read once (B*K*F*T*4 bytes; 1.3 GB at B = 64, K = 25, F = 1024, T = 199),
-// the output is B*F*4 bytes.
+// HBM-bound: the algorithmic traffic is hs read once (B*K*F*T elements: 1.3 GB of fp32 or 0.65 GB of bf16 at B = 64,
+// K = 25, F = 1024, T = 199), the output is B*F*4 bytes.
+//
+// Element type of hs / dhs: fp32 or bf16 (the dtype of a bf16 encoder's output).  bf16 elements are widened to fp32
+// exactly and everything after the load is the fp32 arithmetic in the same order, so a bf16 hs gives bit for bit the
+// pooled values of its fp32 copy, and the bf16 dhs is the fp32 one rounded to nearest even.
 //
 // Layout: hs is (B, K, F, T) contiguous, T innermost.  For one b the (f, t) plane is contiguous, so a block takes
-// `rows` consecutive feature rows = one contiguous run of rows*T floats per layer k (stride F*T between layers),
-// reads it with 128-bit loads when the run is 16-byte aligned, keeps the activated values in shared memory and
-// reduces each row over t in a fixed order (deterministic, no atomics).
+// `rows` consecutive feature rows = one contiguous run of rows*T elements per layer k (stride F*T between layers),
+// reads it with 128-bit loads (4 floats or 8 bf16) when the run allows, keeps the activated values (fp32) in shared
+// memory and reduces each row over t in a fixed order (deterministic, no atomics).
 //
 // Dropout: counter-based Philox4x32-10 keyed by a (seed, offset) pair read from DEVICE memory, so a captured CUDA
 // graph draws a new mask every replay (the caller bumps the offset in-stream).  Element (b,f,t) uses word
 // (i & 3) of the block i >> 2, i = (b*F + f)*T + t; the backward regenerates the same mask.
+#include <type_traits>
+
 #include "supcon_common.cuh"
 #include "supcon_internal.h"
 
@@ -52,62 +58,83 @@ __device__ __forceinline__ float dropout_scale(unsigned long long seed, unsigned
   return u >= p ? keep_scale : 0.0f;
 }
 
+template <typename E>
 struct RunView {            // the contiguous run of one block
-  const float* base;        // hs + ((b*K)*F + f0)*T
+  const E* base;            // hs + ((b*K)*F + f0)*T
   long long plane;          // F*T
   long long first_elem;     // (b*F + f0)*T : index of the run's first element in the (B,F,T) mask space
   int rows, len, f0, b;
 };
 
-__device__ __forceinline__ RunView run_of_block(const HeadPoolArgs& a) {
-  RunView v;
+template <typename E>
+__device__ __forceinline__ RunView<E> run_of_block(const HeadPoolArgs& a) {
+  RunView<E> v;
   v.b = blockIdx.y;
   v.f0 = blockIdx.x * a.rows_per_block;
   v.rows = min(a.rows_per_block, a.F - v.f0);
   v.len = v.rows * a.T;
   v.plane = (long long)a.F * a.T;
-  v.base = a.hs + ((long long)v.b * a.K) * v.plane + (long long)v.f0 * a.T;
+  v.base = static_cast<const E*>(a.hs) + ((long long)v.b * a.K) * v.plane + (long long)v.f0 * a.T;
   v.first_elem = ((long long)v.b * a.F + v.f0) * a.T;
   return v;
 }
 
-template <int VEC>
+// one access of VEC elements of type E: 16 bytes (float4, or eight bf16 in a uint4) or one element
+template <typename E, int VEC>
 struct Pack;
 template <>
-struct Pack<4> { typedef float4 type; };
+struct Pack<float, 4> { typedef float4 type; };
 template <>
-struct Pack<1> { typedef float type; };
+struct Pack<float, 1> { typedef float type; };
+template <>
+struct Pack<__nv_bfloat16, 8> { typedef uint4 type; };
+template <>
+struct Pack<__nv_bfloat16, 1> { typedef __nv_bfloat16 type; };
 
-template <int VEC>
-__device__ __forceinline__ void add_pack(float (&acc)[VEC], const typename Pack<VEC>::type& x) {
+// the two bf16 of a 32-bit word widened to fp32 (exact): element 2i is the low half
+__device__ __forceinline__ float bf16_lo(unsigned w) { return __uint_as_float(w << 16); }
+__device__ __forceinline__ float bf16_hi(unsigned w) { return __uint_as_float(w & 0xFFFF0000u); }
+// and back, rounded to nearest even
+__device__ __forceinline__ unsigned bf16x2_rn(float lo, float hi) {
+  const __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const unsigned*>(&h);
+}
+
+template <typename E, int VEC>
+__device__ __forceinline__ void add_pack(float (&acc)[VEC], const typename Pack<E, VEC>::type& x) {
   if constexpr (VEC == 4) { acc[0] += x.x; acc[1] += x.y; acc[2] += x.z; acc[3] += x.w; }
-  else acc[0] += x;
+  else if constexpr (VEC == 8) {
+    acc[0] += bf16_lo(x.x); acc[1] += bf16_hi(x.x); acc[2] += bf16_lo(x.y); acc[3] += bf16_hi(x.y);
+    acc[4] += bf16_lo(x.z); acc[5] += bf16_hi(x.z); acc[6] += bf16_lo(x.w); acc[7] += bf16_hi(x.w);
+  }
+  else if constexpr (std::is_same<E, float>::value) acc[0] += x;
+  else acc[0] += __bfloat162float(x);
 }
 
 // sum over the K layers of VEC consecutive elements starting at run offset e, layers added in order k = 0..K-1;
 // loads are issued eight layers at a time so that each thread keeps 8 x 16 bytes in flight
-template <int VEC>
-__device__ __forceinline__ void layer_sum(const RunView& v, int K, int e, float (&acc)[VEC]) {
-  typedef typename Pack<VEC>::type pack_t;
+template <typename E, int VEC>
+__device__ __forceinline__ void layer_sum(const RunView<E>& v, int K, int e, float (&acc)[VEC]) {
+  typedef typename Pack<E, VEC>::type pack_t;
   constexpr int BATCH = 8;
 #pragma unroll
   for (int i = 0; i < VEC; ++i) acc[i] = 0.f;
-  const float* p = v.base + e;
+  const E* p = v.base + e;
   int k = 0;
   for (; k + BATCH <= K; k += BATCH) {
     pack_t x[BATCH];
 #pragma unroll
     for (int j = 0; j < BATCH; ++j) x[j] = __ldg(reinterpret_cast<const pack_t*>(p + (long long)(k + j) * v.plane));
 #pragma unroll
-    for (int j = 0; j < BATCH; ++j) add_pack<VEC>(acc, x[j]);
+    for (int j = 0; j < BATCH; ++j) add_pack<E, VEC>(acc, x[j]);
   }
-  for (; k < K; ++k) add_pack<VEC>(acc, __ldg(reinterpret_cast<const pack_t*>(p + (long long)k * v.plane)));
+  for (; k < K; ++k) add_pack<E, VEC>(acc, __ldg(reinterpret_cast<const pack_t*>(p + (long long)k * v.plane)));
 }
 
-template <int VEC>
+template <typename E, int VEC>
 __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolArgs a) {
   extern __shared__ float act[];                      // [rows*T] activated values of this block's run
-  const RunView v = run_of_block(a);
+  const RunView<E> v = run_of_block<E>(a);
   const bool drop = a.dropout_p > 0.f && a.rng_state != nullptr;
   unsigned long long seed = 0, offset = 0;
   if (drop) { seed = a.rng_state[0]; offset = a.rng_state[1]; }
@@ -116,7 +143,7 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolAr
 
   for (int e = threadIdx.x * VEC; e < v.len; e += HP_THREADS * VEC) {
     float acc[VEC];
-    layer_sum<VEC>(v, a.K, e, acc);
+    layer_sum<E, VEC>(v, a.K, e, acc);
 #pragma unroll
     for (int i = 0; i < VEC; ++i) {
       float x = acc[i] * inv_k;
@@ -136,22 +163,23 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolAr
   }
 }
 
-// dhs[b,k,f,t] = dpooled[b,f] * (1/T) * LeakyReLU'(x) * dropout multiplier * (1/K), the same for every k
-template <int VEC>
+// dhs[b,k,f,t] = dpooled[b,f] * (1/T) * LeakyReLU'(x) * dropout multiplier * (1/K), the same for every k; computed
+// in fp32 and stored in E (bf16: round to nearest even)
+template <typename E, int VEC>
 __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_bwd_kernel(HeadPoolArgs a, const float* __restrict__ dpooled,
-                                                                   float* __restrict__ dhs) {
-  const RunView v = run_of_block(a);
+                                                                   E* __restrict__ dhs) {
+  const RunView<E> v = run_of_block<E>(a);
   const bool drop = a.dropout_p > 0.f && a.rng_state != nullptr;
   unsigned long long seed = 0, offset = 0;
   if (drop) { seed = a.rng_state[0]; offset = a.rng_state[1]; }
   const float inv_k = 1.0f / (float)a.K;
   const float keep_scale = drop ? 1.0f / (1.0f - a.dropout_p) : 1.0f;
   const float inv_kt = inv_k / (float)a.T;
-  float* out = dhs + (v.base - a.hs);
+  E* out = dhs + (v.base - static_cast<const E*>(a.hs));
 
   for (int e = threadIdx.x * VEC; e < v.len; e += HP_THREADS * VEC) {
     float acc[VEC], g[VEC];
-    layer_sum<VEC>(v, a.K, e, acc);
+    layer_sum<E, VEC>(v, a.K, e, acc);
 #pragma unroll
     for (int i = 0; i < VEC; ++i) {
       const float m = drop ? dropout_scale(seed, offset, v.first_elem + e + i, a.dropout_p, keep_scale) : 1.0f;
@@ -159,58 +187,81 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_bwd_kernel(HeadPoolAr
       const float up = dpooled[(long long)v.b * a.F + v.f0 + (e + i) / a.T];
       g[i] = up * inv_kt * m * (x > 0.f ? 1.0f : a.negative_slope);
     }
-    float* q = out + e;
-    for (int k = 0; k < a.K; ++k) {
-      if constexpr (VEC == 4)
-        *reinterpret_cast<float4*>(q + (long long)k * v.plane) = make_float4(g[0], g[1], g[2], g[3]);
-      else
-        q[(long long)k * v.plane] = g[0];
+    E* q = out + e;
+    if constexpr (VEC == 8) {
+      const uint4 w = make_uint4(bf16x2_rn(g[0], g[1]), bf16x2_rn(g[2], g[3]), bf16x2_rn(g[4], g[5]),
+                                 bf16x2_rn(g[6], g[7]));
+      for (int k = 0; k < a.K; ++k) *reinterpret_cast<uint4*>(q + (long long)k * v.plane) = w;
+    } else {
+      for (int k = 0; k < a.K; ++k) {
+        if constexpr (VEC == 4)
+          *reinterpret_cast<float4*>(q + (long long)k * v.plane) = make_float4(g[0], g[1], g[2], g[3]);
+        else if constexpr (std::is_same<E, float>::value)
+          q[(long long)k * v.plane] = g[0];
+        else
+          q[(long long)k * v.plane] = __float2bfloat16_rn(g[0]);
+      }
     }
   }
 }
 
 // 128-bit accesses need every run (and every layer plane) to start on a 16-byte boundary and to hold a multiple of
-// four floats - including the shorter run of the last block of a row of blocks.
-bool vector_ok(const HeadPoolArgs& a, const void* other) {
+// `width` elements (four floats, eight bf16) - including the shorter run of the last block of a row of blocks.
+bool vector_ok(const HeadPoolArgs& a, const void* other, int width) {
   auto aligned = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   const long long run = (long long)a.rows_per_block * a.T;
   const long long tail = (long long)(a.F % a.rows_per_block) * a.T;
-  return aligned(a.hs) && (other == nullptr || aligned(other)) && ((long long)a.F * a.T) % 4 == 0 && run % 4 == 0 &&
-         tail % 4 == 0;
+  return aligned(a.hs) && (other == nullptr || aligned(other)) && ((long long)a.F * a.T) % width == 0 &&
+         run % width == 0 && tail % width == 0;
 }
 
 }  // namespace
 
-int head_pool_rows_per_block(int F, int T) {
+int head_pool_rows_per_block(int F, int T, int hs_dtype) {
   // 16 rows per block when they fit 48 KB of shared memory (T <= 768), fewer for longer clips; 0 = unsupported
   if (T < 1 || F < 1) return 0;
   int rows = 12288 / T;
   if (rows < 1) return 0;
   if (rows > 16) rows = 16;
-  if (rows > 4) rows &= ~3;           // keep runs a multiple of four floats for any T
+  // keep runs a multiple of one 128-bit access for any T: four floats, eight bf16 (from 8 rows up)
+  if (hs_dtype == SUPCON_BF16 && rows >= 8) rows &= ~7;
+  else if (rows > 4) rows &= ~3;
   return rows < F ? rows : F;
 }
 
 cudaError_t head_pool_forward(HeadPoolArgs a, cudaStream_t stream) {
-  a.rows_per_block = head_pool_rows_per_block(a.F, a.T);
+  a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
   if (a.rows_per_block < 1) return cudaErrorInvalidValue;
   dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
   const size_t smem = (size_t)a.rows_per_block * a.T * sizeof(float);
-  if (vector_ok(a, nullptr))
-    head_pool_fwd_kernel<4><<<grid, HP_THREADS, smem, stream>>>(a);
-  else
-    head_pool_fwd_kernel<1><<<grid, HP_THREADS, smem, stream>>>(a);
+  if (a.hs_dtype == SUPCON_BF16) {
+    if (vector_ok(a, nullptr, 8))
+      head_pool_fwd_kernel<__nv_bfloat16, 8><<<grid, HP_THREADS, smem, stream>>>(a);
+    else
+      head_pool_fwd_kernel<__nv_bfloat16, 1><<<grid, HP_THREADS, smem, stream>>>(a);
+  } else if (vector_ok(a, nullptr, 4)) {
+    head_pool_fwd_kernel<float, 4><<<grid, HP_THREADS, smem, stream>>>(a);
+  } else {
+    head_pool_fwd_kernel<float, 1><<<grid, HP_THREADS, smem, stream>>>(a);
+  }
   return cudaGetLastError();
 }
 
-cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, float* dhs, cudaStream_t stream) {
-  a.rows_per_block = head_pool_rows_per_block(a.F, a.T);
+cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, void* dhs, cudaStream_t stream) {
+  a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
   if (a.rows_per_block < 1) return cudaErrorInvalidValue;
   dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
-  if (vector_ok(a, dhs))
-    head_pool_bwd_kernel<4><<<grid, HP_THREADS, 0, stream>>>(a, dpooled, dhs);
-  else
-    head_pool_bwd_kernel<1><<<grid, HP_THREADS, 0, stream>>>(a, dpooled, dhs);
+  if (a.hs_dtype == SUPCON_BF16) {
+    __nv_bfloat16* d = static_cast<__nv_bfloat16*>(dhs);
+    if (vector_ok(a, dhs, 8))
+      head_pool_bwd_kernel<__nv_bfloat16, 8><<<grid, HP_THREADS, 0, stream>>>(a, dpooled, d);
+    else
+      head_pool_bwd_kernel<__nv_bfloat16, 1><<<grid, HP_THREADS, 0, stream>>>(a, dpooled, d);
+  } else if (vector_ok(a, dhs, 4)) {
+    head_pool_bwd_kernel<float, 4><<<grid, HP_THREADS, 0, stream>>>(a, dpooled, static_cast<float*>(dhs));
+  } else {
+    head_pool_bwd_kernel<float, 1><<<grid, HP_THREADS, 0, stream>>>(a, dpooled, static_cast<float*>(dhs));
+  }
   return cudaGetLastError();
 }
 

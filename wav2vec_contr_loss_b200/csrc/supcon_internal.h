@@ -200,16 +200,17 @@ cudaError_t mid_launch(const SmallArgs& a, cudaStream_t stream, bool* taken);
 
 // ---- producer of z: compression head up to the Linear layer, fused with the time mean (supcon_head.cu) ----
 struct HeadPoolArgs {
-  const float* hs;                      // [B][K][F][T]
+  const void* hs;                       // [B][K][F][T] of hs_dtype
   float* pooled;                        // fwd out [B][F]
   const unsigned long long* rng_state;  // device {seed, offset}; NULL = no dropout
   int B, K, F, T;
   float dropout_p, negative_slope;
   int rows_per_block;                   // filled by the launcher
+  int hs_dtype;                         // SUPCON_F32 | SUPCON_BF16: element type of hs and dhs
 };
-int head_pool_rows_per_block(int F, int T);
+int head_pool_rows_per_block(int F, int T, int hs_dtype);
 cudaError_t head_pool_forward(HeadPoolArgs a, cudaStream_t stream);
-cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, float* dhs, cudaStream_t stream);
+cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, void* dhs, cudaStream_t stream);
 
 // tcgen05 building-block diagnostic (supcon_tc_debug.cu)
 int tc_debug_tile(const void* z_bf16, int n, int d, int row_i, int row_j, float* s_out, float* o_out,

@@ -8,8 +8,9 @@ The reference builds z as (compression_module.py:48-65, stage1_utils.py:122-123)
 
 ``mlp3`` and the time mean are both linear, so ``seq.mean(-1) == mlp3(x.mean(-1))``: the per-frame GEMM over
 B*T rows collapses to one over B rows and everything left of it is a single pass over ``hs``, which is what
-``supcon_head_pool_forward`` (csrc/supcon_head.cu) does - hs read once, (B, F) floats written.  The (B, F) x (F, D)
-product that remains is a plain library GEMM (``F.linear``: autograd gives the weight/bias gradients), and the row
+``supcon_head_pool_forward_typed`` (csrc/supcon_head.cu) does - hs read once, (B, F) floats written.  ``hs`` is read
+in its own dtype when that is fp32 or bf16 (the output of an encoder run in bf16: no fp32 copy, and d loss / d hs comes
+back in bf16); other dtypes are converted to fp32 first.  The (B, F) x (F, D) product that remains is a plain library GEMM (``F.linear``: autograd gives the weight/bias gradients), and the row
 normalisation is this library's kernel.
 
 ``FusedCompressionHead`` has the reference module's parameters under the same names (``mlp3.weight``,
@@ -32,7 +33,8 @@ from . import functional as Fn
 
 
 class _LayerTimePool(torch.autograd.Function):
-    """pooled[b, f] = mean_t LeakyReLU(Dropout(mean_k hs[b, k, f, t]))."""
+    """pooled[b, f] = mean_t LeakyReLU(Dropout(mean_k hs[b, k, f, t])).  fp32 and bf16 hs go to the kernel as they
+    are (bf16 is widened exactly inside it, and dhs is returned in bf16); other dtypes through an fp32 copy."""
 
     @staticmethod
     def forward(ctx, hs, dropout_p, negative_slope, rng_state):
@@ -41,9 +43,10 @@ class _LayerTimePool(torch.autograd.Function):
             raise ValueError(f"hs must be (batch, layers, feat, frames), got {tuple(hs.shape)}")
         lib = _cabi.load()
         x = hs.detach()
-        if x.dtype != torch.float32:
+        if x.dtype not in (torch.float32, torch.bfloat16):
             x = x.float()
         x = x.contiguous()
+        dtype_code = _cabi.BF16 if x.dtype == torch.bfloat16 else _cabi.F32
         b, k, f, t = x.shape
         dev = x.device
         rng = None
@@ -53,33 +56,35 @@ class _LayerTimePool(torch.autograd.Function):
             rng = rng_state.clone()                    # the backward must see the values this forward used
         with torch.cuda.device(dev):
             pooled = torch.empty((b, f), dtype=torch.float32, device=dev)
-            _cabi.check(lib.supcon_head_pool_forward(Fn._p(x), b, k, f, t, float(dropout_p), float(negative_slope),
-                                                     Fn._p(rng), Fn._p(pooled), Fn._stream(dev)),
-                        "supcon_head_pool_forward")
+            _cabi.check(lib.supcon_head_pool_forward_typed(Fn._p(x), dtype_code, b, k, f, t, float(dropout_p),
+                                                           float(negative_slope), Fn._p(rng), Fn._p(pooled),
+                                                           Fn._stream(dev)),
+                        "supcon_head_pool_forward_typed")
         if ctx.needs_input_grad[0]:
             ctx.save_for_backward(x, rng if rng is not None else torch.empty(0, device=dev))
-            ctx.cfg = (float(dropout_p), float(negative_slope), rng is not None, hs.dtype)
+            ctx.cfg = (float(dropout_p), float(negative_slope), rng is not None, hs.dtype, dtype_code)
         return pooled
 
     @staticmethod
     def backward(ctx, dpooled):
         x, rng = ctx.saved_tensors
-        dropout_p, negative_slope, has_rng, in_dtype = ctx.cfg
+        dropout_p, negative_slope, has_rng, in_dtype, dtype_code = ctx.cfg
         lib = _cabi.load()
         b, k, f, t = x.shape
         dev = x.device
         g = dpooled.detach().float().contiguous()
         with torch.cuda.device(dev):
-            dhs = torch.empty_like(x)
-            _cabi.check(lib.supcon_head_pool_backward(Fn._p(x), b, k, f, t, dropout_p, negative_slope,
-                                                      Fn._p(rng) if has_rng else None, Fn._p(g),
-                                                      Fn._p(dhs), Fn._stream(dev)),
-                        "supcon_head_pool_backward")
+            dhs = torch.empty_like(x)                  # in x's dtype: the kernel writes bf16 for a bf16 hs
+            _cabi.check(lib.supcon_head_pool_backward_typed(Fn._p(x), dtype_code, b, k, f, t, dropout_p,
+                                                            negative_slope, Fn._p(rng) if has_rng else None,
+                                                            Fn._p(g), Fn._p(dhs), Fn._stream(dev)),
+                        "supcon_head_pool_backward_typed")
         return dhs.to(in_dtype), None, None, None
 
 
 def layer_time_pool(hs: torch.Tensor, dropout_p: float = 0.0, negative_slope: float = 0.01, rng_state=None):
-    """One pass over hs (B, K, F, T): ``LeakyReLU(Dropout(hs.mean(1))).mean(-1)`` -> (B, F) fp32."""
+    """One pass over hs (B, K, F, T): ``LeakyReLU(Dropout(hs.mean(1))).mean(-1)`` -> (B, F) fp32.  hs may be fp32 or
+    bf16 (read natively, with the layer sum in fp32); any other dtype is converted to fp32 first."""
     return _LayerTimePool.apply(hs, float(dropout_p), float(negative_slope), rng_state)
 
 
