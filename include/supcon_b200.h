@@ -201,6 +201,26 @@ int supcon_backward_rows_remote(const supcon_problem_t* p, const void* z_all, co
                                 void* dz_out, int32_t dz_dtype, void* workspace, size_t workspace_bytes,
                                 void* stream);
 
+/* supcon_forward_rows / supcon_backward_rows for a memory that is still filling, with its fill level in DEVICE
+ * memory, so that one captured CUDA graph serves every fill level (a training step replayed as a graph while its
+ * cross-batch memory fills).  Both need SUPCON_FLAG_MEMORY_COLUMNS (SUPCON_E_INVALID before any CUDA call without
+ * it).  n_total is the CAPACITY, n_rows + memory size; the plan, the workspace and the route depend on it alone.
+ *   mem_filled  DEVICE int32, read by the kernels only: columns [n_rows + *mem_filled, n_total) are absent.  They
+ *               enter no sum, no count (|pos_i|, |neg_i|, the class sizes), no top-K list and not the fixed maximum,
+ *               and they get no gradient.  Their rows of z_all must still hold finite values (the tensor path reads
+ *               whole tiles).  A count outside [0, n_total - n_rows] makes the loss and dz NaN (no device fault).
+ *               NULL = a full memory: the call is then supcon_forward_rows / supcon_backward_rows.
+ * Results equal those of the plain calls with n_total = n_rows + *mem_filled on the same route, up to the order of
+ * the column splits' sums.  On the tensor path the tiles of absent columns still run (masked): a call costs what a
+ * full memory costs. */
+int supcon_forward_rows_memory(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
+                               const int32_t* mem_filled, float* row_stats, double* partials, float* loss_out,
+                               void* workspace, size_t workspace_bytes, void* stream);
+int supcon_backward_rows_memory(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
+                                const int32_t* mem_filled, const float* stats_all, const double* partials_global,
+                                const float* grad_out, void* dz_out, int32_t dz_dtype, void* workspace,
+                                size_t workspace_bytes, void* stream);
+
 /* ---- exchange between ranks through peer memory (NVLink / NVSwitch), see csrc/supcon_peer.cu -------------
  * The host maps every rank's exchange buffer into every process (a symmetric allocation, e.g.
  * torch.distributed._symmetric_memory) and describes it here.  All kernels are this library's own: plain

@@ -1,6 +1,8 @@
 """Head step of BASELINE configs[4] (frozen encoder): eager launches vs one CUDA-graph replay.
 
     python tools/graphed_step_bench.py [--batch 64] [--iters 30] [--head fused] [--hs-dtype bfloat16]
+    python tools/graphed_step_bench.py --head fused --memory 4096,16384,65536
+
 
 hs is the encoder output the reference hands the head: (B, 25, 1024, 199) fp32 (1.3 GB at B = 64), synthetic; with
 --hs-dtype bfloat16 it is the output of an encoder run in bf16 (0.65 GB), which the fused head reads as it is.
@@ -10,6 +12,11 @@ Times are CUDA events on the launching stream, median of --iters steps after war
 so every pass reads it from HBM.  Rates are over algorithmic bytes: hs read once by the forward; hs read once and d hs
 (K copies of the (B, F, T) gradient) written once by the backward.  The card's name and power limit are read in the
 same run and printed with the times.
+
+--memory M,...: the step with MemorySupConLoss (cross-batch memory of M rows) instead, for fp32 z and for bf16 z with
+unit rows, alpha 0 and 0.5: one graph replay with the memory full, one while it fills (reset to empty before the
+timed window, which enqueues fewer than M rows), the eager step with the memory full, and the graphed step with
+SupConBinaryLoss on the same batch.
 """
 import argparse
 import json
@@ -59,6 +66,58 @@ def card():
     return out
 
 
+def memory_steps(args, hs, y, sizes):
+    from wav2vec_contr_loss_b200 import FusedCompressionHead, SupConBinaryLoss
+    from wav2vec_contr_loss_b200 import functional as Fn
+    from wav2vec_contr_loss_b200 import stage1 as S
+    from wav2vec_contr_loss_b200.memory import MemorySupConLoss
+    dev, B, res = hs.device, hs.size(0), []
+    for z_dtype in (torch.float32, torch.bfloat16):
+        normalize = (lambda x: Fn.l2_normalize(x, torch.bfloat16)) if z_dtype == torch.bfloat16 else None
+        for alpha in (0.0, 0.5):
+            def make(loss_fn):
+                head = (FusedCompressionHead() if args.head == "fused" else LayerMeanHead()).to(dev).train()
+                opt = torch.optim.AdamW(head.parameters(), lr=5e-3, weight_decay=3e-3, capturable=True)
+                return head, opt, S.GraphedHeadStep(head, loss_fn, opt, hs, y, topk_neg=15, normalize=normalize)
+
+            _, _, plain = make(SupConBinaryLoss(temperature=0.07, similarity="cosine"))
+            t_plain = median_ms(lambda: plain(plain.hs, plain.labels, alpha), args.iters)
+            del plain
+            for m in sizes:
+                loss_fn = MemorySupConLoss(0.07, "cosine", memory_size=m)
+                head, opt, step = make(loss_fn)
+                mem = loss_fn.memory
+                g = torch.Generator(device=dev).manual_seed(m)
+                fill = _unit_rows(torch.randn(m, 256, device=dev, generator=g)).to(z_dtype)
+                mem.enqueue(fill, torch.randint(0, 2, (m,), device=dev, generator=g), unit_rows=True)
+                t_full = median_ms(lambda: step(step.hs, step.labels, alpha), args.iters)
+                mem.reset()
+                t_fill = median_ms(lambda: step(step.hs, step.labels, alpha), args.iters)
+                filled_after = mem.filled
+
+                def eager_step():
+                    z = S.embed(head, hs, normalize)
+                    loss = loss_fn(z, y, topk_neg=15, alpha=alpha)
+                    opt.zero_grad(set_to_none=True)
+                    loss.backward()
+                    torch.nn.utils.clip_grad_norm_(head.parameters(), 5.0)
+                    opt.step()
+
+                mem.enqueue(fill, torch.randint(0, 2, (m,), device=dev, generator=g), unit_rows=True)
+                t_eager = median_ms(eager_step, args.iters)
+                res.append({"z_dtype": str(z_dtype).replace("torch.", ""), "alpha": alpha, "memory_size": m,
+                            "graphed_memory_full_ms": t_full, "graphed_memory_filling_ms": t_fill,
+                            "filling_window_ends_at_rows": filled_after, "eager_memory_full_ms": t_eager,
+                            "graphed_without_memory_ms": t_plain})
+                print(json.dumps(res[-1]), file=sys.stderr, flush=True)
+                del step, head, opt, loss_fn, mem, fill
+    return res
+
+
+def _unit_rows(x):
+    return torch.nn.functional.normalize(x, dim=1)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", type=int, default=64)
@@ -68,6 +127,7 @@ def main():
                     help="torch: the reference's op chain; fused: FusedCompressionHead (csrc/supcon_head.cu)")
     ap.add_argument("--hs-dtype", choices=("float32", "bfloat16"), default="float32",
                     help="element type of the encoder output hs (bfloat16 needs --head fused)")
+    ap.add_argument("--memory", default="", help="comma-separated memory sizes: time the cross-batch memory step")
     args = ap.parse_args()
     if args.hs_dtype == "bfloat16" and args.head != "fused":
         ap.error("--hs-dtype bfloat16 needs --head fused (the torch op chain's Linear layer is fp32)")
@@ -85,6 +145,10 @@ def main():
     hs_bytes = hs.numel() * hs.element_size()
     out = {"batch": B, "hs_shape": list(hs.shape), "hs_dtype": args.hs_dtype, "hs_GB": hs_bytes / 1e9,
            "iters": args.iters, "head": args.head, "card": card()}
+    if args.memory:
+        out["memory"] = memory_steps(args, hs, y, [int(m) for m in args.memory.split(",")])
+        print(json.dumps(out))
+        return
     if args.head == "fused":
         rng = torch.tensor([1337, 0], dtype=torch.int64, device=dev)
         with torch.no_grad():

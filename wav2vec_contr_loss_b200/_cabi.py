@@ -34,6 +34,7 @@ EXPORTS = (
     "supcon_finalize_sets", "supcon_backward_rows_local", "supcon_backward_rows_remote",
     "supcon_peer_push", "supcon_peer_wait", "supcon_peer_end_step", "supcon_label_keys",
     "supcon_head_pool_forward_typed", "supcon_head_pool_backward_typed",
+    "supcon_forward_rows_memory", "supcon_backward_rows_memory",
 )
 
 
@@ -86,6 +87,9 @@ def load():
     lib.supcon_forward_rows.restype = c_int32
     lib.supcon_forward_rows.argtypes = [P, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                         c_size_t, c_void_p]
+    lib.supcon_forward_rows_memory.restype = c_int32
+    lib.supcon_forward_rows_memory.argtypes = [P, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                               c_void_p, c_size_t, c_void_p]
     lib.supcon_forward_rows_local.restype = c_int32
     lib.supcon_forward_rows_local.argtypes = [P, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
     lib.supcon_forward_rows_remote.restype = c_int32
@@ -95,6 +99,9 @@ def load():
     lib.supcon_backward_rows.restype = c_int32
     lib.supcon_backward_rows.argtypes = [P, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_int32, c_void_p, c_size_t, c_void_p]
+    lib.supcon_backward_rows_memory.restype = c_int32
+    lib.supcon_backward_rows_memory.argtypes = [P, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                c_void_p, c_int32, c_void_p, c_size_t, c_void_p]
     lib.supcon_loss_and_grad.restype = c_int32
     lib.supcon_loss_and_grad.argtypes = [P, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p,
                                          c_void_p, c_void_p, c_size_t, c_void_p]

@@ -236,12 +236,16 @@ int supcon_workspace_bytes(const supcon_problem_t* p, size_t* bytes_out) {
   return 0;
 }
 
-int supcon_forward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
-                        float* row_stats, double* partials, float* loss_out, void* workspace,
-                        size_t workspace_bytes, void* stream) {
-  if (int rc = validate(p)) return rc;
+}  // extern "C"
+
+namespace {
+// supcon_forward_rows (mem_filled == NULL) and supcon_forward_rows_memory: the plan, the workspace and the route
+// depend on the problem alone, never on the device fill level, so one captured graph serves every fill level
+int forward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const int32_t* mem_filled,
+                 float* row_stats, double* partials, float* loss_out, void* workspace, size_t workspace_bytes,
+                 void* stream, const char* who) {
   if (!z_all || !labels_all || !row_stats || !partials || !workspace)
-    return fail(SUPCON_E_INVALID, "NULL buffer passed to supcon_forward_rows");
+    return fail(SUPCON_E_INVALID, "NULL buffer passed to %s", who);
   if (workspace_bytes < workspace_need(p))
     return fail(SUPCON_E_WORKSPACE, "workspace too small: %zu < %zu", workspace_bytes, workspace_need(p));
   if ((p->flags & SUPCON_FLAG_FORCE_TENSOR) && !tc_supported(p))
@@ -266,17 +270,38 @@ int supcon_forward_rows(const supcon_problem_t* p, const void* z_all, const int3
   }
   if (use_tc(p, false)) {
     const char* err = "";
-    int rc = tc_forward(p, z_all, labels_all, row_stats, partials, loss_out, workspace, st, &err);
+    int rc = tc_forward(p, z_all, labels_all, row_stats, partials, loss_out, workspace, st, &err, 0, mem_filled);
     if (rc) return fail(rc, "tc_forward: %s", err);
     return 0;
   }
   cudaError_t e = cudaMemsetAsync(workspace, 0, 256, st);
   if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
   FfmaArgs a = make_ffma(p, z_all, labels_all, workspace);
-  a.row_stats = row_stats; a.partials = partials; a.loss_out = loss_out;
+  a.row_stats = row_stats; a.partials = partials; a.loss_out = loss_out; a.mem_filled = mem_filled;
   e = ffma_forward(a, st);
   if (e != cudaSuccess) return cuda_fail(e, "ffma_forward");
   return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int supcon_forward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
+                        float* row_stats, double* partials, float* loss_out, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+  if (int rc = validate(p)) return rc;
+  return forward_rows(p, z_all, labels_all, nullptr, row_stats, partials, loss_out, workspace, workspace_bytes,
+                      stream, "supcon_forward_rows");
+}
+
+int supcon_forward_rows_memory(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
+                               const int32_t* mem_filled, float* row_stats, double* partials, float* loss_out,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  if (int rc = validate(p)) return rc;
+  if (!(p->flags & SUPCON_FLAG_MEMORY_COLUMNS))
+    return fail(SUPCON_E_INVALID, "supcon_forward_rows_memory needs SUPCON_FLAG_MEMORY_COLUMNS");
+  return forward_rows(p, z_all, labels_all, mem_filled, row_stats, partials, loss_out, workspace, workspace_bytes,
+                      stream, "supcon_forward_rows_memory");
 }
 
 int supcon_forward_rows_local(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
@@ -372,13 +397,15 @@ int supcon_backward_rows_remote(const supcon_problem_t* p, const void* z_all, co
   return 0;
 }
 
-int supcon_backward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
-                         const float* stats_all, const double* partials_global, const float* grad_out,
-                         void* dz_out, int32_t dz_dtype, void* workspace, size_t workspace_bytes,
-                         void* stream) {
-  if (int rc = validate(p)) return rc;
+}  // extern "C"
+
+namespace {
+// supcon_backward_rows (mem_filled == NULL) and supcon_backward_rows_memory
+int backward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const int32_t* mem_filled,
+                  const float* stats_all, const double* partials_global, const float* grad_out, void* dz_out,
+                  int32_t dz_dtype, void* workspace, size_t workspace_bytes, void* stream, const char* who) {
   if (!z_all || !labels_all || !stats_all || !partials_global || !dz_out)
-    return fail(SUPCON_E_INVALID, "NULL buffer passed to supcon_backward_rows");
+    return fail(SUPCON_E_INVALID, "NULL buffer passed to %s", who);
   if (dz_dtype != SUPCON_F32 && dz_dtype != SUPCON_BF16)
     return fail(SUPCON_E_INVALID, "unknown dz_dtype %d", dz_dtype);
   if (use_tc(p, true)) {
@@ -386,7 +413,7 @@ int supcon_backward_rows(const supcon_problem_t* p, const void* z_all, const int
       return fail(SUPCON_E_WORKSPACE, "workspace too small: %zu < %zu", workspace_bytes, workspace_need(p));
     const char* err = "";
     int rc = tc_backward(p, z_all, labels_all, stats_all, partials_global, grad_out, dz_out, dz_dtype, workspace,
-                         reinterpret_cast<cudaStream_t>(stream), &err);
+                         reinterpret_cast<cudaStream_t>(stream), &err, 0, mem_filled);
     if (rc) return fail(rc, "tc_backward: %s", err);
     return 0;
   }
@@ -395,10 +422,33 @@ int supcon_backward_rows(const supcon_problem_t* p, const void* z_all, const int
   FfmaArgs a = make_ffma(p, z_all, labels_all, workspace, /*backward=*/true);
   a.stats_all = stats_all;
   a.partials = const_cast<double*>(partials_global);
-  a.grad_out = grad_out; a.dz_out = dz_out;
+  a.grad_out = grad_out; a.dz_out = dz_out; a.mem_filled = mem_filled;
   cudaError_t e = ffma_backward(a, dz_dtype, reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "ffma_backward");
   return 0;
+}
+}  // namespace
+
+extern "C" {
+
+int supcon_backward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
+                         const float* stats_all, const double* partials_global, const float* grad_out,
+                         void* dz_out, int32_t dz_dtype, void* workspace, size_t workspace_bytes,
+                         void* stream) {
+  if (int rc = validate(p)) return rc;
+  return backward_rows(p, z_all, labels_all, nullptr, stats_all, partials_global, grad_out, dz_out, dz_dtype,
+                       workspace, workspace_bytes, stream, "supcon_backward_rows");
+}
+
+int supcon_backward_rows_memory(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,
+                                const int32_t* mem_filled, const float* stats_all, const double* partials_global,
+                                const float* grad_out, void* dz_out, int32_t dz_dtype, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+  if (int rc = validate(p)) return rc;
+  if (!(p->flags & SUPCON_FLAG_MEMORY_COLUMNS))
+    return fail(SUPCON_E_INVALID, "supcon_backward_rows_memory needs SUPCON_FLAG_MEMORY_COLUMNS");
+  return backward_rows(p, z_all, labels_all, mem_filled, stats_all, partials_global, grad_out, dz_out, dz_dtype,
+                       workspace, workspace_bytes, stream, "supcon_backward_rows_memory");
 }
 
 int supcon_loss_and_grad(const supcon_problem_t* p, const void* z, const int32_t* labels, float* loss_out,

@@ -39,6 +39,15 @@ __device__ __forceinline__ float geodesic_slope_exact(float c) {
   return __fdiv_rn(SUPCON_2_OVER_PI_F, sqrtf(fmaf(-c, c, 1.0f)));
 }
 
+// Columns a kernel sweeps when the memory's fill level is read on the device (supcon_forward_rows_memory):
+// n_rows + *mem_filled, or -1 when the count lies outside [0, n_total - n_rows] (the caller poisons its results
+// with NaN and sweeps every column).  mem_filled == NULL: n_total, a full memory or none.
+__device__ __forceinline__ int live_columns(const int32_t* mem_filled, int n_rows, int n_total) {
+  if (mem_filled == nullptr) return n_total;
+  const int f = *mem_filled;
+  return (f >= 0 && f <= n_total - n_rows) ? n_rows + f : -1;
+}
+
 // Global coefficients of the backward pass, derived from the (all-reduced)
 // partial sums exactly as loss.py:137-151 blends the two means.
 struct GlobalCoef {

@@ -117,6 +117,10 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
   const bool geo = a.similarity == SUPCON_GEODESIC;
   const bool uni = a.lambda_uni > 0.f;
   const bool mine = a.mine != 0;
+  // columns [n_cols, n_total) are absent (a memory that is not full yet); bad: the fill level is out of range
+  const int n_live = live_columns(a.mem_filled, a.n_rows, a.n_total);
+  const bool bad = n_live < 0;
+  const int n_cols = bad ? a.n_total : n_live;
 
   // phase-2 mapping: 4 threads per row, thread q takes columns q, q+4, ...
   const int pr = tid >> 2, pq = tid & 3;
@@ -141,7 +145,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
   // column range of this CTA (blockIdx.y = column split; one split = the whole sweep)
   const int split = blockIdx.y;
   const int c_lo = (int)(((int64_t)a.col_tiles * split) / a.splits) * BN;
-  const int c_hi = min(a.n_total, (int)(((int64_t)a.col_tiles * (split + 1)) / a.splits) * BN);
+  const int c_hi = min(n_cols, (int)(((int64_t)a.col_tiles * (split + 1)) / a.splits) * BN);
 
   float acc[4][4];
   for (int round = 0; round < rounds_total; ++round) {
@@ -151,8 +155,8 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
     if (tid < BM) cnt[tid] = 0;
     __syncthreads();
     for (int col0 = c_lo; col0 < c_hi; col0 += BN) {
-      gram_tile<T>(z, a.d, a.vec_ok, row0, row_end, col0, a.n_total, As, Bs, acc, nrm_r, nrm_c, uni && first);
-      if (tid < BN) lab_c[tid] = (col0 + tid < a.n_total) ? a.labels[col0 + tid] : 0;
+      gram_tile<T>(z, a.d, a.vec_ok, row0, row_end, col0, n_cols, As, Bs, acc, nrm_r, nrm_c, uni && first);
+      if (tid < BN) lab_c[tid] = (col0 + tid < n_cols) ? a.labels[col0 + tid] : 0;
       __syncthreads();  // norms + labels visible
 #pragma unroll
       for (int i = 0; i < 4; ++i)
@@ -174,7 +178,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
 #pragma unroll 4
         for (int t = 0; t < BN / 4; ++t) {
           int c = pq + 4 * t, gj = col0 + c;
-          if (row_ok && gj < a.n_total && gj != gi) tmax = fmaxf(tmax, __fdiv_rn(Ss[pr * LDS_ + c], a.tau));
+          if (row_ok && gj < n_cols && gj != gi) tmax = fmaxf(tmax, __fdiv_rn(Ss[pr * LDS_ + c], a.tau));
         }
         if (tmax > st.m) {
           float f = rescale(st.m, tmax);
@@ -183,7 +187,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
 #pragma unroll 4
         for (int t = 0; t < BN / 4; ++t) {
           int c = pq + 4 * t, gj = col0 + c;
-          if (row_ok && gj < a.n_total && gj != gi) {
+          if (row_ok && gj < n_cols && gj != gi) {
             float s = Ss[pr * LDS_ + c];
             float e = expf(__fdiv_rn(s, a.tau) - st.m);
             st.sum_all += e;
@@ -204,7 +208,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
 #pragma unroll 4
           for (int t = 0; t < BN / 4; ++t) {
             int c = pq + 4 * t, gj = col0 + c;
-            if (gj < a.n_total && lab_c[c] != lab_r) {
+            if (gj < n_cols && lab_c[c] != lab_r) {
               float s = Ss[pr * LDS_ + c];
               bool elig = (s < bound_v) || (s == bound_v && gj > bound_i);
               if (elig && (have < Kr || s > thr)) cand = true;
@@ -221,7 +225,7 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
           int cn = have;
           for (int c = 0; c < BN; ++c) {
             int gj = col0 + c;
-            if (gj >= a.n_total || lab_c[c] == lab_r) continue;
+            if (gj >= n_cols || lab_c[c] == lab_r) continue;
             float s = Ss[pr * LDS_ + c];
             if (!((s < bound_v) || (s == bound_v && gj > bound_i))) continue;
             int p;
@@ -315,6 +319,10 @@ __global__ void __launch_bounds__(NT) ffma_fwd_kernel(FfmaArgs a) {
         if (nneg > 0 && a.topk >= 1) { l_mined = (double)(lse_m - pos_mean); c_mined = 1.0; }
       }
       w = (double)wsum;
+      if (bad) {   // fill level out of range: NaN loss (c_full = 1 so that the loss reads the NaN sum)
+        so[SUPCON_ST_LSE] = so[SUPCON_ST_LSE_M] = NAN;
+        l_full = l_mined = w = NAN; c_full = 1.0;
+      }
     }
     red[0 * BM + pr] = l_full; red[1 * BM + pr] = c_full; red[2 * BM + pr] = l_mined;
     red[3 * BM + pr] = c_mined; red[4 * BM + pr] = w;
@@ -382,6 +390,10 @@ __global__ void __launch_bounds__(128) ffma_fwd_merge_kernel(FfmaArgs a) {
       if (nneg > 0 && a.topk >= 1) { l_mined = (double)(lse_m - pos_mean); c_mined = 1.0; }
     }
     w = (double)wsum;
+    if (live_columns(a.mem_filled, a.n_rows, a.n_total) < 0) {   // as in ffma_fwd_kernel
+      so[SUPCON_ST_LSE] = so[SUPCON_ST_LSE_M] = NAN;
+      l_full = l_mined = w = NAN; c_full = 1.0;
+    }
   }
   red[0 * 128 + threadIdx.x] = l_full; red[1 * 128 + threadIdx.x] = c_full; red[2 * 128 + threadIdx.x] = l_mined;
   red[3 * 128 + threadIdx.x] = c_mined; red[4 * 128 + threadIdx.x] = w;
@@ -404,6 +416,7 @@ __global__ void __launch_bounds__(256) ffma_bwd_reduce_kernel(FfmaArgs a) {
     v = fmaf(g.cu * a.stats_all[(int64_t)gi * SUPCON_STATS_STRIDE + SUPCON_ST_WSUM],
              ld_elem<T>(reinterpret_cast<const T*>(a.z) + (int64_t)gi * a.d + dd), v);
   v *= a.grad_out ? *a.grad_out : 1.0f;
+  if (live_columns(a.mem_filled, a.n_rows, a.n_total) < 0) v = NAN;
   TO* out = reinterpret_cast<TO*>(a.dz_out);
   if constexpr (sizeof(TO) == 4) out[idx] = v;
   else out[idx] = __float2bfloat16(v);
@@ -468,6 +481,8 @@ __global__ void __launch_bounds__(NT) ffma_bwd_kernel(FfmaArgs a) {
   const GlobalCoef g = global_coef(a.partials, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t);
   const bool uni = g.cu != 0.f;
   const bool mining = g.a_mined != 0.f;
+  const int n_live = live_columns(a.mem_filled, a.n_rows, a.n_total);
+  const int n_cols = n_live < 0 ? a.n_total : n_live;   // columns [n_cols, n_total) are absent
 
   if (tid < BM) load_coef(a, g, row0 + tid, row0 + tid < row_end, rf, rn, tid, BM);
 
@@ -479,16 +494,16 @@ __global__ void __launch_bounds__(NT) ffma_bwd_kernel(FfmaArgs a) {
 
   const int split = blockIdx.z;
   const int c_lo = (int)(((int64_t)a.col_tiles * split) / a.splits) * BN;
-  const int c_hi = min(a.n_total, (int)(((int64_t)a.col_tiles * (split + 1)) / a.splits) * BN);
+  const int c_hi = min(n_cols, (int)(((int64_t)a.col_tiles * (split + 1)) / a.splits) * BN);
   float acc[4][4];
   for (int col0 = c_lo; col0 < c_hi; col0 += BN) {
-    gram_tile<T>(z, a.d, a.vec_ok, row0, row_end, col0, a.n_total, As, Bs, acc, nrm_r, nrm_c, uni);
-    if (tid < BN) load_coef(a, g, col0 + tid, col0 + tid < a.n_total, cf, cn, tid, BN);
+    gram_tile<T>(z, a.d, a.vec_ok, row0, row_end, col0, n_cols, As, Bs, acc, nrm_r, nrm_c, uni);
+    if (tid < BN) load_coef(a, g, col0 + tid, col0 + tid < n_cols, cf, cn, tid, BN);
     // stage Z_J[:, dc0:dc0+DC] (fp32) for the H.Z product
     for (int idx = tid; idx < BN * (DC / 4); idx += NT) {
       int r = idx / (DC / 4), q = idx % (DC / 4);
       int gc = col0 + r;
-      float4 v = ld_row4<T>(z, gc, gc < a.n_total, dc0 + 4 * q, a.d, a.vec_ok);
+      float4 v = ld_row4<T>(z, gc, gc < n_cols, dc0 + 4 * q, a.d, a.vec_ok);
       *reinterpret_cast<float4*>(&Zs[r * DC + 4 * q]) = v;
     }
     __syncthreads();
@@ -499,7 +514,7 @@ __global__ void __launch_bounds__(NT) ffma_bwd_kernel(FfmaArgs a) {
         const int r = ty + 16 * i, c = tx + 16 * j;
         const int gi = row0 + r, gj = col0 + c;
         float h = 0.f;
-        if (gi < row_end && gj < a.n_total && gi != gj) {
+        if (gi < row_end && gj < n_cols && gi != gj) {
           const float cv = acc[i][j];
           const float s = geo ? geodesic_sim(cv) : cv;
           const float lg = __fdiv_rn(s, a.tau);
@@ -566,7 +581,7 @@ __global__ void __launch_bounds__(NT) ffma_bwd_kernel(FfmaArgs a) {
     }
     return;
   }
-  const float gscale = a.grad_out ? *a.grad_out : 1.0f;
+  const float gscale = n_live < 0 ? NAN : (a.grad_out ? *a.grad_out : 1.0f);
   TO* out = reinterpret_cast<TO*>(a.dz_out);
 #pragma unroll
   for (int i = 0; i < 4; ++i) {

@@ -28,6 +28,7 @@ struct FfmaArgs {
   void* dz_out;              // bwd: [n_rows][d]
   int n_total, row_offset, n_rows, d;
   int n_batch;               // batch_columns(): columns from n_batch on are memory (no statistics, no uniformity)
+  const int32_t* mem_filled; // device fill level of the memory (live_columns()); nullptr: all n_total columns
   int z_dtype, similarity, topk, kcap, mine, vec_ok;
   float tau, alpha, lambda_uni, uni_t;
   // column splits (ffma_plan): partial records / candidate lists / partial dz in the workspace
@@ -108,6 +109,7 @@ struct TcFwdArgs {
   int n_total, n_pad, row_offset, n_rows, rows_pad, topk, mine, kcap;
   float inv_tau, c1, c0, ut2;
   float m_limit;     // tau / 0.025: largest fixed maximum that cannot underflow a row's dominant terms
+  const int32_t* mem_filled;   // device fill level of the memory (live_columns()); nullptr: all n_total columns
 };
 struct TcBwdPrepArgs {
   const float* stats;        // statistics of rows [stats_row0, ...): [..][STRIDE]
@@ -126,6 +128,8 @@ struct TcBwdPrepArgs {
   float* scalars;
   int n_total, n_pad, topk;
   int n_batch;               // batch_columns(): columns from n_batch on are memory (zero coefficients, no statistics)
+  int n_rows;
+  const int32_t* mem_filled; // as in TcFwdArgs
   float tau, alpha, lambda_uni, uni_t;
 };
 struct TcBwdArgs {
@@ -152,6 +156,7 @@ struct TcBwdArgs {
   const float* csum;     // [TC_CMAX][256]
   const int32_t* cls_pad;  // dense class id per column (tc_prep_bwd_kernel)
   int plin_twin;
+  const int32_t* mem_filled;   // as in TcFwdArgs
 };
 TcPlan tc_plan(const supcon_problem_t* p);
 bool tc_supported(const supcon_problem_t* p);
@@ -160,15 +165,17 @@ bool tc_bwd_two_phase(const supcon_problem_t* p);
 int tc_debug_plan(const supcon_problem_t* p, int32_t* out, int n_out);
 int tc_debug_sched(int T, int P, long long U, int cta, int row_block, long long* range_begin, long long* range_end,
                    int* first_cta, int* last_cta);
+// mem_filled (SUPCON_FLAG_MEMORY_COLUMNS, phase 0 only): device fill level of the memory; columns
+// [n_rows + *mem_filled, n_total) are absent.  nullptr: every column is there.
 int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, float* row_stats,
                double* partials, float* loss_out, void* workspace, cudaStream_t stream, const char** err,
-               int phase = 0);
+               int phase = 0, const int32_t* mem_filled = nullptr);
 // phase: 0 = whole backward; 1 = only the columns this rank owns (`stats` = the rank's OWN statistics
 // [n_rows][STRIDE], `partials` = its own forward partials; partial dz records, nothing else is written);
 // 2 = all other columns (`stats` = everyone's, `partials` = the global sums) + reduce over both phases.
 int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const float* stats,
                 const double* partials, const float* grad_out, void* dz_out, int dz_dtype, void* workspace,
-                cudaStream_t stream, const char** err, int phase = 0);
+                cudaStream_t stream, const char** err, int phase = 0, const int32_t* mem_filled = nullptr);
 
 // ---- exchange through peer memory (supcon_peer.cu) ----
 int peer_check(const supcon_peer_t* pe, const char** err);

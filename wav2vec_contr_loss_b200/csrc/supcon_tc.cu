@@ -155,14 +155,20 @@ __device__ __forceinline__ float fixmax_from_bits(unsigned bits, float m_limit) 
 // Memory columns [mem_lo, n) (SUPCON_FLAG_MEMORY_COLUMNS) feed the maximum but store nrm_pad = +inf: the sweeps'
 // uniformity weight ex2(-ut2 * max(n_i + n_j - 2 c, 0)) is then exactly 0 for them (ut2 > 0 is validated), so
 // they drop out of the uniformity sums without a test in the sweep kernels.
+// mem_filled (live_columns()): absent columns [n_live, n) are padding here: no load, no share in the maximum.  A fill
+// level out of range poisons the maximum with NaN, like a broken unit-rows promise.
 __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* __restrict__ z,
                                                           const int32_t* __restrict__ labels, int n, int n_pad, int d,
                                                           int32_t* __restrict__ lab_pad, float* __restrict__ nrm_pad,
                                                           unsigned* __restrict__ nrm2_max, int count, int j_lo = 0,
                                                           int ex_lo = 0x7fffffff, int ex_len = 0,
-                                                          int track_max = 1, int mem_lo = 0x7fffffff) {
+                                                          int track_max = 1, int mem_lo = 0x7fffffff,
+                                                          const int32_t* mem_filled = nullptr, int n_rows = 0) {
   __shared__ float wmax[8];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int n_live = live_columns(mem_filled, n_rows, n);
+  if (n_live < 0 && blockIdx.x == 0 && threadIdx.x == 0) atomicMax(nrm2_max, 0x7fc00000u);
+  if (n_live >= 0) n = n_live;
   float mx = 0.f;
   for (int w = blockIdx.x * 8 + wib; w < count; w += gridDim.x * 8) {
     int j = j_lo + w;
@@ -201,9 +207,13 @@ __global__ void __launch_bounds__(256) tc_prep_fwd_kernel(const __nv_bfloat16* _
 // class sizes: one thread per column of [j_lo, n) minus the excluded window; lanes holding the same label are
 // aggregated (__match_any_sync) so a binary batch costs two atomics per warp instead of 32 on two addresses
 // hids / n_classes (optional): the thread that claims a slot also gives it the next dense class id
+// mem_filled: only the live columns of [0, n) count (live_columns())
 __global__ void tc_label_table_kernel(const int32_t* __restrict__ labels, int n, unsigned long long* hkeys,
                                       int* hcounts, uint32_t hmask, int j_lo, int ex_lo, int ex_len,
-                                      int* hids = nullptr, int* n_classes = nullptr) {
+                                      int* hids = nullptr, int* n_classes = nullptr,
+                                      const int32_t* mem_filled = nullptr, int n_rows = 0) {
+  const int n_live = live_columns(mem_filled, n_rows, n);
+  if (n_live >= 0) n = n_live;
   int j = j_lo + blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= ex_lo) j += ex_len;
   const bool ok = j < n;
@@ -247,13 +257,17 @@ __global__ void __launch_bounds__(256) tc_class_sum_kernel(const __nv_bfloat16* 
                                                            const unsigned long long* __restrict__ hkeys,
                                                            const int* __restrict__ hids, uint32_t hmask,
                                                            const int* __restrict__ n_classes,
-                                                           float* __restrict__ part) {
+                                                           float* __restrict__ part,
+                                                           const int32_t* __restrict__ mem_filled = nullptr,
+                                                           int n_rows = 0) {
   __shared__ float acc[TC_CMAX * TD];   // thread k owns element k of every class sum
   __shared__ int ids_s[CS_COLS];
   const int nc = *n_classes;
   if (nc > TC_CMAX) return;
+  const int n_live = live_columns(mem_filled, n_rows, n);
+  if (n_live >= 0) n = n_live;          // absent columns: in no class sum
   const int tid = threadIdx.x;
-  const int j0 = blockIdx.x * CS_COLS, cnt = min(CS_COLS, n - j0);
+  const int j0 = blockIdx.x * CS_COLS, cnt = max(0, min(CS_COLS, n - j0));
   if (tid < CS_COLS) ids_s[tid] = tid < cnt ? label_table_id(hkeys, hids, hmask, labels[j0 + tid]) : 0;
   for (int c = 0; c < nc; ++c) acc[c * TD + tid] = 0.f;
   __syncthreads();
@@ -292,16 +306,18 @@ __global__ void __launch_bounds__(1024) tc_class_reduce_kernel(const float* __re
 //   e0_ij = exp((s_ij - 1)/tau);  H_ij = e0 (A_i + A_j) [+ mined terms] - pos_ij (B_i + B_j)
 //   A = a_f exp(1/tau - lse),  Am = a_m exp(1/tau - lse_m),  B = (a_f + a_m)/|pos|
 // Memory columns [n_batch, n_total) (SUPCON_FLAG_MEMORY_COLUMNS) are constants: A = Am = B = 0, thr = +inf, idx = -1
-// and no statistics are read; only their label is needed (positives of the rows).
+// and no statistics are read; only their label is needed (positives of the rows).  Absent columns [n_live, n_total)
+// (live_columns()) are padding; a fill level out of range makes M NaN.
 __global__ void tc_prep_bwd_kernel(TcBwdPrepArgs a) {
   int j = a.j_lo + blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= a.j_lo + a.j_cnt) return;
   float A = 0.f, Am = 0.f, B = 0.f, thr = INFINITY;
   int ti = -1, lab = 0;
+  const int n_live = live_columns(a.mem_filled, a.n_rows, a.n_total);
   // fixed maximum the forward used (tensor-path statistics carry it; statistics of another path: M = 1)
-  const float Mp = (float)a.partials[SUPCON_P_FIXMAX];   // NaN = the forward poisoned the result: stays NaN
+  const float Mp = n_live < 0 ? NAN : (float)a.partials[SUPCON_P_FIXMAX];   // NaN = poisoned: stays NaN
   const float M = (Mp >= 1.0f || Mp != Mp) ? Mp : 1.0f;
-  if (j < a.n_total) {
+  if (j < (n_live < 0 ? a.n_total : n_live)) {
     const GlobalCoef g = global_coef(a.partials, a.n_batch, a.tau, a.alpha, a.lambda_uni, a.uni_t,
                                      a.use_label_counts != 0);
     if (j < a.n_batch) {
@@ -542,9 +558,11 @@ __device__ __forceinline__ void load_rows_to_tmem(const __nv_bfloat16* __restric
 // releases the TMEM buffer at once (the next MMA into it overlaps the exp work) and then reduces
 // from registers.  All pipeline barriers are indexed by a running tile counter, so segments
 // follow each other without draining the TMA ring.
-template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
-__global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid_constant__ CUtensorMap tmap,
-                                                                    const __nv_bfloat16* __restrict__ z, TcFwdArgs a) {
+// LIVE: columns [n_cols, n_total) are absent (live_columns(): a memory that is not full yet) and masked; the tiles
+// holding them run the masked path.  Only tc_fwd_live_kernel has it: the other sweeps compile as without a memory.
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN, bool LIVE>
+__device__ __forceinline__ void tc_fwd_sweep(const CUtensorMap& tmap, const __nv_bfloat16* __restrict__ z,
+                                             const TcFwdArgs& a) {
   static_assert(NCH == 1 || (NCH == 2 && !MINE), "the top-K lists are kept by one thread per row");
   static_assert(!PLIN || (SIM == SUPCON_COSINE && !MINE), "positives by linearity: cosine, no per-pair positive terms");
   // positives by linearity: this kernel and its per-pair twin are both launched, the class count picks one
@@ -655,6 +673,11 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid
     const uint32_t taddr = tmem + lane_addr + TM_S + wg * BN + ch * CW;
     // exponent offset of this launch: -M/tau * log2(e) with the fixed maximum as of this phase's prep kernel
     const float c0 = -a.c1 * fixmax_from_bits(*a.nrm2_max, a.m_limit);
+    int n_cols = a.n_total;
+    if (LIVE) {
+      const int n_live = live_columns(a.mem_filled, a.n_rows, a.n_total);
+      if (n_live >= 0) n_cols = n_live;
+    }
     int g = 0;
     for (long long u = u_begin; u < u_end;) {
       const int rb = (int)(u / sc.T), ct0 = (int)(u % sc.T);
@@ -691,23 +714,23 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid
           ptx::tc_fence_before_sync();
           ptx::mbar_arrive(&bar_tempty[wg]);   // S_g is free again: the next MMA overlaps the work below
         }
-        const bool masked = (col0 + BN > a.n_total) || (col0 < rblk0 + TBM && rblk0 < col0 + BN);
+        const bool masked = (col0 + BN > n_cols) || (col0 < rblk0 + TBM && rblk0 < col0 + BN);
         const int cc = ch * CW;                // first tile column of this thread
         const int32_t* lab_s = lab_ring[slot] + cc;
         const float* nrm_s = nrm_ring[UNI ? slot : 0] + cc;
         if (masked) {
-          fwd_chunk<SIM, UNI, MINE, true, PLIN>(r0, col0 + cc, gi, a.n_total, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
-          fwd_chunk<SIM, UNI, MINE, true, PLIN>(r1, col0 + cc + 32, gi, a.n_total, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
+          fwd_chunk<SIM, UNI, MINE, true, PLIN>(r0, col0 + cc, gi, n_cols, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
+          fwd_chunk<SIM, UNI, MINE, true, PLIN>(r1, col0 + cc + 32, gi, n_cols, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
           if constexpr (NCH == 1) {
-            fwd_chunk<SIM, UNI, MINE, true, PLIN>(r2, col0 + 64, gi, a.n_total, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
-            fwd_chunk<SIM, UNI, MINE, true, PLIN>(r3, col0 + 96, gi, a.n_total, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
+            fwd_chunk<SIM, UNI, MINE, true, PLIN>(r2, col0 + 64, gi, n_cols, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
+            fwd_chunk<SIM, UNI, MINE, true, PLIN>(r3, col0 + 96, gi, n_cols, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
           }
         } else {
-          fwd_chunk<SIM, UNI, MINE, false, PLIN>(r0, col0 + cc, gi, a.n_total, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
-          fwd_chunk<SIM, UNI, MINE, false, PLIN>(r1, col0 + cc + 32, gi, a.n_total, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
+          fwd_chunk<SIM, UNI, MINE, false, PLIN>(r0, col0 + cc, gi, n_cols, lab_r, nrm_r, lab_s, nrm_s, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr);
+          fwd_chunk<SIM, UNI, MINE, false, PLIN>(r1, col0 + cc + 32, gi, n_cols, lab_r, nrm_r, lab_s + 32, nrm_s + 32, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 32);
           if constexpr (NCH == 1) {
-            fwd_chunk<SIM, UNI, MINE, false, PLIN>(r2, col0 + 64, gi, a.n_total, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
-            fwd_chunk<SIM, UNI, MINE, false, PLIN>(r3, col0 + 96, gi, a.n_total, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
+            fwd_chunk<SIM, UNI, MINE, false, PLIN>(r2, col0 + 64, gi, n_cols, lab_r, nrm_r, lab_s + 64, nrm_s + 64, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 64);
+            fwd_chunk<SIM, UNI, MINE, false, PLIN>(r3, col0 + 96, gi, n_cols, lab_r, nrm_r, lab_s + 96, nrm_s + 96, a.c1, c0, a.ut2, st, ms, wl_v, wl_i, lane, K, taddr + 96);
           }
         }
         if (MINE) {   // candidates re-read S from tensor memory: release the buffer only now
@@ -750,6 +773,17 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid
   ptx::tc_fence_before_sync();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc<512>(tmem);
+}
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
+__global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_kernel(const __grid_constant__ CUtensorMap tmap,
+                                                                    const __nv_bfloat16* __restrict__ z, TcFwdArgs a) {
+  tc_fwd_sweep<SIM, UNI, MINE, NCH, PLIN, false>(tmap, z, a);
+}
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
+__global__ void __launch_bounds__(tc_threads(NCH), 1) tc_fwd_live_kernel(const __grid_constant__ CUtensorMap tmap,
+                                                                         const __nv_bfloat16* __restrict__ z,
+                                                                         TcFwdArgs a) {
+  tc_fwd_sweep<SIM, UNI, MINE, NCH, PLIN, true>(tmap, z, a);
 }
 
 // merge the column splits into row statistics + loss partial sums
@@ -794,6 +828,8 @@ __global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishAr
   // final fixed maximum (all columns seen): records of an earlier phase may carry a smaller one and are rescaled
   const float M = fixmax_from_bits(*a.nrm2_max, a.m_limit);
   const float c0 = -a.c1 * M, m_tau = M * a.inv_tau;
+  const int n_live = live_columns(a.mem_filled, a.n_rows, a.n_total);
+  const int n_cols = n_live < 0 ? a.n_total : n_live;
   if (lr < a.n_rows) {
     float sum_all = 0.f, sum_pos_s = 0.f, wsum = 0.f, sum_pos_e = 0.f;
     const int npos = label_table_count(a.hkeys, a.hcounts, a.hmask, a.lab_pad[a.row_offset + lr]) - 1;
@@ -820,7 +856,7 @@ __global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishAr
         sum_pos_e = fmaf(rec[4], scale, sum_pos_e);
       }
     if (plin) sum_pos_s = posdot_s[threadIdx.x] - a.nrm_pad[a.row_offset + lr];   // minus the self term z_i . z_i
-    const int nneg = a.n_total - 1 - npos;
+    const int nneg = n_cols - 1 - npos;
     const float lse = logf(sum_all) + m_tau;   // fixed maximum M/tau folded back in
     const float pos_mean = npos > 0 ? (sum_pos_s * a.inv_tau) / (float)npos : 0.f;
     float lse_m = lse;
@@ -870,6 +906,7 @@ __global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishAr
       if (nneg > 0 && a.topk >= 1) { l_mined = (double)(lse_m - pos_mean); c_mined = 1.0; }
     }
     w = (double)wsum;
+    if (n_live < 0) { l_full = l_mined = w = NAN; c_full = 1.0; }   // fill level out of range: NaN loss
   }
   // |A_f|, |A_m| of the GLOBAL batch from the class-size table (it holds every column by now): a class of
   // size c contributes its c rows to A_f when c >= 2 and to A_m when also c < N (some negative exists).
@@ -885,7 +922,7 @@ __global__ void __launch_bounds__(128) tc_fwd_merge_kernel(TcFwdArgs a, FinishAr
       const int c = a.hcounts[h];
       if (c >= 2) {
         g_full += (double)c;
-        if (c < a.n_total && a.topk >= 1) g_mined += (double)c;
+        if (c < n_cols && a.topk >= 1) g_mined += (double)c;
       }
     }
   }
@@ -910,10 +947,11 @@ struct RowMine {  // the same for this thread's row
   int thr_idx;
 };
 
-template <int SIM, bool UNI, bool MINE, bool MASKED, int NQ, bool PLIN>
+// MASKED: the tile holds the diagonal or (LIVE) absent columns [n_cols, n_total); both get H = 0
+template <int SIM, bool UNI, bool MINE, bool MASKED, int NQ, bool PLIN, bool LIVE>
 __device__ __forceinline__ void bwd_chunk(const uint32_t (&r)[4 * NQ], uint32_t (&hw)[2 * NQ], int gj0, int gi, int lab_r,
                                           float A_r, float B_r, float nrm_r, float cu, float c0, const ColVecs& cv,
-                                          const RowMine& rm, const TcBwdArgs& a) {
+                                          const RowMine& rm, const TcBwdArgs& a, int n_cols) {
   if constexpr (SIM == SUPCON_COSINE && !MINE && !MASKED) {
     // packed pairs: exponent arguments, A_i + A_j and the product, two columns per instruction
     const f32x2 c1p = pk2(a.c1, a.c1), c0p = pk2(c0, c0), Arp = pk2(A_r, A_r);
@@ -995,7 +1033,7 @@ __device__ __forceinline__ void bwd_chunk(const uint32_t (&r)[4 * NQ], uint32_t 
       if (!PLIN && labs[e] == lab_r) v -= B_r + Bs[e];   // PLIN: the reduce kernel adds the positives' term
       if (SIM == SUPCON_GEODESIC) v *= geodesic_slope_fast(c);
       if (UNI) v = fmaf(-cu, ex2f(-a.ut2 * fmaxf(nrm_r + njs[e] - 2.f * c, 0.f)), v);
-      if (MASKED) v = (gj0 + 4 * q + e == gi) ? 0.f : v;
+      if (MASKED) v = (gj0 + 4 * q + e == gi || (LIVE && gj0 + 4 * q + e >= n_cols)) ? 0.f : v;
       h[e] = v;
     }
     __nv_bfloat162 p0 = __floats2bfloat162_rn(h[0], h[1]);
@@ -1033,9 +1071,10 @@ __device__ __forceinline__ int bwd_col_tile(const TcBwdArgs& a, int ct) {
 // Later in round 2 the chain itself got shorter instead -- the positives' term left the loop (PLIN) and the fp32
 // arithmetic went to packed pairs: 1433 M -> ~930 M instructions, tensor pipe 73.5 % -> 80.9 %, 3.19 -> 2.87 ms
 // (profiles/r02_fwd_pos_by_linearity.md, r02_packed_pairs_ab.md).
-template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
-__global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_kernel(const __grid_constant__ CUtensorMap tmapJ,
-                                                                    const __nv_bfloat16* __restrict__ z, TcBwdArgs a) {
+// LIVE: as in tc_fwd_sweep (tc_bwd_live_kernel only)
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN, bool LIVE>
+__device__ __forceinline__ void tc_bwd_sweep(const CUtensorMap& tmapJ, const __nv_bfloat16* __restrict__ z,
+                                             const TcBwdArgs& a) {
   static_assert(NCH == 1 || NCH == 2, "one or two threads per tile row");
   static_assert(!PLIN || (SIM == SUPCON_COSINE && !MINE), "positives by linearity: cosine, no mining");
   // positives by linearity: this kernel and its per-pair twin are both launched, the class count picks one
@@ -1053,6 +1092,7 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_kernel(const __grid
   __shared__ __align__(8) uint64_t bar_a, bar_full[STAGES], bar_empty[STAGES], bar_sfull[2], bar_hfull[2],
       bar_done, bar_dzfree, bar_col[RING];
   __shared__ uint32_t tmem_base_s;
+  __shared__ int n_cols_s;   // LIVE: live columns, in shared memory rather than in a register of the H warps
   __shared__ __align__(16) int32_t lab_ring[RING][BN];
   __shared__ __align__(16) float colA_ring[RING][BN], colB_ring[RING][BN];
   __shared__ __align__(16) float nrm_ring[UNI ? RING : 1][BN];
@@ -1072,6 +1112,10 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_kernel(const __grid
     for (int b = 0; b < RING; ++b) ptx::mbar_init(&bar_col[b], 1);
     ptx::fence_mbar_init();
     ptx::tma_prefetch_desc(&tmapJ);
+    if (LIVE) {
+      const int n_live = live_columns(a.mem_filled, a.n_rows, a.n_total);
+      n_cols_s = n_live < 0 ? a.n_total : n_live;
+    }
   }
   if (warp == 1) ptx::tmem_alloc<512>(&tmem_base_s);
   ptx::tc_fence_before_sync();
@@ -1222,18 +1266,18 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_kernel(const __grid
         cv0.thr_idx = thridx_ring[MINE ? slot : 0] + cc;
         cv1.lab = cv0.lab + 32; cv1.A = cv0.A + 32; cv1.B = cv0.B + 32; cv1.nrm = cv0.nrm + 32;
         cv1.Am = cv0.Am + 32; cv1.thr = cv0.thr + 32; cv1.thr_idx = cv0.thr_idx + 32;
-        const bool masked = (col0 < row0 + TBM && row0 < col0 + BN);
+        const bool masked = (col0 < row0 + TBM && row0 < col0 + BN) || (LIVE && col0 + BN > n_cols_s);
         if (masked) {
-          bwd_chunk<SIM, UNI, MINE, true, 8, PLIN>(r0, h0, col0 + cc, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv0, rm, a);
+          bwd_chunk<SIM, UNI, MINE, true, 8, PLIN, LIVE>(r0, h0, col0 + cc, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv0, rm, a, n_cols_s);
         } else {
-          bwd_chunk<SIM, UNI, MINE, false, 8, PLIN>(r0, h0, col0 + cc, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv0, rm, a);
+          bwd_chunk<SIM, UNI, MINE, false, 8, PLIN, LIVE>(r0, h0, col0 + cc, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv0, rm, a, n_cols_s);
         }
         if constexpr (NCH == 1) {
           uint32_t (&h1)[16] = *reinterpret_cast<uint32_t (*)[16]>(&hw[16]);
           if (masked) {
-            bwd_chunk<SIM, UNI, MINE, true, 8, PLIN>(r1, h1, col0 + 32, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv1, rm, a);
+            bwd_chunk<SIM, UNI, MINE, true, 8, PLIN, LIVE>(r1, h1, col0 + 32, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv1, rm, a, n_cols_s);
           } else {
-            bwd_chunk<SIM, UNI, MINE, false, 8, PLIN>(r1, h1, col0 + 32, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv1, rm, a);
+            bwd_chunk<SIM, UNI, MINE, false, 8, PLIN, LIVE>(r1, h1, col0 + 32, gi, lab_r, A_r, B_r, nrm_r, cu, c0, cv1, rm, a, n_cols_s);
           }
           ptx::tmem_st32(sbuf, hw);          // H(t): 64 bf16 = 32 packed columns over S(t)
         } else {
@@ -1275,6 +1319,17 @@ __global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_kernel(const __grid
   ptx::tc_fence_before_sync();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc<512>(tmem);
+}
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
+__global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_kernel(const __grid_constant__ CUtensorMap tmapJ,
+                                                                    const __nv_bfloat16* __restrict__ z, TcBwdArgs a) {
+  tc_bwd_sweep<SIM, UNI, MINE, NCH, PLIN, false>(tmapJ, z, a);
+}
+template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN>
+__global__ void __launch_bounds__(tc_threads(NCH), 1) tc_bwd_live_kernel(const __grid_constant__ CUtensorMap tmapJ,
+                                                                         const __nv_bfloat16* __restrict__ z,
+                                                                         TcBwdArgs a) {
+  tc_bwd_sweep<SIM, UNI, MINE, NCH, PLIN, true>(tmapJ, z, a);
 }
 
 // sum the column splits, add the uniformity diagonal term, scale by grad_out, convert
@@ -1323,7 +1378,7 @@ __global__ void __launch_bounds__(256) tc_bwd_reduce_kernel(TcBwdArgs a, const _
     acc.x = fmaf(wd, __bfloat162float(zr[0]), acc.x); acc.y = fmaf(wd, __bfloat162float(zr[1]), acc.y);
     acc.z = fmaf(wd, __bfloat162float(zr[2]), acc.z); acc.w = fmaf(wd, __bfloat162float(zr[3]), acc.w);
   }
-  const float g = grad_out ? *grad_out : 1.0f;
+  const float g = live_columns(a.mem_filled, a.n_rows, a.n_total) < 0 ? NAN : (grad_out ? *grad_out : 1.0f);
   acc.x *= g; acc.y *= g; acc.z *= g; acc.w *= g;
   if constexpr (sizeof(TO) == 4) {
     *reinterpret_cast<float4*>(out + (int64_t)lr * TD + 4 * c4) = acc;
@@ -1535,10 +1590,11 @@ constexpr int FWD_NCH = 2, BWD_NCH = 1, BWD_MINE_NCH = 2;
 template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN = false>
 static cudaError_t launch_fwd(const CUtensorMap& tm, const __nv_bfloat16* z, const TcFwdArgs& a, int ctas, size_t smem,
                               cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute(tc_fwd_kernel<SIM, UNI, MINE, NCH, PLIN>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  // a device fill level (supcon_forward_rows_memory): the sweep that masks absent columns
+  auto kernel = a.mem_filled ? tc_fwd_live_kernel<SIM, UNI, MINE, NCH, PLIN> : tc_fwd_kernel<SIM, UNI, MINE, NCH, PLIN>;
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  tc_fwd_kernel<SIM, UNI, MINE, NCH, PLIN><<<ctas, tc_threads(NCH), smem, st>>>(tm, z, a);
+  kernel<<<ctas, tc_threads(NCH), smem, st>>>(tm, z, a);
   return cudaGetLastError();
 }
 template <int SIM, bool UNI>
@@ -1578,6 +1634,7 @@ static TcFwdArgs fwd_base_args(const supcon_problem_t* p, const TcPlan& pl, char
   a.nrm_pad = reinterpret_cast<const float*>(ws + pl.off_nrm);
   a.part = reinterpret_cast<float*>(ws + pl.off_part);
   a.n_total = p->n_total; a.n_pad = pl.n_pad; a.row_offset = p->row_offset; a.n_rows = p->n_rows;
+  a.mem_filled = nullptr;
   a.rows_pad = pl.rows_pad; a.sched = pl.fwd_sched; a.topk = p->topk;
   a.inv_tau = 1.0f / p->tau;
   a.c1 = LOG2E / p->tau; a.c0 = -a.c1; a.ut2 = p->uni_t * LOG2E;   // c0: unit-row value; kernels derive theirs
@@ -1614,7 +1671,8 @@ static bool fwd_class_sums(const supcon_problem_t* p, int phase) {
 }
 
 int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, float* row_stats,
-               double* partials, float* loss_out, void* workspace, cudaStream_t stream, const char** err, int phase) {
+               double* partials, float* loss_out, void* workspace, cudaStream_t stream, const char** err, int phase,
+               const int32_t* mem_filled) {
   const TcPlan pl = tc_plan(p);
   char* ws = reinterpret_cast<char*>(workspace);
   CUtensorMap tm;
@@ -1644,7 +1702,7 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
                                                      reinterpret_cast<int32_t*>(ws + pl.off_lab),
                                                      reinterpret_cast<float*>(ws + pl.off_nrm), nrm2_max, count, j_lo,
                                                      ex_lo, ex_len, p->similarity == SUPCON_COSINE ? 1 : 0,
-                                                     batch_columns(p));
+                                                     batch_columns(p), mem_filled, p->n_rows);
     }
     // class-size table over the (real) columns of this phase
     int jn_lo = j_lo, jn_ex_lo = ex_lo, jn_ex_len = ex_len, jn_count = p->n_total;
@@ -1658,18 +1716,19 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
       tc_label_table_kernel<<<(jn_count + 255) / 256, 256, 0, stream>>>(
           labels_all, p->n_total, reinterpret_cast<unsigned long long*>(ws + pl.off_hkeys),
           reinterpret_cast<int*>(ws + pl.off_hcounts), pl.hash_size - 1, jn_lo, jn_ex_lo, jn_ex_len,
-          plin ? hids : nullptr, plin ? n_classes : nullptr);
+          plin ? hids : nullptr, plin ? n_classes : nullptr, mem_filled, p->n_rows);
     if (plin) {
       tc_class_sum_kernel<<<pl.csum_blocks, 256, 0, stream>>>(
           reinterpret_cast<const __nv_bfloat16*>(z_all), labels_all, p->n_total,
           reinterpret_cast<const unsigned long long*>(ws + pl.off_hkeys), hids, pl.hash_size - 1, n_classes,
-          reinterpret_cast<float*>(ws + pl.off_csum_part));
+          reinterpret_cast<float*>(ws + pl.off_csum_part), mem_filled, p->n_rows);
       tc_class_reduce_kernel<<<TC_CMAX, 1024, 0, stream>>>(reinterpret_cast<const float*>(ws + pl.off_csum_part),
                                                          pl.csum_blocks, n_classes,
                                                          reinterpret_cast<float*>(ws + pl.off_csum));
     }
   }
   TcFwdArgs a = fwd_base_args(p, pl, ws);
+  a.mem_filled = mem_filled;
   if (fwd_class_sums(p, phase)) {
     a.n_classes = reinterpret_cast<const int*>(ws) + WS_NCLASSES_WORD;
     a.hids = reinterpret_cast<const int*>(ws + pl.off_hids);
@@ -1702,10 +1761,10 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
 template <int SIM, bool UNI, bool MINE, int NCH, bool PLIN = false>
 static cudaError_t launch_bwd(const CUtensorMap& tmJ, const __nv_bfloat16* z, const TcBwdArgs& a, int ctas, size_t smem,
                               cudaStream_t st) {
-  cudaError_t e = cudaFuncSetAttribute(tc_bwd_kernel<SIM, UNI, MINE, NCH, PLIN>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  auto kernel = a.mem_filled ? tc_bwd_live_kernel<SIM, UNI, MINE, NCH, PLIN> : tc_bwd_kernel<SIM, UNI, MINE, NCH, PLIN>;
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  tc_bwd_kernel<SIM, UNI, MINE, NCH, PLIN><<<ctas, tc_threads(NCH), smem, st>>>(tmJ, z, a);
+  kernel<<<ctas, tc_threads(NCH), smem, st>>>(tmJ, z, a);
   return cudaGetLastError();
 }
 template <int SIM, bool UNI>
@@ -1725,7 +1784,7 @@ static cudaError_t launch_bwd_m(bool mine, const CUtensorMap& tmJ, const __nv_bf
 
 int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all, const float* stats,
                 const double* partials, const float* grad_out, void* dz_out, int dz_dtype, void* workspace,
-                cudaStream_t stream, const char** err, int phase) {
+                cudaStream_t stream, const char** err, int phase, const int32_t* mem_filled) {
   const TcPlan pl = tc_plan(p);
   char* ws = reinterpret_cast<char*>(workspace);
   CUtensorMap tmJ;
@@ -1745,7 +1804,7 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
                                                    reinterpret_cast<int32_t*>(ws + pl.off_lab),
                                                    reinterpret_cast<float*>(ws + pl.off_nrm),
                                                    reinterpret_cast<unsigned*>(ws + pl.off_scalars) + 8, pl.n_pad,
-                                                   0, 0x7fffffff, 0, 1, batch_columns(p));
+                                                   0, 0x7fffffff, 0, 1, batch_columns(p), mem_filled, p->n_rows);
   }
   // positives by linearity: single-phase cosine backward without mining, when the sweep is long enough.  Not with
   // SUPCON_FLAG_MEMORY_COLUMNS: -2 B_i (C[c] - z_i) assumes every same-class column j carries B_j = B_i, and a memory
@@ -1783,6 +1842,7 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
   pa.lab_pad = reinterpret_cast<int32_t*>(ws + pl.off_lab);
   pa.scalars = reinterpret_cast<float*>(ws + pl.off_scalars);
   pa.n_total = p->n_total; pa.n_pad = pl.n_pad; pa.topk = p->topk; pa.n_batch = batch_columns(p);
+  pa.n_rows = p->n_rows; pa.mem_filled = mem_filled;
   pa.tau = p->tau; pa.alpha = p->alpha; pa.lambda_uni = p->lambda_uni; pa.uni_t = p->uni_t;
   pa.hkeys = plin ? reinterpret_cast<const unsigned long long*>(ws + pl.off_hkeys) : nullptr;
   pa.hids = hids; pa.hmask = pl.hash_size - 1;
@@ -1797,6 +1857,7 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
   a.colAm = pa.colAm; a.colThr = pa.colThr; a.colThrIdx = pa.colThrIdx;
   a.dz_part = reinterpret_cast<float*>(ws + pl.off_part);
   a.n_total = p->n_total; a.n_pad = pl.n_pad; a.row_offset = p->row_offset; a.n_rows = p->n_rows;
+  a.mem_filled = mem_filled;
   a.rows_pad = pl.rows_pad; a.sched = pl.bwd_sched;
   a.sched_b.P = 0; a.sched_b.T = 1; a.sched_b.U = 1; a.sched_b.RB = 1; a.sched_b.NP = 1; a.sched_b.Tp = 1;
   a.slot_base_b = 0;

@@ -193,19 +193,27 @@ def with_flags(prob: _cabi.Problem, extra: int) -> _cabi.Problem:
 
 
 def forward_rows(z_all: torch.Tensor, labels_i32: torch.Tensor, prob: _cabi.Problem, want_loss: bool,
-                 keep_ws: bool = False):
+                 keep_ws: bool = False, mem_filled: Optional[torch.Tensor] = None):
     """Row-block forward. Returns (row_stats [n_rows,8] f32, partials [8] f64, loss or None) and, with
     ``keep_ws``, the workspace as a fourth item: handed to backward_rows(ws=...) untouched, it lets the backward
-    reuse the label table and class sums the forward built (SUPCON_FLAG_WS_FROM_FORWARD)."""
+    reuse the label table and class sums the forward built (SUPCON_FLAG_WS_FROM_FORWARD).
+    ``mem_filled``: a one-element int32 CUDA tensor, the fill level of a memory problem's columns
+    (supcon_forward_rows_memory); ``prob.n_total`` is then the capacity."""
     _require_cuda(z_all, "z")
     lib = _cabi.load()
     dev = z_all.device
     with _on(dev):
         stats, partials, loss = _stats_buffers(prob.n_rows, dev, want_loss)
         ws = workspace_for(prob, dev)
-        _cabi.check(lib.supcon_forward_rows(ctypes.byref(prob), _p(z_all), _p(labels_i32), _p(stats),
-                                            _p(partials), _p(loss), _p(ws), ws.numel(), _stream(dev)),
-                    "supcon_forward_rows")
+        if mem_filled is None:
+            _cabi.check(lib.supcon_forward_rows(ctypes.byref(prob), _p(z_all), _p(labels_i32), _p(stats),
+                                                _p(partials), _p(loss), _p(ws), ws.numel(), _stream(dev)),
+                        "supcon_forward_rows")
+        else:
+            _cabi.check(lib.supcon_forward_rows_memory(ctypes.byref(prob), _p(z_all), _p(labels_i32), _p(mem_filled),
+                                                       _p(stats), _p(partials), _p(loss), _p(ws), ws.numel(),
+                                                       _stream(dev)),
+                        "supcon_forward_rows_memory")
     if keep_ws:
         return stats, partials, loss, ws
     return stats, partials, loss
@@ -337,9 +345,11 @@ def backward_rows_remote(z_all, labels_i32, stats_all, partials_global, grad_out
 
 
 def backward_rows(z_all, labels_i32, stats_all, partials_global, grad_out, prob: _cabi.Problem,
-                  out_dtype=torch.float32, ws: Optional[torch.Tensor] = None) -> torch.Tensor:
+                  out_dtype=torch.float32, ws: Optional[torch.Tensor] = None,
+                  mem_filled: Optional[torch.Tensor] = None) -> torch.Tensor:
     """``ws``: the workspace forward_rows(..., keep_ws=True) returned for the SAME problem, untouched since (the
-    backward then reuses what the forward built there); None = a fresh one."""
+    backward then reuses what the forward built there); None = a fresh one.  ``mem_filled``: as in forward_rows
+    (supcon_backward_rows_memory)."""
     lib = _cabi.load()
     dev = z_all.device
     with _on(dev):
@@ -351,10 +361,16 @@ def backward_rows(z_all, labels_i32, stats_all, partials_global, grad_out, prob:
         g = None
         if grad_out is not None:
             g = grad_out.detach().reshape(()).to(device=dev, dtype=torch.float32)
-        _cabi.check(lib.supcon_backward_rows(ctypes.byref(prob), _p(z_all), _p(labels_i32), _p(stats_all),
-                                             _p(partials_global), _p(g), _p(dz), _dtype_id(dz), _p(ws),
-                                             ws.numel(), _stream(dev)),
-                    "supcon_backward_rows")
+        if mem_filled is None:
+            _cabi.check(lib.supcon_backward_rows(ctypes.byref(prob), _p(z_all), _p(labels_i32), _p(stats_all),
+                                                 _p(partials_global), _p(g), _p(dz), _dtype_id(dz), _p(ws),
+                                                 ws.numel(), _stream(dev)),
+                        "supcon_backward_rows")
+        else:
+            _cabi.check(lib.supcon_backward_rows_memory(ctypes.byref(prob), _p(z_all), _p(labels_i32), _p(mem_filled),
+                                                        _p(stats_all), _p(partials_global), _p(g), _p(dz),
+                                                        _dtype_id(dz), _p(ws), ws.numel(), _stream(dev)),
+                        "supcon_backward_rows_memory")
     return dz
 
 

@@ -329,7 +329,15 @@ class GraphedHeadStep:
     parameters and the optimizer state are put back afterwards, in place, so constructing the object does not
     train.  ``grad_sync`` (``GradSync``) is captured into the graph when given (NCCL collectives capture).
     Inputs are copied into the static buffers ``step.hs`` / ``step.labels`` unless they ARE those buffers (an
-    encoder that writes its output there saves the copy)."""
+    encoder that writes its output there saves the copy).
+
+    A ``loss_fn`` with a cross-batch ``memory`` (``MemorySupConLoss``) is captured at the memory's capacity and reads
+    its fill level and ring head on the device, so one graph serves the memory while it fills, once it is full and
+    as it wraps.  Construction and capture leave the memory's contents and state as they were (the warm-up and
+    the captured step enqueue nothing that stays).  Each replay enqueues its batch on the device and advances the
+    host ``filled`` / ``head`` by B, so ``memory.embeddings`` / ``memory.keys`` describe what the device holds.
+    The graphs of different alphas share that one memory.  Eager calls of the loss between replays stay valid as
+    long as the batch size does not grow (a larger batch reallocates the buffers the graphs use)."""
 
     def __init__(self, head, loss_fn, optimizer, hs_example: torch.Tensor, labels_example: torch.Tensor, *,
                  topk_neg: int = 32, max_grad_norm: float = 5.0, normalize: Optional[Callable] = None,
@@ -344,6 +352,7 @@ class GraphedHeadStep:
         self.normalize, self.grad_sync, self.warmup = normalize, grad_sync, max(1, int(warmup))
         self.hs = hs_example.detach().clone()
         self.labels = labels_example.detach().clone().long()
+        self.memory = getattr(loss_fn, "memory", None)
         self._graphs = {}
 
     def _eager(self, alpha: float) -> torch.Tensor:
@@ -362,10 +371,13 @@ class GraphedHeadStep:
         buffers = [b.detach().clone() for b in self.head.buffers()]
         state = {p: {k: (v.detach().clone() if torch.is_tensor(v) else v) for k, v in st.items()}
                  for p, st in self.optimizer.state.items()}
-        return params, buffers, state
+        memory = self.memory.snapshot() if self.memory is not None else None
+        return params, buffers, state, memory
 
     def _restore(self, snap) -> None:
-        params, buffers, state = snap
+        params, buffers, state, memory = snap
+        if self.memory is not None:
+            self.memory.restore(memory)
         with torch.no_grad():
             for p, saved in zip(self.head.parameters(), params):
                 p.copy_(saved)
@@ -395,8 +407,9 @@ class GraphedHeadStep:
         self.optimizer.zero_grad(set_to_none=True)
         with torch.cuda.graph(graph, capture_error_mode="thread_local"):
             loss = self._eager(alpha)
+        push = self.memory.last_push if self.memory is not None else None   # what each replay enqueues
         self._restore(snap)
-        return graph, loss
+        return graph, loss, push
 
     def __call__(self, hs: torch.Tensor, labels: torch.Tensor, alpha: float = 0.0) -> torch.Tensor:
         if hs.shape != self.hs.shape or labels.shape != self.labels.shape:
@@ -405,10 +418,12 @@ class GraphedHeadStep:
         key = float(alpha)
         if key not in self._graphs:
             self._graphs[key] = self._capture(key)
-        graph, loss = self._graphs[key]
+        graph, loss, push = self._graphs[key]
         if hs.data_ptr() != self.hs.data_ptr():         # producers may write straight into step.hs / step.labels
             self.hs.copy_(hs, non_blocking=True)
         if labels.data_ptr() != self.labels.data_ptr():
             self.labels.copy_(labels, non_blocking=True)
         graph.replay()
+        if push is not None:
+            self.memory.advance_host(*push)
         return loss
