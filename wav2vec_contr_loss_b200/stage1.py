@@ -39,7 +39,18 @@ from . import functional as Fn
 
 __all__ = ["alpha_for_epoch", "BalancedBatchSampler", "RunningLoss", "GradSync", "embed", "call_loss",
            "normalized_supcon_loss",
-           "train_one_epoch", "evaluate", "setup_distributed", "export_embeddings", "GraphedHeadStep"]
+           "train_one_epoch", "evaluate", "setup_distributed", "export_embeddings", "GraphedHeadStep",
+           "CachedBatchStep", "train_one_epoch_cached"]
+
+_CACHED_BATCH = ("CachedBatchStep", "train_one_epoch_cached")
+
+
+def __getattr__(name):
+    """Re-export of ``cached_batch`` (global batches of k micro-batches), which itself builds on this module."""
+    if name in _CACHED_BATCH:
+        from . import cached_batch
+        return getattr(cached_batch, name)
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")
 
 
 # ------------------------------------------------------------------------------------------------ schedule
