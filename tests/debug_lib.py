@@ -24,6 +24,8 @@ def load():
         lib.supcon_debug_plan.argtypes = [P, c_void_p, c_int32]
         lib.supcon_debug_ffma_plan.restype = c_int32
         lib.supcon_debug_ffma_plan.argtypes = [P, c_void_p, c_int32]
+        lib.supcon_debug_route.restype = c_int32
+        lib.supcon_debug_route.argtypes = [P, c_void_p, c_void_p, c_int32]
         lib.supcon_debug_sched.restype = c_int32
         lib.supcon_debug_sched.argtypes = [c_int32, c_int32, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                            c_void_p]
@@ -34,3 +36,17 @@ def load():
 def check(rc, what):
     if rc != 0:
         raise RuntimeError(f"{what} failed (code {rc}): {load().supcon_debug_last_error().decode()}")
+
+
+SMALL, MID, TENSOR, TILED = range(4)        # routes of supcon_debug_route
+ROUTE_NAMES = ("small", "mid", "tensor", "tiled")
+
+
+def route(prob, z):
+    """supcon_debug_route of ``prob`` for rows at ``z`` (a tensor, or an address: only its alignment matters):
+    dict(loss_and_grad, forward_rows, backward_rows, cluster, vec, fwd_class_sums, bwd_class_sums)"""
+    out = (c_int32 * 7)()
+    addr = z if isinstance(z, int) else z.data_ptr()
+    check(load().supcon_debug_route(ctypes.byref(prob), c_void_p(addr), out, 7), "supcon_debug_route")
+    keys = ("loss_and_grad", "forward_rows", "backward_rows", "cluster", "vec", "fwd_class_sums", "bwd_class_sums")
+    return dict(zip(keys, list(out)))

@@ -64,14 +64,6 @@ bool owns_all_anchors(const supcon_problem_t* p) {
 
 constexpr uint32_t FLAG_TC_FWD_ONLY = SUPCON_FLAG_DEBUG_TC_FWD_ONLY, FLAG_TC_BWD_ONLY = SUPCON_FLAG_DEBUG_TC_BWD_ONLY;
 
-bool use_tc(const supcon_problem_t* p, bool backward) {
-  if (p->flags & SUPCON_FLAG_FORCE_EXACT) return false;
-  if (!tc_supported(p)) return false;
-  if (backward && (p->flags & FLAG_TC_FWD_ONLY)) return false;
-  if (!backward && (p->flags & FLAG_TC_BWD_ONLY)) return false;
-  return true;
-}
-
 size_t workspace_need(const supcon_problem_t* p) {
   size_t need = ffma_workspace_bytes(p);
   if (!(p->flags & SUPCON_FLAG_FORCE_EXACT) && tc_supported(p)) {
@@ -83,26 +75,10 @@ size_t workspace_need(const supcon_problem_t* p) {
 
 bool needs_mining(const supcon_problem_t* p) { return p->alpha != 0.f && p->topk >= 1; }
 
-bool vec_ok(const void* z, const supcon_problem_t* p) {
-  size_t al = p->z_dtype == SUPCON_BF16 ? 8 : 16;
-  return (p->d % 4 == 0) && ((reinterpret_cast<uintptr_t>(z) % al) == 0);
-}
-
 // A memory problem (SUPCON_FLAG_MEMORY_COLUMNS) never takes the single-launch kernels, not even with an empty memory
 // (n_rows == n_total): its forward and backward are separate calls, and the backward's hard-negative membership test
 // (s == thr) needs the forward's Gram arithmetic, which the small / mid kernels do not share with the tiled ones.
 constexpr uint32_t NOT_SINGLE_LAUNCH = SUPCON_FLAG_NO_SMALL | SUPCON_FLAG_FORCE_TENSOR | SUPCON_FLAG_MEMORY_COLUMNS;
-
-bool use_small(const supcon_problem_t* p, const void* z) {
-  if (p->flags & NOT_SINGLE_LAUNCH) return false;
-  return small_supported(p, z);
-}
-// mid-size single-launch kernel: exact fp32 math, so it yields to the tensor path where that one is eligible
-bool use_mid(const supcon_problem_t* p, const void* z) {
-  if (p->flags & NOT_SINGLE_LAUNCH) return false;
-  if (use_tc(p, false) || use_tc(p, true)) return false;
-  return !small_supported(p, z) && mid_supported(p, z);
-}
 
 SmallArgs make_small(const supcon_problem_t* p, const void* z, const int32_t* labels) {
   SmallArgs s;
@@ -220,6 +196,40 @@ __global__ void normalize_bwd_kernel(const TZ* __restrict__ z, const float* __re
 }
 
 }  // namespace
+
+// ---- route predicates (declared in supcon_internal.h: the test library's route report calls these same ones) ----
+bool use_tc(const supcon_problem_t* p, bool backward) {
+  if (p->flags & SUPCON_FLAG_FORCE_EXACT) return false;
+  if (!tc_supported(p)) return false;
+  if (backward && (p->flags & FLAG_TC_FWD_ONLY)) return false;
+  if (!backward && (p->flags & FLAG_TC_BWD_ONLY)) return false;
+  return true;
+}
+
+bool vec_ok(const void* z, const supcon_problem_t* p) {
+  size_t al = p->z_dtype == SUPCON_BF16 ? 8 : 16;
+  return (p->d % 4 == 0) && ((reinterpret_cast<uintptr_t>(z) % al) == 0);
+}
+
+bool use_small(const supcon_problem_t* p, const void* z) {
+  if (p->flags & NOT_SINGLE_LAUNCH) return false;
+  return small_supported(p, z);
+}
+// supcon_forward_rows' statistics feed a supcon_backward_rows on the tiled kernels, whose hard-negative membership test
+// (s > thr || s == thr && j <= thr_idx) recomputes s as one fma chain over k.  Below 129 rows the small kernel sums
+// each dot product from 2 or 4 k-slices, so its threshold can differ from the tiled s in the last bit and drop the K-th
+// negative from the backward's set: a mining forward there runs on the tiled kernels.  (The mid kernel's chain is the
+// tiled kernels' own; supcon_loss_and_grad's small-kernel backward reuses its own Gram.)
+bool use_small_forward_rows(const supcon_problem_t* p, const void* z) {
+  return use_small(p, z) && !needs_mining(p);
+}
+// mid-size single-launch kernel: exact fp32 math, so it yields to the tensor path where that one is eligible
+bool use_mid(const supcon_problem_t* p, const void* z) {
+  if (p->flags & NOT_SINGLE_LAUNCH) return false;
+  if (use_tc(p, false) || use_tc(p, true)) return false;
+  return !small_supported(p, z) && mid_supported(p, z);
+}
+
 }  // namespace supcon
 
 using namespace supcon;
@@ -253,7 +263,7 @@ int forward_rows(const supcon_problem_t* p, const void* z_all, const int32_t* la
   if (loss_out && !owns_all_anchors(p))
     return fail(SUPCON_E_INVALID, "loss_out needs a rank that owns every row; use supcon_finalize");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (use_small(p, z_all)) {   // whole batch on this rank, small N: one launch, statistics + loss only
+  if (use_small_forward_rows(p, z_all)) {   // whole batch on this rank, small N: one launch, statistics + loss only
     SmallArgs s = make_small(p, z_all, labels_all);
     s.row_stats = row_stats; s.partials = partials; s.loss_out = loss_out;
     cudaError_t es = small_launch(s, st);

@@ -1,6 +1,6 @@
 // TEST-ONLY entry points (libsupcon_b200_test.so; declared in csrc/supcon_debug.h, not in the public header):
-// the tcgen05/TMA building-block diagnostic, host-side introspection of the tensor path's work distribution and
-// of the exact path's column splits and top-K selection rounds.
+// the tcgen05/TMA building-block diagnostic, host-side introspection of the tensor path's work distribution, of
+// the exact path's column splits and top-K selection rounds, and of the route the dispatcher picks.
 // The product library libsupcon_b200.so does not contain this file.
 #include <string>
 
@@ -52,6 +52,34 @@ int supcon_debug_ffma_plan(const supcon_problem_t* p, int32_t* out, int32_t n_ou
   out[1] = pl.bwd_splits;
   out[2] = pl.kcap;
   out[3] = mine ? (p->topk + pl.kcap - 1) / pl.kcap : 0;
+  return 0;
+}
+
+int supcon_debug_route(const supcon_problem_t* p, const void* z, int32_t* out, int32_t n_out) {
+  if (int rc = dbg_validate(p)) return rc;
+  if (!out || n_out < 7) return dbg_fail(SUPCON_E_INVALID, "bad arguments to supcon_debug_route");
+  enum { SMALL = 0, MID = 1, TENSOR = 2, TILED = 3 };
+  int devices = 0;
+  if (cudaGetDeviceCount(&devices) != cudaSuccess) { cudaGetLastError(); devices = 0; }
+  const bool mid = use_mid(p, z);
+  int cluster = -1;
+  if (devices > 0) {
+    cluster = 0;
+    if (mid) {   // the occupancy query of pick_cluster, for a problem the mid kernel can hold
+      SmallArgs s{};
+      s.n = p->n_total; s.d = p->d; s.z_dtype = p->z_dtype; s.dz_dtype = SUPCON_F32;
+      cluster = mid_cluster_ctas(s);
+    }
+  }
+  // forward of supcon_loss_and_grad and supcon_forward_rows (the single-launch kernels also do the former's backward)
+  const int after_small = mid && cluster != 0 ? MID : use_tc(p, false) ? TENSOR : TILED;
+  out[0] = use_small(p, z) ? SMALL : after_small;
+  out[1] = use_small_forward_rows(p, z) ? SMALL : after_small;
+  out[2] = use_tc(p, true) ? TENSOR : TILED;
+  out[3] = cluster;
+  out[4] = vec_ok(z, p) ? 1 : 0;
+  out[5] = use_tc(p, false) && tc_class_sums(p, false, 0) ? 1 : 0;
+  out[6] = use_tc(p, true) && tc_class_sums(p, true, 0) ? 1 : 0;
   return 0;
 }
 

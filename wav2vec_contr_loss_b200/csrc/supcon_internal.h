@@ -204,6 +204,21 @@ cudaError_t small_launch(const SmallArgs& a, cudaStream_t stream);
 //      co-schedule the cluster (the caller then uses the tiled kernels) ----
 bool mid_supported(const supcon_problem_t* p, const void* z);
 cudaError_t mid_launch(const SmallArgs& a, cudaStream_t stream, bool* taken);
+// The route decisions below are shared with the test library's route report (supcon_debug_route); hidden, so that
+// the product library exports nothing beyond its C ABI on their account.
+#define SUPCON_HIDDEN __attribute__((visibility("hidden")))
+// CTAs of the mid kernel's cluster on the current device: 16, 8, or 0 when it cannot take a.n rows
+SUPCON_HIDDEN int mid_cluster_ctas(const SmallArgs& a);
+
+// ---- route predicates of the dispatcher (supcon_api.cu) ----
+SUPCON_HIDDEN bool use_tc(const supcon_problem_t* p, bool backward);     // tensor-core forward / backward
+SUPCON_HIDDEN bool use_small(const supcon_problem_t* p, const void* z);  // single-launch small kernel
+SUPCON_HIDDEN bool use_small_forward_rows(const supcon_problem_t* p, const void* z);   // ... in supcon_forward_rows
+SUPCON_HIDDEN bool use_mid(const supcon_problem_t* p, const void* z);    // mid kernel (if mid_cluster_ctas > 0)
+SUPCON_HIDDEN bool vec_ok(const void* z, const supcon_problem_t* p);     // tiled kernels: vector row loads
+// tensor path: positives by linearity (class sums) in the forward / backward of this phase; the device still falls
+// back to per-pair sums above TC_CMAX classes
+SUPCON_HIDDEN bool tc_class_sums(const supcon_problem_t* p, bool backward, int phase);
 
 // ---- producer of z: compression head up to the Linear layer, fused with the time mean (supcon_head.cu) ----
 struct HeadPoolArgs {

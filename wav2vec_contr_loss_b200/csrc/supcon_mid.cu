@@ -370,15 +370,21 @@ bool mid_supported(const supcon_problem_t* p, const void* z) {
   return mid_layout(p->n_total, p->d, MMAXR).total <= 224 * 1024;
 }
 
+int mid_cluster_ctas(const SmallArgs& a) {
+  typedef __nv_bfloat16 bf;
+  if (a.z_dtype == SUPCON_BF16) return a.dz_dtype == SUPCON_BF16 ? pick_cluster<bf, bf>(a) : pick_cluster<bf, float>(a);
+  return a.dz_dtype == SUPCON_BF16 ? pick_cluster<float, bf>(a) : pick_cluster<float, float>(a);
+}
+
 cudaError_t mid_launch(const SmallArgs& a, cudaStream_t stream, bool* taken) {
   *taken = false;
+  const int sc = mid_cluster_ctas(a);
+  if (sc == 0) return cudaSuccess;
+  const size_t smem = mid_layout(a.n, a.d, (a.n + sc - 1) / sc).total;
   cudaError_t e = cudaSuccess;
 #define SUPCON_MID(TI, TO)                                                          \
   do {                                                                              \
-    const int sc = pick_cluster<TI, TO>(a);                                         \
-    if (sc == 0) return cudaSuccess;                                                \
-    const int rows = (a.n + sc - 1) / sc;                                           \
-    e = launch_mid<TI, TO>(a, sc, mid_layout(a.n, a.d, rows).total, stream, false, nullptr); \
+    e = launch_mid<TI, TO>(a, sc, smem, stream, false, nullptr);                    \
     *taken = (e == cudaSuccess);                                                    \
   } while (0)
   if (a.z_dtype == SUPCON_BF16) {

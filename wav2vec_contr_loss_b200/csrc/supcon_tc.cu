@@ -1664,8 +1664,11 @@ constexpr long long PLIN_MIN_PAIRS = 1ll << 30;
 static bool plin_size_ok(const supcon_problem_t* p) {
   return (long long)p->n_rows * p->n_total >= PLIN_MIN_PAIRS || (p->flags & SUPCON_FLAG_CLASS_SUMS);
 }
-// positives by linearity in the forward: whole forward (one phase), cosine, no mining, large enough
-static bool fwd_class_sums(const supcon_problem_t* p, int phase) {
+// positives by linearity: single phase, cosine, no mining, large enough.  Not in a backward with
+// SUPCON_FLAG_MEMORY_COLUMNS: -2 B_i (C[c] - z_i) assumes every same-class column j carries B_j = B_i, and a memory
+// column carries B_j = 0 (the forward's class sums stay valid: they only need the positives' similarities)
+bool tc_class_sums(const supcon_problem_t* p, bool backward, int phase) {
+  if (backward && (p->flags & SUPCON_FLAG_MEMORY_COLUMNS)) return false;
   return phase == 0 && p->similarity == SUPCON_COSINE && !(p->alpha != 0.f && p->topk >= 1) &&
          !(p->flags & SUPCON_FLAG_NO_CLASS_SUMS) && plin_size_ok(p);
 }
@@ -1709,7 +1712,7 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
     if (phase == 1) { jn_count = p->n_rows; jn_ex_lo = jn_lo + jn_count; jn_ex_len = p->n_total; }
     if (phase == 2) { jn_count = p->n_total - p->n_rows; jn_ex_len = p->n_rows; }
     // positives by linearity: whole forward (one phase), cosine, no mining
-    const bool plin = fwd_class_sums(p, phase);
+    const bool plin = tc_class_sums(p, false, phase);
     int* n_classes = reinterpret_cast<int*>(ws) + WS_NCLASSES_WORD;
     int* hids = reinterpret_cast<int*>(ws + pl.off_hids);
     if (jn_count > 0)
@@ -1729,7 +1732,7 @@ int tc_forward(const supcon_problem_t* p, const void* z_all, const int32_t* labe
   }
   TcFwdArgs a = fwd_base_args(p, pl, ws);
   a.mem_filled = mem_filled;
-  if (fwd_class_sums(p, phase)) {
+  if (tc_class_sums(p, false, phase)) {
     a.n_classes = reinterpret_cast<const int*>(ws) + WS_NCLASSES_WORD;
     a.hids = reinterpret_cast<const int*>(ws + pl.off_hids);
     a.csum = reinterpret_cast<const float*>(ws + pl.off_csum);
@@ -1806,16 +1809,11 @@ int tc_backward(const supcon_problem_t* p, const void* z_all, const int32_t* lab
                                                    reinterpret_cast<unsigned*>(ws + pl.off_scalars) + 8, pl.n_pad,
                                                    0, 0x7fffffff, 0, 1, batch_columns(p), mem_filled, p->n_rows);
   }
-  // positives by linearity: single-phase cosine backward without mining, when the sweep is long enough.  Not with
-  // SUPCON_FLAG_MEMORY_COLUMNS: -2 B_i (C[c] - z_i) assumes every same-class column j carries B_j = B_i, and a memory
-  // column carries B_j = 0 (the forward's class sums stay valid: they only need the positives' similarities)
-  const bool mine_b = p->alpha != 0.f && p->topk >= 1;
-  const bool plin = phase == 0 && p->similarity == SUPCON_COSINE && !mine_b &&
-                    !(p->flags & (SUPCON_FLAG_NO_CLASS_SUMS | SUPCON_FLAG_MEMORY_COLUMNS)) && plin_size_ok(p);
+  const bool plin = tc_class_sums(p, true, phase);
   int* n_classes = reinterpret_cast<int*>(ws) + WS_NCLASSES_WORD;
   int* hids = reinterpret_cast<int*>(ws + pl.off_hids);
   // the forward of the same problem left its label table and class sums in this very workspace (caller's promise)
-  const bool from_fwd = plin && (p->flags & SUPCON_FLAG_WS_FROM_FORWARD) && fwd_class_sums(p, 0) &&
+  const bool from_fwd = plin && (p->flags & SUPCON_FLAG_WS_FROM_FORWARD) && tc_class_sums(p, false, 0) &&
                         !(p->flags & (SUPCON_FLAG_DEBUG_TC_FWD_ONLY | SUPCON_FLAG_DEBUG_TC_BWD_ONLY));
   if (plin && !from_fwd) {
     e = cudaMemsetAsync(workspace, 0, 256, stream);
