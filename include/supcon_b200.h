@@ -308,6 +308,27 @@ int supcon_head_pool_backward(const float* hs, int32_t batch, int32_t layers, in
                               float dropout_p, float negative_slope, const uint64_t* rng_state,
                               const float* dpooled /*[batch][feat]*/, float* dhs_out, void* stream);
 
+/* Training the head on a frozen encoder from a store of its layer means, m[c] = (1/K) sum_k hs[c][k] (feat, frames)
+ * fp32 per clip: everything of the head after the layer mean is recomputed from m every epoch, fresh dropout masks
+ * included, without running the encoder again.
+ *
+ * supcon_head_layer_mean_typed writes store_rows[b] = (1/K) sum_k hs[b][k] for the batch's hs (hs_dtype as above);
+ * store_rows is the store's row of the batch's first clip (store + slot0 * feat * frames).  The sum is in fp32 over
+ * k = 0..K-1 in order, then times (1/K): the arithmetic of supcon_head_pool_forward_typed, bit for bit.
+ *
+ * supcon_head_store_pool_forward is supcon_head_pool_forward_typed on the store rows idx[0..batch) (int64, on the
+ * device, so a captured graph takes new indices every replay):
+ *   pooled[b][f] = (1/T) sum_t LeakyReLU(Dropout(store[idx[b]][f][t]))
+ * The dropout mask of element (b, f, t) is the one supcon_head_pool_forward_typed draws for batch position b with the
+ * same rng_state, so pooled_out equals bit for bit that call's on hs[idx[0..batch)].  An index outside [0, n_store)
+ * writes NaN into its pooled row; the other rows are unaffected.  The store is a constant: there is no backward. */
+int supcon_head_layer_mean_typed(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                                 int32_t frames, float* store_rows /*[batch][feat][frames]*/, void* stream);
+int supcon_head_store_pool_forward(const float* store /*[n_store][feat][frames]*/, int64_t n_store, int32_t feat,
+                                   int32_t frames, const int64_t* idx /*[batch]*/, int32_t batch, float dropout_p,
+                                   float negative_slope, const uint64_t* rng_state,
+                                   float* pooled_out /*[batch][feat]*/, void* stream);
+
 /* Diagnostics used by the parity tests: hard-negative index sets of the owned
  * rows, recomputed from the statistics (index ascending, -1 padded). */
 int supcon_topk_indices(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,

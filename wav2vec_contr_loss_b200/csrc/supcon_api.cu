@@ -614,6 +614,36 @@ int supcon_head_pool_backward(const float* hs, int32_t batch, int32_t layers, in
                        dhs_out, stream, "supcon_head_pool_backward");
 }
 
+int supcon_head_layer_mean_typed(const void* hs, int32_t hs_dtype, int32_t batch, int32_t layers, int32_t feat,
+                                 int32_t frames, float* store_rows, void* stream) {
+  const char* who = "supcon_head_layer_mean_typed";
+  if (int rc = head_pool_check(hs, hs_dtype, batch, layers, feat, frames, 0.f, store_rows, who)) return rc;
+  HeadPoolArgs a{};
+  a.hs = hs; a.hs_dtype = hs_dtype;
+  a.B = batch; a.K = layers; a.F = feat; a.T = frames;
+  cudaError_t e = head_layer_mean(a, store_rows, reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "head_layer_mean_kernel");
+  return 0;
+}
+
+int supcon_head_store_pool_forward(const float* store, int64_t n_store, int32_t feat, int32_t frames,
+                                   const int64_t* idx, int32_t batch, float dropout_p, float negative_slope,
+                                   const uint64_t* rng_state, float* pooled_out, void* stream) {
+  const char* who = "supcon_head_store_pool_forward";
+  if (!idx) return fail(SUPCON_E_INVALID, "NULL idx passed to %s", who);
+  if (n_store < 1) return fail(SUPCON_E_INVALID, "%s: bad store size %lld", who, (long long)n_store);
+  if (int rc = head_pool_check(store, SUPCON_F32, batch, 1, feat, frames, dropout_p, pooled_out, who)) return rc;
+  HeadPoolArgs a{};
+  a.hs = store; a.pooled = pooled_out;
+  a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
+  a.B = batch; a.F = feat; a.T = frames;
+  a.dropout_p = dropout_p; a.negative_slope = negative_slope;
+  cudaError_t e = head_store_pool_forward(a, reinterpret_cast<const long long*>(idx), n_store,
+                                          reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "head_store_pool_fwd_kernel");
+  return 0;
+}
+
 int supcon_peer_push(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0, const void* src1,
                      size_t bytes1, uint64_t dst_off1, int32_t flag_id, int32_t wait_flag_id, int32_t include_self,
                      void* stream) {

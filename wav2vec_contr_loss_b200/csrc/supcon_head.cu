@@ -7,7 +7,9 @@
 // The Linear layer and the time mean are both linear, so  mean_t seq = W * (mean_t x) + bias : the per-frame
 // GEMM over (B*T, F) collapses to one over (B, F), and everything left of it is ONE pass over hs:
 //     pooled[b,f] = (1/T) sum_t LeakyReLU(Dropout((1/K) sum_k hs[b,k,f,t]))
-// This file is that pass (forward) and its transpose (backward, only needed when the encoder is fine-tuned).
+// This file is that pass (forward) and its transpose (backward, only needed when the encoder is fine-tuned), and the
+// same forward split in two for a frozen encoder: the layer mean written once per clip into a store, and the rest of
+// the pass run on store rows gathered by index every epoch.
 // HBM-bound: the algorithmic traffic is hs read once (B*K*F*T elements: 1.3 GB of fp32 or 0.65 GB of bf16 at B = 64,
 // K = 25, F = 1024, T = 199), the output is B*F*4 bytes.
 //
@@ -131,10 +133,24 @@ __device__ __forceinline__ void layer_sum(const RunView<E>& v, int K, int e, flo
   for (; k < K; ++k) add_pack<E, VEC>(acc, __ldg(reinterpret_cast<const pack_t*>(p + (long long)k * v.plane)));
 }
 
-template <typename E, int VEC>
-__global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolArgs a) {
+// VEC consecutive fp32 values of a stored layer-mean row, starting at run offset e
+template <int VEC>
+__device__ __forceinline__ void stored_mean(const RunView<float>& v, int e, float (&x)[VEC]) {
+  if constexpr (VEC == 4) {
+    const float4 q = __ldg(reinterpret_cast<const float4*>(v.base + e));
+    x[0] = q.x; x[1] = q.y; x[2] = q.z; x[3] = q.w;
+  } else {
+    x[0] = __ldg(v.base + e);
+  }
+}
+
+// The forward of one block after its run is located: Dropout, LeakyReLU, and the time mean of each row.  STORED
+// picks the source of the layer mean: false = the K-layer sum of hs times 1/K, true = a row of a layer-mean store
+// (head_layer_mean_kernel wrote exactly that product, so both sources give the same bits).  The mask index is
+// always the batch position's, so a gathered batch draws the mask of the same batch read from hs.
+template <typename E, int VEC, bool STORED>
+__device__ __forceinline__ void pool_run(const HeadPoolArgs& a, const RunView<E>& v) {
   extern __shared__ float act[];                      // [rows*T] activated values of this block's run
-  const RunView<E> v = run_of_block<E>(a);
   const bool drop = a.dropout_p > 0.f && a.rng_state != nullptr;
   unsigned long long seed = 0, offset = 0;
   if (drop) { seed = a.rng_state[0]; offset = a.rng_state[1]; }
@@ -143,10 +159,12 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolAr
 
   for (int e = threadIdx.x * VEC; e < v.len; e += HP_THREADS * VEC) {
     float acc[VEC];
-    layer_sum<E, VEC>(v, a.K, e, acc);
+    if constexpr (STORED) stored_mean<VEC>(v, e, acc);
+    else layer_sum<E, VEC>(v, a.K, e, acc);
 #pragma unroll
     for (int i = 0; i < VEC; ++i) {
-      float x = acc[i] * inv_k;
+      float x = acc[i];
+      if constexpr (!STORED) x *= inv_k;
       if (drop) x *= dropout_scale(seed, offset, v.first_elem + e + i, a.dropout_p, keep_scale);
       act[e + i] = x > 0.f ? x : x * a.negative_slope;
     }
@@ -160,6 +178,50 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolAr
     for (int t = lane; t < a.T; t += 32) s += act[r * a.T + t];
     s = warp_sum(s);
     if (lane == 0) a.pooled[(long long)v.b * a.F + v.f0 + r] = s * inv_t;
+  }
+}
+
+template <typename E, int VEC>
+__global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolArgs a) {
+  pool_run<E, VEC, false>(a, run_of_block<E>(a));
+}
+
+// Gather-pool: batch position b reads store row idx[b] (a.hs = the (n_store, F, T) store, a.K = 1; idx on the
+// device, so a captured graph takes new rows every replay).  A row index
+// outside [0, n_store) poisons pooled row b with NaN (the other rows stay exact); nothing is read for it.
+template <int VEC>
+__global__ void __launch_bounds__(HP_THREADS, 4) head_store_pool_fwd_kernel(HeadPoolArgs a,
+                                                                         const long long* __restrict__ idx,
+                                                                         long long n_store) {
+  RunView<float> v = run_of_block<float>(a);
+  const long long row = idx[v.b];
+  if (row < 0 || row >= n_store) {
+    for (int r = threadIdx.x; r < v.rows; r += HP_THREADS) a.pooled[(long long)v.b * a.F + v.f0 + r] = NAN;
+    return;
+  }
+  v.base = static_cast<const float*>(a.hs) + row * v.plane + (long long)v.f0 * a.T;
+  pool_run<float, VEC, true>(a, v);
+}
+
+// store_rows[b] = (1/K) sum_k hs[b, k] in fp32, layers added in order: the layer mean of head_pool_fwd_kernel, bit
+// for bit, written out instead of activated
+template <typename E, int VEC>
+__global__ void __launch_bounds__(HP_THREADS, 4) head_layer_mean_kernel(HeadPoolArgs a, float* __restrict__ rows) {
+  const RunView<E> v = run_of_block<E>(a);
+  const float inv_k = 1.0f / (float)a.K;
+  float* out = rows + (long long)v.b * v.plane + (long long)v.f0 * a.T;
+  for (int e = threadIdx.x * VEC; e < v.len; e += HP_THREADS * VEC) {
+    float acc[VEC];
+    layer_sum<E, VEC>(v, a.K, e, acc);
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) acc[i] *= inv_k;
+    if constexpr (VEC == 1) {
+      out[e] = acc[0];
+    } else {
+#pragma unroll
+      for (int i = 0; i < VEC; i += 4)
+        *reinterpret_cast<float4*>(out + e + i) = make_float4(acc[i], acc[i + 1], acc[i + 2], acc[i + 3]);
+    }
   }
 }
 
@@ -244,6 +306,37 @@ cudaError_t head_pool_forward(HeadPoolArgs a, cudaStream_t stream) {
   } else {
     head_pool_fwd_kernel<float, 1><<<grid, HP_THREADS, smem, stream>>>(a);
   }
+  return cudaGetLastError();
+}
+
+cudaError_t head_layer_mean(HeadPoolArgs a, float* rows, cudaStream_t stream) {
+  a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
+  if (a.rows_per_block < 1) return cudaErrorInvalidValue;
+  dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
+  if (a.hs_dtype == SUPCON_BF16) {
+    if (vector_ok(a, rows, 8))
+      head_layer_mean_kernel<__nv_bfloat16, 8><<<grid, HP_THREADS, 0, stream>>>(a, rows);
+    else
+      head_layer_mean_kernel<__nv_bfloat16, 1><<<grid, HP_THREADS, 0, stream>>>(a, rows);
+  } else if (vector_ok(a, rows, 4)) {
+    head_layer_mean_kernel<float, 4><<<grid, HP_THREADS, 0, stream>>>(a, rows);
+  } else {
+    head_layer_mean_kernel<float, 1><<<grid, HP_THREADS, 0, stream>>>(a, rows);
+  }
+  return cudaGetLastError();
+}
+
+cudaError_t head_store_pool_forward(HeadPoolArgs a, const long long* idx, long long n_store, cudaStream_t stream) {
+  a.K = 1;
+  a.hs_dtype = SUPCON_F32;
+  a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
+  if (a.rows_per_block < 1) return cudaErrorInvalidValue;
+  dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
+  const size_t smem = (size_t)a.rows_per_block * a.T * sizeof(float);
+  if (vector_ok(a, nullptr, 4))
+    head_store_pool_fwd_kernel<4><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+  else
+    head_store_pool_fwd_kernel<1><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
   return cudaGetLastError();
 }
 

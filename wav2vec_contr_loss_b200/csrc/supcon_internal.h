@@ -232,6 +232,9 @@ struct HeadPoolArgs {
 };
 int head_pool_rows_per_block(int F, int T, int hs_dtype);
 cudaError_t head_pool_forward(HeadPoolArgs a, cudaStream_t stream);
+cudaError_t head_layer_mean(HeadPoolArgs a, float* rows, cudaStream_t stream);   // rows [B][F][T] fp32
+// a.hs = the fp32 (n_store, F, T) store, idx = [B] store row of each batch position
+cudaError_t head_store_pool_forward(HeadPoolArgs a, const long long* idx, long long n_store, cudaStream_t stream);
 cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, void* dhs, cudaStream_t stream);
 
 // tcgen05 building-block diagnostic (supcon_tc_debug.cu)

@@ -143,6 +143,20 @@ class FusedCompressionHead(nn.Module):
         """(B, D) == ``CompressionModule(hs).mean(dim=-1)`` of the reference."""
         return F.linear(self.pooled_features(hs), self.mlp3.weight, self.mlp3.bias)
 
+    def pooled_features_from_store(self, store, idx: torch.Tensor) -> torch.Tensor:
+        """``pooled_features`` of the clips in slots ``idx`` (device int64) of a ``feature_store.LayerMeanStore``:
+        the same values, bit for bit, and the same dropout stream (one offset per call in train mode)."""
+        p = self.dropout_head.p if self.training else 0.0
+        if p > 0.0:
+            out = store.pool(idx, p, self.activation_head.negative_slope, self.rng_state)
+            self.rng_state[1] += 1
+            return out
+        return store.pool(idx, 0.0, self.activation_head.negative_slope, None)
+
+    def pooled_embedding_from_store(self, store, idx: torch.Tensor) -> torch.Tensor:
+        """(B, D) == ``pooled_embedding`` of the clips in slots ``idx`` of the store."""
+        return F.linear(self.pooled_features_from_store(store, idx), self.mlp3.weight, self.mlp3.bias)
+
     def forward(self, hs: torch.Tensor) -> torch.Tensor:
         """(B, D, 1): the reference's (B, D, T) sequence already averaged over T, so that the unchanged caller's
         ``seq.mean(dim=-1)`` (stage1_utils.py:123) is the pooled embedding."""

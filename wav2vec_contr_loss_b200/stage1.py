@@ -9,6 +9,9 @@ What the reference keeps in ``stage1_utils.py`` around ``loss_fn(z, labels, topk
   setup_distributed      torchrun / SLURM rendezvous           stage1_utils.py:156-172
   export_embeddings      (N, 256) fp32 .npy for Stage 2        extract_stage1_embeddings.py:148-163,220-231
   GraphedHeadStep        head+loss+optimizer step, one CUDA graph replay (no reference counterpart)
+  train_one_epoch_from_store / evaluate_from_store
+                         the epoch functions for a frozen encoder whose layer means are held in a
+                         feature_store.LayerMeanStore (train_stage1_from_emb.py trains from disk features)
 
 Same names, positional arguments and return values, so a caller that does
 ``from stage1_utils import train_one_epoch`` can import it from here instead.  What differs, on purpose:
@@ -40,7 +43,7 @@ from . import functional as Fn
 __all__ = ["alpha_for_epoch", "BalancedBatchSampler", "RunningLoss", "GradSync", "embed", "call_loss",
            "normalized_supcon_loss",
            "train_one_epoch", "evaluate", "setup_distributed", "export_embeddings", "GraphedHeadStep",
-           "CachedBatchStep", "train_one_epoch_cached"]
+           "CachedBatchStep", "train_one_epoch_cached", "train_one_epoch_from_store", "evaluate_from_store"]
 
 _CACHED_BATCH = ("CachedBatchStep", "train_one_epoch_cached")
 
@@ -263,6 +266,67 @@ def evaluate(encoder, head, loss_fn, loader, device, cfg, *, normalize: Optional
     return running.average()
 
 
+# ------------------------------------------------------------------ epochs from a store of layer means
+
+def _check_store_cfg(cfg, training: bool) -> None:
+    if getattr(cfg, "finetune_encoder", False):
+        raise ValueError("cfg.finetune_encoder is set: the encoder's output changes every step, so a store of its "
+                         "layer means would be stale; train with train_one_epoch")
+    if training and getattr(cfg, "use_rawboost", False):
+        raise ValueError("cfg.use_rawboost is set: augmented waveforms give new hidden states every epoch, so a store "
+                         "of layer means would be stale; train with train_one_epoch")
+
+
+def _store_indices(store, batch, device) -> torch.Tensor:
+    rows = [int(i) for i in batch]
+    if rows and not (0 <= min(rows) and max(rows) < store.filled):
+        raise IndexError(f"batch indices must lie in [0, {store.filled}), the clips in the store")
+    return torch.tensor(rows, dtype=torch.int64).to(device, non_blocking=True)
+
+
+def _store_embed(head, store, idx: torch.Tensor, normalize: Optional[Callable] = None) -> torch.Tensor:
+    return (normalize or Fn.l2_normalize)(head.pooled_embedding_from_store(store, idx))
+
+
+def train_one_epoch_from_store(head, loss_fn, store, batches, optimizer, device, epoch, cfg, *,
+                               normalize: Optional[Callable] = None, max_grad_norm: float = 5.0):
+    """``train_one_epoch`` for a frozen encoder whose layer means are in ``store``
+    (``feature_store.build_layer_mean_store``): no encoder call.  ``batches`` are index lists into the store, e.g.
+    the batches of the same ``BalancedBatchSampler``; labels are gathered from the store on the device.  ``head`` is
+    a ``FusedCompressionHead``.  With the same batches, seeds and dropout stream the epoch is ``train_one_epoch``'s
+    whenever the encoder's output for a clip does not depend on its batch mates.  Returns ``(mean loss, alpha)``.
+    Raises when ``cfg.finetune_encoder`` or ``cfg.use_rawboost`` is set: the store would be stale."""
+    _check_store_cfg(cfg, training=True)
+    head.train()
+    alpha = alpha_for_epoch(epoch, cfg)
+    running = RunningLoss(device)
+    for batch in batches:
+        idx = _store_indices(store, batch, device)
+        z = _store_embed(head, store, idx, normalize)
+        loss = call_loss(loss_fn, z, store.labels_of(idx), cfg.topk_neg, alpha)
+
+        optimizer.zero_grad(set_to_none=True)
+        loss.backward()
+        torch.nn.utils.clip_grad_norm_(head.parameters(), max_grad_norm)
+        optimizer.step()
+        running.add(loss)
+    return running.average(), alpha
+
+
+@torch.no_grad()
+def evaluate_from_store(head, loss_fn, store, batches, device, cfg, *, normalize: Optional[Callable] = None):
+    """``evaluate`` over index lists into a store of layer means (alpha = 0, no graph).  Raises when
+    ``cfg.finetune_encoder`` is set."""
+    _check_store_cfg(cfg, training=False)
+    head.eval()
+    running = RunningLoss(device)
+    for batch in batches:
+        idx = _store_indices(store, batch, device)
+        running.add(call_loss(loss_fn, _store_embed(head, store, idx, normalize), store.labels_of(idx),
+                              cfg.topk_neg, 0.0))
+    return running.average()
+
+
 # --------------------------------------------------------------------------------------------- rendezvous
 
 def setup_distributed(backend: str = "nccl"):
@@ -348,11 +412,16 @@ class GraphedHeadStep:
     the captured step enqueue nothing that stays).  Each replay enqueues its batch on the device and advances the
     host ``filled`` / ``head`` by B, so ``memory.embeddings`` / ``memory.keys`` describe what the device holds.
     The graphs of different alphas share that one memory.  Eager calls of the loss between replays stay valid as
-    long as the batch size does not grow (a larger batch reallocates the buffers the graphs use)."""
+    long as the batch size does not grow (a larger batch reallocates the buffers the graphs use).
 
-    def __init__(self, head, loss_fn, optimizer, hs_example: torch.Tensor, labels_example: torch.Tensor, *,
-                 topk_neg: int = 32, max_grad_norm: float = 5.0, normalize: Optional[Callable] = None,
-                 grad_sync: Optional[Callable] = None, warmup: int = 3):
+    ``store=`` (a ``feature_store.LayerMeanStore``, head = ``FusedCompressionHead``) captures the step of
+    ``train_one_epoch_from_store`` instead: the graph gathers and pools the store rows ``step.idx`` and their labels,
+    so the static input is the (B,) int64 index vector.  Pass an index example in place of ``hs_example``, no
+    labels, and call ``step(idx, alpha=alpha)``: a replay copies ``idx`` and runs."""
+
+    def __init__(self, head, loss_fn, optimizer, hs_example: torch.Tensor, labels_example: Optional[torch.Tensor] = None,
+                 *, topk_neg: int = 32, max_grad_norm: float = 5.0, normalize: Optional[Callable] = None,
+                 grad_sync: Optional[Callable] = None, warmup: int = 3, store=None):
         if hs_example.device.type != "cuda":
             raise RuntimeError("GraphedHeadStep needs CUDA tensors (there is no CPU path)")
         for group in optimizer.param_groups:
@@ -361,14 +430,30 @@ class GraphedHeadStep:
         self.head, self.loss_fn, self.optimizer = head, loss_fn, optimizer
         self.topk_neg, self.max_grad_norm = int(topk_neg), float(max_grad_norm)
         self.normalize, self.grad_sync, self.warmup = normalize, grad_sync, max(1, int(warmup))
-        self.hs = hs_example.detach().clone()
-        self.labels = labels_example.detach().clone().long()
+        self.store = store
+        if store is not None:
+            if labels_example is not None:
+                raise ValueError("with store= the labels come from the store: pass no labels_example")
+            if hs_example.dim() != 1 or hs_example.dtype != torch.int64:
+                raise ValueError("with store= the example is the (B,) int64 vector of store rows")
+            self.idx = hs_example.detach().clone()
+            self.hs = self.labels = None
+        else:
+            if labels_example is None:
+                raise ValueError("GraphedHeadStep needs labels_example (or store=)")
+            self.hs = hs_example.detach().clone()
+            self.labels = labels_example.detach().clone().long()
         self.memory = getattr(loss_fn, "memory", None)
         self._graphs = {}
 
     def _eager(self, alpha: float) -> torch.Tensor:
-        z = embed(self.head, self.hs, self.normalize)
-        loss = call_loss(self.loss_fn, z, self.labels, self.topk_neg, alpha)
+        if self.store is not None:
+            z = _store_embed(self.head, self.store, self.idx, self.normalize)
+            labels = self.store.labels_of(self.idx)
+        else:
+            z = embed(self.head, self.hs, self.normalize)
+            labels = self.labels
+        loss = call_loss(self.loss_fn, z, labels, self.topk_neg, alpha)
         self.optimizer.zero_grad(set_to_none=True)
         loss.backward()
         if self.grad_sync is not None:
@@ -405,7 +490,7 @@ class GraphedHeadStep:
                         v.zero_()                   # state created by the warm-up: back to its initial zeros
 
     def _capture(self, alpha: float):
-        dev = self.hs.device
+        dev = (self.idx if self.store is not None else self.hs).device
         snap = self._snapshot()
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
@@ -422,18 +507,28 @@ class GraphedHeadStep:
         self._restore(snap)
         return graph, loss, push
 
-    def __call__(self, hs: torch.Tensor, labels: torch.Tensor, alpha: float = 0.0) -> torch.Tensor:
-        if hs.shape != self.hs.shape or labels.shape != self.labels.shape:
+    def __call__(self, hs: torch.Tensor, labels: Optional[torch.Tensor] = None, alpha: float = 0.0) -> torch.Tensor:
+        if self.store is not None:
+            if labels is not None or hs.shape != self.idx.shape or hs.dtype != torch.int64:
+                raise ValueError(f"GraphedHeadStep was captured for store rows of shape {tuple(self.idx.shape)} "
+                                 f"(int64, no labels), got {hs.dtype} {tuple(hs.shape)}"
+                                 + (" and labels" if labels is not None else ""))
+        elif labels is None or hs.shape != self.hs.shape or labels.shape != self.labels.shape:
             raise ValueError(f"GraphedHeadStep was captured for hs {tuple(self.hs.shape)} / labels "
-                             f"{tuple(self.labels.shape)}, got {tuple(hs.shape)} / {tuple(labels.shape)}")
+                             f"{tuple(self.labels.shape)}, got {tuple(hs.shape)} / "
+                             f"{tuple(labels.shape) if labels is not None else None}")
         key = float(alpha)
         if key not in self._graphs:
             self._graphs[key] = self._capture(key)
         graph, loss, push = self._graphs[key]
-        if hs.data_ptr() != self.hs.data_ptr():         # producers may write straight into step.hs / step.labels
-            self.hs.copy_(hs, non_blocking=True)
-        if labels.data_ptr() != self.labels.data_ptr():
-            self.labels.copy_(labels, non_blocking=True)
+        if self.store is not None:
+            if hs.data_ptr() != self.idx.data_ptr():
+                self.idx.copy_(hs, non_blocking=True)
+        else:
+            if hs.data_ptr() != self.hs.data_ptr():     # producers may write straight into step.hs / step.labels
+                self.hs.copy_(hs, non_blocking=True)
+            if labels.data_ptr() != self.labels.data_ptr():
+                self.labels.copy_(labels, non_blocking=True)
         graph.replay()
         if push is not None:
             self.memory.advance_host(*push)
