@@ -329,6 +329,20 @@ int supcon_head_store_pool_forward(const float* store /*[n_store][feat][frames]*
                                    float negative_slope, const uint64_t* rng_state,
                                    float* pooled_out /*[batch][feat]*/, void* stream);
 
+/* supcon_head_sharded_store_pool_forward is supcon_head_store_pool_forward on a store sharded over the n_ranks GPUs
+ * of one node: row i lives in the shard of rank i % n_ranks, at local row i / n_ranks (64-bit offsets).
+ * shard_bases[r] (a device table of n_ranks addresses, so a captured graph reads it at every replay) is the address
+ * of rank r's shard in the calling process: its own allocation, or a peer's mapped into it (CUDA IPC, symmetric
+ * memory).  Every base must be 16-byte aligned and every shard hold ceil(n_store / n_ranks) rows of feat * frames
+ * floats.  pooled_out equals bit for bit supcon_head_store_pool_forward's on a single store of the same n_store rows;
+ * an index outside [0, n_store) writes NaN into its pooled row and reads nothing.  Returns SUPCON_E_INVALID, before
+ * any CUDA call, for n_ranks < 1, n_store < n_ranks, a NULL table and the arguments the single-store call rejects. */
+int supcon_head_sharded_store_pool_forward(const uint64_t* shard_bases /*device [n_ranks]*/, int32_t n_ranks,
+                                           int64_t n_store, int32_t feat, int32_t frames,
+                                           const int64_t* idx /*[batch]*/, int32_t batch, float dropout_p,
+                                           float negative_slope, const uint64_t* rng_state,
+                                           float* pooled_out /*[batch][feat]*/, void* stream);
+
 /* Diagnostics used by the parity tests: hard-negative index sets of the owned
  * rows, recomputed from the statistics (index ascending, -1 padded). */
 int supcon_topk_indices(const supcon_problem_t* p, const void* z_all, const int32_t* labels_all,

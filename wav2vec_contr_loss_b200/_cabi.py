@@ -35,7 +35,7 @@ EXPORTS = (
     "supcon_peer_push", "supcon_peer_wait", "supcon_peer_end_step", "supcon_label_keys",
     "supcon_head_pool_forward_typed", "supcon_head_pool_backward_typed",
     "supcon_forward_rows_memory", "supcon_backward_rows_memory",
-    "supcon_head_layer_mean_typed", "supcon_head_store_pool_forward",
+    "supcon_head_layer_mean_typed", "supcon_head_store_pool_forward", "supcon_head_sharded_store_pool_forward",
 )
 
 
@@ -138,6 +138,10 @@ def load():
     lib.supcon_head_store_pool_forward.restype = c_int32
     lib.supcon_head_store_pool_forward.argtypes = [c_void_p, ctypes.c_int64, c_int32, c_int32, c_void_p, c_int32,
                                                    c_float, c_float, c_void_p, c_void_p, c_void_p]
+    lib.supcon_head_sharded_store_pool_forward.restype = c_int32
+    lib.supcon_head_sharded_store_pool_forward.argtypes = [c_void_p, c_int32, ctypes.c_int64, c_int32, c_int32,
+                                                           c_void_p, c_int32, c_float, c_float, c_void_p, c_void_p,
+                                                           c_void_p]
     lib.supcon_label_keys.restype = c_int32
     lib.supcon_label_keys.argtypes = [c_void_p, c_int32, c_int32, c_void_p, c_void_p]
     PP = POINTER(Peer)

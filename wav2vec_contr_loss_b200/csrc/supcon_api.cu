@@ -644,6 +644,28 @@ int supcon_head_store_pool_forward(const float* store, int64_t n_store, int32_t 
   return 0;
 }
 
+int supcon_head_sharded_store_pool_forward(const uint64_t* shard_bases, int32_t n_ranks, int64_t n_store,
+                                           int32_t feat, int32_t frames, const int64_t* idx, int32_t batch,
+                                           float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                           float* pooled_out, void* stream) {
+  const char* who = "supcon_head_sharded_store_pool_forward";
+  if (!idx) return fail(SUPCON_E_INVALID, "NULL idx passed to %s", who);
+  if (n_ranks < 1) return fail(SUPCON_E_INVALID, "%s: bad rank count %d", who, n_ranks);
+  if (n_store < n_ranks)
+    return fail(SUPCON_E_INVALID, "%s: bad store size %lld for %d ranks", who, (long long)n_store, n_ranks);
+  if (int rc = head_pool_check(shard_bases, SUPCON_F32, batch, 1, feat, frames, dropout_p, pooled_out, who)) return rc;
+  HeadPoolArgs a{};
+  a.pooled = pooled_out;
+  a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
+  a.B = batch; a.F = feat; a.T = frames;
+  a.dropout_p = dropout_p; a.negative_slope = negative_slope;
+  cudaError_t e = head_sharded_store_pool_forward(a, reinterpret_cast<const unsigned long long*>(shard_bases),
+                                                  n_ranks, reinterpret_cast<const long long*>(idx), n_store,
+                                                  reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return cuda_fail(e, "head_sharded_store_pool_fwd_kernel");
+  return 0;
+}
+
 int supcon_peer_push(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0, const void* src1,
                      size_t bytes1, uint64_t dst_off1, int32_t flag_id, int32_t wait_flag_id, int32_t include_self,
                      void* stream) {

@@ -9,7 +9,7 @@
 //     pooled[b,f] = (1/T) sum_t LeakyReLU(Dropout((1/K) sum_k hs[b,k,f,t]))
 // This file is that pass (forward) and its transpose (backward, only needed when the encoder is fine-tuned), and the
 // same forward split in two for a frozen encoder: the layer mean written once per clip into a store, and the rest of
-// the pass run on store rows gathered by index every epoch.
+// the pass run on store rows gathered by index every epoch (one GPU's store, or one sharded over a node's GPUs).
 // HBM-bound: the algorithmic traffic is hs read once (B*K*F*T elements: 1.3 GB of fp32 or 0.65 GB of bf16 at B = 64,
 // K = 25, F = 1024, T = 199), the output is B*F*4 bytes.
 //
@@ -186,21 +186,41 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolAr
   pool_run<E, VEC, false>(a, run_of_block<E>(a));
 }
 
-// Gather-pool: batch position b reads store row idx[b] (a.hs = the (n_store, F, T) store, a.K = 1; idx on the
-// device, so a captured graph takes new rows every replay).  A row index
-// outside [0, n_store) poisons pooled row b with NaN (the other rows stay exact); nothing is read for it.
-template <int VEC>
-__global__ void __launch_bounds__(HP_THREADS, 4) head_store_pool_fwd_kernel(HeadPoolArgs a,
-                                                                         const long long* __restrict__ idx,
-                                                                         long long n_store) {
+// Gather-pool: batch position b reads store row idx[b] (idx on the device, so a captured graph takes new rows every
+// replay; a.K = 1).  row_of(row, plane) is the address of a row's (F, T) plane.  A row index outside [0, n_store)
+// poisons pooled row b with NaN (the other rows stay exact); nothing is read for it.
+template <int VEC, typename RowOf>
+__device__ __forceinline__ void store_pool_run(const HeadPoolArgs& a, const long long* __restrict__ idx,
+                                               long long n_store, RowOf row_of) {
   RunView<float> v = run_of_block<float>(a);
   const long long row = idx[v.b];
   if (row < 0 || row >= n_store) {
     for (int r = threadIdx.x; r < v.rows; r += HP_THREADS) a.pooled[(long long)v.b * a.F + v.f0 + r] = NAN;
     return;
   }
-  v.base = static_cast<const float*>(a.hs) + row * v.plane + (long long)v.f0 * a.T;
+  v.base = row_of(row, v.plane) + (long long)v.f0 * a.T;
   pool_run<float, VEC, true>(a, v);
+}
+
+// a.hs = the (n_store, F, T) store
+template <int VEC>
+__global__ void __launch_bounds__(HP_THREADS, 4) head_store_pool_fwd_kernel(HeadPoolArgs a,
+                                                                         const long long* __restrict__ idx,
+                                                                         long long n_store) {
+  store_pool_run<VEC>(a, idx, n_store, [&](long long row, long long plane) {
+    return static_cast<const float*>(a.hs) + row * plane;
+  });
+}
+
+// The store sharded over n_ranks GPUs: row i is local row i / n_ranks of the shard at bases[i % n_ranks], a device
+// address in this process (its own shard, or a peer's mapped over NVLink)
+template <int VEC>
+__global__ void __launch_bounds__(HP_THREADS, 4) head_sharded_store_pool_fwd_kernel(
+    HeadPoolArgs a, const unsigned long long* __restrict__ bases, int n_ranks, const long long* __restrict__ idx,
+    long long n_store) {
+  store_pool_run<VEC>(a, idx, n_store, [&](long long row, long long plane) {
+    return reinterpret_cast<const float*>(bases[row % n_ranks]) + (row / n_ranks) * plane;
+  });
 }
 
 // store_rows[b] = (1/K) sum_k hs[b, k] in fp32, layers added in order: the layer mean of head_pool_fwd_kernel, bit
@@ -337,6 +357,22 @@ cudaError_t head_store_pool_forward(HeadPoolArgs a, const long long* idx, long l
     head_store_pool_fwd_kernel<4><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
   else
     head_store_pool_fwd_kernel<1><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+  return cudaGetLastError();
+}
+
+cudaError_t head_sharded_store_pool_forward(HeadPoolArgs a, const unsigned long long* bases, int n_ranks,
+                                            const long long* idx, long long n_store, cudaStream_t stream) {
+  a.hs = nullptr;           // the shard bases are on the device: 16-byte alignment is the caller's promise
+  a.K = 1;
+  a.hs_dtype = SUPCON_F32;
+  a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
+  if (a.rows_per_block < 1) return cudaErrorInvalidValue;
+  dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
+  const size_t smem = (size_t)a.rows_per_block * a.T * sizeof(float);
+  if (vector_ok(a, nullptr, 4))
+    head_sharded_store_pool_fwd_kernel<4><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx, n_store);
+  else
+    head_sharded_store_pool_fwd_kernel<1><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx, n_store);
   return cudaGetLastError();
 }
 

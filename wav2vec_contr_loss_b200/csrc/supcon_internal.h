@@ -235,6 +235,9 @@ cudaError_t head_pool_forward(HeadPoolArgs a, cudaStream_t stream);
 cudaError_t head_layer_mean(HeadPoolArgs a, float* rows, cudaStream_t stream);   // rows [B][F][T] fp32
 // a.hs = the fp32 (n_store, F, T) store, idx = [B] store row of each batch position
 cudaError_t head_store_pool_forward(HeadPoolArgs a, const long long* idx, long long n_store, cudaStream_t stream);
+// the same on a store sharded over n_ranks GPUs: row i at bases[i % n_ranks] + (i / n_ranks) * F * T (device table)
+cudaError_t head_sharded_store_pool_forward(HeadPoolArgs a, const unsigned long long* bases, int n_ranks,
+                                            const long long* idx, long long n_store, cudaStream_t stream);
 cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, void* dhs, cudaStream_t stream);
 
 // tcgen05 building-block diagnostic (supcon_tc_debug.cu)

@@ -16,15 +16,23 @@ the rows of a batch and pools them with the arithmetic and the dropout masks of 
 same batch read from hs.  Training from the store therefore walks the trajectory of ``stage1.train_one_epoch``
 whenever the encoder's output for a clip does not depend on the other clips of its batch.
 
+``ShardedLayerMeanStore`` / ``build_sharded_layer_mean_store`` split the store over the GPUs of one node: slot i
+lives on rank i % R, each rank encodes only its own clips, and ``pool`` reads the other ranks' rows through peer
+memory (``supcon_head_sharded_store_pool_forward``), with the same bits as ``LayerMeanStore.pool``.
+
 Preconditions: frozen encoder, no waveform augmentation, the same crop / pad of each clip in every epoch.  The rows
 are fp32 (a bf16 store would round the mean and lose that equality).  There is no backward: the store is a constant.
 """
+import socket
+
 import torch
+import torch.distributed as dist
 
 from . import _cabi
 from . import functional as Fn
 
-__all__ = ["LayerMeanStore", "build_layer_mean_store"]
+__all__ = ["LayerMeanStore", "build_layer_mean_store", "ShardedLayerMeanStore", "build_sharded_layer_mean_store",
+           "shard_slots"]
 
 
 class LayerMeanStore:
@@ -38,12 +46,9 @@ class LayerMeanStore:
         if n < 1 or feat < 1 or frames < 1:
             raise ValueError(f"bad store shape ({n}, {feat}, {frames})")
         device = torch.device(device)
-        need = store_bytes(n, feat, frames)
-        if device.type == "cuda":
-            free, _ = torch.cuda.mem_get_info(device)
-            if need > free:
-                raise MemoryError(f"a store of {n} clips x ({feat}, {frames}) fp32 takes {need / 1e9:.2f} GB; "
-                                  f"{free / 1e9:.2f} GB are free on {device}")
+        too_big = _fit_error(n, feat, frames, device, store_bytes(n, feat, frames))
+        if too_big:
+            raise MemoryError(too_big)
         self.rows = torch.empty((n, feat, frames), dtype=torch.float32, device=device)
         self.labels = torch.full((n,), -1, dtype=torch.int64, device=device)
         self.filled = 0
@@ -67,28 +72,13 @@ class LayerMeanStore:
     def append(self, hs: torch.Tensor, labels: torch.Tensor) -> int:
         """Write ``mean_k hs[b, k]`` (hs = (B, K, F, T), fp32 or bf16; other dtypes through an fp32 copy) and
         ``labels[b]`` at slot ``filled + b``; returns the first slot written."""
-        if hs.dim() != 4:
-            raise ValueError(f"hs must be (batch, layers, feat, frames), got {tuple(hs.shape)}")
-        b, k, f, t = hs.shape
-        if (f, t) != (self.feat, self.frames):
-            raise ValueError(f"clips {self.filled}..{self.filled + b - 1}: hidden states of (F, T) = ({f}, {t}), "
-                             f"the store holds ({self.feat}, {self.frames})")
+        b = _check_hs(hs, self.feat, self.frames, self.filled)
         if tuple(labels.shape) != (b,):
             raise ValueError(f"labels must be ({b},), got {tuple(labels.shape)}")
         if self.filled + b > self.n:
             raise ValueError(f"the store holds {self.n} clips: no room for {b} more after {self.filled}")
-        Fn._require_cuda(hs, "hs")
-        if hs.device != self.device:
-            raise ValueError(f"hs is on {hs.device}, the store on {self.device}")
-        x = hs.detach()
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        x = x.contiguous()
         slot0 = self.filled
-        with torch.cuda.device(self.device):
-            _cabi.check(_cabi.load().supcon_head_layer_mean_typed(
-                Fn._p(x), _cabi.BF16 if x.dtype == torch.bfloat16 else _cabi.F32, b, k, f, t,
-                Fn._p(self.rows[slot0]), Fn._stream(self.device)), "supcon_head_layer_mean_typed")
+        write_layer_means(self.rows, slot0, hs)
         self.labels[slot0:slot0 + b].copy_(labels.detach().long(), non_blocking=True)
         self.filled += b
         return slot0
@@ -102,17 +92,7 @@ class LayerMeanStore:
              rng_state=None) -> torch.Tensor:
         """(B, F) fp32: ``LeakyReLU(Dropout(rows[idx])).mean(-1)``, equal bit for bit to ``head.layer_time_pool``
         on the hs of those clips with the same ``rng_state`` {seed, offset}.  No host sync."""
-        if idx.dim() != 1 or idx.dtype != torch.int64 or idx.device != self.device:
-            raise ValueError(f"idx must be a 1-D int64 tensor on {self.device}, got {idx.dtype} "
-                             f"{tuple(idx.shape)} on {idx.device}")
-        Fn._require_cuda(self.rows, "the store")
-        rng = None
-        if dropout_p > 0.0:
-            if (rng_state is None or rng_state.dtype != torch.int64 or rng_state.numel() != 2
-                    or rng_state.device != self.device):
-                raise ValueError("dropout needs rng_state = int64 tensor {seed, offset} on the store's device")
-            rng = rng_state
-        idx = idx.contiguous()
+        idx, rng = _pool_args(self.rows, idx, dropout_p, rng_state)
         with torch.cuda.device(self.device):
             pooled = torch.empty((idx.shape[0], self.feat), dtype=torch.float32, device=self.device)
             _cabi.check(_cabi.load().supcon_head_store_pool_forward(
@@ -125,6 +105,65 @@ class LayerMeanStore:
 def store_bytes(n: int, feat: int, frames: int) -> int:
     """device bytes of a store of n clips: fp32 rows and int64 labels"""
     return n * feat * frames * 4 + n * 8
+
+
+def _fit_error(n: int, feat: int, frames: int, device: torch.device, need: int) -> str:
+    """why ``need`` bytes for a store of n clips do not fit the free memory of ``device`` ("" when they do)"""
+    if device.type != "cuda":
+        return ""
+    free, _ = torch.cuda.mem_get_info(device)
+    if need <= free:
+        return ""
+    return (f"a store of {n} clips x ({feat}, {frames}) fp32 takes {need / 1e9:.2f} GB; {free / 1e9:.2f} GB are free "
+            f"on {device}")
+
+
+def _check_hs(hs: torch.Tensor, feat: int, frames: int, slot0: int) -> int:
+    """the batch size of hidden states (B, K, F, T) that fit a store of (feat, frames) rows"""
+    if hs.dim() != 4:
+        raise ValueError(f"hs must be (batch, layers, feat, frames), got {tuple(hs.shape)}")
+    b, _, f, t = hs.shape
+    if (f, t) != (feat, frames):
+        raise ValueError(f"clips {slot0}..{slot0 + b - 1}: hidden states of (F, T) = ({f}, {t}), "
+                         f"the store holds ({feat}, {frames})")
+    return b
+
+
+def write_layer_means(rows: torch.Tensor, slot0: int, hs: torch.Tensor) -> None:
+    """``rows[slot0 + b] = mean_k hs[b, k]`` with ``supcon_head_layer_mean_typed`` (hs fp32 or bf16; other dtypes
+    through an fp32 copy); the caller has checked the shape and the room"""
+    Fn._require_cuda(hs, "hs")
+    if hs.device != rows.device:
+        raise ValueError(f"hs is on {hs.device}, the store on {rows.device}")
+    x = hs.detach()
+    if x.dtype not in (torch.float32, torch.bfloat16):
+        x = x.float()
+    x = x.contiguous()
+    b, k, f, t = x.shape
+    with torch.cuda.device(rows.device):
+        _cabi.check(_cabi.load().supcon_head_layer_mean_typed(
+            Fn._p(x), _cabi.BF16 if x.dtype == torch.bfloat16 else _cabi.F32, b, k, f, t,
+            Fn._p(rows[slot0]), Fn._stream(rows.device)), "supcon_head_layer_mean_typed")
+
+
+def _pool_args(rows: torch.Tensor, idx: torch.Tensor, dropout_p: float, rng_state):
+    """(contiguous idx, rng_state or None) of a pool call on a store whose rows are on ``rows.device``"""
+    device = rows.device
+    if idx.dim() != 1 or idx.dtype != torch.int64 or idx.device != device:
+        raise ValueError(f"idx must be a 1-D int64 tensor on {device}, got {idx.dtype} "
+                         f"{tuple(idx.shape)} on {idx.device}")
+    Fn._require_cuda(rows, "the store")
+    rng = None
+    if dropout_p > 0.0:
+        if (rng_state is None or rng_state.dtype != torch.int64 or rng_state.numel() != 2
+                or rng_state.device != device):
+            raise ValueError("dropout needs rng_state = int64 tensor {seed, offset} on the store's device")
+        rng = rng_state
+    return idx.contiguous(), rng
+
+
+def _labels_of(labels: torch.Tensor, filled: int, idx: torch.Tensor) -> torch.Tensor:
+    return labels.index_select(0, idx.clamp(0, max(filled, 1) - 1))
 
 
 @torch.no_grad()
@@ -152,4 +191,198 @@ def build_layer_mean_store(encoder, loader, device, *, label_index: int = 1, n=N
         store.append(hs, labels)
     if store is None:
         raise ValueError("the loader yielded no clips")
+    return store
+
+
+# ---------------------------------------------------------------------- the store sharded over one node's GPUs
+
+def shard_slots(n: int, rank: int, world: int) -> range:
+    """the dataset indices (slots) rank ``rank`` of ``world`` holds, in the order of its local rows: slot i lives on
+    rank i % world at local row i // world.  ``build_sharded_layer_mean_store``'s loader yields these clips."""
+    return range(rank, n, world)
+
+
+def _agree(problem, group) -> None:
+    """Every rank passes its own failed check (an exception, or None); raises the same error on every rank when any
+    rank has one.  Checks that can fail on one rank alone go through here, so that no rank is left waiting in a
+    collective that the failing rank never joins."""
+    got = [None] * dist.get_world_size(group)
+    dist.all_gather_object(got, None if problem is None else (type(problem).__name__, str(problem)), group=group)
+    bad = [(r, p) for r, p in enumerate(got) if p is not None]
+    if bad:
+        kind = {"MemoryError": MemoryError, "RuntimeError": RuntimeError}.get(bad[0][1][0], ValueError)
+        raise kind("; ".join(f"rank {r}: {msg}" for r, (_, msg) in bad))
+
+
+class _SymmetricShard:
+    """This rank's (rows, F, T) fp32 shard in symmetric memory (``torch.distributed._symmetric_memory``, as the peer
+    exchange of ``distributed.py`` allocates its buffers): the same size on every rank and mapped into every process,
+    so ``bases[r]`` is rank r's shard as seen from this one."""
+
+    def __init__(self, rows: int, feat: int, frames: int, device, group):
+        import torch.distributed._symmetric_memory as symm
+        problem = None
+        try:
+            self.buf = symm.empty(rows * feat * frames, dtype=torch.float32, device=device)
+        except Exception as exc:  # noqa: BLE001  (refused by the allocator: every rank must hear of it)
+            self.buf, problem = None, RuntimeError(f"symmetric allocation of {rows} x ({feat}, {frames}) fp32: {exc}")
+        _agree(problem, group)
+        self.handle = symm.rendezvous(self.buf, group if group is not None else dist.group.WORLD)
+        self.rows = self.buf.view(rows, feat, frames)
+        self.bases = [int(p) for p in self.handle.buffer_ptrs]
+
+    def write(self, row0: int, hs: torch.Tensor) -> None:
+        write_layer_means(self.rows, row0, hs)
+
+    def close(self) -> None:
+        self.rows = self.buf = self.handle = None
+
+
+class ShardedLayerMeanStore:
+    """A ``LayerMeanStore`` of n clips split over the R ranks of ``group`` on one node: slot i is row i // R of the
+    shard of rank i % R.  Every rank allocates ceil(n / R) rows; ``rows`` is this rank's shard, ``labels`` (n,) a
+    full copy on every rank.  ``pool`` gathers any slot, reading the other ranks' rows through peer memory over
+    NVLink, with the values and dropout masks of ``LayerMeanStore.pool`` bit for bit; ``labels_of`` is a local
+    gather.  It offers the interface the Stage-1 code calls on a ``LayerMeanStore`` (``pool``, ``labels_of``,
+    ``filled``, ``n``, ``feat``, ``frames``, ``device``), so ``FusedCompressionHead.pooled_features_from_store``,
+    ``train_one_epoch_from_store``, ``evaluate_from_store`` and ``GraphedHeadStep(store=)`` take it unchanged.
+
+    Construction is collective: every rank passes the same (n, feat, frames) with its own device.  The checks --
+    n >= R, the same shape on every rank, the shard fits free memory, one host, every pair of GPUs peer-capable --
+    are agreed on first and raise on every rank.  ``close()`` (collective) releases the mapping; call it before
+    ``destroy_process_group``.  ``allocate`` replaces the symmetric allocation (tests without a GPU)."""
+
+    def __init__(self, n: int, feat: int, frames: int, device, group=None, *, allocate=None):
+        self.group = group
+        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
+        device = torch.device(device)
+        self.n, self.feat, self.frames = n, feat, frames
+        self.local_rows = -(-n // self.world) if n > 0 else 0
+        where = [None] * self.world
+        dist.all_gather_object(where, ((n, feat, frames), socket.gethostname(), device.index), group=group)
+        _agree(self._local_problem(device, where), group)
+        self._shard = (allocate or _SymmetricShard)(self.local_rows, feat, frames, device, group)
+        self.rows = self._shard.rows
+        self.bases = torch.tensor(self._shard.bases, dtype=torch.int64, device=device)
+        self.labels = torch.full((n,), -1, dtype=torch.int64, device=device)
+        self.filled = 0
+
+    @property
+    def device(self) -> torch.device:
+        return self.labels.device
+
+    def _local_problem(self, device, where):
+        """this rank's failed precondition, or None; ``where`` = every rank's ((n, F, T), host, device index)"""
+        if self.n < self.world:
+            return ValueError(f"a store sharded over {self.world} ranks needs at least {self.world} clips, "
+                              f"got {self.n}")
+        shapes = [s for s, _, _ in where]
+        if len(set(shapes)) != 1:
+            return ValueError("the ranks disagree on the store's (n, F, T): " +
+                              ", ".join(f"rank {r} {s}" for r, s in enumerate(shapes)))
+        if self.feat < 1 or self.frames < 1:
+            return ValueError(f"bad store shape ({self.n}, {self.feat}, {self.frames})")
+        too_big = _fit_error(self.local_rows, self.feat, self.frames, device,
+                             store_bytes(self.local_rows, self.feat, self.frames) + self.n * 8)
+        if too_big:
+            return MemoryError(f"the shard of {too_big}")
+        if device.type != "cuda":
+            return None
+        # the shards are read over NVLink: one host, and this GPU reaches every other rank's
+        alone = "; a sharded store needs the GPUs of one node with peer access: use feature_store.LayerMeanStore"
+        if len({h for _, h, _ in where}) != 1:
+            return RuntimeError("the ranks run on several hosts" + alone)
+        blocked = [r for r, (_, _, d) in enumerate(where)
+                   if d != device.index and not torch.cuda.can_device_access_peer(device.index, d)]
+        if blocked:
+            return RuntimeError(f"cuda:{device.index} has no peer access to the GPU of rank(s) {blocked}" + alone)
+        return None
+
+    def labels_of(self, idx: torch.Tensor) -> torch.Tensor:
+        """labels of the slots ``idx`` (device int64), from this rank's full copy (clamped as in
+        ``LayerMeanStore.labels_of``)"""
+        return _labels_of(self.labels, self.filled, idx)
+
+    def pool(self, idx: torch.Tensor, dropout_p: float = 0.0, negative_slope: float = 0.01,
+             rng_state=None) -> torch.Tensor:
+        """(B, F) fp32, ``LayerMeanStore.pool`` of the slots ``idx`` wherever they live.  No host sync, no
+        collective: the other ranks' shards are read in place."""
+        if self._shard is None:
+            raise RuntimeError("the sharded store is closed")
+        idx, rng = _pool_args(self.rows, idx, dropout_p, rng_state)
+        with torch.cuda.device(self.device):
+            pooled = torch.empty((idx.shape[0], self.feat), dtype=torch.float32, device=self.device)
+            _cabi.check(_cabi.load().supcon_head_sharded_store_pool_forward(
+                Fn._p(self.bases), self.world, self.filled, self.feat, self.frames, Fn._p(idx), idx.shape[0],
+                float(dropout_p), float(negative_slope), Fn._p(rng), Fn._p(pooled), Fn._stream(self.device)),
+                "supcon_head_sharded_store_pool_forward")
+        return pooled
+
+    def gather_labels(self, local_labels: torch.Tensor) -> None:
+        """``labels`` = every rank's ``local_labels`` (ceil(n / R),) in slot order, through one all-gather"""
+        parts = [torch.empty_like(local_labels) for _ in range(self.world)]
+        dist.all_gather(parts, local_labels.contiguous(), group=self.group)
+        self.labels.copy_(torch.stack(parts, dim=1).reshape(-1)[:self.n])
+
+    def close(self) -> None:
+        """Release this rank's shard and its mapping of the others' (collective: waits until no rank still reads a
+        shard).  The store cannot pool afterwards."""
+        if self._shard is None:
+            return
+        if self.device.type == "cuda":
+            torch.cuda.synchronize(self.device)
+        dist.barrier(group=self.group)
+        self._shard.close()
+        self._shard = self.rows = None
+
+
+@torch.no_grad()
+def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=None, label_index: int = 1,
+                                   allocate=None) -> ShardedLayerMeanStore:
+    """``build_layer_mean_store`` split over the ranks of ``group`` (collective): each rank runs ``encoder`` on its
+    own share of the n clips, so the build takes 1 / R of the time and the node holds R times the clips.
+    ``loader`` yields this rank's clips in the order ``shard_slots(n, rank, R)`` lists them (e.g. a
+    ``DataLoader(Subset(dataset, shard_slots(...)), shuffle=False)``); the encoder is called as
+    ``build_layer_mean_store`` calls it.  Raises on every rank when the ranks' (F, T) differ, a shard does not fit
+    free memory, a rank's loader yields more or fewer clips than its share, n < R, or the GPUs cannot reach each
+    other's memory.  Afterwards ``filled == n`` and ``labels`` holds every slot's label on every rank."""
+    from .stage1 import _to_device
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    encoder.eval()
+
+    def encoded(batch):
+        waveforms, labels = _to_device(batch[0], batch[label_index], device)
+        return encoder(waveforms, attention_mask=(waveforms != 0.0).long()), labels
+
+    batches = iter(loader)
+    first = next(batches, None)
+    hs, labels = encoded(first) if first is not None else (None, None)
+    shape = tuple(hs.shape[-2:]) if hs is not None else (0, 0)
+    store = ShardedLayerMeanStore(n, *shape, device, group, allocate=allocate)
+    share = len(shard_slots(n, rank, world))
+    local_labels = torch.full((store.local_rows,), -1, dtype=torch.int64, device=store.device)
+    filled, problem = 0, None
+    try:
+        while hs is not None:
+            b = _check_hs(hs, store.feat, store.frames, filled)
+            if tuple(labels.shape) != (b,):
+                raise ValueError(f"labels must be ({b},), got {tuple(labels.shape)}")
+            if filled + b > share:
+                raise ValueError(f"the loader yields more than this rank's {share} clips of {n}")
+            store._shard.write(filled, hs)
+            local_labels[filled:filled + b].copy_(labels.detach().long(), non_blocking=True)
+            filled += b
+            batch = next(batches, None)
+            hs, labels = encoded(batch) if batch is not None else (None, None)
+        if filled != share:
+            raise ValueError(f"the loader yielded {filled} clips, this rank's share of {n} is {share}")
+    except ValueError as exc:
+        problem = exc
+    try:
+        _agree(problem, group)
+    except Exception:
+        store.close()
+        raise
+    store.gather_labels(local_labels)
+    store.filled = n
     return store

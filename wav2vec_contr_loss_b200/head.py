@@ -144,7 +144,7 @@ class FusedCompressionHead(nn.Module):
         return F.linear(self.pooled_features(hs), self.mlp3.weight, self.mlp3.bias)
 
     def pooled_features_from_store(self, store, idx: torch.Tensor) -> torch.Tensor:
-        """``pooled_features`` of the clips in slots ``idx`` (device int64) of a ``feature_store.LayerMeanStore``:
+        """``pooled_features`` of the clips in slots ``idx`` (device int64) of a ``feature_store.LayerMeanStore`` (or ``ShardedLayerMeanStore``):
         the same values, bit for bit, and the same dropout stream (one offset per call in train mode)."""
         p = self.dropout_head.p if self.training else 0.0
         if p > 0.0:

@@ -289,13 +289,16 @@ def _store_embed(head, store, idx: torch.Tensor, normalize: Optional[Callable] =
 
 
 def train_one_epoch_from_store(head, loss_fn, store, batches, optimizer, device, epoch, cfg, *,
-                               normalize: Optional[Callable] = None, max_grad_norm: float = 5.0):
+                               normalize: Optional[Callable] = None, grad_sync: Optional[Callable] = None,
+                               max_grad_norm: float = 5.0):
     """``train_one_epoch`` for a frozen encoder whose layer means are in ``store``
     (``feature_store.build_layer_mean_store``): no encoder call.  ``batches`` are index lists into the store, e.g.
     the batches of the same ``BalancedBatchSampler``; labels are gathered from the store on the device.  ``head`` is
     a ``FusedCompressionHead``.  With the same batches, seeds and dropout stream the epoch is ``train_one_epoch``'s
     whenever the encoder's output for a clip does not depend on its batch mates.  Returns ``(mean loss, alpha)``.
-    Raises when ``cfg.finetune_encoder`` or ``cfg.use_rawboost`` is set: the store would be stale."""
+    On several ranks (a ``feature_store.ShardedLayerMeanStore``, ``BalancedBatchSampler(rank=, world_size=)`` batches,
+    ``ShardedSupConLoss``) pass ``grad_sync=GradSync(head.parameters())``: it runs after ``backward`` as in
+    ``train_one_epoch``.  Raises when ``cfg.finetune_encoder`` or ``cfg.use_rawboost`` is set: the store would be stale."""
     _check_store_cfg(cfg, training=True)
     head.train()
     alpha = alpha_for_epoch(epoch, cfg)
@@ -307,6 +310,8 @@ def train_one_epoch_from_store(head, loss_fn, store, batches, optimizer, device,
 
         optimizer.zero_grad(set_to_none=True)
         loss.backward()
+        if grad_sync is not None:
+            grad_sync()
         torch.nn.utils.clip_grad_norm_(head.parameters(), max_grad_norm)
         optimizer.step()
         running.add(loss)
@@ -414,7 +419,7 @@ class GraphedHeadStep:
     The graphs of different alphas share that one memory.  Eager calls of the loss between replays stay valid as
     long as the batch size does not grow (a larger batch reallocates the buffers the graphs use).
 
-    ``store=`` (a ``feature_store.LayerMeanStore``, head = ``FusedCompressionHead``) captures the step of
+    ``store=`` (a ``feature_store.LayerMeanStore`` or ``ShardedLayerMeanStore``, head = ``FusedCompressionHead``) captures the step of
     ``train_one_epoch_from_store`` instead: the graph gathers and pools the store rows ``step.idx`` and their labels,
     so the static input is the (B,) int64 index vector.  Pass an index example in place of ``hs_example``, no
     labels, and call ``step(idx, alpha=alpha)``: a replay copies ``idx`` and runs."""
