@@ -22,9 +22,20 @@ memory (``supcon_head_sharded_store_pool_forward``), with the same bits as ``Lay
 
 Preconditions: frozen encoder, no waveform augmentation, the same crop / pad of each clip in every epoch.  The rows
 are fp32 (a bf16 store would round the mean and lose that equality).  There is no backward: the store is a constant.
+
+On disk a store is a directory of two ``.npy`` files, ``rows.npy`` (n, F, T) fp32 in C order and ``labels.npy``
+(n,) int64, in slot order whatever the number of ranks that wrote it: the layout of the reference's layer-mean
+feature memmap (extract_encoder_embeddings.py).  ``save`` / ``load_layer_mean_store`` /
+``load_sharded_layer_mean_store`` stream the rows between the file and the device through two pinned staging
+buffers, so the host never holds the array.
 """
+import io
+import mmap
+import os
+import shutil
 import socket
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -32,7 +43,10 @@ from . import _cabi
 from . import functional as Fn
 
 __all__ = ["LayerMeanStore", "build_layer_mean_store", "ShardedLayerMeanStore", "build_sharded_layer_mean_store",
-           "shard_slots"]
+           "shard_slots", "load_layer_mean_store", "load_sharded_layer_mean_store"]
+
+ROWS_FILE, LABELS_FILE = "rows.npy", "labels.npy"
+STAGE_BYTES = 64 << 20      # each of the two pinned staging buffers of a save or load
 
 
 class LayerMeanStore:
@@ -100,6 +114,49 @@ class LayerMeanStore:
                 float(negative_slope), Fn._p(rng), Fn._p(pooled), Fn._stream(self.device)),
                 "supcon_head_store_pool_forward")
         return pooled
+
+    def save(self, path, overwrite: bool = False):
+        """Write slots ``[0, filled)`` to the directory ``path`` (``rows.npy``, ``labels.npy``; module docstring).
+        The files are written into ``<path>.partial``, fsynced and then renamed to ``path``, so a save that dies
+        leaves nothing that loads.  An existing ``path`` is kept unless ``overwrite`` (as ``export_embeddings``
+        keeps its files): returns None then, else the number of clips written.  Raises on an empty store."""
+        path = os.fspath(path)
+        if self.filled < 1:
+            raise ValueError("the store is empty: nothing to save")
+        if os.path.exists(path) and not overwrite:
+            return None
+        partial = path + ".partial"
+        try:
+            header = _create_rows_file(partial, (self.filled, self.feat, self.frames))
+            _write_rows(self.rows, range(self.filled), partial, header)
+            _finish_save(partial, path, self.labels[:self.filled])
+        except BaseException:
+            _discard(partial)
+            raise
+        return self.filled
+
+    @classmethod
+    def from_arrays(cls, rows, labels, device) -> "LayerMeanStore":
+        """A store of ``n == filled`` clips from host arrays: ``rows`` (n, F, T) float32 (copied bit for bit) or
+        float16 (widened exactly) as a numpy array, memmap or CPU tensor, ``labels`` (n,) integers.  A memmap of a
+        whole ``.npy`` file is read from the file in chunks, any other array copied in chunks; either way through
+        the pinned staging buffers, never as a whole.  Raises on another dtype (float64 would round), another rank
+        and labels that are not (n,) integers."""
+        src = _RowSource(rows)
+        lab = _label_tensor(labels, src.n)
+        store = cls(src.n, src.feat, src.frames, device)
+        _read_rows(src, range(src.n), store.rows)
+        store.labels.copy_(lab)
+        store.filled = src.n
+        return store
+
+
+def load_layer_mean_store(path, device) -> LayerMeanStore:
+    """The store that ``LayerMeanStore.save`` or ``ShardedLayerMeanStore.save`` (any number of ranks) wrote to
+    ``path``, or layer means extracted elsewhere in that layout, on ``device``: ``n == filled ==`` the file's row
+    count.  Raises FileNotFoundError on a missing store and ValueError naming the file on a truncated or unreadable
+    one, besides the checks of ``LayerMeanStore.from_arrays``."""
+    return LayerMeanStore.from_arrays(*_open_store(path), device)
 
 
 def store_bytes(n: int, feat: int, frames: int) -> int:
@@ -335,6 +392,75 @@ class ShardedLayerMeanStore:
         self._shard.close()
         self._shard = self.rows = None
 
+    def save(self, path, overwrite: bool = False):
+        """``LayerMeanStore.save`` of slots ``[0, filled)`` (collective), in the same format: the file does not
+        depend on R.  Rank 0 creates and sizes ``<path>.partial/rows.npy``; then every rank writes its own rows at
+        their slots (local row j is slot rank + j R) and fsyncs; then rank 0 writes ``labels.npy`` and renames.  A
+        failure on any rank raises on every rank and removes the partial directory.  Whether ``path`` exists is
+        rank 0's view."""
+        if self._shard is None:
+            raise RuntimeError("the sharded store is closed")
+        path = os.fspath(path)
+        if self.filled < 1:
+            raise ValueError("the store is empty: nothing to save")
+        seen = [None] * self.world
+        dist.all_gather_object(seen, os.path.exists(path), group=self.group)
+        if seen[0] and not overwrite:
+            return None
+        partial, lead = path + ".partial", self.rank == 0
+        header = len(_npy_header((self.filled, self.feat, self.frames)))
+
+        def step(fn):
+            problem = None
+            try:
+                fn()
+            except (OSError, ValueError, RuntimeError) as exc:
+                problem = exc
+            try:
+                _agree(problem, self.group)
+            except Exception:
+                if lead:
+                    _discard(partial)
+                raise
+
+        step(lambda: _create_rows_file(partial, (self.filled, self.feat, self.frames)) if lead else None)
+        step(lambda: _write_rows(self.rows, shard_slots(self.filled, self.rank, self.world), partial, header))
+        step(lambda: _finish_save(partial, path, self.labels[:self.filled]) if lead else None)
+        return self.filled
+
+    @classmethod
+    def from_arrays(cls, rows, labels, device, group=None, *, allocate=None) -> "ShardedLayerMeanStore":
+        """``LayerMeanStore.from_arrays`` split over the ranks of ``group`` (collective): every rank passes the
+        whole (n, F, T) array (typically a memmap of the same file) and reads only its slots
+        ``shard_slots(n, rank, R)`` into its shard, in place.  Besides ``from_arrays``' checks and the
+        constructor's, the ranks must agree on the dtype; every check raises on every rank."""
+        src, lab, problem = None, None, None
+        try:
+            src = _RowSource(rows)
+            lab = _label_tensor(labels, src.n)
+        except ValueError as exc:
+            problem = exc
+        _agree(problem, group)
+        kinds = [None] * dist.get_world_size(group)
+        dist.all_gather_object(kinds, str(src.rows.dtype), group=group)
+        if len(set(kinds)) != 1:
+            raise ValueError("the ranks disagree on the rows' dtype: " +
+                             ", ".join(f"rank {r} {k}" for r, k in enumerate(kinds)))
+        store = cls(src.n, src.feat, src.frames, device, group, allocate=allocate)
+        problem = None
+        try:
+            _read_rows(src, shard_slots(store.n, store.rank, store.world), store.rows)
+            store.labels.copy_(lab)
+        except (OSError, ValueError, RuntimeError) as exc:
+            problem = exc
+        try:
+            _agree(problem, group)                  # also the barrier before any rank reads a peer's shard
+        except Exception:
+            store.close()
+            raise
+        store.filled = store.n
+        return store
+
 
 @torch.no_grad()
 def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=None, label_index: int = 1,
@@ -386,3 +512,256 @@ def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=Non
     store.gather_labels(local_labels)
     store.filled = n
     return store
+
+
+def load_sharded_layer_mean_store(path, device, group=None, *, allocate=None) -> ShardedLayerMeanStore:
+    """``load_layer_mean_store`` into a store sharded over the ranks of ``group`` (collective): the file may have
+    been written by any number of ranks, one included, and rank r reads only its own slots.  A missing, truncated
+    or unreadable file on any rank raises on every rank, as do the checks of ``ShardedLayerMeanStore.from_arrays``.
+    ``allocate`` as in ``ShardedLayerMeanStore``."""
+    arrays, problem = None, None
+    try:
+        arrays = _open_store(path)
+    except (OSError, ValueError) as exc:
+        problem = exc
+    _agree(problem, group)
+    return ShardedLayerMeanStore.from_arrays(*arrays, device, group, allocate=allocate)
+
+
+# ---------------------------------------------------------------------------------- the store on disk
+
+def _open_store(path):
+    """(rows, labels) memmaps of the store directory ``path``; np.load checks each header against the file's size"""
+    path = os.fspath(path)
+    if not os.path.isdir(path):
+        raise FileNotFoundError(f"no layer-mean store at {path}")
+    arrays = []
+    for name in (ROWS_FILE, LABELS_FILE):
+        file = os.path.join(path, name)
+        try:
+            arrays.append(np.load(file, mmap_mode="r"))
+        except FileNotFoundError:
+            raise
+        except (OSError, ValueError) as exc:
+            raise ValueError(f"{file} is not a readable .npy array: {exc}") from exc
+    return arrays
+
+
+class _RowSource:
+    """(n, F, T) float32 or float16 rows from the host: a memmap of a whole file (what np.load returns) is read from
+    the file with readinto, which keeps its pages out of this process; any other array is copied row by row."""
+
+    def __init__(self, rows):
+        if isinstance(rows, torch.Tensor):
+            if rows.device.type != "cpu" or rows.dtype not in (torch.float32, torch.float16):
+                raise ValueError(f"rows must be a float32 or float16 CPU tensor, got {rows.dtype} on {rows.device}")
+            rows = rows.detach().numpy()
+        if not isinstance(rows, np.ndarray):
+            raise ValueError(f"rows must be a numpy array or a CPU tensor, got {type(rows).__name__}")
+        if rows.dtype not in (np.dtype(np.float32), np.dtype(np.float16)):
+            raise ValueError(f"rows must be float32 or float16 (another dtype would be rounded), got {rows.dtype}")
+        if rows.ndim != 3:
+            raise ValueError(f"rows must be (n, F, T), got {rows.shape}")
+        self.rows = rows
+        self.n, self.feat, self.frames = rows.shape
+        self.row = self.feat * self.frames
+        self.file = self.offset = None
+        if (isinstance(rows, np.memmap) and isinstance(rows.base, mmap.mmap) and rows.flags.c_contiguous
+                and rows.filename):
+            self.file, self.offset = rows.filename, rows.offset
+        # float16 is read here and widened into the fp32 staging buffer (exact); float32 is read into it directly
+        self.raw = None if rows.dtype == np.float32 else np.empty(0, np.float16)
+
+    def fill(self, out: np.ndarray, pieces, fd) -> None:
+        """``out`` (m,) fp32 = the source's elements ``pieces`` [(flat offset, count), ...] in order"""
+        if self.raw is not None and self.raw.size < out.size:
+            self.raw = np.empty(out.size, np.float16)
+        dst = out if self.raw is None else self.raw[:out.size]
+        pos = 0
+        for start, count in pieces:
+            if fd is not None:
+                _read_exactly(fd, dst[pos:pos + count], self.offset + start * dst.itemsize, self.file)
+            else:
+                done = 0
+                while done < count:                         # rows, so that a strided array is never copied whole
+                    i, lo = divmod(start + done, self.row)
+                    k = min(self.row - lo, count - done)
+                    np.copyto(dst[pos + done:pos + done + k], self.rows[i].reshape(-1)[lo:lo + k])
+                    done += k
+            pos += count
+        if self.raw is not None:
+            np.copyto(out, dst)
+
+
+def _read_exactly(fd: int, out: np.ndarray, offset: int, file: str) -> None:
+    view = memoryview(out).cast("B")
+    while view.nbytes:
+        got = os.preadv(fd, [view], offset)
+        if got == 0:
+            raise ValueError(f"{file} ends at byte {offset}, before the rows its header declares")
+        view, offset = view[got:], offset + got
+
+
+def _write_all(fd: int, data: np.ndarray, offset: int) -> None:
+    view = memoryview(data).cast("B")
+    while view.nbytes:
+        put = os.pwrite(fd, view, offset)
+        view, offset = view[put:], offset + put
+
+
+def _label_tensor(labels, n: int) -> torch.Tensor:
+    """(n,) int64 CPU tensor of labels given as integers of any width (numpy array, memmap or tensor)"""
+    lab = labels.detach().cpu().numpy() if isinstance(labels, torch.Tensor) else np.asarray(labels)
+    if lab.shape != (n,) or lab.dtype.kind not in "iu":
+        raise ValueError(f"labels must be ({n},) integers, got {lab.dtype} {lab.shape}")
+    return torch.from_numpy(lab.astype(np.int64))
+
+
+def _chunks(slots, row: int, chunk: int):
+    """(device element offset, [(file element offset, count), ...]) of at most ``chunk`` elements each, in order:
+    the device tensor's local row j is slot ``slots[j]`` of the file.  A chunk may split a row."""
+    runs = ([(slots.start * row, len(slots) * row)] if isinstance(slots, range) and slots.step == 1
+            else [(s * row, row) for s in slots])
+    d0, pieces, size = 0, [], 0
+    for f0, count in runs:
+        while count:
+            k = min(count, chunk - size)
+            pieces.append((f0, k))
+            size, f0, count = size + k, f0 + k, count - k
+            if size == chunk:
+                yield d0, pieces
+                d0, pieces, size = d0 + size, [], 0
+    if pieces:
+        yield d0, pieces
+
+
+class _Staging:
+    """Two fp32 host buffers of ``STAGE_BYTES`` (pinned when the store is on a GPU) and a side stream for their
+    copies to and from the device, each a ``cudaMemcpyAsync``; an event per buffer guards its reuse, so the file
+    I/O of one chunk overlaps the copy of the other."""
+
+    def __init__(self, device):
+        self.chunk = max(STAGE_BYTES // 4, 1)
+        self.cuda = device.type == "cuda"
+        self.bufs = [torch.empty(self.chunk, dtype=torch.float32, pin_memory=self.cuda) for _ in range(2)]
+        self.events = [None, None]
+        if self.cuda:
+            self.stream = torch.cuda.Stream(device)
+            self.stream.wait_stream(torch.cuda.current_stream(device))
+
+    def host(self, c: int) -> torch.Tensor:
+        """the buffer of chunk c, once the last copy into or out of it has completed"""
+        if self.events[c % 2] is not None:
+            self.events[c % 2].synchronize()
+        return self.bufs[c % 2]
+
+    def copy(self, c: int, dst: torch.Tensor, src: torch.Tensor) -> None:
+        if not self.cuda:
+            dst.copy_(src)
+            return
+        with torch.cuda.stream(self.stream):
+            dst.copy_(src, non_blocking=True)
+            self.events[c % 2] = torch.cuda.Event()
+            self.events[c % 2].record(self.stream)
+
+    def finish(self) -> None:
+        if self.cuda:
+            self.stream.synchronize()
+
+
+def _read_rows(src: _RowSource, slots, rows: torch.Tensor) -> None:
+    """``rows[j] = src[slots[j]]`` (rows contiguous fp32, on a GPU or the CPU); returns when the copies are done"""
+    dst = rows.view(-1)
+    st = _Staging(rows.device)
+    fd = os.open(src.file, os.O_RDONLY) if src.file else None
+    try:
+        for c, (d0, pieces) in enumerate(_chunks(slots, src.row, st.chunk)):
+            m = sum(k for _, k in pieces)
+            buf = st.host(c)[:m]
+            src.fill(buf.numpy(), pieces, fd)
+            st.copy(c, dst[d0:d0 + m], buf)
+        st.finish()
+    finally:
+        if fd is not None:
+            os.close(fd)
+
+
+def _write_rows(rows: torch.Tensor, slots, partial: str, header: int) -> None:
+    """write ``rows[j]`` at slot ``slots[j]`` of ``<partial>/rows.npy`` (sized by ``_create_rows_file``; its data
+    starts at byte ``header``) and fsync it"""
+    row = rows.shape[1] * rows.shape[2]
+    src = rows.view(-1)
+    st = _Staging(rows.device)
+    chunks = list(_chunks(slots, row, st.chunk))
+    sizes = [sum(k for _, k in pieces) for _, pieces in chunks]
+
+    def issue(c):
+        st.copy(c, st.host(c)[:sizes[c]], src[chunks[c][0]:chunks[c][0] + sizes[c]])
+
+    fd = os.open(os.path.join(partial, ROWS_FILE), os.O_WRONLY)
+    try:
+        if chunks:
+            issue(0)
+        for c, (_, pieces) in enumerate(chunks):
+            if c + 1 < len(chunks):
+                issue(c + 1)                                # its buffer was written to the file one chunk ago
+            buf, pos = st.host(c).numpy(), 0
+            for f0, k in pieces:
+                _write_all(fd, buf[pos:pos + k], header + 4 * f0)
+                pos += k
+        st.finish()
+        os.fsync(fd)
+    finally:
+        os.close(fd)
+
+
+def _npy_header(shape) -> bytes:
+    """the .npy header of a C-order little-endian fp32 array of ``shape``: the same bytes on every rank"""
+    out = io.BytesIO()
+    np.lib.format.write_array_header_1_0(out, {"descr": "<f4", "fortran_order": False, "shape": tuple(shape)})
+    return out.getvalue()
+
+
+def _create_rows_file(partial: str, shape) -> int:
+    """a fresh ``<partial>/rows.npy`` of ``shape`` fp32 (header written, data sized, not yet filled); returns the
+    header's length.  A ``partial`` left by a save that died is removed first."""
+    _discard(partial)
+    os.makedirs(partial)
+    header = _npy_header(shape)
+    with open(os.path.join(partial, ROWS_FILE), "wb") as fh:
+        fh.write(header)
+        fh.truncate(len(header) + 4 * int(np.prod(shape)))
+    return len(header)
+
+
+def _fsync_dir(path: str) -> None:
+    fd = os.open(path, os.O_RDONLY)
+    try:
+        os.fsync(fd)
+    finally:
+        os.close(fd)
+
+
+def _finish_save(partial: str, path: str, labels: torch.Tensor) -> None:
+    """write ``labels.npy``, fsync, and rename ``partial`` to ``path`` (replacing what is there)"""
+    with open(os.path.join(partial, LABELS_FILE), "wb") as fh:
+        np.save(fh, labels.detach().cpu().numpy().astype(np.int64))
+        fh.flush()
+        os.fsync(fh.fileno())
+    _fsync_dir(partial)
+    old = None
+    if os.path.lexists(path):
+        old = path + ".old"
+        _discard(old)
+        os.rename(path, old)
+    os.rename(partial, path)
+    _fsync_dir(os.path.dirname(os.path.abspath(path)))
+    if old is not None:
+        _discard(old)
+
+
+def _discard(path: str) -> None:
+    if os.path.isdir(path) and not os.path.islink(path):
+        shutil.rmtree(path)
+    elif os.path.lexists(path):
+        os.remove(path)
