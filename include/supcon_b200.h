@@ -34,6 +34,9 @@ extern "C" {
 /* element type of z / dz buffers */
 #define SUPCON_F32 0
 #define SUPCON_BF16 1
+/* fp16: the element type of a layer-mean store's rows only (the store_dtype of the _store_pool_forward_typed entries);
+ * every z / dz / hs dtype argument rejects it */
+#define SUPCON_F16 2
 
 /* similarity (reference loss.py:96-107) */
 #define SUPCON_COSINE 0
@@ -342,6 +345,23 @@ int supcon_head_sharded_store_pool_forward(const uint64_t* shard_bases /*device 
                                            const int64_t* idx /*[batch]*/, int32_t batch, float dropout_p,
                                            float negative_slope, const uint64_t* rng_state,
                                            float* pooled_out /*[batch][feat]*/, void* stream);
+
+/* store_dtype (the _typed entry points) is the element type of the store's rows: SUPCON_F32, or SUPCON_F16 for a
+ * store kept at half the bytes.  fp16 elements are widened to fp32 exactly and the arithmetic after the load is the
+ * fp32 one, so pooled_out equals bit for bit that of the SUPCON_F32 call on a store holding the widened values.
+ * Shard offsets count elements of store_dtype.  Any other store_dtype, SUPCON_BF16 included, returns
+ * SUPCON_E_INVALID before any CUDA call, as do the arguments the untyped entries reject.
+ * supcon_head_store_pool_forward / supcon_head_sharded_store_pool_forward are the SUPCON_F32 case. */
+int supcon_head_store_pool_forward_typed(const void* store /*[n_store][feat][frames]*/, int32_t store_dtype,
+                                         int64_t n_store, int32_t feat, int32_t frames,
+                                         const int64_t* idx /*[batch]*/, int32_t batch, float dropout_p,
+                                         float negative_slope, const uint64_t* rng_state,
+                                         float* pooled_out /*[batch][feat]*/, void* stream);
+int supcon_head_sharded_store_pool_forward_typed(const uint64_t* shard_bases /*device [n_ranks]*/, int32_t n_ranks,
+                                                 int32_t store_dtype, int64_t n_store, int32_t feat, int32_t frames,
+                                                 const int64_t* idx /*[batch]*/, int32_t batch, float dropout_p,
+                                                 float negative_slope, const uint64_t* rng_state,
+                                                 float* pooled_out /*[batch][feat]*/, void* stream);
 
 /* Diagnostics used by the parity tests: hard-negative index sets of the owned
  * rows, recomputed from the statistics (index ascending, -1 padded). */

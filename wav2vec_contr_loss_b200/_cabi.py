@@ -12,6 +12,7 @@ from ctypes import POINTER, c_char_p, c_float, c_int32, c_size_t, c_uint32, c_vo
 _LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libsupcon_b200.so")
 
 F32, BF16 = 0, 1
+F16 = 2                 # a layer-mean store's element type only
 COSINE, GEODESIC = 0, 1
 FLAG_FORCE_EXACT, FLAG_FORCE_TENSOR, FLAG_NO_SMALL = 1, 2, 4
 LABEL_I64, LABEL_F32, LABEL_F64 = 1, 2, 3
@@ -36,6 +37,7 @@ EXPORTS = (
     "supcon_head_pool_forward_typed", "supcon_head_pool_backward_typed",
     "supcon_forward_rows_memory", "supcon_backward_rows_memory",
     "supcon_head_layer_mean_typed", "supcon_head_store_pool_forward", "supcon_head_sharded_store_pool_forward",
+    "supcon_head_store_pool_forward_typed", "supcon_head_sharded_store_pool_forward_typed",
 )
 
 
@@ -142,6 +144,14 @@ def load():
     lib.supcon_head_sharded_store_pool_forward.argtypes = [c_void_p, c_int32, ctypes.c_int64, c_int32, c_int32,
                                                            c_void_p, c_int32, c_float, c_float, c_void_p, c_void_p,
                                                            c_void_p]
+    lib.supcon_head_store_pool_forward_typed.restype = c_int32
+    lib.supcon_head_store_pool_forward_typed.argtypes = [c_void_p, c_int32, ctypes.c_int64, c_int32, c_int32,
+                                                         c_void_p, c_int32, c_float, c_float, c_void_p, c_void_p,
+                                                         c_void_p]
+    lib.supcon_head_sharded_store_pool_forward_typed.restype = c_int32
+    lib.supcon_head_sharded_store_pool_forward_typed.argtypes = [c_void_p, c_int32, c_int32, ctypes.c_int64,
+                                                                 c_int32, c_int32, c_void_p, c_int32, c_float,
+                                                                 c_float, c_void_p, c_void_p, c_void_p]
     lib.supcon_label_keys.restype = c_int32
     lib.supcon_label_keys.argtypes = [c_void_p, c_int32, c_int32, c_void_p, c_void_p]
     PP = POINTER(Peer)

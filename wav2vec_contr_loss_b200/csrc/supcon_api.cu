@@ -626,10 +626,17 @@ int supcon_head_layer_mean_typed(const void* hs, int32_t hs_dtype, int32_t batch
   return 0;
 }
 
-int supcon_head_store_pool_forward(const float* store, int64_t n_store, int32_t feat, int32_t frames,
-                                   const int64_t* idx, int32_t batch, float dropout_p, float negative_slope,
-                                   const uint64_t* rng_state, float* pooled_out, void* stream) {
-  const char* who = "supcon_head_store_pool_forward";
+// the element type of a layer-mean store's rows: SUPCON_F32 or SUPCON_F16 (SUPCON_BF16 is an hs / z type only)
+static int store_dtype_check(int32_t store_dtype, const char* who) {
+  if (store_dtype != SUPCON_F32 && store_dtype != SUPCON_F16)
+    return fail(SUPCON_E_INVALID, "%s: unknown store_dtype %d (SUPCON_F32 or SUPCON_F16)", who, store_dtype);
+  return 0;
+}
+
+static int store_pool_fwd(const void* store, int32_t store_dtype, int64_t n_store, int32_t feat, int32_t frames,
+                          const int64_t* idx, int32_t batch, float dropout_p, float negative_slope,
+                          const uint64_t* rng_state, float* pooled_out, void* stream, const char* who) {
+  if (int rc = store_dtype_check(store_dtype, who)) return rc;
   if (!idx) return fail(SUPCON_E_INVALID, "NULL idx passed to %s", who);
   if (n_store < 1) return fail(SUPCON_E_INVALID, "%s: bad store size %lld", who, (long long)n_store);
   if (int rc = head_pool_check(store, SUPCON_F32, batch, 1, feat, frames, dropout_p, pooled_out, who)) return rc;
@@ -638,17 +645,17 @@ int supcon_head_store_pool_forward(const float* store, int64_t n_store, int32_t 
   a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
   a.B = batch; a.F = feat; a.T = frames;
   a.dropout_p = dropout_p; a.negative_slope = negative_slope;
-  cudaError_t e = head_store_pool_forward(a, reinterpret_cast<const long long*>(idx), n_store,
+  cudaError_t e = head_store_pool_forward(a, store_dtype, reinterpret_cast<const long long*>(idx), n_store,
                                           reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "head_store_pool_fwd_kernel");
   return 0;
 }
 
-int supcon_head_sharded_store_pool_forward(const uint64_t* shard_bases, int32_t n_ranks, int64_t n_store,
-                                           int32_t feat, int32_t frames, const int64_t* idx, int32_t batch,
-                                           float dropout_p, float negative_slope, const uint64_t* rng_state,
-                                           float* pooled_out, void* stream) {
-  const char* who = "supcon_head_sharded_store_pool_forward";
+static int sharded_store_pool_fwd(const uint64_t* shard_bases, int32_t n_ranks, int32_t store_dtype,
+                                  int64_t n_store, int32_t feat, int32_t frames, const int64_t* idx, int32_t batch,
+                                  float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                  float* pooled_out, void* stream, const char* who) {
+  if (int rc = store_dtype_check(store_dtype, who)) return rc;
   if (!idx) return fail(SUPCON_E_INVALID, "NULL idx passed to %s", who);
   if (n_ranks < 1) return fail(SUPCON_E_INVALID, "%s: bad rank count %d", who, n_ranks);
   if (n_store < n_ranks)
@@ -659,11 +666,44 @@ int supcon_head_sharded_store_pool_forward(const uint64_t* shard_bases, int32_t 
   a.rng_state = reinterpret_cast<const unsigned long long*>(rng_state);
   a.B = batch; a.F = feat; a.T = frames;
   a.dropout_p = dropout_p; a.negative_slope = negative_slope;
-  cudaError_t e = head_sharded_store_pool_forward(a, reinterpret_cast<const unsigned long long*>(shard_bases),
-                                                  n_ranks, reinterpret_cast<const long long*>(idx), n_store,
+  cudaError_t e = head_sharded_store_pool_forward(a, store_dtype,
+                                                  reinterpret_cast<const unsigned long long*>(shard_bases), n_ranks,
+                                                  reinterpret_cast<const long long*>(idx), n_store,
                                                   reinterpret_cast<cudaStream_t>(stream));
   if (e != cudaSuccess) return cuda_fail(e, "head_sharded_store_pool_fwd_kernel");
   return 0;
+}
+
+int supcon_head_store_pool_forward_typed(const void* store, int32_t store_dtype, int64_t n_store, int32_t feat,
+                                         int32_t frames, const int64_t* idx, int32_t batch, float dropout_p,
+                                         float negative_slope, const uint64_t* rng_state, float* pooled_out,
+                                         void* stream) {
+  return store_pool_fwd(store, store_dtype, n_store, feat, frames, idx, batch, dropout_p, negative_slope, rng_state,
+                        pooled_out, stream, "supcon_head_store_pool_forward_typed");
+}
+
+int supcon_head_store_pool_forward(const float* store, int64_t n_store, int32_t feat, int32_t frames,
+                                   const int64_t* idx, int32_t batch, float dropout_p, float negative_slope,
+                                   const uint64_t* rng_state, float* pooled_out, void* stream) {
+  return store_pool_fwd(store, SUPCON_F32, n_store, feat, frames, idx, batch, dropout_p, negative_slope, rng_state,
+                        pooled_out, stream, "supcon_head_store_pool_forward");
+}
+
+int supcon_head_sharded_store_pool_forward_typed(const uint64_t* shard_bases, int32_t n_ranks, int32_t store_dtype,
+                                                 int64_t n_store, int32_t feat, int32_t frames, const int64_t* idx,
+                                                 int32_t batch, float dropout_p, float negative_slope,
+                                                 const uint64_t* rng_state, float* pooled_out, void* stream) {
+  return sharded_store_pool_fwd(shard_bases, n_ranks, store_dtype, n_store, feat, frames, idx, batch, dropout_p,
+                                negative_slope, rng_state, pooled_out, stream,
+                                "supcon_head_sharded_store_pool_forward_typed");
+}
+
+int supcon_head_sharded_store_pool_forward(const uint64_t* shard_bases, int32_t n_ranks, int64_t n_store,
+                                           int32_t feat, int32_t frames, const int64_t* idx, int32_t batch,
+                                           float dropout_p, float negative_slope, const uint64_t* rng_state,
+                                           float* pooled_out, void* stream) {
+  return sharded_store_pool_fwd(shard_bases, n_ranks, SUPCON_F32, n_store, feat, frames, idx, batch, dropout_p,
+                                negative_slope, rng_state, pooled_out, stream, "supcon_head_sharded_store_pool_forward");
 }
 
 int supcon_peer_push(const supcon_peer_t* pe, const void* src0, size_t bytes0, uint64_t dst_off0, const void* src1,

@@ -27,6 +27,8 @@
 // (i & 3) of the block i >> 2, i = (b*F + f)*T + t; the backward regenerates the same mask.
 #include <type_traits>
 
+#include <cuda_fp16.h>
+
 #include "supcon_common.cuh"
 #include "supcon_internal.h"
 
@@ -81,7 +83,7 @@ __device__ __forceinline__ RunView<E> run_of_block(const HeadPoolArgs& a) {
   return v;
 }
 
-// one access of VEC elements of type E: 16 bytes (float4, or eight bf16 in a uint4) or one element
+// one access of VEC elements of type E: 16 bytes (float4, or eight bf16 / fp16 in a uint4) or one element
 template <typename E, int VEC>
 struct Pack;
 template <>
@@ -92,6 +94,10 @@ template <>
 struct Pack<__nv_bfloat16, 8> { typedef uint4 type; };
 template <>
 struct Pack<__nv_bfloat16, 1> { typedef __nv_bfloat16 type; };
+template <>
+struct Pack<__half, 8> { typedef uint4 type; };
+template <>
+struct Pack<__half, 1> { typedef __half type; };
 
 // the two bf16 of a 32-bit word widened to fp32 (exact): element 2i is the low half
 __device__ __forceinline__ float bf16_lo(unsigned w) { return __uint_as_float(w << 16); }
@@ -133,14 +139,30 @@ __device__ __forceinline__ void layer_sum(const RunView<E>& v, int K, int e, flo
   for (; k < K; ++k) add_pack<E, VEC>(acc, __ldg(reinterpret_cast<const pack_t*>(p + (long long)k * v.plane)));
 }
 
-// VEC consecutive fp32 values of a stored layer-mean row, starting at run offset e
-template <int VEC>
-__device__ __forceinline__ void stored_mean(const RunView<float>& v, int e, float (&x)[VEC]) {
+// the two fp16 of a 32-bit word widened to fp32 (exact): element 2i is the low half
+__device__ __forceinline__ float2 f16x2_to_float2(unsigned w) {
+  return __half22float2(*reinterpret_cast<const __half2*>(&w));
+}
+
+// VEC consecutive values of a stored layer-mean row of element type S (fp32, or fp16 widened to fp32 exactly),
+// starting at run offset e
+template <typename S, int VEC>
+__device__ __forceinline__ void stored_mean(const RunView<S>& v, int e, float (&x)[VEC]) {
+  typedef typename Pack<S, VEC>::type pack_t;
+  const pack_t q = __ldg(reinterpret_cast<const pack_t*>(v.base + e));
   if constexpr (VEC == 4) {
-    const float4 q = __ldg(reinterpret_cast<const float4*>(v.base + e));
     x[0] = q.x; x[1] = q.y; x[2] = q.z; x[3] = q.w;
+  } else if constexpr (VEC == 8) {
+    const unsigned w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const float2 f = f16x2_to_float2(w[i]);
+      x[2 * i] = f.x; x[2 * i + 1] = f.y;
+    }
+  } else if constexpr (std::is_same<S, float>::value) {
+    x[0] = q;
   } else {
-    x[0] = __ldg(v.base + e);
+    x[0] = __half2float(q);
   }
 }
 
@@ -159,7 +181,7 @@ __device__ __forceinline__ void pool_run(const HeadPoolArgs& a, const RunView<E>
 
   for (int e = threadIdx.x * VEC; e < v.len; e += HP_THREADS * VEC) {
     float acc[VEC];
-    if constexpr (STORED) stored_mean<VEC>(v, e, acc);
+    if constexpr (STORED) stored_mean<E, VEC>(v, e, acc);
     else layer_sum<E, VEC>(v, a.K, e, acc);
 #pragma unroll
     for (int i = 0; i < VEC; ++i) {
@@ -187,39 +209,40 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_fwd_kernel(HeadPoolAr
 }
 
 // Gather-pool: batch position b reads store row idx[b] (idx on the device, so a captured graph takes new rows every
-// replay; a.K = 1).  row_of(row, plane) is the address of a row's (F, T) plane.  A row index outside [0, n_store)
-// poisons pooled row b with NaN (the other rows stay exact); nothing is read for it.
-template <int VEC, typename RowOf>
+// replay; a.K = 1).  S is the store's element type (float, or __half widened exactly on the load).  row_of(row,
+// plane) is the address of a row's (F, T) plane.  A row index outside [0, n_store) poisons pooled row b with NaN (the
+// other rows stay exact); nothing is read for it.
+template <typename S, int VEC, typename RowOf>
 __device__ __forceinline__ void store_pool_run(const HeadPoolArgs& a, const long long* __restrict__ idx,
                                                long long n_store, RowOf row_of) {
-  RunView<float> v = run_of_block<float>(a);
+  RunView<S> v = run_of_block<S>(a);
   const long long row = idx[v.b];
   if (row < 0 || row >= n_store) {
     for (int r = threadIdx.x; r < v.rows; r += HP_THREADS) a.pooled[(long long)v.b * a.F + v.f0 + r] = NAN;
     return;
   }
   v.base = row_of(row, v.plane) + (long long)v.f0 * a.T;
-  pool_run<float, VEC, true>(a, v);
+  pool_run<S, VEC, true>(a, v);
 }
 
-// a.hs = the (n_store, F, T) store
-template <int VEC>
+// a.hs = the (n_store, F, T) store of S
+template <typename S, int VEC>
 __global__ void __launch_bounds__(HP_THREADS, 4) head_store_pool_fwd_kernel(HeadPoolArgs a,
                                                                          const long long* __restrict__ idx,
                                                                          long long n_store) {
-  store_pool_run<VEC>(a, idx, n_store, [&](long long row, long long plane) {
-    return static_cast<const float*>(a.hs) + row * plane;
+  store_pool_run<S, VEC>(a, idx, n_store, [&](long long row, long long plane) {
+    return static_cast<const S*>(a.hs) + row * plane;
   });
 }
 
 // The store sharded over n_ranks GPUs: row i is local row i / n_ranks of the shard at bases[i % n_ranks], a device
-// address in this process (its own shard, or a peer's mapped over NVLink)
-template <int VEC>
+// address in this process (its own shard, or a peer's mapped over NVLink); offsets are in elements of S
+template <typename S, int VEC>
 __global__ void __launch_bounds__(HP_THREADS, 4) head_sharded_store_pool_fwd_kernel(
     HeadPoolArgs a, const unsigned long long* __restrict__ bases, int n_ranks, const long long* __restrict__ idx,
     long long n_store) {
-  store_pool_run<VEC>(a, idx, n_store, [&](long long row, long long plane) {
-    return reinterpret_cast<const float*>(bases[row % n_ranks]) + (row / n_ranks) * plane;
+  store_pool_run<S, VEC>(a, idx, n_store, [&](long long row, long long plane) {
+    return reinterpret_cast<const S*>(bases[row % n_ranks]) + (row / n_ranks) * plane;
   });
 }
 
@@ -288,7 +311,7 @@ __global__ void __launch_bounds__(HP_THREADS, 4) head_pool_bwd_kernel(HeadPoolAr
 }
 
 // 128-bit accesses need every run (and every layer plane) to start on a 16-byte boundary and to hold a multiple of
-// `width` elements (four floats, eight bf16) - including the shorter run of the last block of a row of blocks.
+// `width` elements (four floats, eight bf16 or fp16) - including the shorter run of the last block of a row of blocks.
 bool vector_ok(const HeadPoolArgs& a, const void* other, int width) {
   auto aligned = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   const long long run = (long long)a.rows_per_block * a.T;
@@ -305,8 +328,8 @@ int head_pool_rows_per_block(int F, int T, int hs_dtype) {
   int rows = 12288 / T;
   if (rows < 1) return 0;
   if (rows > 16) rows = 16;
-  // keep runs a multiple of one 128-bit access for any T: four floats, eight bf16 (from 8 rows up)
-  if (hs_dtype == SUPCON_BF16 && rows >= 8) rows &= ~7;
+  // keep runs a multiple of one 128-bit access for any T: four floats, eight 16-bit elements (from 8 rows up)
+  if ((hs_dtype == SUPCON_BF16 || hs_dtype == SUPCON_F16) && rows >= 8) rows &= ~7;
   else if (rows > 4) rows &= ~3;
   return rows < F ? rows : F;
 }
@@ -346,33 +369,51 @@ cudaError_t head_layer_mean(HeadPoolArgs a, float* rows, cudaStream_t stream) {
   return cudaGetLastError();
 }
 
-cudaError_t head_store_pool_forward(HeadPoolArgs a, const long long* idx, long long n_store, cudaStream_t stream) {
+cudaError_t head_store_pool_forward(HeadPoolArgs a, int store_dtype, const long long* idx, long long n_store,
+                                    cudaStream_t stream) {
   a.K = 1;
-  a.hs_dtype = SUPCON_F32;
+  a.hs_dtype = store_dtype;
   a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
   if (a.rows_per_block < 1) return cudaErrorInvalidValue;
   dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
   const size_t smem = (size_t)a.rows_per_block * a.T * sizeof(float);
-  if (vector_ok(a, nullptr, 4))
-    head_store_pool_fwd_kernel<4><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
-  else
-    head_store_pool_fwd_kernel<1><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+  if (store_dtype == SUPCON_F16) {
+    if (vector_ok(a, nullptr, 8))
+      head_store_pool_fwd_kernel<__half, 8><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+    else
+      head_store_pool_fwd_kernel<__half, 1><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+  } else if (vector_ok(a, nullptr, 4)) {
+    head_store_pool_fwd_kernel<float, 4><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+  } else {
+    head_store_pool_fwd_kernel<float, 1><<<grid, HP_THREADS, smem, stream>>>(a, idx, n_store);
+  }
   return cudaGetLastError();
 }
 
-cudaError_t head_sharded_store_pool_forward(HeadPoolArgs a, const unsigned long long* bases, int n_ranks,
-                                            const long long* idx, long long n_store, cudaStream_t stream) {
+cudaError_t head_sharded_store_pool_forward(HeadPoolArgs a, int store_dtype, const unsigned long long* bases,
+                                            int n_ranks, const long long* idx, long long n_store,
+                                            cudaStream_t stream) {
   a.hs = nullptr;           // the shard bases are on the device: 16-byte alignment is the caller's promise
   a.K = 1;
-  a.hs_dtype = SUPCON_F32;
+  a.hs_dtype = store_dtype;
   a.rows_per_block = head_pool_rows_per_block(a.F, a.T, a.hs_dtype);
   if (a.rows_per_block < 1) return cudaErrorInvalidValue;
   dim3 grid((a.F + a.rows_per_block - 1) / a.rows_per_block, a.B);
   const size_t smem = (size_t)a.rows_per_block * a.T * sizeof(float);
-  if (vector_ok(a, nullptr, 4))
-    head_sharded_store_pool_fwd_kernel<4><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx, n_store);
-  else
-    head_sharded_store_pool_fwd_kernel<1><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx, n_store);
+  if (store_dtype == SUPCON_F16) {
+    if (vector_ok(a, nullptr, 8))
+      head_sharded_store_pool_fwd_kernel<__half, 8><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx,
+                                                                                         n_store);
+    else
+      head_sharded_store_pool_fwd_kernel<__half, 1><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx,
+                                                                                         n_store);
+  } else if (vector_ok(a, nullptr, 4)) {
+    head_sharded_store_pool_fwd_kernel<float, 4><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx,
+                                                                                      n_store);
+  } else {
+    head_sharded_store_pool_fwd_kernel<float, 1><<<grid, HP_THREADS, smem, stream>>>(a, bases, n_ranks, idx,
+                                                                                      n_store);
+  }
   return cudaGetLastError();
 }
 

@@ -228,16 +228,20 @@ struct HeadPoolArgs {
   int B, K, F, T;
   float dropout_p, negative_slope;
   int rows_per_block;                   // filled by the launcher
-  int hs_dtype;                         // SUPCON_F32 | SUPCON_BF16: element type of hs and dhs
+  int hs_dtype;                         // SUPCON_F32 | SUPCON_BF16: element type of hs and dhs (a store's: | F16)
 };
 int head_pool_rows_per_block(int F, int T, int hs_dtype);
 cudaError_t head_pool_forward(HeadPoolArgs a, cudaStream_t stream);
 cudaError_t head_layer_mean(HeadPoolArgs a, float* rows, cudaStream_t stream);   // rows [B][F][T] fp32
-// a.hs = the fp32 (n_store, F, T) store, idx = [B] store row of each batch position
-cudaError_t head_store_pool_forward(HeadPoolArgs a, const long long* idx, long long n_store, cudaStream_t stream);
-// the same on a store sharded over n_ranks GPUs: row i at bases[i % n_ranks] + (i / n_ranks) * F * T (device table)
-cudaError_t head_sharded_store_pool_forward(HeadPoolArgs a, const unsigned long long* bases, int n_ranks,
-                                            const long long* idx, long long n_store, cudaStream_t stream);
+// a.hs = the (n_store, F, T) store of store_dtype (SUPCON_F32 | SUPCON_F16), idx = [B] store row of each batch
+// position
+cudaError_t head_store_pool_forward(HeadPoolArgs a, int store_dtype, const long long* idx, long long n_store,
+                                    cudaStream_t stream);
+// the same on a store sharded over n_ranks GPUs: row i at bases[i % n_ranks] + (i / n_ranks) * F * T elements
+// (device table)
+cudaError_t head_sharded_store_pool_forward(HeadPoolArgs a, int store_dtype, const unsigned long long* bases,
+                                            int n_ranks, const long long* idx, long long n_store,
+                                            cudaStream_t stream);
 cudaError_t head_pool_backward(HeadPoolArgs a, const float* dpooled, void* dhs, cudaStream_t stream);
 
 // tcgen05 building-block diagnostic (supcon_tc_debug.cu)

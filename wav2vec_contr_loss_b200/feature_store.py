@@ -21,11 +21,16 @@ lives on rank i % R, each rank encodes only its own clips, and ``pool`` reads th
 memory (``supcon_head_sharded_store_pool_forward``), with the same bits as ``LayerMeanStore.pool``.
 
 Preconditions: frozen encoder, no waveform augmentation, the same crop / pad of each clip in every epoch.  The rows
-are fp32 (a bf16 store would round the mean and lose that equality).  There is no backward: the store is a constant.
+are fp32 by default, which keeps that equality (a rounded mean would lose it).  ``dtype=torch.float16`` keeps them
+in fp16 instead, at half the bytes: twice the clips per GPU.  Each layer mean is then rounded once, to nearest even
+(``rows32.half()``), and the kernel widens it back exactly, so pooling an fp16 store gives bit for bit what pooling
+an fp32 store of the same widened values gives.  A finite mean beyond fp16's range (|m| >= 65520 rounds to inf) is
+an error: the build and a load raise naming the slot, and ``save`` refuses.  There is no backward: the store is a
+constant.
 
-On disk a store is a directory of two ``.npy`` files, ``rows.npy`` (n, F, T) fp32 in C order and ``labels.npy``
-(n,) int64, in slot order whatever the number of ranks that wrote it: the layout of the reference's layer-mean
-feature memmap (extract_encoder_embeddings.py).  ``save`` / ``load_layer_mean_store`` /
+On disk a store is a directory of two ``.npy`` files, ``rows.npy`` (n, F, T) in C order, fp32 (``<f4``) or for an
+fp16 store ``<f2``, and ``labels.npy`` (n,) int64, in slot order whatever the number of ranks that wrote it: the
+layout of the reference's layer-mean feature memmap (extract_encoder_embeddings.py).  ``save`` / ``load_layer_mean_store`` /
 ``load_sharded_layer_mean_store`` stream the rows between the file and the device through two pinned staging
 buffers, so the host never holds the array.
 """
@@ -47,25 +52,36 @@ __all__ = ["LayerMeanStore", "build_layer_mean_store", "ShardedLayerMeanStore", 
 
 ROWS_FILE, LABELS_FILE = "rows.npy", "labels.npy"
 STAGE_BYTES = 64 << 20      # each of the two pinned staging buffers of a save or load
+# the element types of a store's rows: C-ABI store_dtype, .npy descr, name
+_STORE_DTYPES = {torch.float32: (_cabi.F32, "<f4", "fp32"), torch.float16: (_cabi.F16, "<f2", "fp16")}
+
+
+def _store_dtype(dtype) -> torch.dtype:
+    if dtype not in _STORE_DTYPES:
+        raise ValueError(f"the store dtype must be torch.float32 or torch.float16, got {dtype}")
+    return dtype
 
 
 class LayerMeanStore:
-    """``rows`` (n, F, T) fp32 and ``labels`` (n,) int64, both on one device; slots ``[0, filled)`` are written.
+    """``rows`` (n, F, T) of ``dtype`` (fp32, or fp16 at half the bytes: module docstring) and ``labels`` (n,)
+    int64, both on one device; slots ``[0, filled)`` are written.
 
     ``append`` writes the layer means of a batch of hidden states at the next ``B`` slots.  ``pool`` and
     ``labels_of`` take a device int64 index vector, so both can be captured in a CUDA graph and fed new indices
     every replay.  An index outside ``[0, filled)`` gives a NaN pooled row (the loss turns NaN) instead of a fault."""
 
-    def __init__(self, n: int, feat: int, frames: int, device):
+    def __init__(self, n: int, feat: int, frames: int, device, dtype=torch.float32):
         if n < 1 or feat < 1 or frames < 1:
             raise ValueError(f"bad store shape ({n}, {feat}, {frames})")
+        dtype = _store_dtype(dtype)
         device = torch.device(device)
-        too_big = _fit_error(n, feat, frames, device, store_bytes(n, feat, frames))
+        too_big = _fit_error(n, feat, frames, device, store_bytes(n, feat, frames, dtype), dtype)
         if too_big:
             raise MemoryError(too_big)
-        self.rows = torch.empty((n, feat, frames), dtype=torch.float32, device=device)
+        self.rows = torch.empty((n, feat, frames), dtype=dtype, device=device)
         self.labels = torch.full((n,), -1, dtype=torch.int64, device=device)
         self.filled = 0
+        self._rounding = _Rounding(self.rows)
 
     @property
     def n(self) -> int:
@@ -83,16 +99,22 @@ class LayerMeanStore:
     def device(self) -> torch.device:
         return self.rows.device
 
+    @property
+    def dtype(self) -> torch.dtype:
+        return self.rows.dtype
+
     def append(self, hs: torch.Tensor, labels: torch.Tensor) -> int:
         """Write ``mean_k hs[b, k]`` (hs = (B, K, F, T), fp32 or bf16; other dtypes through an fp32 copy) and
-        ``labels[b]`` at slot ``filled + b``; returns the first slot written."""
+        ``labels[b]`` at slot ``filled + b``; returns the first slot written.  An fp16 store rounds the fp32 mean to
+        nearest even and notes, on the device, a finite mean that became inf (``build_layer_mean_store`` and
+        ``save`` raise on it)."""
         b = _check_hs(hs, self.feat, self.frames, self.filled)
         if tuple(labels.shape) != (b,):
             raise ValueError(f"labels must be ({b},), got {tuple(labels.shape)}")
         if self.filled + b > self.n:
             raise ValueError(f"the store holds {self.n} clips: no room for {b} more after {self.filled}")
         slot0 = self.filled
-        write_layer_means(self.rows, slot0, hs)
+        self._rounding.write_means(slot0, hs)
         self.labels[slot0:slot0 + b].copy_(labels.detach().long(), non_blocking=True)
         self.filled += b
         return slot0
@@ -109,25 +131,29 @@ class LayerMeanStore:
         idx, rng = _pool_args(self.rows, idx, dropout_p, rng_state)
         with torch.cuda.device(self.device):
             pooled = torch.empty((idx.shape[0], self.feat), dtype=torch.float32, device=self.device)
-            _cabi.check(_cabi.load().supcon_head_store_pool_forward(
-                Fn._p(self.rows), self.filled, self.feat, self.frames, Fn._p(idx), idx.shape[0], float(dropout_p),
-                float(negative_slope), Fn._p(rng), Fn._p(pooled), Fn._stream(self.device)),
-                "supcon_head_store_pool_forward")
+            _cabi.check(_cabi.load().supcon_head_store_pool_forward_typed(
+                Fn._p(self.rows), _STORE_DTYPES[self.dtype][0], self.filled, self.feat, self.frames, Fn._p(idx),
+                idx.shape[0], float(dropout_p), float(negative_slope), Fn._p(rng), Fn._p(pooled),
+                Fn._stream(self.device)), "supcon_head_store_pool_forward_typed")
         return pooled
 
     def save(self, path, overwrite: bool = False):
         """Write slots ``[0, filled)`` to the directory ``path`` (``rows.npy``, ``labels.npy``; module docstring).
         The files are written into ``<path>.partial``, fsynced and then renamed to ``path``, so a save that dies
         leaves nothing that loads.  An existing ``path`` is kept unless ``overwrite`` (as ``export_embeddings``
-        keeps its files): returns None then, else the number of clips written.  Raises on an empty store."""
+        keeps its files): returns None then, else the number of clips written.  Raises on an empty store and on an
+        fp16 store holding a mean that rounded to inf."""
         path = os.fspath(path)
         if self.filled < 1:
             raise ValueError("the store is empty: nothing to save")
+        bad = self._rounding.first_overflow()
+        if bad is not None:
+            raise ValueError(_overflow_message(bad) + ": not saved")
         if os.path.exists(path) and not overwrite:
             return None
         partial = path + ".partial"
         try:
-            header = _create_rows_file(partial, (self.filled, self.feat, self.frames))
+            header = _create_rows_file(partial, (self.filled, self.feat, self.frames), _STORE_DTYPES[self.dtype][1])
             _write_rows(self.rows, range(self.filled), partial, header)
             _finish_save(partial, path, self.labels[:self.filled])
         except BaseException:
@@ -136,43 +162,100 @@ class LayerMeanStore:
         return self.filled
 
     @classmethod
-    def from_arrays(cls, rows, labels, device) -> "LayerMeanStore":
-        """A store of ``n == filled`` clips from host arrays: ``rows`` (n, F, T) float32 (copied bit for bit) or
-        float16 (widened exactly) as a numpy array, memmap or CPU tensor, ``labels`` (n,) integers.  A memmap of a
-        whole ``.npy`` file is read from the file in chunks, any other array copied in chunks; either way through
-        the pinned staging buffers, never as a whole.  Raises on another dtype (float64 would round), another rank
-        and labels that are not (n,) integers."""
+    def from_arrays(cls, rows, labels, device, dtype=torch.float32) -> "LayerMeanStore":
+        """A store of ``n == filled`` clips from host arrays: ``rows`` (n, F, T) float32 or float16 as a numpy
+        array, memmap or CPU tensor, ``labels`` (n,) integers.  Into the default fp32 store float32 is copied bit
+        for bit and float16 widened exactly; into an fp16 store (``dtype=torch.float16``) float16 is copied bit for
+        bit and float32 rounded to nearest even on the store's device (``rows.half()``).  A memmap of a whole
+        ``.npy`` file is read from the file in chunks, any other array copied in chunks; either way through the
+        pinned staging buffers, never as a whole.  Raises on another dtype (float64 would round), another rank,
+        labels that are not (n,) integers and a float32 value that rounds to inf in fp16 (naming the file and the
+        slot)."""
         src = _RowSource(rows)
         lab = _label_tensor(labels, src.n)
-        store = cls(src.n, src.feat, src.frames, device)
-        _read_rows(src, range(src.n), store.rows)
+        store = cls(src.n, src.feat, src.frames, device, dtype)
+        _read_rows(src, range(src.n), store._rounding)
+        bad = store._rounding.first_overflow()
+        if bad is not None:
+            raise ValueError(f"{src.name}: {_overflow_message(bad)}")
         store.labels.copy_(lab)
         store.filled = src.n
         return store
 
 
-def load_layer_mean_store(path, device) -> LayerMeanStore:
+def load_layer_mean_store(path, device, dtype=torch.float32) -> LayerMeanStore:
     """The store that ``LayerMeanStore.save`` or ``ShardedLayerMeanStore.save`` (any number of ranks) wrote to
     ``path``, or layer means extracted elsewhere in that layout, on ``device``: ``n == filled ==`` the file's row
-    count.  Raises FileNotFoundError on a missing store and ValueError naming the file on a truncated or unreadable
-    one, besides the checks of ``LayerMeanStore.from_arrays``."""
-    return LayerMeanStore.from_arrays(*_open_store(path), device)
+    count; ``dtype`` the store's (``from_arrays``), whatever the file's.  Raises FileNotFoundError on a missing store
+    and ValueError naming the file on a truncated or unreadable one, besides the checks of
+    ``LayerMeanStore.from_arrays``."""
+    return LayerMeanStore.from_arrays(*_open_store(path), device, dtype)
 
 
-def store_bytes(n: int, feat: int, frames: int) -> int:
-    """device bytes of a store of n clips: fp32 rows and int64 labels"""
-    return n * feat * frames * 4 + n * 8
+def store_bytes(n: int, feat: int, frames: int, dtype=torch.float32) -> int:
+    """device bytes of a store of n clips: rows of ``dtype`` (4 or 2 bytes an element) and int64 labels"""
+    return n * feat * frames * _store_dtype(dtype).itemsize + n * 8
 
 
-def _fit_error(n: int, feat: int, frames: int, device: torch.device, need: int) -> str:
+def _fit_error(n: int, feat: int, frames: int, device: torch.device, need: int, dtype=torch.float32) -> str:
     """why ``need`` bytes for a store of n clips do not fit the free memory of ``device`` ("" when they do)"""
     if device.type != "cuda":
         return ""
     free, _ = torch.cuda.mem_get_info(device)
     if need <= free:
         return ""
-    return (f"a store of {n} clips x ({feat}, {frames}) fp32 takes {need / 1e9:.2f} GB; {free / 1e9:.2f} GB are free "
-            f"on {device}")
+    return (f"a store of {n} clips x ({feat}, {frames}) {_STORE_DTYPES[dtype][2]} takes {need / 1e9:.2f} GB; "
+            f"{free / 1e9:.2f} GB are free on {device}")
+
+
+def _overflow_message(slot: int) -> str:
+    return (f"slot {slot}: a finite layer mean rounds to inf in fp16 (largest finite value 65504); "
+            f"keep this store in fp32")
+
+
+class _Rounding:
+    """Writes fp32 values into the rows of a store.  An fp32 store takes them as they are; an fp16 store rounds them
+    to nearest even (torch's ``copy_``, so the rows equal ``rows32.half()``) and keeps on the device the first
+    element where a finite value became inf: no host sync until ``first_overflow``.  Shared by ``append``, the
+    sharded build and the loads."""
+    NONE = 1 << 62
+
+    def __init__(self, rows: torch.Tensor):
+        self.rows = rows
+        self.row = rows.shape[1] * rows.shape[2]
+        self.scratch = None                                  # fp16: (B, F, T) fp32 layer means, kept between calls
+        self.first = (torch.full((), self.NONE, dtype=torch.int64, device=rows.device)
+                      if rows.dtype == torch.float16 else None)
+
+    def write_means(self, row0: int, hs: torch.Tensor) -> None:
+        """``rows[row0 + b] = mean_k hs[b, k]`` with ``write_layer_means``: in place, or for fp16 through the fp32
+        scratch and ``put``"""
+        if self.first is None:
+            write_layer_means(self.rows, row0, hs)
+            return
+        b = hs.shape[0]
+        if self.scratch is None or self.scratch.shape[0] < b:
+            self.scratch = torch.empty((b,) + tuple(self.rows.shape[1:]), dtype=torch.float32,
+                                       device=self.rows.device)
+        write_layer_means(self.scratch, 0, hs)
+        self.put(row0 * self.row, self.scratch[:b].view(-1))
+
+    def put(self, offset: int, src: torch.Tensor) -> None:
+        """the rows' flat elements ``[offset, offset + src.numel())`` = ``src`` (fp32, on the rows' device),
+        rounded to the store dtype, in the current stream"""
+        dst = self.rows.view(-1)[offset:offset + src.numel()]
+        dst.copy_(src)
+        if self.first is None:
+            return
+        hit, i = (dst.isinf() & src.isfinite()).to(torch.uint8).max(0)       # i: the first hit, if any
+        torch.minimum(self.first, torch.where(hit.bool(), i + offset, self.NONE), out=self.first)
+
+    def first_overflow(self):
+        """the first row holding a finite value rounded to inf, or None (always None for fp32; syncs for fp16)"""
+        if self.first is None:
+            return None
+        first = int(self.first)
+        return None if first == self.NONE else first // self.row
 
 
 def _check_hs(hs: torch.Tensor, feat: int, frames: int, slot0: int) -> int:
@@ -224,14 +307,16 @@ def _labels_of(labels: torch.Tensor, filled: int, idx: torch.Tensor) -> torch.Te
 
 
 @torch.no_grad()
-def build_layer_mean_store(encoder, loader, device, *, label_index: int = 1, n=None) -> LayerMeanStore:
+def build_layer_mean_store(encoder, loader, device, *, label_index: int = 1, n=None,
+                           dtype=torch.float32) -> LayerMeanStore:
     """Run ``encoder`` once over ``loader`` as ``stage1.train_one_epoch`` runs a frozen one (eval mode, no grad,
     ``attention_mask = (waveforms != 0).long()``) and store each clip's layer mean.  Slot i holds the loader's i-th
     clip, so a sequential loader over the dataset gives slot = dataset index.  ``n`` (default
     ``len(loader.dataset)``) is the number of clips to allocate for; a loader that yields fewer leaves the store
     ``filled`` short of ``n``.  Raises on a clip whose (F, T) differs from the first one, on more clips than ``n``
     and on a store that does not fit the device's free memory.  ``label_index`` picks the label column of the batch
-    tuple, as in ``train_one_epoch``."""
+    tuple, as in ``train_one_epoch``.  ``dtype`` is the store's (``LayerMeanStore``); an fp16 store raises at the
+    end, naming the first slot, when a finite layer mean rounded to inf."""
     from .stage1 import _to_device
     if n is None:
         dataset = getattr(loader, "dataset", None)
@@ -244,10 +329,13 @@ def build_layer_mean_store(encoder, loader, device, *, label_index: int = 1, n=N
         waveforms, labels = _to_device(batch[0], batch[label_index], device)
         hs = encoder(waveforms, attention_mask=(waveforms != 0.0).long())
         if store is None:
-            store = LayerMeanStore(n, hs.shape[-2], hs.shape[-1], device)
+            store = LayerMeanStore(n, hs.shape[-2], hs.shape[-1], device, dtype)
         store.append(hs, labels)
     if store is None:
         raise ValueError("the loader yielded no clips")
+    bad = store._rounding.first_overflow()
+    if bad is not None:
+        raise ValueError(_overflow_message(bad))
     return store
 
 
@@ -272,23 +360,25 @@ def _agree(problem, group) -> None:
 
 
 class _SymmetricShard:
-    """This rank's (rows, F, T) fp32 shard in symmetric memory (``torch.distributed._symmetric_memory``, as the peer
-    exchange of ``distributed.py`` allocates its buffers): the same size on every rank and mapped into every process,
-    so ``bases[r]`` is rank r's shard as seen from this one."""
+    """This rank's (rows, F, T) shard of ``dtype`` in symmetric memory (``torch.distributed._symmetric_memory``, as
+    the peer exchange of ``distributed.py`` allocates its buffers): the same size on every rank and mapped into every
+    process, so ``bases[r]`` is rank r's shard as seen from this one."""
 
-    def __init__(self, rows: int, feat: int, frames: int, device, group):
+    def __init__(self, rows: int, feat: int, frames: int, device, group, *, dtype=torch.float32):
         import torch.distributed._symmetric_memory as symm
         problem = None
         try:
-            self.buf = symm.empty(rows * feat * frames, dtype=torch.float32, device=device)
+            self.buf = symm.empty(rows * feat * frames, dtype=dtype, device=device)
         except Exception as exc:  # noqa: BLE001  (refused by the allocator: every rank must hear of it)
-            self.buf, problem = None, RuntimeError(f"symmetric allocation of {rows} x ({feat}, {frames}) fp32: {exc}")
+            self.buf, problem = None, RuntimeError(f"symmetric allocation of {rows} x ({feat}, {frames}) "
+                                                   f"{_STORE_DTYPES[dtype][2]}: {exc}")
         _agree(problem, group)
         self.handle = symm.rendezvous(self.buf, group if group is not None else dist.group.WORLD)
         self.rows = self.buf.view(rows, feat, frames)
         self.bases = [int(p) for p in self.handle.buffer_ptrs]
 
     def write(self, row0: int, hs: torch.Tensor) -> None:
+        """fp32 shards: ``rows[row0 + b] = mean_k hs[b, k]`` (the store writes an fp16 shard itself)"""
         write_layer_means(self.rows, row0, hs)
 
     def close(self) -> None:
@@ -307,19 +397,26 @@ class ShardedLayerMeanStore:
     Construction is collective: every rank passes the same (n, feat, frames) with its own device.  The checks --
     n >= R, the same shape on every rank, the shard fits free memory, one host, every pair of GPUs peer-capable --
     are agreed on first and raise on every rank.  ``close()`` (collective) releases the mapping; call it before
-    ``destroy_process_group``.  ``allocate`` replaces the symmetric allocation (tests without a GPU)."""
+    ``destroy_process_group``.  ``allocate`` replaces the symmetric allocation (tests without a GPU): it is called
+    as ``allocate(local_rows, feat, frames, device, group)``, with ``dtype=torch.float16`` added for an fp16 store.
+    ``dtype`` (the same on every rank) is the rows' element type, as in ``LayerMeanStore``."""
 
-    def __init__(self, n: int, feat: int, frames: int, device, group=None, *, allocate=None):
+    def __init__(self, n: int, feat: int, frames: int, device, group=None, *, allocate=None, dtype=torch.float32):
         self.group = group
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
         device = torch.device(device)
         self.n, self.feat, self.frames = n, feat, frames
         self.local_rows = -(-n // self.world) if n > 0 else 0
         where = [None] * self.world
-        dist.all_gather_object(where, ((n, feat, frames), socket.gethostname(), device.index), group=group)
-        _agree(self._local_problem(device, where), group)
-        self._shard = (allocate or _SymmetricShard)(self.local_rows, feat, frames, device, group)
+        dist.all_gather_object(where, ((n, feat, frames), socket.gethostname(), device.index, str(dtype)),
+                               group=group)
+        _agree(self._local_problem(device, where, dtype), group)
+        self.dtype = dtype
+        alloc = allocate or _SymmetricShard
+        kw = {} if dtype == torch.float32 else {"dtype": dtype}
+        self._shard = alloc(self.local_rows, feat, frames, device, group, **kw)
         self.rows = self._shard.rows
+        self._rounding = _Rounding(self.rows)
         self.bases = torch.tensor(self._shard.bases, dtype=torch.int64, device=device)
         self.labels = torch.full((n,), -1, dtype=torch.int64, device=device)
         self.filled = 0
@@ -328,28 +425,37 @@ class ShardedLayerMeanStore:
     def device(self) -> torch.device:
         return self.labels.device
 
-    def _local_problem(self, device, where):
-        """this rank's failed precondition, or None; ``where`` = every rank's ((n, F, T), host, device index)"""
+    def _local_problem(self, device, where, dtype):
+        """this rank's failed precondition, or None; ``where`` = every rank's ((n, F, T), host, device index,
+        dtype)"""
         if self.n < self.world:
             return ValueError(f"a store sharded over {self.world} ranks needs at least {self.world} clips, "
                               f"got {self.n}")
-        shapes = [s for s, _, _ in where]
+        shapes = [w[0] for w in where]
         if len(set(shapes)) != 1:
             return ValueError("the ranks disagree on the store's (n, F, T): " +
                               ", ".join(f"rank {r} {s}" for r, s in enumerate(shapes)))
+        kinds = [w[3] for w in where]
+        if len(set(kinds)) != 1:
+            return ValueError("the ranks disagree on the store dtype: " +
+                              ", ".join(f"rank {r} {k}" for r, k in enumerate(kinds)))
+        try:
+            _store_dtype(dtype)
+        except ValueError as exc:
+            return exc
         if self.feat < 1 or self.frames < 1:
             return ValueError(f"bad store shape ({self.n}, {self.feat}, {self.frames})")
         too_big = _fit_error(self.local_rows, self.feat, self.frames, device,
-                             store_bytes(self.local_rows, self.feat, self.frames) + self.n * 8)
+                             store_bytes(self.local_rows, self.feat, self.frames, dtype) + self.n * 8, dtype)
         if too_big:
             return MemoryError(f"the shard of {too_big}")
         if device.type != "cuda":
             return None
         # the shards are read over NVLink: one host, and this GPU reaches every other rank's
         alone = "; a sharded store needs the GPUs of one node with peer access: use feature_store.LayerMeanStore"
-        if len({h for _, h, _ in where}) != 1:
+        if len({w[1] for w in where}) != 1:
             return RuntimeError("the ranks run on several hosts" + alone)
-        blocked = [r for r, (_, _, d) in enumerate(where)
+        blocked = [r for r, (_, _, d, _) in enumerate(where)
                    if d != device.index and not torch.cuda.can_device_access_peer(device.index, d)]
         if blocked:
             return RuntimeError(f"cuda:{device.index} has no peer access to the GPU of rank(s) {blocked}" + alone)
@@ -369,11 +475,25 @@ class ShardedLayerMeanStore:
         idx, rng = _pool_args(self.rows, idx, dropout_p, rng_state)
         with torch.cuda.device(self.device):
             pooled = torch.empty((idx.shape[0], self.feat), dtype=torch.float32, device=self.device)
-            _cabi.check(_cabi.load().supcon_head_sharded_store_pool_forward(
-                Fn._p(self.bases), self.world, self.filled, self.feat, self.frames, Fn._p(idx), idx.shape[0],
-                float(dropout_p), float(negative_slope), Fn._p(rng), Fn._p(pooled), Fn._stream(self.device)),
-                "supcon_head_sharded_store_pool_forward")
+            _cabi.check(_cabi.load().supcon_head_sharded_store_pool_forward_typed(
+                Fn._p(self.bases), self.world, _STORE_DTYPES[self.dtype][0], self.filled, self.feat, self.frames,
+                Fn._p(idx), idx.shape[0], float(dropout_p), float(negative_slope), Fn._p(rng), Fn._p(pooled),
+                Fn._stream(self.device)), "supcon_head_sharded_store_pool_forward_typed")
         return pooled
+
+    def _write(self, row0: int, hs: torch.Tensor) -> None:
+        """local rows ``row0 + b`` = the layer means of hs: through the allocation's own ``write`` for fp32, through
+        ``_Rounding`` (as ``LayerMeanStore.append``) for fp16"""
+        if self.dtype == torch.float32:
+            self._shard.write(row0, hs)
+        else:
+            self._rounding.write_means(row0, hs)
+
+    def _overflow_problem(self, where: str = ""):
+        """a ValueError naming the first slot of this rank whose fp16 row holds a finite value rounded to inf, or
+        None"""
+        bad = self._rounding.first_overflow()
+        return None if bad is None else ValueError(where + _overflow_message(self.rank + bad * self.world))
 
     def gather_labels(self, local_labels: torch.Tensor) -> None:
         """``labels`` = every rank's ``local_labels`` (ceil(n / R),) in slot order, through one all-gather"""
@@ -403,12 +523,15 @@ class ShardedLayerMeanStore:
         path = os.fspath(path)
         if self.filled < 1:
             raise ValueError("the store is empty: nothing to save")
+        problem = self._overflow_problem()
+        _agree(problem and ValueError(f"{problem}: not saved"), self.group)
         seen = [None] * self.world
         dist.all_gather_object(seen, os.path.exists(path), group=self.group)
         if seen[0] and not overwrite:
             return None
         partial, lead = path + ".partial", self.rank == 0
-        header = len(_npy_header((self.filled, self.feat, self.frames)))
+        descr = _STORE_DTYPES[self.dtype][1]
+        header = len(_npy_header((self.filled, self.feat, self.frames), descr))
 
         def step(fn):
             problem = None
@@ -423,17 +546,18 @@ class ShardedLayerMeanStore:
                     _discard(partial)
                 raise
 
-        step(lambda: _create_rows_file(partial, (self.filled, self.feat, self.frames)) if lead else None)
+        step(lambda: _create_rows_file(partial, (self.filled, self.feat, self.frames), descr) if lead else None)
         step(lambda: _write_rows(self.rows, shard_slots(self.filled, self.rank, self.world), partial, header))
         step(lambda: _finish_save(partial, path, self.labels[:self.filled]) if lead else None)
         return self.filled
 
     @classmethod
-    def from_arrays(cls, rows, labels, device, group=None, *, allocate=None) -> "ShardedLayerMeanStore":
+    def from_arrays(cls, rows, labels, device, group=None, *, allocate=None,
+                    dtype=torch.float32) -> "ShardedLayerMeanStore":
         """``LayerMeanStore.from_arrays`` split over the ranks of ``group`` (collective): every rank passes the
         whole (n, F, T) array (typically a memmap of the same file) and reads only its slots
-        ``shard_slots(n, rank, R)`` into its shard, in place.  Besides ``from_arrays``' checks and the
-        constructor's, the ranks must agree on the dtype; every check raises on every rank."""
+        ``shard_slots(n, rank, R)`` into its shard, in place; ``dtype`` is the store's.  Besides ``from_arrays``'
+        checks and the constructor's, the ranks must agree on the rows' dtype; every check raises on every rank."""
         src, lab, problem = None, None, None
         try:
             src = _RowSource(rows)
@@ -446,10 +570,11 @@ class ShardedLayerMeanStore:
         if len(set(kinds)) != 1:
             raise ValueError("the ranks disagree on the rows' dtype: " +
                              ", ".join(f"rank {r} {k}" for r, k in enumerate(kinds)))
-        store = cls(src.n, src.feat, src.frames, device, group, allocate=allocate)
+        store = cls(src.n, src.feat, src.frames, device, group, allocate=allocate, dtype=dtype)
         problem = None
         try:
-            _read_rows(src, shard_slots(store.n, store.rank, store.world), store.rows)
+            _read_rows(src, shard_slots(store.n, store.rank, store.world), store._rounding)
+            problem = store._overflow_problem(f"{src.name}: ")
             store.labels.copy_(lab)
         except (OSError, ValueError, RuntimeError) as exc:
             problem = exc
@@ -464,14 +589,16 @@ class ShardedLayerMeanStore:
 
 @torch.no_grad()
 def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=None, label_index: int = 1,
-                                   allocate=None) -> ShardedLayerMeanStore:
+                                   allocate=None, dtype=torch.float32) -> ShardedLayerMeanStore:
     """``build_layer_mean_store`` split over the ranks of ``group`` (collective): each rank runs ``encoder`` on its
     own share of the n clips, so the build takes 1 / R of the time and the node holds R times the clips.
     ``loader`` yields this rank's clips in the order ``shard_slots(n, rank, R)`` lists them (e.g. a
     ``DataLoader(Subset(dataset, shard_slots(...)), shuffle=False)``); the encoder is called as
     ``build_layer_mean_store`` calls it.  Raises on every rank when the ranks' (F, T) differ, a shard does not fit
     free memory, a rank's loader yields more or fewer clips than its share, n < R, or the GPUs cannot reach each
-    other's memory.  Afterwards ``filled == n`` and ``labels`` holds every slot's label on every rank."""
+    other's memory, and, for an fp16 store (``dtype``, the same on every rank), when a finite layer mean rounded to
+    inf (naming the first such slot of each rank).  Afterwards ``filled == n`` and ``labels`` holds every slot's
+    label on every rank."""
     from .stage1 import _to_device
     world, rank = dist.get_world_size(group), dist.get_rank(group)
     encoder.eval()
@@ -484,7 +611,7 @@ def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=Non
     first = next(batches, None)
     hs, labels = encoded(first) if first is not None else (None, None)
     shape = tuple(hs.shape[-2:]) if hs is not None else (0, 0)
-    store = ShardedLayerMeanStore(n, *shape, device, group, allocate=allocate)
+    store = ShardedLayerMeanStore(n, *shape, device, group, allocate=allocate, dtype=dtype)
     share = len(shard_slots(n, rank, world))
     local_labels = torch.full((store.local_rows,), -1, dtype=torch.int64, device=store.device)
     filled, problem = 0, None
@@ -495,13 +622,14 @@ def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=Non
                 raise ValueError(f"labels must be ({b},), got {tuple(labels.shape)}")
             if filled + b > share:
                 raise ValueError(f"the loader yields more than this rank's {share} clips of {n}")
-            store._shard.write(filled, hs)
+            store._write(filled, hs)
             local_labels[filled:filled + b].copy_(labels.detach().long(), non_blocking=True)
             filled += b
             batch = next(batches, None)
             hs, labels = encoded(batch) if batch is not None else (None, None)
         if filled != share:
             raise ValueError(f"the loader yielded {filled} clips, this rank's share of {n} is {share}")
+        problem = store._overflow_problem()
     except ValueError as exc:
         problem = exc
     try:
@@ -514,18 +642,19 @@ def build_sharded_layer_mean_store(encoder, loader, device, *, n: int, group=Non
     return store
 
 
-def load_sharded_layer_mean_store(path, device, group=None, *, allocate=None) -> ShardedLayerMeanStore:
+def load_sharded_layer_mean_store(path, device, group=None, *, allocate=None,
+                                  dtype=torch.float32) -> ShardedLayerMeanStore:
     """``load_layer_mean_store`` into a store sharded over the ranks of ``group`` (collective): the file may have
     been written by any number of ranks, one included, and rank r reads only its own slots.  A missing, truncated
     or unreadable file on any rank raises on every rank, as do the checks of ``ShardedLayerMeanStore.from_arrays``.
-    ``allocate`` as in ``ShardedLayerMeanStore``."""
+    ``allocate`` and ``dtype`` as in ``ShardedLayerMeanStore``."""
     arrays, problem = None, None
     try:
         arrays = _open_store(path)
     except (OSError, ValueError) as exc:
         problem = exc
     _agree(problem, group)
-    return ShardedLayerMeanStore.from_arrays(*arrays, device, group, allocate=allocate)
+    return ShardedLayerMeanStore.from_arrays(*arrays, device, group, allocate=allocate, dtype=dtype)
 
 
 # ---------------------------------------------------------------------------------- the store on disk
@@ -549,7 +678,7 @@ def _open_store(path):
 
 class _RowSource:
     """(n, F, T) float32 or float16 rows from the host: a memmap of a whole file (what np.load returns) is read from
-    the file with readinto, which keeps its pages out of this process; any other array is copied row by row."""
+    the file with preadv, which keeps its pages out of this process; any other array is copied row by row."""
 
     def __init__(self, rows):
         if isinstance(rows, torch.Tensor):
@@ -569,14 +698,17 @@ class _RowSource:
         if (isinstance(rows, np.memmap) and isinstance(rows.base, mmap.mmap) and rows.flags.c_contiguous
                 and rows.filename):
             self.file, self.offset = rows.filename, rows.offset
-        # float16 is read here and widened into the fp32 staging buffer (exact); float32 is read into it directly
-        self.raw = None if rows.dtype == np.float32 else np.empty(0, np.float16)
+        self.name = self.file or "rows"
+        # a float16 source bound for a float32 staging buffer is read here and widened (exact)
+        self.raw = np.empty(0, rows.dtype)
 
     def fill(self, out: np.ndarray, pieces, fd) -> None:
-        """``out`` (m,) fp32 = the source's elements ``pieces`` [(flat offset, count), ...] in order"""
-        if self.raw is not None and self.raw.size < out.size:
-            self.raw = np.empty(out.size, np.float16)
-        dst = out if self.raw is None else self.raw[:out.size]
+        """``out`` (m,) = the source's elements ``pieces`` [(flat offset, count), ...] in order: ``out`` has the
+        source's dtype, or is float32 for a float16 source"""
+        widen = out.dtype != self.rows.dtype
+        if widen and self.raw.size < out.size:
+            self.raw = np.empty(out.size, self.rows.dtype)
+        dst = self.raw[:out.size] if widen else out
         pos = 0
         for start, count in pieces:
             if fd is not None:
@@ -589,7 +721,7 @@ class _RowSource:
                     np.copyto(dst[pos + done:pos + done + k], self.rows[i].reshape(-1)[lo:lo + k])
                     done += k
             pos += count
-        if self.raw is not None:
+        if widen:
             np.copyto(out, dst)
 
 
@@ -636,14 +768,19 @@ def _chunks(slots, row: int, chunk: int):
 
 
 class _Staging:
-    """Two fp32 host buffers of ``STAGE_BYTES`` (pinned when the store is on a GPU) and a side stream for their
-    copies to and from the device, each a ``cudaMemcpyAsync``; an event per buffer guards its reuse, so the file
-    I/O of one chunk overlaps the copy of the other."""
+    """Two host byte buffers of ``STAGE_BYTES`` (pinned when the store is on a GPU), each holding a chunk of
+    elements of ``dtype``, and a side stream for their copies to and from the device, each a ``cudaMemcpyAsync``;
+    an event per buffer guards its reuse, so the file I/O of one chunk overlaps the copy of the other.  ``rounded``
+    adds a device fp32 buffer per host buffer, for chunks that ``round`` puts into an fp16 store."""
 
-    def __init__(self, device):
-        self.chunk = max(STAGE_BYTES // 4, 1)
+    def __init__(self, device, dtype=torch.float32, rounded: bool = False):
+        self.dtype = dtype
+        self.chunk = max(STAGE_BYTES // dtype.itemsize, 1)
         self.cuda = device.type == "cuda"
-        self.bufs = [torch.empty(self.chunk, dtype=torch.float32, pin_memory=self.cuda) for _ in range(2)]
+        self.bufs = [torch.empty(self.chunk * dtype.itemsize, dtype=torch.uint8, pin_memory=self.cuda)
+                     for _ in range(2)]
+        self.dev = ([torch.empty(self.chunk, dtype=torch.float32, device=device) for _ in range(2)]
+                    if rounded and self.cuda else None)
         self.events = [None, None]
         if self.cuda:
             self.stream = torch.cuda.Stream(device)
@@ -653,7 +790,7 @@ class _Staging:
         """the buffer of chunk c, once the last copy into or out of it has completed"""
         if self.events[c % 2] is not None:
             self.events[c % 2].synchronize()
-        return self.bufs[c % 2]
+        return self.bufs[c % 2].view(self.dtype)
 
     def copy(self, c: int, dst: torch.Tensor, src: torch.Tensor) -> None:
         if not self.cuda:
@@ -664,22 +801,41 @@ class _Staging:
             self.events[c % 2] = torch.cuda.Event()
             self.events[c % 2].record(self.stream)
 
+    def round(self, c: int, rounding: "_Rounding", offset: int, src: torch.Tensor) -> None:
+        """``rounding.put(offset, src)`` of the host fp32 chunk ``src``, on the device"""
+        if not self.cuda:
+            rounding.put(offset, src)
+            return
+        with torch.cuda.stream(self.stream):
+            dev = self.dev[c % 2][:src.numel()]
+            dev.copy_(src, non_blocking=True)
+            rounding.put(offset, dev)
+            self.events[c % 2] = torch.cuda.Event()
+            self.events[c % 2].record(self.stream)
+
     def finish(self) -> None:
         if self.cuda:
             self.stream.synchronize()
 
 
-def _read_rows(src: _RowSource, slots, rows: torch.Tensor) -> None:
-    """``rows[j] = src[slots[j]]`` (rows contiguous fp32, on a GPU or the CPU); returns when the copies are done"""
-    dst = rows.view(-1)
-    st = _Staging(rows.device)
+def _read_rows(src: _RowSource, slots, rounding: "_Rounding") -> None:
+    """``rows[j] = src[slots[j]]`` for the rows of ``rounding`` (contiguous, on a GPU or the CPU); returns when the
+    copies are done.  The chunks travel in the source's dtype, except a float16 source for an fp32 store (widened on
+    the host, exactly); a float32 source for an fp16 store is rounded on the device by ``rounding.put``."""
+    dst = rounding.rows.view(-1)
+    rounded = rounding.rows.dtype == torch.float16 and src.rows.dtype == np.float32
+    wire = torch.float16 if rounding.rows.dtype == torch.float16 and not rounded else torch.float32
+    st = _Staging(dst.device, wire, rounded)
     fd = os.open(src.file, os.O_RDONLY) if src.file else None
     try:
         for c, (d0, pieces) in enumerate(_chunks(slots, src.row, st.chunk)):
             m = sum(k for _, k in pieces)
             buf = st.host(c)[:m]
             src.fill(buf.numpy(), pieces, fd)
-            st.copy(c, dst[d0:d0 + m], buf)
+            if rounded:
+                st.round(c, rounding, d0, buf)
+            else:
+                st.copy(c, dst[d0:d0 + m], buf)
         st.finish()
     finally:
         if fd is not None:
@@ -691,7 +847,7 @@ def _write_rows(rows: torch.Tensor, slots, partial: str, header: int) -> None:
     starts at byte ``header``) and fsync it"""
     row = rows.shape[1] * rows.shape[2]
     src = rows.view(-1)
-    st = _Staging(rows.device)
+    st = _Staging(rows.device, rows.dtype)
     chunks = list(_chunks(slots, row, st.chunk))
     sizes = [sum(k for _, k in pieces) for _, pieces in chunks]
 
@@ -707,7 +863,7 @@ def _write_rows(rows: torch.Tensor, slots, partial: str, header: int) -> None:
                 issue(c + 1)                                # its buffer was written to the file one chunk ago
             buf, pos = st.host(c).numpy(), 0
             for f0, k in pieces:
-                _write_all(fd, buf[pos:pos + k], header + 4 * f0)
+                _write_all(fd, buf[pos:pos + k], header + rows.element_size() * f0)
                 pos += k
         st.finish()
         os.fsync(fd)
@@ -715,22 +871,23 @@ def _write_rows(rows: torch.Tensor, slots, partial: str, header: int) -> None:
         os.close(fd)
 
 
-def _npy_header(shape) -> bytes:
-    """the .npy header of a C-order little-endian fp32 array of ``shape``: the same bytes on every rank"""
+def _npy_header(shape, descr: str = "<f4") -> bytes:
+    """the .npy header of a C-order array of ``shape`` and ``descr`` (``<f4`` or ``<f2``): the same bytes on every
+    rank"""
     out = io.BytesIO()
-    np.lib.format.write_array_header_1_0(out, {"descr": "<f4", "fortran_order": False, "shape": tuple(shape)})
+    np.lib.format.write_array_header_1_0(out, {"descr": descr, "fortran_order": False, "shape": tuple(shape)})
     return out.getvalue()
 
 
-def _create_rows_file(partial: str, shape) -> int:
-    """a fresh ``<partial>/rows.npy`` of ``shape`` fp32 (header written, data sized, not yet filled); returns the
-    header's length.  A ``partial`` left by a save that died is removed first."""
+def _create_rows_file(partial: str, shape, descr: str = "<f4") -> int:
+    """a fresh ``<partial>/rows.npy`` of ``shape`` and ``descr`` (header written, data sized, not yet filled);
+    returns the header's length.  A ``partial`` left by a save that died is removed first."""
     _discard(partial)
     os.makedirs(partial)
-    header = _npy_header(shape)
+    header = _npy_header(shape, descr)
     with open(os.path.join(partial, ROWS_FILE), "wb") as fh:
         fh.write(header)
-        fh.truncate(len(header) + 4 * int(np.prod(shape)))
+        fh.truncate(len(header) + np.dtype(descr).itemsize * int(np.prod(shape)))
     return len(header)
 
 
